@@ -73,12 +73,17 @@ def parse():
     ap.add_argument("--hyp", type=int, default=1, help="RANSAC hypotheses per landmark (reference: 1)")
     ap.add_argument("--skip-cpu", action="store_true", help="omit the cpu_baseline leg")
     ap.add_argument("--profile", action="store_true", help="ncu mode: exact --warmup, no e2e / cpu legs")
-    ap.add_argument("--no-traffic", action="store_true", help="skip the ncu child run that measures the CNN's DRAM bytes")
+    ap.add_argument("--dump-outputs", metavar="DIR", type=Path,
+                    help="write the landmarks of the last timed step to DIR/landmarks.npy (float64; one file per rank "
+                         "for N > 1) so that two builds can be compared on identical seeded inputs")
     ap.add_argument("--no-view-split", action="store_true", help="skip the config-4 leg (one scan's views split over the ranks)")
     ap.add_argument("--vs-views", type=int, default=200)
     ap.add_argument("--vs-size", type=int, default=512)
     ap.add_argument("--vs-grid", type=int, default=1001, help="1001 -> 1 002 001 vertices / 2 000 000 triangles")
-    return ap.parse_args()
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def peaks_file():
@@ -190,63 +195,6 @@ def cpu_path_seconds_per_scan(args, mesh, sample_views: int):
     native.snap_to_mesh(mesh.verts, mesh.tris, lm)
     t["snap"] = time.perf_counter() - t0
     return sum(t.values()), t, torch.get_num_threads()
-
-
-def measure_cnn_dram_traffic(args, timeout_s=300):
-    """DRAM bytes the CNN stage moves per scan, MEASURED for this build: a child run of this script
-    (--profile: one warm-up + one timed step, no other legs) under `ncu --metrics dram__bytes_read.sum,
-    dram__bytes_write.sum`; the bytes of every CNN kernel are summed and divided by the number of
-    network passes the child executed (= launches of the peak kernel that ends each pass).
-    Returns (bytes_per_scan | None, note)."""
-    import csv
-    import shutil
-    import tempfile
-
-    ncu = shutil.which("ncu") or "/usr/local/cuda/bin/ncu"
-    if not Path(ncu).exists():
-        return None, "ncu not found"
-    with tempfile.TemporaryDirectory() as tmp:
-        log = Path(tmp) / "dram.csv"
-        cmd = [ncu, "--metrics", "dram__bytes_read.sum,dram__bytes_write.sum", "--clock-control", "none", "--csv",
-               "--log-file", str(log), sys.executable, str(ROOT / "bench.py"), "--profile", "--steps", "1", "--warmup", "1",
-               "--views", str(args.views), "--size", str(args.size), "--grid", str(args.grid), "--hyp", str(args.hyp)]
-        env = dict(os.environ)
-        for k in ("RANK", "WORLD_SIZE", "LOCAL_RANK", "MASTER_ADDR", "MASTER_PORT"):
-            env.pop(k, None)
-        try:
-            r = subprocess.run(cmd, capture_output=True, text=True, timeout=timeout_s, env=env)
-        except subprocess.TimeoutExpired:
-            return None, f"ncu child run exceeded {timeout_s} s"
-        if r.returncode != 0 or not log.exists():
-            return None, f"ncu child run failed (rc {r.returncode})"
-        rows = [ln for ln in log.read_text().splitlines() if ln.startswith('"')]
-        rd = csv.DictReader(rows)
-        cnn = ("conv_umma_kernel", "conv_flow_kernel", "pool2_act_kernel", "bn_relu_kernel", "image_to_hilo16_kernel",
-               "peaks_from_keys_kernel")
-        total = {"read": 0.0, "write": 0.0}
-        passes = 0
-        unit_scale = {"byte": 1.0, "Kbyte": 1e3, "Mbyte": 1e6, "Gbyte": 1e9}
-        seen_peaks = set()
-        for row in rd:
-            name = row.get("Kernel Name", "")
-            if not any(k in name for k in cnn):
-                continue
-            try:
-                val = float(row["Metric Value"].replace(",", "")) * unit_scale.get(row.get("Metric Unit", "byte"), 1.0)
-            except (KeyError, ValueError):
-                continue
-            if row["Metric Name"] == "dram__bytes_read.sum":
-                total["read"] += val
-            elif row["Metric Name"] == "dram__bytes_write.sum":
-                total["write"] += val
-            if "peaks_from_keys_kernel" in name and row.get("ID") not in seen_peaks:
-                seen_peaks.add(row.get("ID"))
-                passes += 1
-        if passes == 0:
-            return None, "no CNN pass found in the ncu log"
-        per = (total["read"] + total["write"]) / passes
-        return per, (f"ncu child run of this command: {total['read'] / passes / 1e9:.2f} GB read + {total['write'] / passes / 1e9:.2f} GB "
-                     f"written per scan over {passes} network passes")
 
 
 def run_reference(args):
@@ -467,7 +415,7 @@ def run_ours(args):
     t_start.record()
     pending = []
     for _ in range(args.steps):
-        device_step(record=True)
+        landmarks = device_step(record=True)
         # per-stage events are read after the loop; keep fresh pairs per step
         pending.append({k: ev[k] for k in ev})
         ev = {k: (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for k in ev}
@@ -485,6 +433,10 @@ def run_ours(args):
         dist.all_reduce(tmax, op=dist.ReduceOp.MAX)
     ms_total = float(tmax.item())
     value = world * args.steps / (ms_total / 1e3)
+    if args.dump_outputs is not None:
+        args.dump_outputs.mkdir(parents=True, exist_ok=True)
+        name = "landmarks" if world == 1 else f"landmarks_rank{rank}"
+        np.save(args.dump_outputs / f"{name}.npy", landmarks.cpu().numpy())
 
     # ---- end to end through the plugin call with host (pinned) buffers
     from mvlm_b200.io_obj import Mesh
@@ -589,13 +541,6 @@ def run_ours(args):
             "clocks": clocks,
             "view_split": view_split,
         }
-        if world == 1 and not args.profile and not args.no_traffic:
-            # dram__bytes_read.sum + dram__bytes_write.sum over every CNN launch of one scan, measured now by an ncu
-            # child run of this same script (never a constant carried over from an older build)
-            traffic, note = measure_cnn_dram_traffic(args)
-            line["roofline"]["traffic"] = traffic
-            line["roofline"]["traffic_note"] = note + ("" if traffic is None else "; = %.0f%% of the measured HBM peak at this "
-                                                       "stage time" % (100 * traffic / (stage_ms["cnn"] / 1e3) / 1e9 / pk["hbm_gbs"]))
         if world == 1 and not args.skip_cpu and not args.profile:
             try:
                 cores = use_all_host_threads()
