@@ -99,6 +99,32 @@ int mvlm_obj_counts(const mvlm_obj* obj, int* n_verts, int* n_tris, int* has_uv)
 int mvlm_obj_copy(const mvlm_obj* obj, float* verts, float* uvs, int32_t* tris);
 void mvlm_obj_free(mvlm_obj* obj);
 
+/* Scan loader on the GPU (obj_parse.cu): the same language, arrays and error messages as mvlm_obj_load, bit for bit, */
+/* parsed from the file's bytes in device memory.  Two phases on the caller's stream:                                 */
+/*   mvlm_obj_parse_device  parses up to the output sizes, synchronises `stream` and fills *info; the error of a bad   */
+/*                          file (malformed line, no points, out-of-range index) is returned like mvlm_obj_load's,     */
+/*                          `path` only names the file in it.  info->fallback = 1: the file holds a number of more   */
+/*                          than 19 significant digits (or exceeds the parser's capacity): parse it with mvlm_obj_load */
+/*   mvlm_obj_parse_write   writes verts f32[n_verts*3], uvs f32[n_verts*2] (only when has_uv), tris i32[n_tris*3]    */
+/*                          into device buffers; asynchronous, reads the workspace of the first phase.                 */
+/* workspace: mvlm_obj_parse_workspace_bytes(n_bytes) bytes of device memory, 256-byte aligned (0: beyond capacity). */
+typedef struct mvlm_obj_parse_info {
+  int32_t n_verts, n_tris, has_uv, fallback;
+  int32_t n_positions; /* `v` lines */
+  size_t n_bytes;
+} mvlm_obj_parse_info;
+size_t mvlm_obj_parse_workspace_bytes(size_t n_bytes);
+int mvlm_obj_parse_device(const char* text_dev, size_t n_bytes, const char* path, void* workspace,
+                          size_t workspace_bytes, void* stream, mvlm_obj_parse_info* info);
+int mvlm_obj_parse_write(const mvlm_obj_parse_info* info, const void* workspace, float* verts, float* uvs,
+                         int32_t* tris, void* stream);
+/* Debug (host memory, no GPU): the GPU parser's per-line code run serially over text[0, len).  Per line: kind (0 other, */
+/* 1 v, 2 vt, 3 f), status (0 ok, 1 malformed, 2 host fallback), values f32[3] (v: x y z, vt: u v), n_tris (f), and   */
+/* for f lines the raw (a, b) of each triangulated corner appended to corners i64[2*max_corners] (b = 0: no uv).      */
+int mvlm_debug_obj_parse_lines(const char* text, size_t len, int max_lines, int* n_lines, int32_t* kind,
+                               int32_t* status, float* values, int32_t* n_tris, long long* corners,
+                               long long max_corners);
+
 /* Texture decode on the GPU (nvJPEG); replaces vtkJPEGReader in obj_to_actor, src/mvlm/utils/utils3d.py:26-36.  */
 /* data/len: the compressed file in host memory; out_rgb_dev: device buffer u8[height][width][3], row 0 = top.    */
 /* Thread-safe (one decoder state per calling thread); asynchronous on `stream` after the host-side parse.        */

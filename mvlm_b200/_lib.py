@@ -42,6 +42,12 @@ class ConvArgs(C.Structure):
     ]
 
 
+class ObjParseInfo(C.Structure):
+    """mvlm_obj_parse_info: what the first phase of the GPU OBJ parser found."""
+    _fields_ = [("n_verts", C.c_int32), ("n_tris", C.c_int32), ("has_uv", C.c_int32), ("fallback", C.c_int32),
+                ("n_positions", C.c_int32), ("n_bytes", C.c_size_t)]
+
+
 _lib = None
 
 
@@ -92,6 +98,11 @@ def _declare(lib: C.CDLL) -> None:
         "mvlm_obj_counts": ([vp, C.POINTER(i32), C.POINTER(i32), C.POINTER(i32)], i32),
         "mvlm_obj_copy": ([vp, vp, vp, vp], i32),
         "mvlm_obj_free": ([vp], None),
+        "mvlm_obj_parse_workspace_bytes": ([C.c_size_t], C.c_size_t),
+        "mvlm_obj_parse_device": ([vp, C.c_size_t, C.c_char_p, vp, C.c_size_t, vp, C.POINTER(ObjParseInfo)], i32),
+        "mvlm_obj_parse_write": ([C.POINTER(ObjParseInfo), vp, vp, vp, vp, vp], i32),
+        "mvlm_debug_obj_parse_lines": ([C.c_char_p, C.c_size_t, i32, C.POINTER(i32), vp, vp, vp, vp, vp, C.c_longlong],
+                                       i32),
         "mvlm_jpeg_info": ([C.c_char_p, C.c_size_t, C.POINTER(i32), C.POINTER(i32)], i32),
         "mvlm_jpeg_decode_rgb": ([C.c_char_p, C.c_size_t, vp, i32, i32, vp], i32),
         "mvlm_heatmap_peaks": ([vp, i32, i32, i32, i32, i32, vp, vp], i32),

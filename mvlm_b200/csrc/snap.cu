@@ -16,9 +16,9 @@
 // best < lb(r) - tau STRICTLY, candidates are compared as (dist^2, triangle id) with the same arithmetic as
 // the brute-force scan, so both paths return the same triangle and the same point bit for bit.
 #include <cub/block/block_reduce.cuh>
-#include <cub/block/block_scan.cuh>
 
 #include "common.cuh"
+#include "scan.cuh"
 #include "stages.cuh"
 
 namespace mvlm {
@@ -178,7 +178,6 @@ int snap_launch(const float* verts, const int* tris, int nt, const double* lm, i
 // ---------------------------------------------------------------------------------------------------------
 namespace {
 
-constexpr int kScanItems = 4096;  // cells per scan block (256 threads x 16)
 constexpr int kMaxShells = 8;     // shells walked before a query hands its landmark to the full scan (see 7c: a long walk
                                   // costs more than the scan, which then bounds the worst case at scan + ~50 us)
 constexpr int kGridHdrBytes = 256;
@@ -341,67 +340,6 @@ __global__ void __launch_bounds__(256) grid_count_kernel(const float* __restrict
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) tau = fmaxf(tau, __shfl_xor_sync(0xffffffffu, tau, o));
   if ((threadIdx.x & 31) == 0 && tau > 0.f) atomicMax(&hdr->tau_key, float_key(tau));
-}
-
-__global__ void __launch_bounds__(256) grid_scan_a_kernel(const int* __restrict__ counts, int* __restrict__ block_sums) {
-  using Reduce = cub::BlockReduce<int, 256>;
-  __shared__ typename Reduce::TempStorage tmp;
-  const int4* src = reinterpret_cast<const int4*>(counts + static_cast<size_t>(blockIdx.x) * kScanItems) + threadIdx.x * 4;
-  int sum = 0;
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    const int4 v = src[i];
-    sum += v.x + v.y + v.z + v.w;
-  }
-  const int total = Reduce(tmp).Sum(sum);
-  if (threadIdx.x == 0) block_sums[blockIdx.x] = total;
-}
-
-__global__ void __launch_bounds__(1024) grid_scan_b_kernel(int* __restrict__ block_sums, int nb, int* __restrict__ total_out) {
-  using Scan = cub::BlockScan<int, 1024>;
-  __shared__ typename Scan::TempStorage tmp;
-  int v[4], sum = 0;
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    const int j = threadIdx.x * 4 + i;
-    v[i] = j < nb ? block_sums[j] : 0;
-    sum += v[i];
-  }
-  int excl, total;
-  Scan(tmp).ExclusiveSum(sum, excl, total);
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    const int j = threadIdx.x * 4 + i;
-    if (j < nb) block_sums[j] = excl;
-    excl += v[i];
-  }
-  if (threadIdx.x == 0) *total_out = total;
-}
-
-__global__ void __launch_bounds__(256) grid_scan_c_kernel(const int* __restrict__ counts, const int* __restrict__ block_sums,
-                                                          int* __restrict__ cell_start) {
-  using Scan = cub::BlockScan<int, 256>;
-  __shared__ typename Scan::TempStorage tmp;
-  const size_t base = static_cast<size_t>(blockIdx.x) * kScanItems + threadIdx.x * 16;
-  int v[16], sum = 0;
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    const int4 q = reinterpret_cast<const int4*>(counts + base)[i];
-    v[4 * i] = q.x; v[4 * i + 1] = q.y; v[4 * i + 2] = q.z; v[4 * i + 3] = q.w;
-    sum += q.x + q.y + q.z + q.w;
-  }
-  int excl;
-  Scan(tmp).ExclusiveSum(sum, excl);
-  excl += block_sums[blockIdx.x];
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    int4 q;
-    q.x = excl; excl += v[4 * i];
-    q.y = excl; excl += v[4 * i + 1];
-    q.z = excl; excl += v[4 * i + 2];
-    q.w = excl; excl += v[4 * i + 3];
-    reinterpret_cast<int4*>(cell_start + base)[i] = q;
-  }
 }
 
 __global__ void __launch_bounds__(256) grid_fill_kernel(const float* __restrict__ verts, const int* __restrict__ tris,
@@ -568,13 +506,10 @@ int snap_grid_build(const float* verts, const int* tris, int nt, void* grid, siz
   int* over = reinterpret_cast<int*>(base + g.over);
   MVLM_CHECK_CUDA(cudaMemsetAsync(base, 0, g.cell_start, s));  // header + counts
   const int blocks = min(ceil_div(nt, 256), 4 * sm_count());
-  const int nb = g.cap_cells / kScanItems;
   grid_bounds_kernel<<<blocks, 256, 0, s>>>(verts, tris, nt, hdr);
   grid_setup_kernel<<<1, 1, 0, s>>>(hdr, nt, g.cap_cells);
   grid_count_kernel<<<blocks, 256, 0, s>>>(verts, tris, nt, hdr, counts, over);
-  grid_scan_a_kernel<<<nb, 256, 0, s>>>(counts, block_sums);
-  grid_scan_b_kernel<<<1, 1024, 0, s>>>(block_sums, nb, cell_start + g.cap_cells);
-  grid_scan_c_kernel<<<nb, 256, 0, s>>>(counts, block_sums, cell_start);
+  exclusive_scan(counts, g.cap_cells, block_sums, cell_start, cell_start + g.cap_cells, s);
   grid_fill_kernel<<<blocks, 256, 0, s>>>(verts, tris, nt, hdr, counts, cell_start, sorted);
   count_launch(7);
   MVLM_CHECK_CUDA(cudaGetLastError());

@@ -77,7 +77,7 @@ class Pipeline(abc.ABC, TimeMixin):
                  screenshot_folder: Path | None = None, *, image_size: tuple = (256, 256),
                  channel_mode: str = "RGB+depth", n_hypotheses: int = 1, seed: int | None = None,
                  transforms: np.ndarray | None = None, device: str = "cuda", verbose: bool = True,
-                 texture_decoder: str = "pil", pre_align: dict | None = None):
+                 texture_decoder: str = "pil", pre_align: dict | None = None, obj_parser: str = "host"):
         TimeMixin.__init__(self)
         self.render_image_stack = render_image_stack
         self.render_image_folder = render_image_folder
@@ -88,6 +88,13 @@ class Pipeline(abc.ABC, TimeMixin):
         self.device = torch.device(device)
         # "pil": host decode (shared with the parity oracle); "nvjpeg": decode on the GPU into device memory
         self.texture_decoder = texture_decoder
+        # "host": csrc/obj_loader.cu (numpy arrays); "gpu": csrc/obj_parse.cu, the same arrays bit for bit parsed on the
+        # device (the host only reads the file).  Used by predict_one_file's fused path and predict_files /
+        # predict_folder; the seam path (custom components, render_image_stack) and the view-split upload
+        # (sharding.upload_mesh_sharded) take host arrays and keep the host parser.
+        if obj_parser not in ("host", "gpu"):
+            raise ValueError(f"Unknown OBJ parser: {obj_parser}")
+        self.obj_parser = obj_parser
         # legacy "pre-align" block (configs/*.json:59-84): {"align_center_of_mass", "rot_x", "rot_y", "rot_z", "scale"};
         # None / identity = off, see utils/prealign.py
         self.pre_align = None if prealign.is_identity(pre_align) else dict(pre_align)
@@ -136,7 +143,8 @@ class Pipeline(abc.ABC, TimeMixin):
                 if not file_name.suffix == ".obj":
                     raise ValueError(f"File {file_name} is not an .obj file. Only .obj files are supported.")
                 self.tic()
-                mesh = load_obj(file_name, texture_decoder=self.texture_decoder, device=self.device)
+                mesh = load_obj(file_name, texture_decoder=self.texture_decoder, device=self.device,
+                                parser=self.obj_parser)
                 self._print("Render [1] - Setup time: ", self.toc_p())
                 landmarks = self.predict_mesh(mesh)
                 self._print("Landmarks 3D Total: ", self.p_time(time.time() - full_s))
@@ -164,7 +172,8 @@ class Pipeline(abc.ABC, TimeMixin):
                     raise ValueError(f"File {f} is not an .obj file. Only .obj files are supported.")
                 # four parser threads per scan: with more, the loaders of `prefetch` scans oversubscribe the host and the
                 # thread that feeds the GPU gets descheduled (measured on the 16-core box: 36 scans/s with 16, 51 with 4)
-                return load_obj(f, n_threads=4, texture_decoder=self.texture_decoder, device=self.device)
+                return load_obj(f, n_threads=4, texture_decoder=self.texture_decoder, device=self.device,
+                                parser=self.obj_parser)
 
             def meshes():
                 with ThreadPoolExecutor(max_workers=max(1, prefetch)) as pool:
@@ -215,8 +224,14 @@ class Pipeline(abc.ABC, TimeMixin):
         back = None
         if self.pre_align is not None:
             # the whole path runs on the pre-aligned scan; the snapped landmarks are mapped back in _finish
-            a, b = prealign.affine(mesh.verts, self.pre_align)
-            mesh = dataclasses.replace(mesh, verts=prealign.apply(mesh.verts, a, b))
+            verts = mesh.verts
+            if isinstance(verts, torch.Tensor):
+                # parser="gpu": prealign runs on numpy, so the vertices come back to the host (12 bytes per vertex, and
+                # this thread waits for the scan's parse); the aligned copy is uploaded like host-parsed vertices
+                mesh.geometry_ready.synchronize()
+                verts = verts.cpu().numpy()
+            a, b = prealign.affine(verts, self.pre_align)
+            mesh = dataclasses.replace(mesh, verts=prealign.apply(verts, a, b))
             back = (a, b)
         dmesh = r.upload(mesh)
         out = r.render_device(dmesh, transforms)

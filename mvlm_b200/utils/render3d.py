@@ -101,9 +101,10 @@ class DeviceMesh:
         def up(name, a):
             if a is None:
                 return None
-            if isinstance(a, torch.Tensor):  # texture decoded on the device (nvJPEG) on the loader's side stream
-                if mesh.texture_ready is not None:
-                    torch.cuda.current_stream().wait_event(mesh.texture_ready)
+            if isinstance(a, torch.Tensor):  # decoded (nvJPEG) or parsed (parser="gpu") on the loader's side stream
+                ready = mesh.texture_ready if name == "tex" else mesh.geometry_ready
+                if ready is not None:
+                    torch.cuda.current_stream().wait_event(ready)
                 a.record_stream(torch.cuda.current_stream())
                 return a
             a = np.ascontiguousarray(a)
