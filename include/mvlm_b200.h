@@ -172,7 +172,7 @@ int mvlm_hourglass_create(const char* const* names, const void* const* ptrs, con
                           size_t workspace_bytes, mvlm_hourglass** out);
 int mvlm_hourglass_forward(mvlm_hourglass* net, const uint8_t* img_u8, const float* img_f32,
                            float* out_heatmaps, float* out_peaks, void* stream);
-/* Same result as mvlm_hourglass_forward; the ~155 launches are captured into a CUDA graph per distinct
+/* Same result as mvlm_hourglass_forward; the 144 launches are captured into a CUDA graph per distinct
  * (img, out) pointer tuple on first use and replayed afterwards (buffers must stay valid and unchanged). */
 int mvlm_hourglass_forward_graph(mvlm_hourglass* net, const uint8_t* img_u8, const float* img_f32,
                                  float* out_heatmaps, float* out_peaks, void* stream);
@@ -193,9 +193,6 @@ int mvlm_hourglass_forward_keys(mvlm_hourglass* net, const uint8_t* img_u8, cons
 int mvlm_peaks_from_gathered_keys(const uint64_t* keys, int n_views, int n_landmarks, int w, int world, int slot_views,
                                   float* out_peaks /* (L, V, 3) */, void* stream);
 int mvlm_hourglass_num_launches(const mvlm_hourglass* net);
-/* number of dataflow segments of the plan (csrc/conv_flow.cuh): runs of layers executed by one persistent launch
- * over small view batches so that their intermediate tensors stay in L2; 0 = every layer is its own launch */
-int mvlm_hourglass_num_segments(const mvlm_hourglass* net);
 /* Debug aids: per-op mean milliseconds over `reps` passes (ms_out[num_launches], host memory; out_peaks (L,V,3)
  * device), optionally the conv kernel's per-role stall cycles (roles_out[num_launches*8] host doubles, layout of
  * mvlm_debug_conv_profile, mean over CTAs), and a one-line description of op `op`. */

@@ -87,7 +87,6 @@ def _declare(lib: C.CDLL) -> None:
         "mvlm_hourglass_forward_keys": ([vp, vp, vp, vp, vp], i32),
         "mvlm_peaks_from_gathered_keys": ([vp, i32, i32, i32, i32, i32, vp, vp], i32),
         "mvlm_hourglass_num_launches": ([vp], i32),
-        "mvlm_hourglass_num_segments": ([vp], i32),
         "mvlm_debug_hourglass_profile": ([vp, vp, vp, vp, i32, C.POINTER(C.c_float), C.POINTER(C.c_double), i32,
                                          C.POINTER(C.c_longlong), vp], i32),
         "mvlm_debug_conv_profile_ints": ([], i32),

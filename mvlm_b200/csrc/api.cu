@@ -213,8 +213,6 @@ int mvlm_debug_hourglass_describe(const mvlm_hourglass* net, int op, char* buf, 
 
 int mvlm_hourglass_num_launches(const mvlm_hourglass* net) { return net ? net->net.n_ops() : 0; }
 
-int mvlm_hourglass_num_segments(const mvlm_hourglass* net) { return net ? net->net.n_segments() : 0; }
-
 int mvlm_hourglass_probe(const mvlm_hourglass* net, const char* name, const void** ptr, int* h, int* w, int* c) {
   MVLM_REQUIRE(net && name && ptr && h && w && c, "mvlm_hourglass_probe: null pointer");
   auto it = net->net.probes.find(name);

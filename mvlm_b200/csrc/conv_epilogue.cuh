@@ -1,15 +1,10 @@
-// Epilogue of the tcgen05 convolution kernels, shared by the per-layer kernel (conv_umma.cu) and the
-// multi-layer dataflow kernel (conv_flow.cu): accumulator tile in TMEM -> bias / BatchNorm / ReLU /
-// residuals / 2x2 max-pool / arg-max -> NHWC bf16 (or fp32 NCHW) stores.  See conv_umma.cu for the tile
+// Epilogue of the tcgen05 convolution kernel (conv_umma.cu): accumulator tile in TMEM -> bias / BatchNorm /
+// ReLU / residuals / 2x2 max-pool / arg-max -> NHWC bf16 (or fp32 NCHW) stores.  See conv_umma.cu for the tile
 // geometry and DESIGN.md section 4 for why it looks the way it does.
 #pragma once
 #include "conv_umma.cuh"
 
 #include <type_traits>
-
-#ifndef MVLM_FLOW_RES_BUDGET
-#define MVLM_FLOW_RES_BUDGET 32  // registers of the residual prefetch buffer in the dataflow kernel's variants
-#endif
 
 namespace mvlm {
 namespace epi {
@@ -31,7 +26,7 @@ enum : int { F_PRE = 1, F_RES1 = 2, F_RES2 = 4, F_RAW = 8, F_POST = 16, F_F32 = 
               F_M64 = 1024 /* cout <= 64: tcgen05.mma.ws with M = 64 / 32, the tile's pixels split over the TMEM lane groups */,
               F_POST2 = 2048 /* second full-resolution act copy (aux_mode 1) */,
               F_POOLX = 4096 /* additional pooled raw + pooled act copies (aux_mode 2) */,
-              F_STAT = 8192 /* (per-layer kernel only) 3 x 3 taps over stationary weights: straight-line MMA issue */ };
+              F_STAT = 8192 /* 3 x 3 taps over stationary weights: straight-line MMA issue */ };
 constexpr int F_HEAD = F_F32 | F_ARGMAX;
 
 // feature mask of a planned layer (without F_M64)
@@ -126,8 +121,7 @@ struct TileCoord {
   int mt, tx, ty, img;
 };
 
-// Per-output-channel parameter arrays, never null, at least cout_pad long (shared memory in the per-layer
-// kernel, global memory in the dataflow kernel).
+// Per-output-channel parameter arrays in shared memory, never null, at least cout_pad long.
 struct ChannelParams {
   const float* bias;
   const float* mid_s;  // F_MID parameters, or the aux_scale / aux_shift of F_POST2 / F_POOLX (never both)
@@ -136,12 +130,6 @@ struct ChannelParams {
   const float* pre_t;
   const float* post_s;
   const float* post_t;
-};
-
-// Image index of the tile inside each tensor the epilogue touches (ring buffers of the dataflow plan hold
-// fewer images than the layer processes; the per-layer kernel uses the tile's image for all of them).
-struct ImageSlots {
-  int pre, raw, post, res1, res2, up, aux1, aux2;
 };
 
 // running arg-max of the F_ARGMAX variants (lane = channel), flushed when the CTA moves to another image
@@ -162,14 +150,6 @@ struct EpiTrace {
     if (tr.on && tr.trace && tr.trace_i < kTraceTiles) tr.trace[tr.trace_i * 16 + (slot)] = clock64() - tr.t0; \
   } while (0)
 
-// 16-byte residual load: plain in the per-layer kernel; L1-bypassing in the dataflow kernel, where the producer
-// of the data is another CTA of the same launch
-template <bool kFlow>
-__device__ __forceinline__ uint4 load_res(const uint8_t* p) {
-  if constexpr (kFlow) return __ldcg(reinterpret_cast<const uint4*>(p));
-  else return *reinterpret_cast<const uint4*>(p);
-}
-
 // One accumulator tile.  Pixel n of the tile = 8 * (row in tile) + (pixel in row).  One "unit" (one TMEM load,
 // one transpose) = 16 pixels = 2 image rows x 8 px of the warp's 32 channels.
 //   M = 128 (plain tcgen05.mma): TMEM lane = output channel, TMEM column = pixel n.
@@ -183,9 +163,9 @@ __device__ __forceinline__ uint4 load_res(const uint8_t* p) {
 //
 // `tmem_acc` = TMEM address of column 0 of this tile's accumulator stage; `t_full` / `parity` = the barrier the
 // MMA warp commits to.  The caller releases the stage (tcgen05 fence + arrive on its t_empty barrier) afterwards.
-template <int F, bool kFlow>
+template <int F>
 __device__ __forceinline__ void epilogue_tile(const ConvShape& s, const ConvEpilogue& e, const int tile_h,
-                                              const ChannelParams& ep, const TileCoord& tc, const ImageSlots& is,
+                                              const ChannelParams& ep, const TileCoord& tc,
                                               uint64_t* t_full, const uint32_t parity, const uint32_t tmem_acc,
                                               float* stage, const int ew, const int lane_grp, const int lane,
                                               ArgmaxState& am, const bool prof, long long& w0, EpiTrace& tr) {
@@ -197,7 +177,7 @@ __device__ __forceinline__ void epilogue_tile(const ConvShape& s, const ConvEpil
   constexpr int kUnitRows = kCols / 8;       // image rows per unit
   static_assert(kCols * kPitch <= kStageFloats, "transpose buffer");
   // F_M64: `rep` = 2 (M = 64: 33 .. 64 channels) or 4 (M = 32) lane groups hold the same channels and different pixel
-  // rows of the tile.  Shifts, not divisions: in the dataflow kernel this runs once per tile.
+  // rows of the tile.  A shift count, so that the per-tile index arithmetic below needs no integer division.
   const int rep_log2 = !WS ? 0 : (s.cout_pad <= 32 ? 2 : 1);
   // ew = index of this epilogue warp (0..7), lane_grp = its hardware warp id % 4: the TMEM lanes it may read are
   // 32 * lane_grp ..
@@ -233,12 +213,7 @@ __device__ __forceinline__ void epilogue_tile(const ConvShape& s, const ConvEpil
   constexpr bool kHasRes = (F & (F_RES1 | F_RES2 | F_UP)) != 0;
   constexpr int kMaxUpw = WS ? 4 : 8;  // units per warp at N = 256
   constexpr int kResRegs = 4 * (2 * (((F & F_RES1) ? 1 : 0) + ((F & F_RES2) ? 1 : 0)) + ((F & F_UP) ? 1 : 0));
-  // Dataflow kernel: the first batch is issued AFTER the accumulator wait (below).  Issued before it, as in the
-  // per-layer kernel, the buffer is live across the wait loop and ptxas keeps it on the stack in the dataflow kernel's
-  // many-variant epilogue: every prefetched line was stored to local memory as it arrived, one exposed L2 round trip
-  // per load (measured: 19k cycles before the first unit of a 16-load tile).  Residuals come from L2 there, and one
-  // exposed round trip per tile (~1.5k cycles under load) is the price.
-  constexpr int kResBudget = kFlow ? MVLM_FLOW_RES_BUDGET : 64;
+  constexpr int kResBudget = 64;
   constexpr int kPref = !kHasRes ? 1 : (kResRegs * kMaxUpw <= kResBudget ? kMaxUpw : (kResRegs * kMaxUpw <= 2 * kResBudget ? kMaxUpw / 2 : (kMaxUpw >= 4 ? kMaxUpw / 4 : 1)));  // units per batch
   uint4 r1[kPref][2], r2[(F & F_RES2) ? kPref : 1][2], ru[(F & F_UP) ? kPref : 1][1];
 
@@ -251,12 +226,12 @@ __device__ __forceinline__ void epilogue_tile(const ConvShape& s, const ConvEpil
   const bool ch_ok = c0 < s.cout_pad;  // weight rows beyond cout_pad are never loaded
   const int xa = tc.tx * kTileW + pj;
   const bool vx = ch_ok && xa < s.w;
-  // PIXEL index of my pixel in pass 0 of the first unit of image `img`: (img, y_first, xa); 32-bit (checked in
-  // conv_plan), widened before it is multiplied with a channel stride
-  auto pix_of = [&](int img) __attribute__((always_inline)) { return (static_cast<uint32_t>(img) * s.h + y_first) * s.w + xa; };
-  // element index of the half-resolution pixel (img, y_first/2, xa/2): F_POOL outputs, F_UP input
-  auto ppix_of = [&](int img) __attribute__((always_inline)) {
-    return (static_cast<uint32_t>(img) * (s.h >> 1) + (y_first >> 1)) * (s.w >> 1) + (xa >> 1);
+  // PIXEL index of my pixel in pass 0 of the first unit: (tc.img, y_first, xa); 32-bit (checked in conv_plan),
+  // widened before it is multiplied with a channel stride
+  auto pix = [&]() __attribute__((always_inline)) { return (static_cast<uint32_t>(tc.img) * s.h + y_first) * s.w + xa; };
+  // element index of the half-resolution pixel (tc.img, y_first/2, xa/2): F_POOL outputs, F_UP input
+  auto ppix = [&]() __attribute__((always_inline)) {
+    return (static_cast<uint32_t>(tc.img) * (s.h >> 1) + (y_first >> 1)) * (s.w >> 1) + (xa >> 1);
   };
   if ((F & F_ARGMAX) && tc.img != am.cur_img) {
     if (am.cur_img >= 0 && am.best_hi != 0u && c_lane < e.cout_real)
@@ -266,50 +241,38 @@ __device__ __forceinline__ void epilogue_tile(const ConvShape& s, const ConvEpil
     am.cur_img = tc.img;
   }
   // per-tile base pointers of my (pixel, 8 channels) in the first unit
-  uint8_t* const b_pre = (F & F_PRE) ? reinterpret_cast<uint8_t*>(e.out_pre + e.pre_co + c0 + static_cast<size_t>(pix_of(is.pre)) * e.pre_cs) : nullptr;
-  uint8_t* const b_raw = (F & F_RAW) ? reinterpret_cast<uint8_t*>(e.out_raw + e.raw_co + c0 + static_cast<size_t>((F & F_POOL) ? ppix_of(is.raw) : pix_of(is.raw)) * e.raw_cs) : nullptr;
-  uint8_t* const b_post = (F & F_POST) ? reinterpret_cast<uint8_t*>(e.out_post + e.post_co + c0 + static_cast<size_t>((F & F_POOL) ? ppix_of(is.post) : pix_of(is.post)) * e.post_cs) : nullptr;
-  uint8_t* const b_aux1 = (F & (F_POST2 | F_POOLX)) ? reinterpret_cast<uint8_t*>(e.out_aux1 + e.aux1_co + c0 + static_cast<size_t>((F & F_POOLX) ? ppix_of(is.aux1) : pix_of(is.aux1)) * e.aux1_cs) : nullptr;
-  uint8_t* const b_aux2 = (F & F_POOLX) ? reinterpret_cast<uint8_t*>(e.out_aux2 + e.aux2_co + c0 + static_cast<size_t>(ppix_of(is.aux2)) * e.aux2_cs) : nullptr;
+  uint8_t* const b_pre = (F & F_PRE) ? reinterpret_cast<uint8_t*>(e.out_pre + e.pre_co + c0 + static_cast<size_t>(pix()) * e.pre_cs) : nullptr;
+  uint8_t* const b_raw = (F & F_RAW) ? reinterpret_cast<uint8_t*>(e.out_raw + e.raw_co + c0 + static_cast<size_t>((F & F_POOL) ? ppix() : pix()) * e.raw_cs) : nullptr;
+  uint8_t* const b_post = (F & F_POST) ? reinterpret_cast<uint8_t*>(e.out_post + e.post_co + c0 + static_cast<size_t>((F & F_POOL) ? ppix() : pix()) * e.post_cs) : nullptr;
+  uint8_t* const b_aux1 = (F & (F_POST2 | F_POOLX)) ? reinterpret_cast<uint8_t*>(e.out_aux1 + e.aux1_co + c0 + static_cast<size_t>((F & F_POOLX) ? ppix() : pix()) * e.aux1_cs) : nullptr;
+  uint8_t* const b_aux2 = (F & F_POOLX) ? reinterpret_cast<uint8_t*>(e.out_aux2 + e.aux2_co + c0 + static_cast<size_t>(ppix()) * e.aux2_cs) : nullptr;
   // rows at / below my first pixel that exist in the image (0 when my pixel column / channels do not):
   // unit r, pass ip is valid iff kUnitRows * r + ip < n_rows_ok
   const int n_rows_ok = vx ? s.h - y_first : 0;
-  // (kFlow: lanes whose pixel column / channels / rows do not exist point at the tensor's first element, see
-  // prefetch_batch)
-  const bool res_ok = !kFlow || n_rows_ok > 0;
-  const uint8_t* const b_res1 = (F & F_RES1) ? reinterpret_cast<const uint8_t*>(res_ok ? e.res1 + e.res1_co + c0 + static_cast<size_t>(pix_of(is.res1)) * e.res1_cs : e.res1) : nullptr;
-  const uint8_t* const b_res2 = (F & F_RES2) ? reinterpret_cast<const uint8_t*>(res_ok ? e.res2 + e.res2_co + c0 + static_cast<size_t>(pix_of(is.res2)) * e.res2_cs : e.res2) : nullptr;
-  const uint8_t* const b_up = (F & F_UP) ? reinterpret_cast<const uint8_t*>(res_ok ? e.res_up + e.up_co + c0 + static_cast<size_t>(ppix_of(is.up)) * e.up_cs : e.res_up) : nullptr;
+  const uint8_t* const b_res1 = (F & F_RES1) ? reinterpret_cast<const uint8_t*>(e.res1 + e.res1_co + c0 + static_cast<size_t>(pix()) * e.res1_cs) : nullptr;
+  const uint8_t* const b_res2 = (F & F_RES2) ? reinterpret_cast<const uint8_t*>(e.res2 + e.res2_co + c0 + static_cast<size_t>(pix()) * e.res2_cs) : nullptr;
+  const uint8_t* const b_up = (F & F_UP) ? reinterpret_cast<const uint8_t*>(e.res_up + e.up_co + c0 + static_cast<size_t>(ppix()) * e.up_cs) : nullptr;
   auto prefetch_batch = [&](int u0) __attribute__((always_inline)) {  // units u0 .. u0 + kPref - 1 (u0 compile-time after unrolling)
 #pragma unroll
     for (int q = 0; q < kPref; ++q) {
       const int u = u0 + q;
-      if (kFlow || u < upw) {
+      if (u < upw) {
 #pragma unroll
         for (int ip = 0; ip < 2; ++ip) {
           const int row = kUnitRows * u + ip;
-          if constexpr (kFlow) {
-            // unconditional loads (rows that do not exist re-read the tile's first row and are never used): with
-            // conditionally defined buffer entries ptxas keeps the whole buffer in local memory in the non-inlined
-            // variants of the dataflow kernel (load, store to the stack, reload: one L2 round trip per load)
-            const int rr = (u < upw && row < n_rows_ok) ? row : 0;
-            if (F & F_RES1) r1[q][ip] = load_res<kFlow>(b_res1 + static_cast<size_t>(rr * rs_res1));
-            if (F & F_RES2) r2[q][ip] = load_res<kFlow>(b_res2 + static_cast<size_t>(rr * rs_res2));
-            if ((F & F_UP) && ip == 0)
-              ru[q][0] = load_res<kFlow>(b_up + static_cast<size_t>((rr >> 1) * rs_up));
-          } else if (row < n_rows_ok) {
-            if (F & F_RES1) r1[q][ip] = load_res<kFlow>(b_res1 + static_cast<size_t>(row * rs_res1));
-            if (F & F_RES2) r2[q][ip] = load_res<kFlow>(b_res2 + static_cast<size_t>(row * rs_res2));
+          if (row < n_rows_ok) {
+            if (F & F_RES1) r1[q][ip] = *reinterpret_cast<const uint4*>(b_res1 + static_cast<size_t>(row * rs_res1));
+            if (F & F_RES2) r2[q][ip] = *reinterpret_cast<const uint4*>(b_res2 + static_cast<size_t>(row * rs_res2));
             // nearest x2: rows 2k, 2k+1 and columns xa, xa^1 all read low-res pixel (k, xa/2);
             // both passes share one low-res row per unit
             if ((F & F_UP) && ip == 0)
-              ru[q][0] = load_res<kFlow>(b_up + static_cast<size_t>((row >> 1) * rs_up));
+              ru[q][0] = *reinterpret_cast<const uint4*>(b_up + static_cast<size_t>((row >> 1) * rs_up));
           }
         }
       }
     }
   };
-  if (!kFlow && kHasRes && grp_active && rows_active) prefetch_batch(0);
+  if (kHasRes && grp_active && rows_active) prefetch_batch(0);
   // per-channel parameters of my 8 channels (pixel-major role) and my channel (channel-major role)
   float pre_s[8], pre_t[8], post_s[8], post_t[8];
   const int c0_ok = ch_ok ? c0 : 0;
@@ -318,19 +281,8 @@ __device__ __forceinline__ void epilogue_tile(const ConvShape& s, const ConvEpil
   const int c_lane_ok = c_lane < s.cout_pad ? c_lane : 0;
   const float bias_c = ep.bias[c_lane_ok];
   const float mid_s_c = ep.mid_s[c_lane_ok], mid_t_c = ep.mid_t[c_lane_ok];
-  if constexpr (kFlow) {
-    // no call inside this wait, see ptx::mbar_wait_trap
-    if (!prof) {
-      ptx::mbar_wait_trap(t_full, parity);
-    } else {
-      const long long t0 = clock64();
-      ptx::mbar_wait_trap(t_full, parity);
-      w0 += clock64() - t0;
-    }
-  } else {
-    MVLM_EPI_TRACE(7);  // per-layer kernel: residual prefetch issued, parameters loaded, about to wait
-    timed_wait(t_full, parity, prof, w0);
-  }
+  MVLM_EPI_TRACE(7);  // residual prefetch issued, parameters loaded, about to wait
+  timed_wait(t_full, parity, prof, w0);
   ptx::tc_fence_after();
   MVLM_EPI_TRACE(5);
   if (grp_active && rows_active) {
@@ -344,7 +296,7 @@ __device__ __forceinline__ void epilogue_tile(const ConvShape& s, const ConvEpil
 #pragma unroll
     for (int r = 0; r < kMaxUpw; ++r) {
       if (r < upw) {
-        if (kHasRes && (kPref < kMaxUpw || kFlow) && (kFlow || r > 0) && r % kPref == 0) prefetch_batch(r);  // next batch
+        if (kHasRes && kPref < kMaxUpw && r > 0 && r % kPref == 0) prefetch_batch(r);  // next batch
         const int y = y_first + kUnitRows * r;  // first image row of the unit
         ptx::tmem_ld_wait();
         if (r < 2) MVLM_EPI_TRACE(8 + 4 * r);
@@ -476,8 +428,8 @@ __device__ __forceinline__ void epilogue_tile(const ConvShape& s, const ConvEpil
                 if (F & F_POST)
                   *reinterpret_cast<uint4*>(b_post + static_cast<size_t>(row * rs_post)) = affine_relu_pack8(f, post_s, post_t);
                 if (F & F_POST2) {
-                  // parameters fetched at the point of use (shared memory in the per-layer kernel): 16 registers this
-                  // variant cannot hold across the tile
+                  // parameters fetched from shared memory at the point of use: 16 registers this variant cannot hold
+                  // across the tile
                   // (applied to the bf16-rounded raw value, like the stand-alone pass that reads the stored tensor)
                   float ax_s[8], ax_t[8], g[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
                   add8(pack8(f), g);

@@ -433,7 +433,7 @@ __global__ void __launch_bounds__(kThreads, 1) conv_umma_kernel(const __grid_con
     }
   } else {
     // ===================== epilogue =====================
-    // the per-tile work is epi::epilogue_tile (conv_epilogue.cuh), shared with the dataflow kernel
+    // the per-tile work is epi::epilogue_tile (conv_epilogue.cuh)
     float* stage = stage_all + (warp - 2) * kStageFloats;
     const ChannelParams cp = {ep->bias, ep->mid_s, ep->mid_t, ep->pre_s, ep->pre_t, ep->post_s, ep->post_t};
     int acc = 0;
@@ -444,15 +444,13 @@ __global__ void __launch_bounds__(kThreads, 1) conv_umma_kernel(const __grid_con
     TileIter it(p, t_begin, t_step);
     for (int t = t_begin; t < t_end; t += t_step, it.next()) {
       const TileCoord tc = it.c;
-      const ImageSlots is = {tc.img, tc.img, tc.img, tc.img, tc.img, tc.img, tc.img, tc.img};
       tr.trace_i = trace_i;
       if (p.debug_mode & 2) {  // experiment: accumulators are dropped (results invalid)
         timed_wait(&bar->t_full[acc], pacc, prof, w0);
         ptx::tc_fence_after();
       } else {
-        epilogue_tile<F, false>(s, e, p.tile_h, cp, tc, is, &bar->t_full[acc], pacc,
-                                tmem_base + static_cast<uint32_t>(acc * 256), stage, warp - 2, warp & 3, lane, am, prof, w0,
-                                tr);
+        epilogue_tile<F>(s, e, p.tile_h, cp, tc, &bar->t_full[acc], pacc, tmem_base + static_cast<uint32_t>(acc * 256),
+                         stage, warp - 2, warp & 3, lane, am, prof, w0, tr);
       }
       // all tcgen05.ld of this accumulator stage have completed (wait::ld above)
       ptx::tc_fence_before();

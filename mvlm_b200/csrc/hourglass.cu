@@ -157,17 +157,8 @@ void HourglassNet::note_conv(const void* in, const ConvEpilogue& e) {
 
 void HourglassNet::assign_offsets() {
   const int n_ops = static_cast<int>(ops_.size());
-  // a buffer touched inside a dataflow segment is live for the whole segment (its ops run interleaved)
-  std::vector<int> seg_first(n_segs_, n_ops), seg_last(n_segs_, -1);
-  for (int i = 0; i < n_ops; ++i)
-    if (op_seg_[i] >= 0) {
-      seg_first[op_seg_[i]] = std::min(seg_first[op_seg_[i]], i);
-      seg_last[op_seg_[i]] = std::max(seg_last[op_seg_[i]], i);
-    }
   for (Buf& b : bufs_) {
     if (b.first < 0) { b.first = 0; b.last = n_ops; }  // never referenced by an op: keep it for the whole plan
-    if (b.first < n_ops && op_seg_[b.first] >= 0) b.first = seg_first[op_seg_[b.first]];
-    if (b.last < n_ops && op_seg_[b.last] >= 0) b.last = seg_last[op_seg_[b.last]];
     if (b.pinned || !reuse_) { b.first = 0; b.last = n_ops; }
   }
   // first-fit over a sorted free list, buffers taken in order of their first use
@@ -222,33 +213,6 @@ void HourglassNet::assign_offsets() {
     ws_needed_ = std::max(ws_needed_, top);
     live.push_back(id);
   }
-}
-
-// Output resolution (rows) of an op, the quantity the dataflow window is defined on; -1: the op kind never joins a
-// segment (stem staging, memset, peaks, the arg-max head).
-static int op_out_rows(const NetOp& op) {
-  switch (op.kind) {
-    case NetOp::CONV: return op.is_head ? -1 : op.h;
-    case NetOp::POOL: return op.h / 2;
-    case NetOp::BNRELU: return op.h;
-    default: return -1;
-  }
-}
-
-// Consecutive ops whose output resolution lies in [flow_lo_, flow_hi_] form dataflow segments of at most
-// kFlowMaxLayers layers (a segment boundary is a launch boundary, i.e. a full dependency, so any cut is legal).
-void HourglassNet::push_op(const NetOp& op) {
-  const int rows = op_out_rows(op);
-  const bool in_window = flow_on_ && rows >= flow_lo_ && rows <= flow_hi_;
-  if (!in_window) {
-    cur_seg_ = -1;
-  } else if (cur_seg_ < 0 || cur_seg_layers_ >= kFlowMaxLayers) {
-    cur_seg_ = n_segs_++;
-    cur_seg_layers_ = 0;
-  }
-  if (in_window) ++cur_seg_layers_;
-  ops_.push_back(op);
-  op_seg_.push_back(cur_seg_);
 }
 
 HourglassNet::T HourglassNet::alloc(int h, int w, int c) {
@@ -370,7 +334,7 @@ int HourglassNet::emit_conv(const char* tag, T in, int cin, const std::string& w
     rc = conv_plan(s, e, &op.conv);
     if (rc) return rc;
   }
-  push_op(op);
+  ops_.push_back(op);
   return MVLM_OK;
 }
 
@@ -455,7 +419,7 @@ int HourglassNet::emit_pool(T in, T out_raw, const char* bn_name, T out_act) {
     int rc = bn(bn_name, in.c, &op.scale, &op.shift);
     if (rc) return rc;
   }
-  push_op(op);
+  ops_.push_back(op);
   return MVLM_OK;
 }
 
@@ -539,12 +503,6 @@ int HourglassNet::build(const StateDict* sd, int n_landmarks, int cin, int n_vie
   if (Lp_ == 48) Lp_ = 64;
   if (Lp_ == 16) Lp_ = 32;
   ws_ = static_cast<uint8_t*>(workspace); ws_size_ = workspace_bytes;
-  // experiment knobs of the dataflow plan (defaults in hourglass.cuh)
-  if (const char* v = getenv("MVLM_FLOW")) flow_on_ = atoi(v) != 0;
-  if (const char* v = getenv("MVLM_FLOW_LO")) flow_lo_ = std::max(1, atoi(v));
-  if (const char* v = getenv("MVLM_FLOW_HI")) flow_hi_ = atoi(v);
-  if (const char* v = getenv("MVLM_FLOW_TILES")) flow_tiles_ = std::max(1, atoi(v));
-  if (const char* v = getenv("MVLM_FLOW_K")) flow_interleave_ = std::max(1, atoi(v));
   // MVLM_HG_KEEP_PROBES=1: the probe tensors (layer-wise parity tests) keep their memory for the whole plan;
   // MVLM_HG_NO_REUSE=1: every buffer does (the round-1 layout, for A/B runs)
   keep_probes_ = getenv("MVLM_HG_KEEP_PROBES") != nullptr && atoi(getenv("MVLM_HG_KEEP_PROBES")) != 0;
@@ -579,7 +537,6 @@ int HourglassNet::build(const StateDict* sd, int n_landmarks, int cin, int n_vie
     set_error("hourglass: parameter arena overrun (%zu of %zu bytes)", param_off_, param_bytes);
     rc = MVLM_E_INVALID;
   }
-  if (rc == MVLM_OK) rc = build_segments();
   const cudaError_t ce = cudaStreamSynchronize(build_stream_);
   cudaStreamDestroy(build_stream_);
   build_stream_ = nullptr;
@@ -597,11 +554,10 @@ void HourglassNet::probe(const char* name, const T& t) {
   }
 }
 
-// emits the plan: ops_, op_seg_, probes, flops_ (layout pass: fake addresses, no CUDA calls)
+// emits the plan: ops_, probes, flops_ (layout pass: fake addresses, no CUDA calls)
 int HourglassNet::emit() {
   const int h = H_, w = W_, cin = cin_;
   ops_.clear(); flops_ = 0.0; probes.clear();
-  op_seg_.clear(); segs_.clear(); seg_info_.clear(); cur_seg_ = -1; n_segs_ = 0; cur_seg_layers_ = 0;
   int rc;
   const int F = 256, h2 = h / 2, w2 = w / 2;
 
@@ -614,7 +570,7 @@ int HourglassNet::emit() {
     NetOp op;
     op.kind = NetOp::STEM;
     op.out_raw = img16.p; op.h = h; op.w = w; op.c = cin;
-    push_op(op);
+    ops_.push_back(op);
     flops_ += 2.0 * 64 * cin * 9 * h * w;
     note_use(img16.p); note_use(a_c2.p); note_use(ar_c2.p);
     NetOp cv;
@@ -648,7 +604,7 @@ int HourglassNet::emit() {
       e.out_post = ar_c2.p; e.post_cs = 64; e.post_co = 0;
       if ((rc = conv_plan(s, e, &cv.conv))) return rc;
     }
-    push_op(cv);
+    ops_.push_back(cv);
   }
   T none, y2, y3, r3, a3, a4, a_h1, ar4;
   // conv2 block: its output is only consumed through the max-pool (:411) -> pooled outputs straight from the epilogues
@@ -669,7 +625,7 @@ int HourglassNet::emit() {
     op.kind = NetOp::BNRELU;
     op.in0 = y3.p; op.out_act = ar4.p; op.h = h2; op.w = w2; op.c = 128;
     if ((rc = bn("conv4.resample.0", 128, &op.scale, &op.shift))) return rc;
-    push_op(op);
+    ops_.push_back(op);
   }
   // the first max-pool of each hourglass (:309) is written by the block that produces its input: conv4 / conv7
   T p1, pa1, p2, pa2;
@@ -737,7 +693,7 @@ int HourglassNet::emit() {
     NetOp op;
     op.kind = NetOp::MEMSET;
     op.ptr = keys_; op.bytes = sizeof(unsigned long long) * V_ * L_;
-    push_op(op);
+    ops_.push_back(op);
   }
   flops_ += 2.0 * L_ * L_ * 9 * h * w;  // algorithmic FLOPs of the reference's conv11
   const float* b11 = nullptr;
@@ -772,7 +728,7 @@ int HourglassNet::emit() {
         e.up_sy = 2; e.up_sx = 2; e.up_py = a; e.up_px = b;
         if ((rc = conv_plan(s, e, &op.conv))) return rc;
       }
-      push_op(op);
+      ops_.push_back(op);
     }
   }
   {
@@ -780,72 +736,7 @@ int HourglassNet::emit() {
     note_use(x10.p);  // the "moment" selection re-evaluates windows of the last layer from its input
     NetOp op;
     op.kind = NetOp::PEAKS;
-    push_op(op);
-  }
-  return MVLM_OK;
-}
-
-int HourglassNet::build_segments() {
-  segs_.assign(n_segs_, FlowSegment());
-  seg_info_.assign(n_segs_, SegInfo());
-  if (n_segs_ == 0) return MVLM_OK;
-  {
-    std::vector<float> host(2 * epi::kMaxCout, 0.f);
-    for (int i = 0; i < epi::kMaxCout; ++i) host[epi::kMaxCout + i] = 1.f;
-    MVLM_CHECK_CUDA(cudaMalloc(&zeros_, sizeof(float) * host.size()));
-    owned_.push_back(zeros_);
-    ones_ = zeros_ + epi::kMaxCout;
-    MVLM_CHECK_CUDA(cudaMemcpy(zeros_, host.data(), sizeof(float) * host.size(), cudaMemcpyHostToDevice));
-  }
-  for (int sgm = 0; sgm < n_segs_; ++sgm) {
-    std::vector<FlowLayerDesc> layers;
-    int min_tiles = 1 << 30;
-    for (size_t i = 0; i < ops_.size(); ++i) {
-      if (op_seg_[i] != sgm) continue;
-      if (seg_info_[sgm].first_op < 0) seg_info_[sgm].first_op = static_cast<int>(i);
-      const NetOp& op = ops_[i];
-      FlowLayerDesc d;
-      memset(&d.layer, 0, sizeof(d.layer));
-      FlowLayer& L = d.layer;
-      L.ring_in = L.ring_pre = L.ring_raw = L.ring_post = L.ring_res1 = L.ring_res2 = L.ring_up = L.ring_aux = V_;
-      L.cp = {zeros_, ones_, zeros_, zeros_, zeros_, zeros_, zeros_};
-      if (op.kind == NetOp::CONV) {
-        MVLM_REQUIRE(!op.is_head, "hourglass: head conv inside a dataflow segment");
-        L.p = op.conv;
-        L.kind = FLOW_CONV;
-        const ConvEpilogue& e = op.conv.e;
-        L.f = epi::feature_mask(e) | (op.conv.s.cout_pad <= 64 ? epi::F_M64 : 0);
-        if (e.bias) L.cp.bias = e.bias;
-        if (e.mid_scale) { L.cp.mid_s = e.mid_scale; L.cp.mid_t = e.mid_shift; }
-        if (e.out_pre) { L.cp.pre_s = e.pre_scale; L.cp.pre_t = e.pre_shift; }
-        if (e.out_post) { L.cp.post_s = e.post_scale; L.cp.post_t = e.post_shift; }
-        if (e.aux_mode) { L.cp.mid_s = e.aux_scale; L.cp.mid_t = e.aux_shift; }
-        d.tiles_x = op.conv.tiles_x; d.tiles_y = op.conv.tiles_y; d.n_nt = op.conv.n_nt;
-        min_tiles = std::min(min_tiles, d.tiles_x * d.tiles_y * d.n_nt);
-      } else if (op.kind == NetOp::POOL || op.kind == NetOp::BNRELU) {
-        const bool pool = op.kind == NetOp::POOL;
-        L.kind = pool ? FLOW_POOL : FLOW_BNRELU;
-        L.p.s.in = op.in0; L.p.s.n = V_; L.p.s.h = op.h; L.p.s.w = op.w; L.p.s.cin = op.c; L.p.s.in_cs = op.c;
-        L.p.e.out_raw = op.out_raw;
-        L.p.e.out_post = op.out_act;
-        if (op.out_act) { L.cp.post_s = op.scale; L.cp.post_t = op.shift; }
-        L.p.tile_h = epi::kMaxTileH;
-        d.tiles_x = ceil_div(pool ? op.w / 2 : op.w, epi::kTileW);
-        d.tiles_y = ceil_div(pool ? op.h / 2 : op.h, kFlowEltRows);
-        d.n_nt = 1;
-      } else {
-        MVLM_REQUIRE(false, "hourglass: op kind %d cannot run inside a dataflow segment", static_cast<int>(op.kind));
-      }
-      layers.push_back(d);
-    }
-    MVLM_REQUIRE(!layers.empty() && min_tiles < (1 << 30), "hourglass: empty dataflow segment %d", sgm);
-    // views per batch: enough for flow_tiles_ tiles per group, but at least flow_interleave_ batches (the low
-    // levels have one tile per view: three batches of a third of the views keep their dependent chains overlapped)
-    const int batch = std::max(1, std::min(ceil_div(flow_tiles_, min_tiles), ceil_div(V_, flow_interleave_)));
-    seg_info_[sgm].batch = batch;
-    seg_info_[sgm].n_layers = static_cast<int>(layers.size());
-    const int rc = flow_build_segment(layers, V_, batch, flow_interleave_, &owned_, &segs_[sgm]);
-    if (rc) return rc;
+    ops_.push_back(op);
   }
   return MVLM_OK;
 }
@@ -908,20 +799,10 @@ int HourglassNet::forward(const unsigned char* img_u8, const float* img_f32, flo
                           cudaStream_t stream) {
   MVLM_REQUIRE(!dry_, "hourglass: forward on a dry plan");
   MVLM_REQUIRE(out_peaks || out_heatmaps, "hourglass: no output requested");
-  for (size_t i = 0; i < ops_.size(); ++i) {
-    const int rc = run_step(i, img_u8, img_f32, out_heatmaps, out_peaks, stream);
+  for (NetOp& op : ops_) {
+    const int rc = run_op(op, img_u8, img_f32, out_heatmaps, out_peaks, stream);
     if (rc != MVLM_OK) return rc;
   }
-  return MVLM_OK;
-}
-
-// op i as the plan executes it: the first op of a dataflow segment launches the whole segment, its other ops
-// are part of that launch
-int HourglassNet::run_step(size_t i, const unsigned char* img_u8, const float* img_f32, float* out_heatmaps,
-                           float* out_peaks, cudaStream_t stream) {
-  const int sgm = op_seg_[i];
-  if (sgm < 0) return run_op(ops_[i], img_u8, img_f32, out_heatmaps, out_peaks, stream);
-  if (seg_info_[sgm].first_op == static_cast<int>(i)) return flow_launch(segs_[sgm], stream);
   return MVLM_OK;
 }
 
@@ -937,7 +818,7 @@ int HourglassNet::profile_ops(const unsigned char* img_u8, const float* img_f32,
   for (int r = 0; r < reps && rc == MVLM_OK; ++r) {
     MVLM_CHECK_CUDA(cudaEventRecord(ev[0], stream));
     for (size_t i = 0; i < n && rc == MVLM_OK; ++i) {
-      rc = run_step(i, img_u8, img_f32, nullptr, out_peaks, stream);
+      rc = run_op(ops_[i], img_u8, img_f32, nullptr, out_peaks, stream);
       MVLM_CHECK_CUDA(cudaEventRecord(ev[i + 1], stream));
     }
     MVLM_CHECK_CUDA(cudaStreamSynchronize(stream));
@@ -955,29 +836,6 @@ int HourglassNet::profile_ops(const unsigned char* img_u8, const float* img_f32,
     std::vector<long long> host(kConvProfInts);
     for (size_t i = 0; i < n && rc == MVLM_OK; ++i) {
       for (int k = 0; k < 8; ++k) roles_out[i * 8 + k] = 0.0;
-      if (op_seg_[i] >= 0) {  // dataflow segments: their own counters (conv_flow.cu), reported by the first op
-        const bool first = seg_info_[op_seg_[i]].first_op == static_cast<int>(i);
-        if (first) {
-          MVLM_CHECK_CUDA(cudaMemsetAsync(dev, 0, sizeof(long long) * kConvProfInts, stream));
-          flow_set_profile_buffer(dev);
-        }
-        rc = run_step(i, img_u8, img_f32, nullptr, out_peaks, stream);
-        flow_set_profile_buffer(nullptr);
-        if (first && rc == MVLM_OK) {
-          MVLM_CHECK_CUDA(cudaStreamSynchronize(stream));
-          MVLM_CHECK_CUDA(cudaMemcpy(host.data(), dev, sizeof(long long) * kConvProfInts, cudaMemcpyDeviceToHost));
-          int ctas = 0;
-          for (int c = 0; c < kNumSMs; ++c) {
-            if (host[c * 8 + 7] == 0) continue;
-            ++ctas;
-            for (int k = 0; k < 8; ++k) roles_out[i * 8 + k] += static_cast<double>(host[c * 8 + k]);
-          }
-          for (int k = 0; k < 8; ++k) roles_out[i * 8 + k] /= ctas > 0 ? ctas : 1;
-          if (trace_out && static_cast<int>(i) == trace_op)
-            for (int k = 0; k < kConvTraceTiles * 16; ++k) trace_out[k] = host[kNumSMs * 8 + k];
-        }
-        continue;
-      }
       if (ops_[i].kind == NetOp::CONV) {
         MVLM_CHECK_CUDA(cudaMemsetAsync(dev, 0, sizeof(long long) * kConvProfInts, stream));
         conv_set_profile_buffer(dev);
@@ -1007,25 +865,18 @@ std::string HourglassNet::describe_op(int i) const {
   if (i < 0 || i >= static_cast<int>(ops_.size())) return "";
   const NetOp& op = ops_[i];
   char buf[256];
-  if (op_seg_[i] >= 0 && seg_info_.size() > static_cast<size_t>(op_seg_[i]) && seg_info_[op_seg_[i]].first_op == i) {
-    const SegInfo& si = seg_info_[op_seg_[i]];
-    snprintf(buf, sizeof(buf), "flow segment %d: %d layers, %d view(s) per batch, %d batches in lock step, %d items",
-             op_seg_[i], si.n_layers, si.batch, flow_interleave_, segs_[op_seg_[i]].n_items);
-    return buf;
-  }
-  const char* in_seg = op_seg_[i] >= 0 ? "  (in segment) " : "";
   switch (op.kind) {
     case NetOp::CONV: {
       const ConvShape& s = op.conv.s;
       const ConvEpilogue& e = op.conv.e;
-      snprintf(buf, sizeof(buf), "%sconv %s %dx%d %d->%d k%d%s%s%s%s%s%s%s%s", in_seg, op.tag, s.h, s.w, s.cin, s.cout_pad, s.kh,
+      snprintf(buf, sizeof(buf), "conv %s %dx%d %d->%d k%d%s%s%s%s%s%s%s%s", op.tag, s.h, s.w, s.cin, s.cout_pad, s.kh,
                e.out_pre ? " pre" : "", e.res1 ? " res1" : "", e.res2 ? " res2" : "", e.res_up ? " up" : "", e.out_raw ? " raw" : "",
                e.out_post ? " post" : "", e.pool2 ? " pool" : (e.aux_mode == 2 ? " +pooled" : (e.aux_mode == 1 ? " +act2" : "")),
                e.argmax_keys ? " argmax" : "");
       break;
     }
-    case NetOp::POOL: snprintf(buf, sizeof(buf), "%spool %dx%dx%d", in_seg, op.h, op.w, op.c); break;
-    case NetOp::BNRELU: snprintf(buf, sizeof(buf), "%sbnrelu %dx%dx%d", in_seg, op.h, op.w, op.c); break;
+    case NetOp::POOL: snprintf(buf, sizeof(buf), "pool %dx%dx%d", op.h, op.w, op.c); break;
+    case NetOp::BNRELU: snprintf(buf, sizeof(buf), "bnrelu %dx%dx%d", op.h, op.w, op.c); break;
     case NetOp::STEM: snprintf(buf, sizeof(buf), "stem-stage %dx%dx%d", op.h, op.w, op.c); break;
     case NetOp::MEMSET: snprintf(buf, sizeof(buf), "memset %zu", op.bytes); break;
     case NetOp::PEAKS: snprintf(buf, sizeof(buf), "peaks"); break;

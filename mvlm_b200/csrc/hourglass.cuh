@@ -5,7 +5,6 @@
 #include <string>
 #include <vector>
 
-#include "conv_flow.cuh"
 #include "conv_umma.cuh"
 #include "stages.cuh"
 
@@ -46,10 +45,8 @@ class HourglassNet {
               cudaStream_t stream);
   int run_op(NetOp& op, const unsigned char* img_u8, const float* img_f32, float* out_heatmaps, float* out_peaks,
              cudaStream_t stream);
-  int run_step(size_t i, const unsigned char* img_u8, const float* img_f32, float* out_heatmaps, float* out_peaks,
-               cudaStream_t stream);
   // Captures the launch sequence of forward() into a CUDA graph per distinct argument tuple and replays it
-  // (the plan is static: ~155 launches per call).  Falls back to plain launches if capture is unavailable.
+  // (the plan is static: 144 launches per call).  Falls back to plain launches if capture is unavailable.
   int forward_graph(const unsigned char* img_u8, const float* img_f32, float* out_heatmaps, float* out_peaks,
                     cudaStream_t stream);
 
@@ -75,7 +72,6 @@ class HourglassNet {
   int width() const { return W_; }
   double flops_per_view() const { return flops_; }
   int n_ops() const { return static_cast<int>(ops_.size()); }
-  int n_segments() const { return n_segs_; }
   const std::vector<NetOp>& ops() const { return ops_; }
   // intermediate tensors exposed for layer-wise parity tests: name -> (ptr, h, w, c)
   struct Probe { const __nv_bfloat16* p; int h, w, c; };
@@ -121,29 +117,6 @@ class HourglassNet {
          T* pool_raw = nullptr, const T* up_low = nullptr, const RbAux* aux = nullptr);
   int hourglass(const std::string& p, T x, T a_x, T* out, const T* in_pooled = nullptr, const T* in_pooled_act = nullptr);
   int emit_pool(T in, T out_raw, const char* bn_name, T out_act);
-
-  // ---- dataflow segments (conv_flow.cuh): runs of consecutive ops executed by ONE persistent launch over view
-  // batches with tile-level dependencies instead of one launch per layer.  op_seg_[i] = segment of op i or -1
-  // (per-layer launch); push_op assigns them from the ops' output resolution.
-  void push_op(const NetOp& op);
-  int build_segments();
-  // Off unless MVLM_FLOW=1: measured on the headline workload (profiles/r2_flow_experiments.txt) the segments are
-  // bit-identical to the per-layer launches but not faster -- 18.0 ms against 18.0 ms with the hourglass levels of
-  // <= 32 rows in segments (2 x 55 latency-bound launches become 2 x 3), 20.0 ms with the large layers in them (their
-  // epilogues cannot prefetch residuals across the accumulator wait without spilling) -- so the default plan keeps one
-  // launch per layer.  Ops whose output is flow_lo_ .. flow_hi_ rows high run in segments when it is on.
-  bool flow_on_ = false;
-  int flow_lo_ = 1, flow_hi_ = 32;
-  int cur_seg_layers_ = 0;
-  int flow_tiles_ = 64;      // views per batch = smallest count giving every conv group this many tiles
-  int flow_interleave_ = 3;  // batches advanced in lock step
-  int cur_seg_ = -1, n_segs_ = 0;
-  std::vector<int> op_seg_;
-  std::vector<FlowSegment> segs_;
-  struct SegInfo { int batch = 1, n_layers = 0, first_op = -1; };
-  std::vector<SegInfo> seg_info_;
-  float* zeros_ = nullptr;  // kMaxCout zeros / ones: stand-ins for absent per-channel parameters
-  float* ones_ = nullptr;
 
   const StateDict* sd_ = nullptr;
   // state_dict entry `name` with exactly `numel` elements (a checkpoint of another model must not be misread)

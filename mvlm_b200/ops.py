@@ -168,7 +168,6 @@ class Hourglass:
         self._h = handle
         self.flops_per_view = lib.mvlm_hourglass_flops_per_view(n_landmarks, cin, h, w)
         self.num_launches = lib.mvlm_hourglass_num_launches(handle)
-        self.num_segments = lib.mvlm_hourglass_num_segments(handle)
 
     def forward(self, img, want_heatmaps: bool = False, want_peaks: bool = True, graph: bool = False,
                 selection_method: str = "simple"):

@@ -27,17 +27,7 @@ for a in sys.argv:
 trace = (C.c_longlong * (64 * 16))()
 _lib.check(lib.mvlm_debug_hourglass_profile(net._h, img.data_ptr(), None, peaks.data_ptr(), 5, ms, roles, trace_op, trace,
                                             torch.cuda.current_stream().cuda_stream), "profile")
-if trace_op >= 0 and "--flow" in sys.argv:
-    print(f"timeline of CTA 0 / epilogue warp 2, segment at op {trace_op}: item | layer | fetched, deps-seen, acc-ready, done | "
-          "item-span | unit0: ld sts out end | unit1: ld sts out end")
-    for t in range(64):
-        r = [trace[t * 16 + k] for k in range(16)]
-        if r[3] == 0:
-            continue
-        print(f"  item {r[3]:5d} layer {r[2]:2d} | {r[0]:9d} {r[1] - r[0]:6d} {r[5] - r[0] if r[5] else -1:6d} {r[6] - r[0]:6d} | "
-              f"unit0: ld {r[8] - r[5]:5d} sts {r[9] - r[8]:5d} out {r[10] - r[9]:5d} end {r[11] - r[10]:5d} | unit1: ld {r[12] - r[11]:5d} "
-              f"sts {r[13] - r[12]:5d} out {r[14] - r[13]:5d} end {r[15] - r[14]:5d}")
-elif trace_op >= 0:
+if trace_op >= 0:
     lib.mvlm_debug_hourglass_describe(net._h, trace_op, C.create_string_buffer(256), 256)
     print(f"timeline of CTA 0, op {trace_op} (cycles since kernel start): tile | P halo-issued, P weights-issued | "
           "M acc-acquired, M halo-landed, M issued | E acc-ready, E released")
@@ -64,7 +54,4 @@ print("roles (kcycles per CTA per op): prod-wait-A/B-empty | mma-wait-operands /
 for d, (cnt, t, r) in sorted(agg.items(), key=lambda kv: -kv[1][1]):
     r = [x / cnt / 1e3 for x in r]
     rs = f"  P {r[0]:6.0f} {r[1]:6.0f} | M {r[2]:6.0f} {r[3]:6.0f} {r[4]:6.0f} | E {r[5]:6.0f} {r[6]:6.0f}" if d.startswith("conv") else ""
-    if d.startswith("flow segment"):
-        rs = (f"\n      tracker: dep-wait {r[0]:6.0f} halo-slot-wait {r[1]:6.0f} | MMA: operand-wait {r[2]:6.0f} acc-wait {r[3]:6.0f} "
-              f"total {r[4]:6.0f} | epilogue w2: acc-ready-wait {r[5]:6.0f} dep-flag-wait {r[6]:6.0f} total {r[7]:6.0f} (kcycles)")
     print(f"{t:8.3f} ms {100 * t / total:5.1f}%  x{cnt:3d}  {t / cnt * 1000:8.1f} us/op  {d:62s}{rs}")
