@@ -152,6 +152,28 @@ int mvlm_raster_multiview(const float* verts, int n_verts, const float* uvs, con
                           int32_t* out_tri_id /* (V,H,W) */, float* out_depth /* (V,H,W) */,
                           void* stream);
 
+/* Several scans in one pass (the batch drivers' small-view case: one CNN plan over all views of the pass).  Views   */
+/* are scan-major: global view g = s * n_views + v, rot (S*V,9), outputs (S*V,H,W,...).  Each scan's views are      */
+/* rendered exactly as mvlm_raster_multiview renders them alone.  The table is passed to the kernels by value: up   */
+/* to MVLM_MAX_SCANS entries, host memory, no copy to the device.  workspace:                                       */
+/* mvlm_raster_multiscan_workspace_bytes(S, V, H, W, largest n_verts of the pass); for S = 1 it equals             */
+/* mvlm_raster_workspace_bytes(V, H, W, n_verts).                                                                   */
+#define MVLM_MAX_SCANS 64
+typedef struct mvlm_raster_scan {
+  const float* verts; /* (Nv,3) */
+  int n_verts;
+  const float* uvs;   /* (Nv,2) or NULL */
+  const int32_t* tris; /* (Nt,3) */
+  int n_tris;
+  const uint8_t* tex; /* (Th,Tw,tex_channels) or NULL */
+  int tex_h, tex_w, tex_channels;
+} mvlm_raster_scan;
+size_t mvlm_raster_multiscan_workspace_bytes(int n_scans, int n_views, int h, int w, int max_verts);
+int mvlm_raster_multiscan(const mvlm_raster_scan* scans /* host, n_scans entries */, int n_scans,
+                          const double* rot /* (S*V,9) */, int n_views, int h, int w, int channel_mode, void* workspace,
+                          size_t workspace_bytes, uint8_t* out_u8 /* (S*V,H,W,4) */, float* out_f32 /* (S*V,H,W,C) */,
+                          int32_t* out_tri_id /* (S*V,H,W) */, float* out_depth /* (S*V,H,W) */, void* stream);
+
 /* ------------------------------------------------------------------------- */
 /* Stage 2: stacked-hourglass heat-map CNN (MVLMModel),                       */
 /*   src/mvlm/prediction/paulsenpredictor.py:364-432 driven by                 */
@@ -233,6 +255,18 @@ int mvlm_consensus(const float* peaks, const double* starts, const double* ends,
                    size_t workspace_bytes, double* out_landmarks /* (L,3) */, double* out_errors /* (L) */,
                    int32_t* out_nlines /* (L) or NULL */, void* stream);
 
+/* Several scans of one pass in the same three launches.  peaks / starts / ends are the pass's (L,S*V,3) arrays     */
+/* (scan s at views [s*V, (s+1)*V)); draws: one (L,H,8) table every scan uses (draws_per_scan = 0, the seeded      */
+/* estimator) or one (S,L,H,8) table (draws_per_scan = 1, the reference RNG replay).  Outputs (S,L,3), (S,L), (S,L).*/
+/* Each scan gets exactly what mvlm_consensus returns for it alone.  S = 1 is mvlm_consensus.                       */
+size_t mvlm_consensus_multiscan_workspace_bytes(int n_scans, int n_landmarks, int n_views, int n_hyp);
+int mvlm_consensus_multiscan(const float* peaks, const double* starts, const double* ends, int n_scans,
+                             int n_landmarks, int n_views, int mode, double threshold_quantile,
+                             float threshold_absolute, const uint32_t* draws, int draws_per_scan, int n_hyp,
+                             double dist_thres, void* workspace, size_t workspace_bytes,
+                             double* out_landmarks /* (S,L,3) */, double* out_errors /* (S,L) */,
+                             int32_t* out_nlines /* (S,L) or NULL */, void* stream);
+
 /* ------------------------------------------------------------------------- */
 /* Stage 5b: snap to the mesh surface.  Replaces                               */
 /*   Estimator3D.project_landmarks_to_surface estimator3d.py:252-285.          */
@@ -257,6 +291,21 @@ int mvlm_snap_grid_query(const float* verts, const int32_t* tris, int n_tris, co
                          size_t grid_bytes, const double* landmarks, int n_landmarks, void* workspace,
                          size_t workspace_bytes, double* out /* (L,3) */, int32_t* out_tri /* (L) or NULL */,
                          int32_t* out_stats /* (L,2) or NULL */, void* stream);
+/* Several scans of one pass: landmarks (S,L,3) of scan s snapped to mesh s, the same points and triangles as one  */
+/* mvlm_snap_to_mesh (grid = NULL) or mvlm_snap_grid_query (grid built by mvlm_snap_grid_build) per scan.  The     */
+/* brute-force scan of every scan runs in one launch pair; scans with a grid add one query launch each.  The table */
+/* is host memory (up to MVLM_MAX_SCANS entries).                                                                 */
+typedef struct mvlm_snap_mesh {
+  const float* verts;   /* (Nv,3) */
+  const int32_t* tris;  /* (Nt,3) */
+  int n_tris;
+  const void* grid;     /* NULL or this mesh's grid */
+  size_t grid_bytes;
+} mvlm_snap_mesh;
+size_t mvlm_snap_to_meshes_workspace_bytes(const mvlm_snap_mesh* meshes, int n_scans, int n_landmarks);
+int mvlm_snap_to_meshes(const mvlm_snap_mesh* meshes, int n_scans, const double* landmarks /* (S,L,3) */,
+                        int n_landmarks, void* workspace, size_t workspace_bytes, double* out /* (S,L,3) */,
+                        int32_t* out_tri /* (S,L) or NULL */, void* stream);
 /* debug: grid dims[3] + oversize-list length, cell edge + largest binned triangle radius (synchronises) */
 int mvlm_debug_snap_grid_describe(const void* grid, int32_t* dims_nover /* [4] */, double* edge_tau /* [2] */,
                                   void* stream);

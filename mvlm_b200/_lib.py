@@ -48,6 +48,21 @@ class ObjParseInfo(C.Structure):
                 ("n_positions", C.c_int32), ("n_bytes", C.c_size_t)]
 
 
+class RasterScan(C.Structure):
+    """mvlm_raster_scan: one scan of a multi-scan raster pass (device pointers)."""
+    _fields_ = [("verts", C.c_void_p), ("n_verts", C.c_int), ("uvs", C.c_void_p), ("tris", C.c_void_p),
+                ("n_tris", C.c_int), ("tex", C.c_void_p), ("tex_h", C.c_int), ("tex_w", C.c_int),
+                ("tex_channels", C.c_int)]
+
+
+class SnapMesh(C.Structure):
+    """mvlm_snap_mesh: one mesh of a multi-scan snap (device pointers, grid optional)."""
+    _fields_ = [("verts", C.c_void_p), ("tris", C.c_void_p), ("n_tris", C.c_int), ("grid", C.c_void_p),
+                ("grid_bytes", C.c_size_t)]
+
+
+MAX_SCANS = 64  # MVLM_MAX_SCANS
+
 _lib = None
 
 
@@ -77,6 +92,9 @@ def _declare(lib: C.CDLL) -> None:
         "mvlm_raster_workspace_bytes": ([i32, i32, i32, i32], C.c_size_t),
         "mvlm_raster_multiview": ([vp, i32, vp, vp, i32, vp, i32, i32, i32, vp, i32, i32, i32, i32, vp, C.c_size_t, vp, vp,
                                    vp, vp, vp], i32),
+        "mvlm_raster_multiscan_workspace_bytes": ([i32, i32, i32, i32, i32], C.c_size_t),
+        "mvlm_raster_multiscan": ([C.POINTER(RasterScan), i32, vp, i32, i32, i32, i32, vp, C.c_size_t, vp, vp, vp, vp, vp],
+                                  i32),
         "mvlm_hourglass_workspace_bytes": ([i32, i32, i32, i32, i32], C.c_size_t),
         "mvlm_hourglass_flops_per_view": ([i32, i32, i32, i32], f64),
         "mvlm_hourglass_create": ([C.POINTER(C.c_char_p), C.POINTER(vp), C.POINTER(C.c_longlong), i32, i32, i32, i32,
@@ -108,7 +126,12 @@ def _declare(lib: C.CDLL) -> None:
         "mvlm_rays_from_peaks": ([vp, vp, i32, i32, i32, vp, vp, vp], i32),
         "mvlm_consensus_workspace_bytes": ([i32, i32, i32], C.c_size_t),
         "mvlm_consensus": ([vp, vp, vp, i32, i32, i32, f64, f32, vp, i32, f64, vp, C.c_size_t, vp, vp, vp, vp], i32),
+        "mvlm_consensus_multiscan_workspace_bytes": ([i32, i32, i32, i32], C.c_size_t),
+        "mvlm_consensus_multiscan": ([vp, vp, vp, i32, i32, i32, i32, f64, f32, vp, i32, i32, f64, vp, C.c_size_t, vp, vp,
+                                      vp, vp], i32),
         "mvlm_snap_workspace_bytes": ([i32, i32], C.c_size_t),
+        "mvlm_snap_to_meshes_workspace_bytes": ([C.POINTER(SnapMesh), i32, i32], C.c_size_t),
+        "mvlm_snap_to_meshes": ([C.POINTER(SnapMesh), i32, vp, i32, vp, C.c_size_t, vp, vp, vp], i32),
         "mvlm_snap_to_mesh": ([vp, vp, i32, vp, i32, vp, C.c_size_t, vp, vp, vp], i32),
         "mvlm_snap_grid_bytes": ([i32], C.c_size_t),
         "mvlm_snap_grid_build": ([vp, vp, i32, vp, C.c_size_t, vp], i32),

@@ -55,6 +55,7 @@ __global__ void pack_conv_weight_kernel(const float* __restrict__ w, int cout, i
 }  // namespace mvlm
 
 using namespace mvlm;
+static_assert(kMaxScans == MVLM_MAX_SCANS, "scan table size");
 
 extern "C" {
 
@@ -121,9 +122,28 @@ int mvlm_raster_multiview(const float* verts, int n_verts, const float* uvs, con
                           const uint8_t* tex, int tex_h, int tex_w, int tex_channels, const double* rot, int n_views, int h,
                           int w, int channel_mode, void* workspace, size_t workspace_bytes, uint8_t* out_u8, float* out_f32,
                           int32_t* out_tri_id, float* out_depth, void* stream) {
+  const mvlm_raster_scan scan = {verts, n_verts, uvs, tris, n_tris, tex, tex_h, tex_w, tex_channels};
+  return mvlm_raster_multiscan(&scan, 1, rot, n_views, h, w, channel_mode, workspace, workspace_bytes, out_u8, out_f32,
+                               out_tri_id, out_depth, stream);
+}
+
+size_t mvlm_raster_multiscan_workspace_bytes(int n_scans, int n_views, int h, int w, int max_verts) {
+  return raster_workspace_bytes(n_scans * n_views, h, w, max_verts);
+}
+
+int mvlm_raster_multiscan(const mvlm_raster_scan* scans, int n_scans, const double* rot, int n_views, int h, int w,
+                          int channel_mode, void* workspace, size_t workspace_bytes, uint8_t* out_u8, float* out_f32,
+                          int32_t* out_tri_id, float* out_depth, void* stream) {
+  MVLM_REQUIRE(scans, "mvlm_raster_multiscan: null scan table");
+  MVLM_REQUIRE(n_scans > 0 && n_scans <= kMaxScans, "mvlm_raster_multiscan: 1 to %d scans per pass (got %d)", kMaxScans,
+               n_scans);
+  RasterScan table[kMaxScans];
+  for (int s = 0; s < n_scans; ++s) {
+    const mvlm_raster_scan& q = scans[s];
+    table[s] = RasterScan{q.verts, q.uvs, q.tris, q.tex, q.n_verts, q.n_tris, q.tex_h, q.tex_w, q.tex_channels};
+  }
   RasterArgs a;
-  a.verts = verts; a.nv = n_verts; a.uvs = uvs; a.tris = tris; a.nt = n_tris;
-  a.tex = tex; a.th = tex_h; a.tw = tex_w; a.tex_c = tex_channels;
+  a.scans = table; a.n_scans = n_scans;
   a.rot = rot; a.n_views = n_views; a.h = h; a.w = w; a.channel_mode = channel_mode;
   a.zbuf = static_cast<unsigned long long*>(workspace); a.workspace_bytes = workspace_bytes;
   a.out_u8 = out_u8; a.out_f32 = out_f32; a.out_tri = out_tri_id; a.out_z = out_depth;
@@ -243,10 +263,26 @@ int mvlm_consensus(const float* peaks, const double* starts, const double* ends,
                    int mode, double threshold_quantile, float threshold_absolute, const uint32_t* draws, int n_hyp,
                    double dist_thres, void* workspace, size_t workspace_bytes, double* out_landmarks,
                    double* out_errors, int32_t* out_nlines, void* stream) {
+  return mvlm_consensus_multiscan(peaks, starts, ends, 1, n_landmarks, n_views, mode, threshold_quantile,
+                                  threshold_absolute, draws, 0, n_hyp, dist_thres, workspace, workspace_bytes,
+                                  out_landmarks, out_errors, out_nlines, stream);
+}
+
+size_t mvlm_consensus_multiscan_workspace_bytes(int n_scans, int n_landmarks, int n_views, int n_hyp) {
+  return consensus_workspace_bytes(n_landmarks, n_views, n_hyp, n_scans);
+}
+
+int mvlm_consensus_multiscan(const float* peaks, const double* starts, const double* ends, int n_scans,
+                             int n_landmarks, int n_views, int mode, double threshold_quantile,
+                             float threshold_absolute, const uint32_t* draws, int draws_per_scan, int n_hyp,
+                             double dist_thres, void* workspace, size_t workspace_bytes, double* out_landmarks,
+                             double* out_errors, int32_t* out_nlines, void* stream) {
   ConsensusArgs a;
-  a.peaks = peaks; a.starts = starts; a.ends = ends; a.l = n_landmarks; a.v = n_views; a.mode = mode;
+  a.peaks = peaks; a.starts = starts; a.ends = ends; a.l = n_landmarks; a.v = n_views; a.n_scans = n_scans;
+  a.mode = mode;
   a.threshold_quantile = threshold_quantile; a.threshold_absolute = threshold_absolute;
   a.draws = draws; a.n_hyp = n_hyp; a.dist_thres = dist_thres;
+  a.draws_scan_stride = draws_per_scan ? static_cast<size_t>(n_landmarks) * n_hyp * 8 : 0;
   a.workspace = workspace; a.workspace_bytes = workspace_bytes;
   a.out_landmarks = out_landmarks; a.out_errors = out_errors; a.out_nlines = out_nlines;
   return consensus_launch(a, static_cast<cudaStream_t>(stream));
@@ -275,6 +311,39 @@ int mvlm_snap_grid_query(const float* verts, const int32_t* tris, int n_tris, co
                          int32_t* out_tri, int32_t* out_stats, void* stream) {
   return snap_grid_query(verts, tris, n_tris, grid, grid_bytes, landmarks, n_landmarks, workspace, workspace_bytes, out,
                          out_tri, out_stats, static_cast<cudaStream_t>(stream));
+}
+
+static int snap_table(const mvlm_snap_mesh* meshes, int n_scans, SnapMesh* table, const void** grids) {
+  MVLM_REQUIRE(meshes, "mvlm_snap_to_meshes: null mesh table");
+  MVLM_REQUIRE(n_scans > 0 && n_scans <= kMaxScans, "mvlm_snap_to_meshes: 1 to %d scans per pass (got %d)", kMaxScans,
+               n_scans);
+  for (int i = 0; i < n_scans; ++i) {
+    table[i] = SnapMesh{meshes[i].verts, meshes[i].tris, meshes[i].n_tris};
+    grids[i] = meshes[i].grid;
+    MVLM_REQUIRE(!meshes[i].grid || (meshes[i].n_tris > 0 && meshes[i].grid_bytes >= snap_grid_bytes(meshes[i].n_tris)),
+                 "mvlm_snap_to_meshes: grid buffer of scan %d too small", i);
+  }
+  return MVLM_OK;
+}
+
+size_t mvlm_snap_to_meshes_workspace_bytes(const mvlm_snap_mesh* meshes, int n_scans, int n_landmarks) {
+  SnapMesh table[kMaxScans];
+  const void* grids[kMaxScans];
+  if (snap_table(meshes, n_scans, table, grids) != MVLM_OK) return 0;
+  return snap_meshes_workspace_bytes(table, n_scans, n_landmarks);
+}
+
+int mvlm_snap_to_meshes(const mvlm_snap_mesh* meshes, int n_scans, const double* landmarks, int n_landmarks,
+                        void* workspace, size_t workspace_bytes, double* out, int32_t* out_tri, void* stream) {
+  SnapMesh table[kMaxScans];
+  const void* grids[kMaxScans];
+  const int rc = snap_table(meshes, n_scans, table, grids);
+  if (rc != MVLM_OK) return rc;
+  const cudaStream_t s = static_cast<cudaStream_t>(stream);
+  if (n_scans == 1 && grids[0])  // one scan with a grid: exactly mvlm_snap_grid_query's launches
+    return snap_grid_query(table[0].verts, table[0].tris, table[0].nt, grids[0], meshes[0].grid_bytes, landmarks,
+                           n_landmarks, workspace, workspace_bytes, out, out_tri, nullptr, s);
+  return snap_meshes_launch(table, grids, n_scans, landmarks, n_landmarks, workspace, workspace_bytes, out, out_tri, s);
 }
 
 int mvlm_debug_snap_grid_describe(const void* grid, int32_t* dims_nover, double* edge_tau, void* stream) {

@@ -13,7 +13,11 @@
 // commented-out loop's: first strict minimum of the mean squared inlier distance.
 //
 // Kernels (all fp64; compiled with --fmad=false to round like numpy):
-//   consensus_prepare     one block per landmark: np.quantile('linear', float32) threshold, strict
+// Several scans of one pass run in the same three launches: grid axis z (prepare: y) is the scan, peaks / rays are
+// read with the pass's view stride ((L, S*V, 3), scan s at views [s*V, (s+1)*V)), every per-landmark slot of the
+// workspace and the outputs is (S, L, ...).  A scan's result does not depend on the other scans nor on `splits`.
+//
+//   consensus_prepare     one block per (landmark, scan): np.quantile('linear', float32) threshold, strict
 //                         `>` mask, order-preserving compaction, per-line normal-equation terms
 //                         M_i = n n^T - I and M_i a_i, LSQ over all kept lines (the fallback).
 //   consensus_hypotheses  grid (L, splits): lines of the landmark staged in shared memory, one THREAD
@@ -102,12 +106,13 @@ __device__ __forceinline__ double warp_sum(double x) {
 }
 
 struct Layout {
-  double* lines;  // L * V * 15
-  double* p_all;  // L * 3
-  double* part;   // L * splits * 5
-  int* nl;        // L
+  double* lines;  // S * L * V * 16
+  double* p_all;  // S * L * 3
+  double* part;   // S * L * splits * 5
+  int* nl;        // S * L
 };
 
+// L: landmarks x scans of the pass
 __host__ __device__ inline Layout carve(void* ws, int L, int V, int splits) {
   Layout o;
   double* d = static_cast<double*>(ws);
@@ -127,11 +132,14 @@ __global__ void __launch_bounds__(256) consensus_prepare_kernel(ConsensusArgs g,
   __shared__ float sel[2];
   __shared__ int any_nan;
   __shared__ double red[9][8];
-  const int l = blockIdx.x, V = g.v, tid = threadIdx.x;
+  const int V = g.v, tid = threadIdx.x;
+  const int sl = blockIdx.y * g.l + blockIdx.x;  // (scan, landmark) slot
+  // row of this landmark's views of this scan in the (L, S*V, 3) peaks / rays
+  const size_t row = static_cast<size_t>(blockIdx.x) * g.n_scans * V + static_cast<size_t>(blockIdx.y) * V;
   if (tid == 0) { any_nan = 0; sel[0] = sel[1] = 0.f; }
   __syncthreads();
   for (int i = tid; i < V; i += blockDim.x) {
-    const float x = g.peaks[(static_cast<size_t>(l) * V + i) * 3 + 2];
+    const float x = g.peaks[(row + i) * 3 + 2];
     vals[i] = x;
     if (x != x) any_nan = 1;
   }
@@ -175,12 +183,12 @@ __global__ void __launch_bounds__(256) consensus_prepare_kernel(ConsensusArgs g,
     if (!keep[i]) continue;
     int pos = 0;
     for (int j = 0; j < i; ++j) pos += keep[j];
-    const double* a = g.starts + (static_cast<size_t>(l) * V + i) * 3;
-    const double* b = g.ends + (static_cast<size_t>(l) * V + i) * 3;
+    const double* a = g.starts + (row + i) * 3;
+    const double* b = g.ends + (row + i) * 3;
     const double sx = b[0] - a[0], sy = b[1] - a[1], sz = b[2] - a[2];
     const double nrm = sqrt((sx * sx + sy * sy) + sz * sz);
     const double nx = sx / nrm, ny = sy / nrm, nz = sz / nrm;
-    double* ln = ws.lines + (static_cast<size_t>(l) * V + pos) * kLineDoubles;
+    double* ln = ws.lines + (static_cast<size_t>(sl) * V + pos) * kLineDoubles;
     ln[0] = a[0]; ln[1] = a[1]; ln[2] = a[2];
     ln[3] = b[0]; ln[4] = b[1]; ln[5] = b[2];
     const double mxx = nx * nx - 1.0, myy = ny * ny - 1.0, mzz = nz * nz - 1.0;
@@ -209,9 +217,9 @@ __global__ void __launch_bounds__(256) consensus_prepare_kernel(ConsensusArgs g,
     }
     double p[3];
     sym3_pinv_solve(S, S + 6, p);
-    ws.p_all[3 * l] = p[0]; ws.p_all[3 * l + 1] = p[1]; ws.p_all[3 * l + 2] = p[2];
-    ws.nl[l] = n_kept;
-    if (g.out_nlines) g.out_nlines[l] = n_kept;
+    ws.p_all[3 * sl] = p[0]; ws.p_all[3 * sl + 1] = p[1]; ws.p_all[3 * sl + 2] = p[2];
+    ws.nl[sl] = n_kept;
+    if (g.out_nlines) g.out_nlines[sl] = n_kept;
   }
 }
 
@@ -222,14 +230,17 @@ __global__ void __launch_bounds__(256) consensus_hyp_kernel(ConsensusArgs g, Lay
   extern __shared__ double sl[];  // n * 16
   __shared__ double wbest[8][kPartDoubles];
   const int l = blockIdx.x, split = blockIdx.y;
-  const int n = ws.nl[l];
+  const int slot = blockIdx.z * g.l + l;  // (scan, landmark) slot
+  const int n = ws.nl[slot];
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  double* part = ws.part + (static_cast<size_t>(l) * splits + split) * kPartDoubles;
+  double* part = ws.part + (static_cast<size_t>(slot) * splits + split) * kPartDoubles;
   if (n < 3) {  // plain LSQ, handled by finalize
     if (tid == 0) { part[0] = kNoFit; part[1] = -1.0; part[2] = part[3] = part[4] = 0.0; }
     return;
   }
-  const double* gl = ws.lines + static_cast<size_t>(l) * g.v * kLineDoubles;
+  const double* gl = ws.lines + static_cast<size_t>(slot) * g.v * kLineDoubles;
+  const unsigned int* draws_l = g.draws + static_cast<size_t>(blockIdx.z) * g.draws_scan_stride +
+                                static_cast<size_t>(l) * g.n_hyp * 8;
   for (int i = tid; i < n * kLineDoubles; i += blockDim.x) sl[i] = gl[i];
   __syncthreads();
   const int h_begin = split * chunk;
@@ -240,7 +251,7 @@ __global__ void __launch_bounds__(256) consensus_hyp_kernel(ConsensusArgs g, Lay
   for (int h = h_begin + tid; h < h_end; h += blockDim.x) {
     // --- 8-line LSQ (:105-107)
     double s9[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
-    const uint4* dr = reinterpret_cast<const uint4*>(g.draws + (static_cast<size_t>(l) * g.n_hyp + h) * 8);
+    const uint4* dr = reinterpret_cast<const uint4*>(draws_l + static_cast<size_t>(h) * 8);
     const uint4 d0 = __ldg(dr), d1 = __ldg(dr + 1);
     const unsigned int draws[8] = {d0.x, d0.y, d0.z, d0.w, d1.x, d1.y, d1.z, d1.w};
 #pragma unroll
@@ -302,8 +313,8 @@ __global__ void __launch_bounds__(256) consensus_hyp_kernel(ConsensusArgs g, Lay
 }
 
 __global__ void consensus_finalize_kernel(ConsensusArgs g, Layout ws, int splits) {
-  const int l = blockIdx.x * blockDim.x + threadIdx.x;
-  if (l >= g.l) return;
+  const int l = blockIdx.x * blockDim.x + threadIdx.x;  // (scan, landmark) slot
+  if (l >= g.l * g.n_scans) return;
   const int n = ws.nl[l];
   const double* part = ws.part + static_cast<size_t>(l) * splits * kPartDoubles;
   int bs = -1;
@@ -339,7 +350,8 @@ int pick_splits(int l, int n_hyp) {
 
 }  // namespace
 
-size_t consensus_workspace_bytes(int l, int v, int n_hyp) {
+size_t consensus_workspace_bytes(int l, int v, int n_hyp, int n_scans) {
+  l *= n_scans;
   const int splits = pick_splits(l, n_hyp);
   size_t d = static_cast<size_t>(l) * v * kLineDoubles + static_cast<size_t>(l) * 3 +
              static_cast<size_t>(l) * splits * kPartDoubles;
@@ -349,22 +361,26 @@ size_t consensus_workspace_bytes(int l, int v, int n_hyp) {
 int consensus_launch(const ConsensusArgs& a, cudaStream_t s) {
   MVLM_REQUIRE(a.peaks && a.starts && a.ends && a.draws && a.out_landmarks && a.out_errors && a.workspace,
                "consensus: null pointer");
-  MVLM_REQUIRE(a.l > 0 && a.v > 0 && a.n_hyp > 0, "consensus: bad sizes");
+  MVLM_REQUIRE(a.l > 0 && a.v > 0 && a.n_hyp > 0 && a.n_scans > 0 && a.n_scans <= 65535, "consensus: bad sizes");
+  MVLM_REQUIRE(a.draws_scan_stride == 0 || a.draws_scan_stride == static_cast<size_t>(a.l) * a.n_hyp * 8,
+               "consensus: draws are one shared (L,H,8) table or one (S,L,H,8) table");
   MVLM_REQUIRE(a.v <= kMaxViews, "consensus: at most %d views supported (got %d)", kMaxViews, a.v);
   MVLM_REQUIRE(a.mode == 0 || a.mode == 1, "consensus: Unknown mode for line matching in Estimator: %d", a.mode);
-  MVLM_REQUIRE(a.workspace_bytes >= consensus_workspace_bytes(a.l, a.v, a.n_hyp), "consensus: workspace too small");
-  const int splits = pick_splits(a.l, a.n_hyp);
+  MVLM_REQUIRE(a.workspace_bytes >= consensus_workspace_bytes(a.l, a.v, a.n_hyp, a.n_scans),
+               "consensus: workspace too small");
+  const int slots = a.l * a.n_scans;
+  const int splits = pick_splits(slots, a.n_hyp);
   const int chunk = ceil_div(a.n_hyp, splits);
-  Layout ws = carve(a.workspace, a.l, a.v, splits);
-  consensus_prepare_kernel<<<a.l, 256, 0, s>>>(a, ws);
+  Layout ws = carve(a.workspace, slots, a.v, splits);
+  consensus_prepare_kernel<<<dim3(a.l, a.n_scans), 256, 0, s>>>(a, ws);
   const size_t smem = static_cast<size_t>(a.v) * kLineDoubles * sizeof(double);
   // more than 48 KB (over 384 views): the opt-in attribute is per device, so it is set on every such launch
   // (a host-side call of about a microsecond; the common cases stay below the limit)
   if (smem > 48 * 1024)
     MVLM_CHECK_CUDA(cudaFuncSetAttribute(consensus_hyp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                          static_cast<int>(smem)));
-  consensus_hyp_kernel<<<dim3(a.l, splits), 256, smem, s>>>(a, ws, splits, chunk);
-  consensus_finalize_kernel<<<ceil_div(a.l, 128), 128, 0, s>>>(a, ws, splits);
+  consensus_hyp_kernel<<<dim3(a.l, splits, a.n_scans), 256, smem, s>>>(a, ws, splits, chunk);
+  consensus_finalize_kernel<<<ceil_div(slots, 128), 128, 0, s>>>(a, ws, splits);
   count_launch(3);
   MVLM_CHECK_CUDA(cudaGetLastError());
   return MVLM_OK;

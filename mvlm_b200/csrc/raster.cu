@@ -1,4 +1,6 @@
-// Batched multi-view orthographic rasteriser: all V views of one mesh in one launch sequence.
+// Batched multi-view orthographic rasteriser: all V views of one mesh -- or of the S meshes of a pass, scan-major
+// (global view g = s * V + v) -- in one launch sequence.  The scans of a pass come as a table passed by value
+// (__grid_constant__); each block looks up its scan from g, and the grids cover the largest scan of the pass.
 //
 // Replaces ObjVTKRenderer3D.render_3d_multi_rgb_geometry_depth (reference
 // src/mvlm/utils/render3d.py:114-177; camera :53-59,:136,:150-152; depth byte encoder
@@ -57,17 +59,25 @@ __device__ __forceinline__ SV xform_vertex(const float* __restrict__ v, const do
   return o;
 }
 
-// (view, vertex) -> window position + z-buffer value, computed once (sv[view * nv + vertex])
-__global__ void __launch_bounds__(256) raster_xform_kernel(const float* __restrict__ verts, int nv,
-                                                           const double* __restrict__ rot, int H, int W,
+struct RasterScans {
+  RasterScan s[kMaxScans];
+};
+
+// (view, vertex) -> window position + z-buffer value, computed once (sv[(g - g0) * sv_stride + vertex]).  The grid's x
+// extent covers the largest scan of the pass; threads past their own scan's vertex count do nothing.
+__global__ void __launch_bounds__(256) raster_xform_kernel(const __grid_constant__ RasterScans scans, int n_views, int g0,
+                                                           const double* __restrict__ rot, int H, int W, int sv_stride,
                                                            float4* __restrict__ sv) {
   __shared__ double R[9];
-  const int view = blockIdx.y;
-  if (threadIdx.x < 9) R[threadIdx.x] = rot[view * 9 + threadIdx.x];
+  const int g = g0 + static_cast<int>(blockIdx.y);
+  const RasterScan& sc = scans.s[g / n_views];
+  if (threadIdx.x < 9) R[threadIdx.x] = rot[g * 9 + threadIdx.x];
   __syncthreads();
   const float kx = static_cast<float>(static_cast<double>(W) / 300.0);
   const float ky = static_cast<float>(static_cast<double>(H) / 300.0);
-  float4* out = sv + static_cast<size_t>(view) * nv;
+  float4* out = sv + static_cast<size_t>(blockIdx.y) * sv_stride;
+  const int nv = sc.nv;
+  const float* __restrict__ verts = sc.verts;
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < nv; i += gridDim.x * blockDim.x) {
     const SV a = xform_vertex(verts + 3 * i, R, kx, ky);
     out[i] = make_float4(a.sx, a.sy, a.zb, 0.f);
@@ -81,12 +91,15 @@ __device__ __forceinline__ SV load_sv(const float4* __restrict__ sv, int i) {
   return o;
 }
 
-__global__ void __launch_bounds__(256) raster_tris_kernel(const float4* __restrict__ sv, int nv,
-                                                          const int* __restrict__ tris, int nt, int H, int W,
+__global__ void __launch_bounds__(256) raster_tris_kernel(const __grid_constant__ RasterScans scans, int n_views, int g0,
+                                                          const float4* __restrict__ sv, int sv_stride, int H, int W,
                                                           unsigned long long* __restrict__ zbuf) {
-  const int view = blockIdx.y;
-  const float4* svv = sv + static_cast<size_t>(view) * nv;
-  unsigned long long* zb = zbuf + static_cast<size_t>(view) * H * W;
+  const int g = g0 + static_cast<int>(blockIdx.y);
+  const RasterScan& sc = scans.s[g / n_views];
+  const float4* svv = sv + static_cast<size_t>(blockIdx.y) * sv_stride;
+  unsigned long long* zb = zbuf + static_cast<size_t>(g) * H * W;
+  const int nt = sc.nt;
+  const int* __restrict__ tris = sc.tris;
   for (int t = blockIdx.x * blockDim.x + threadIdx.x; t < nt; t += gridDim.x * blockDim.x) {
     const int i0 = __ldg(tris + 3 * t), i1 = __ldg(tris + 3 * t + 1), i2 = __ldg(tris + 3 * t + 2);
     const SV a = load_sv(svv, i0), b = load_sv(svv, i1), c = load_sv(svv, i2);
@@ -118,14 +131,16 @@ __global__ void __launch_bounds__(256) raster_tris_kernel(const float4* __restri
   }
 }
 
-// views view0 .. view0 + n_chunk - 1 (sv holds the transformed vertices of exactly these views)
-__global__ void __launch_bounds__(256) raster_resolve_kernel(RasterArgs g, const float4* __restrict__ sv, int view0,
+// global views g0 .. g0 + n_chunk - 1 (sv holds the transformed vertices of exactly these views)
+__global__ void __launch_bounds__(256) raster_resolve_kernel(RasterArgs g, const __grid_constant__ RasterScans scans,
+                                                             const float4* __restrict__ sv, int sv_stride, int g0,
                                                              int n_chunk) {
   // grid = (pixel blocks of one view, views of the chunk): 32-bit index arithmetic (three 64-bit divisions per pixel
   // were a large part of this kernel's 275 instructions per pixel)
   const unsigned int vp = blockIdx.x * blockDim.x + threadIdx.x;  // pixel within the view
   if (vp >= static_cast<unsigned int>(g.h * g.w) || static_cast<int>(blockIdx.y) >= n_chunk) return;
-  const int view = view0 + static_cast<int>(blockIdx.y);
+  const int view = g0 + static_cast<int>(blockIdx.y);
+  const RasterScan& sc = scans.s[view / g.n_views];
   const int py = static_cast<int>(vp / static_cast<unsigned int>(g.w));
   const int px = static_cast<int>(vp - static_cast<unsigned int>(py) * static_cast<unsigned int>(g.w));
   const size_t pix = static_cast<size_t>(view) * g.h * g.w + vp;
@@ -137,29 +152,29 @@ __global__ void __launch_bounds__(256) raster_resolve_kernel(RasterArgs g, const
   if (key != kBgKey) {
     tid = static_cast<int>(key & 0xFFFFFFFFu);
     zval = __uint_as_float(static_cast<unsigned int>(key >> 32));
-    const int i0 = __ldg(g.tris + 3 * tid), i1 = __ldg(g.tris + 3 * tid + 1), i2 = __ldg(g.tris + 3 * tid + 2);
+    const int i0 = __ldg(sc.tris + 3 * tid), i1 = __ldg(sc.tris + 3 * tid + 1), i2 = __ldg(sc.tris + 3 * tid + 2);
     const double* R = g.rot + view * 9;
-    if (g.tex && g.uvs && (mode == 0 || mode == 2)) {
-      const float4* svv = sv + static_cast<size_t>(view - view0) * g.nv;
+    if (sc.tex && sc.uvs && (mode == 0 || mode == 2)) {
+      const float4* svv = sv + static_cast<size_t>(blockIdx.y) * sv_stride;
       const SV a = load_sv(svv, i0), b = load_sv(svv, i1), c = load_sv(svv, i2);
       const float cx = static_cast<float>(px) + 0.5f, cy = static_cast<float>(py) + 0.5f;
       const float area = edge_fn(a.sx, a.sy, b.sx, b.sy, c.sx, c.sy);
       const float l0 = edge_fn(b.sx, b.sy, c.sx, c.sy, cx, cy) / area;
       const float l1 = edge_fn(c.sx, c.sy, a.sx, a.sy, cx, cy) / area;
       const float l2 = edge_fn(a.sx, a.sy, b.sx, b.sy, cx, cy) / area;
-      const float u = (l0 * g.uvs[2 * i0] + l1 * g.uvs[2 * i1]) + l2 * g.uvs[2 * i2];
-      const float v = (l0 * g.uvs[2 * i0 + 1] + l1 * g.uvs[2 * i1 + 1]) + l2 * g.uvs[2 * i2 + 1];
-      int tx = static_cast<int>(floorf(u * static_cast<float>(g.tw)));
-      int ty = static_cast<int>(floorf(v * static_cast<float>(g.th)));
+      const float u = (l0 * sc.uvs[2 * i0] + l1 * sc.uvs[2 * i1]) + l2 * sc.uvs[2 * i2];
+      const float v = (l0 * sc.uvs[2 * i0 + 1] + l1 * sc.uvs[2 * i1 + 1]) + l2 * sc.uvs[2 * i2 + 1];
+      int tx = static_cast<int>(floorf(u * static_cast<float>(sc.tw)));
+      int ty = static_cast<int>(floorf(v * static_cast<float>(sc.th)));
       // repeat wrap; texture coordinates inside [0, 1) (the usual case) skip the two integer divisions
-      if (tx < 0 || tx >= g.tw) { tx %= g.tw; if (tx < 0) tx += g.tw; }
-      if (ty < 0 || ty >= g.th) { ty %= g.th; if (ty < 0) ty += g.th; }
-      const size_t ti = static_cast<size_t>(g.th - 1 - ty) * g.tw + tx;
-      if (g.tex_c == 4) {  // RGBA texture: one 4-byte load per texel
-        const uchar4 q4 = __ldg(reinterpret_cast<const uchar4*>(g.tex) + ti);
+      if (tx < 0 || tx >= sc.tw) { tx %= sc.tw; if (tx < 0) tx += sc.tw; }
+      if (ty < 0 || ty >= sc.th) { ty %= sc.th; if (ty < 0) ty += sc.th; }
+      const size_t ti = static_cast<size_t>(sc.th - 1 - ty) * sc.tw + tx;
+      if (sc.tex_c == 4) {  // RGBA texture: one 4-byte load per texel
+        const uchar4 q4 = __ldg(reinterpret_cast<const uchar4*>(sc.tex) + ti);
         r8 = q4.x; g8 = q4.y; b8 = q4.z;
       } else {
-        const unsigned char* texel = g.tex + ti * 3;
+        const unsigned char* texel = sc.tex + ti * 3;
         r8 = texel[0]; g8 = texel[1]; b8 = texel[2];
       }
 
@@ -169,7 +184,7 @@ __global__ void __launch_bounds__(256) raster_resolve_kernel(RasterArgs g, const
       const int idx[3] = {i0, i1, i2};
 #pragma unroll
       for (int k = 0; k < 3; ++k) {
-        const float* v3 = g.verts + 3 * idx[k];
+        const float* v3 = sc.verts + 3 * idx[k];
 #pragma unroll
         for (int rr = 0; rr < 3; ++rr)
           p[k][rr] = (R[3 * rr] * v3[0] + R[3 * rr + 1] * v3[1]) + R[3 * rr + 2] * v3[2];
@@ -235,32 +250,48 @@ static int sv_chunk_views(int n_views, int nv) {
   return static_cast<int>(std::max<size_t>(1, std::min<size_t>(static_cast<size_t>(n_views), fit)));
 }
 
-size_t raster_workspace_bytes(int n_views, int h, int w, int n_verts) {
+size_t raster_workspace_bytes(int n_views, int h, int w, int n_verts) {  // n_views: all views of the pass
   const size_t z = (static_cast<size_t>(n_views) * h * w * sizeof(unsigned long long) + 255) & ~static_cast<size_t>(255);
   return z + static_cast<size_t>(sv_chunk_views(n_views, n_verts)) * n_verts * sizeof(float4);
 }
 
 int raster_launch(const RasterArgs& g, cudaStream_t stream) {
-  MVLM_REQUIRE(g.verts && g.tris && g.rot && g.zbuf, "raster: null pointer");
-  MVLM_REQUIRE(g.nt > 0 && g.nv > 0 && g.n_views > 0 && g.h > 0 && g.w > 0, "raster: bad sizes");
+  MVLM_REQUIRE(g.scans && g.rot && g.zbuf, "raster: null pointer");
+  MVLM_REQUIRE(g.n_scans > 0 && g.n_scans <= kMaxScans, "raster: 1 to %d scans per pass (got %d)", kMaxScans, g.n_scans);
+  MVLM_REQUIRE(g.n_views > 0 && g.h > 0 && g.w > 0, "raster: bad sizes");
+  MVLM_REQUIRE(static_cast<long long>(g.n_scans) * g.n_views <= 65535, "raster: at most 65535 views per pass");
   MVLM_REQUIRE(raster_channels(g.channel_mode) > 0, "raster: unknown channel_mode %d", g.channel_mode);
-  MVLM_REQUIRE(!g.tex || g.tex_c == 3 || g.tex_c == 4, "raster: texture must have 3 or 4 channels (got %d)", g.tex_c);
-  MVLM_REQUIRE(g.workspace_bytes >= raster_workspace_bytes(g.n_views, g.h, g.w, g.nv),
+  RasterScans table;
+  int max_nv = 0, max_nt = 0;
+  for (int s = 0; s < g.n_scans; ++s) {
+    const RasterScan& sc = g.scans[s];
+    MVLM_REQUIRE(sc.verts && sc.tris, "raster: null pointer (scan %d)", s);
+    MVLM_REQUIRE(sc.nt > 0 && sc.nv > 0, "raster: bad sizes (scan %d)", s);
+    MVLM_REQUIRE(!sc.tex || sc.tex_c == 3 || sc.tex_c == 4, "raster: texture must have 3 or 4 channels (got %d)",
+                 sc.tex_c);
+    table.s[s] = sc;
+    max_nv = std::max(max_nv, sc.nv);
+    max_nt = std::max(max_nt, sc.nt);
+  }
+  const int total = g.n_scans * g.n_views;
+  MVLM_REQUIRE(g.workspace_bytes >= raster_workspace_bytes(total, g.h, g.w, max_nv),
                "raster: workspace too small (%zu bytes given, %zu needed)", g.workspace_bytes,
-               raster_workspace_bytes(g.n_views, g.h, g.w, g.nv));
-  const size_t npix = static_cast<size_t>(g.n_views) * g.h * g.w;
+               raster_workspace_bytes(total, g.h, g.w, max_nv));
+  const size_t npix = static_cast<size_t>(total) * g.h * g.w;
   const size_t zbytes = (npix * sizeof(unsigned long long) + 255) & ~static_cast<size_t>(255);
   float4* sv = reinterpret_cast<float4*>(reinterpret_cast<unsigned char*>(g.zbuf) + zbytes);
   MVLM_CHECK_CUDA(cudaMemsetAsync(g.zbuf, 0xFF, npix * sizeof(unsigned long long), stream));
-  const int chunk = sv_chunk_views(g.n_views, g.nv);
+  // chunks of (scan, view) pairs: every view of a chunk keeps max_nv transformed vertices
+  const int chunk = sv_chunk_views(total, max_nv);
   const size_t view_pix = static_cast<size_t>(g.h) * g.w;
-  for (int v0 = 0; v0 < g.n_views; v0 += chunk) {
-    const int nc = std::min(chunk, g.n_views - v0);
-    dim3 gx(std::min(ceil_div(g.nv, 256), 1024), nc);
-    raster_xform_kernel<<<gx, 256, 0, stream>>>(g.verts, g.nv, g.rot + static_cast<size_t>(v0) * 9, g.h, g.w, sv);
-    dim3 gt(std::min(ceil_div(g.nt, 256), 1024), nc);
-    raster_tris_kernel<<<gt, 256, 0, stream>>>(sv, g.nv, g.tris, g.nt, g.h, g.w, g.zbuf + static_cast<size_t>(v0) * view_pix);
-    raster_resolve_kernel<<<dim3(static_cast<unsigned>((view_pix + 255) / 256), nc), 256, 0, stream>>>(g, sv, v0, nc);
+  for (int g0 = 0; g0 < total; g0 += chunk) {
+    const int nc = std::min(chunk, total - g0);
+    dim3 gx(std::min(ceil_div(max_nv, 256), 1024), nc);
+    raster_xform_kernel<<<gx, 256, 0, stream>>>(table, g.n_views, g0, g.rot, g.h, g.w, max_nv, sv);
+    dim3 gt(std::min(ceil_div(max_nt, 256), 1024), nc);
+    raster_tris_kernel<<<gt, 256, 0, stream>>>(table, g.n_views, g0, sv, max_nv, g.h, g.w, g.zbuf);
+    raster_resolve_kernel<<<dim3(static_cast<unsigned>((view_pix + 255) / 256), nc), 256, 0, stream>>>(g, table, sv, max_nv,
+                                                                                                       g0, nc);
     count_launch(3);
   }
   MVLM_CHECK_CUDA(cudaGetLastError());

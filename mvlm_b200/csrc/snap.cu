@@ -92,11 +92,20 @@ __device__ __forceinline__ void tri_closest(const float* __restrict__ verts, con
   closest_on_tri(p, a, b, c, q);
 }
 
-__global__ void __launch_bounds__(256) snap_scan_kernel(const float* __restrict__ verts, const int* __restrict__ tris,
-                                                        int nt, const double* __restrict__ lm, int splits,
+struct SnapMeshes {
+  SnapMesh m[kMaxScans];
+};
+
+// grid (L, splits, S): landmarks lm (S,L,3) of scan s = blockIdx.z against mesh s; partial minima part (S,L,splits,5)
+__global__ void __launch_bounds__(256) snap_scan_kernel(const __grid_constant__ SnapMeshes meshes, int L,
+                                                        const double* __restrict__ lm, int splits,
                                                         double* __restrict__ part, const int* __restrict__ only) {
-  const int l = blockIdx.x, split = blockIdx.y;
+  const int l = blockIdx.z * L + blockIdx.x, split = blockIdx.y;  // (scan, landmark) slot
   if (only && !only[l]) return;  // grid path: only the landmarks its query handed back
+  const SnapMesh& mesh = meshes.m[blockIdx.z];
+  const float* __restrict__ verts = mesh.verts;
+  const int* __restrict__ tris = mesh.tris;
+  const int nt = mesh.nt;
   const double p[3] = {lm[3 * l], lm[3 * l + 1], lm[3 * l + 2]};
   const int chunk = (nt + splits - 1) / splits;
   const int t0 = split * chunk, t1 = min(nt, t0 + chunk);
@@ -131,6 +140,7 @@ __global__ void __launch_bounds__(256) snap_scan_kernel(const float* __restrict_
   }
 }
 
+// one thread per (scan, landmark) slot of the S*L
 __global__ void snap_finalize_kernel(const double* __restrict__ part, int L, int splits, double* __restrict__ out,
                                      int* __restrict__ out_tri, const int* __restrict__ only) {
   const int l = blockIdx.x * blockDim.x + threadIdx.x;
@@ -156,8 +166,46 @@ int snap_splits(int l, int nt) {
 
 }  // namespace
 
+// l: landmarks x scans, nt: the largest triangle count
 size_t snap_workspace_bytes(int l, int nt) {
   return static_cast<size_t>(l) * snap_splits(l, nt) * kSnapPart * sizeof(double) + 64;
+}
+
+size_t snap_meshes_workspace_bytes(const SnapMesh* meshes, int n_scans, int l) {
+  int max_nt = 0;
+  for (int i = 0; i < n_scans; ++i) max_nt = max(max_nt, meshes[i].nt);
+  const size_t part = snap_workspace_bytes(l * n_scans, max_nt);
+  return part + (static_cast<size_t>(l) * n_scans * sizeof(int) + 63) / 64 * 64;
+}
+
+// The scan kernels of every scan of the pass in one launch pair.  `only` (S*L ints, device, or null): slots to do.
+static int snap_scan_launch(const SnapMesh* meshes, int n_scans, const double* lm, int l, double* part, double* out,
+                            int* out_tri, const int* only, cudaStream_t s) {
+  SnapMeshes table;
+  int max_nt = 0;
+  for (int i = 0; i < n_scans; ++i) {
+    table.m[i] = meshes[i];
+    max_nt = max(max_nt, meshes[i].nt);
+  }
+  const int slots = l * n_scans;
+  // splits from all slots of the pass and the largest mesh: a split of a smaller mesh may be empty; the
+  // (dist^2, triangle) minimum does not depend on how the triangles are split
+  const int splits = snap_splits(slots, max_nt);
+  snap_scan_kernel<<<dim3(l, splits, n_scans), 256, 0, s>>>(table, l, lm, splits, part, only);
+  snap_finalize_kernel<<<ceil_div(slots, 128), 128, 0, s>>>(part, slots, splits, out, out_tri, only);
+  count_launch(2);
+  MVLM_CHECK_CUDA(cudaGetLastError());
+  return MVLM_OK;
+}
+
+static int check_meshes(const SnapMesh* meshes, int n_scans) {
+  MVLM_REQUIRE(meshes && n_scans > 0 && n_scans <= kMaxScans, "snap: 1 to %d scans per pass (got %d)", kMaxScans,
+               n_scans);
+  for (int i = 0; i < n_scans; ++i) {
+    MVLM_REQUIRE(meshes[i].verts && meshes[i].tris, "snap: null pointer (scan %d)", i);
+    MVLM_REQUIRE(meshes[i].nt > 0, "snap: bad sizes (scan %d)", i);
+  }
+  return MVLM_OK;
 }
 
 int snap_launch(const float* verts, const int* tris, int nt, const double* lm, int l, void* workspace,
@@ -165,12 +213,8 @@ int snap_launch(const float* verts, const int* tris, int nt, const double* lm, i
   MVLM_REQUIRE(verts && tris && lm && out && workspace, "snap: null pointer");
   MVLM_REQUIRE(nt > 0 && l > 0, "snap: bad sizes");
   MVLM_REQUIRE(workspace_bytes >= snap_workspace_bytes(l, nt), "snap: workspace too small");
-  const int splits = snap_splits(l, nt);
-  snap_scan_kernel<<<dim3(l, splits), 256, 0, s>>>(verts, tris, nt, lm, splits, static_cast<double*>(workspace), nullptr);
-  snap_finalize_kernel<<<ceil_div(l, 128), 128, 0, s>>>(static_cast<double*>(workspace), l, splits, out, out_tri, nullptr);
-  count_launch(2);
-  MVLM_CHECK_CUDA(cudaGetLastError());
-  return MVLM_OK;
+  const SnapMesh mesh = {verts, tris, nt};
+  return snap_scan_launch(&mesh, 1, lm, l, static_cast<double*>(workspace), out, out_tri, nullptr, s);
 }
 
 // ---------------------------------------------------------------------------------------------------------
@@ -537,14 +581,48 @@ int snap_grid_query(const float* verts, const int* tris, int nt, const void* gri
                                       reinterpret_cast<const int*>(base + g.sorted),
                                       reinterpret_cast<const int*>(base + g.over), lm, out, out_tri, out_stats,
                                       handed_back);
+  count_launch(1);
+  MVLM_CHECK_CUDA(cudaGetLastError());
   // landmarks the walk gave up on (more than kMaxShells cells from the surface, non-finite): the full scan, spread over
   // (L, splits) blocks; blocks of the other landmarks return at once
-  const int splits = snap_splits(l, nt);
-  snap_scan_kernel<<<dim3(l, splits), 256, 0, s>>>(verts, tris, nt, lm, splits, part, handed_back);
-  snap_finalize_kernel<<<ceil_div(l, 128), 128, 0, s>>>(part, l, splits, out, out_tri, handed_back);
-  count_launch(3);
-  MVLM_CHECK_CUDA(cudaGetLastError());
-  return MVLM_OK;
+  const SnapMesh mesh = {verts, tris, nt};
+  return snap_scan_launch(&mesh, 1, lm, l, part, out, out_tri, handed_back, s);
+}
+
+int snap_meshes_launch(const SnapMesh* meshes, const void* const* grids, int n_scans, const double* lm, int l,
+                       void* workspace, size_t workspace_bytes, double* out, int* out_tri, cudaStream_t s) {
+  const int rc = check_meshes(meshes, n_scans);
+  if (rc != MVLM_OK) return rc;
+  MVLM_REQUIRE(lm && out && workspace && l > 0, "snap: null pointer");
+  MVLM_REQUIRE(workspace_bytes >= snap_meshes_workspace_bytes(meshes, n_scans, l), "snap: workspace too small");
+  MVLM_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 7) == 0, "snap: workspace must be 8-byte aligned");
+  int max_nt = 0, n_grids = 0;
+  for (int i = 0; i < n_scans; ++i) {
+    max_nt = max(max_nt, meshes[i].nt);
+    n_grids += grids && grids[i] ? 1 : 0;
+  }
+  double* part = static_cast<double*>(workspace);
+  int* only = nullptr;
+  if (n_grids > 0) {
+    // scans without a grid: every landmark goes to the scan kernel (any non-zero int); scans with one: the landmarks
+    // their query hands back
+    only = reinterpret_cast<int*>(static_cast<uint8_t*>(workspace) + snap_workspace_bytes(l * n_scans, max_nt));
+    MVLM_CHECK_CUDA(cudaMemsetAsync(only, 0x01, static_cast<size_t>(l) * n_scans * sizeof(int), s));
+    for (int i = 0; i < n_scans; ++i) {
+      if (!grids || !grids[i]) continue;
+      const uint8_t* base = static_cast<const uint8_t*>(grids[i]);
+      const GridLayout g = grid_layout(meshes[i].nt);
+      const size_t o = static_cast<size_t>(i) * l;
+      grid_query_kernel<<<l, kQueryThreads, 0, s>>>(meshes[i].verts, meshes[i].tris, reinterpret_cast<const GridHdr*>(base),
+                                                    reinterpret_cast<const int*>(base + g.cell_start),
+                                                    reinterpret_cast<const int*>(base + g.sorted),
+                                                    reinterpret_cast<const int*>(base + g.over), lm + 3 * o, out + 3 * o,
+                                                    out_tri ? out_tri + o : nullptr, nullptr, only + o);
+      count_launch(1);
+    }
+    MVLM_CHECK_CUDA(cudaGetLastError());
+  }
+  return snap_scan_launch(meshes, n_scans, lm, l, part, out, out_tri, only, s);
 }
 
 // debug: dims[3], n_over, cell edge, largest binned radius (synchronises the stream)

@@ -5,26 +5,33 @@
 namespace mvlm {
 
 // ---- raster.cu ------------------------------------------------------------
+// Scans of one pass: the kernels take the whole table by value (a __grid_constant__ parameter), so no host -> device
+// copy of it is needed.  Views of a pass are scan-major: global view g = s * n_views + v.
+constexpr int kMaxScans = 64;
+struct RasterScan {
+  const float* verts;          // (Nv,3)
+  const float* uvs;            // (Nv,2) or null
+  const int* tris;             // (Nt,3)
+  const unsigned char* tex;    // (Th,Tw,tex_c) or null
+  int nv, nt;
+  int th, tw, tex_c;           // tex_c = 3 (RGB) or 4 (RGBA: one 4-byte load per texel)
+};
 struct RasterArgs {
-  const float* verts = nullptr;       // (Nv,3)
-  int nv = 0;
-  const float* uvs = nullptr;         // (Nv,2) or null
-  const int* tris = nullptr;          // (Nt,3)
-  int nt = 0;
-  const unsigned char* tex = nullptr;  // (Th,Tw,tex_c) or null
-  int th = 0, tw = 0, tex_c = 3;       // tex_c = 3 (RGB) or 4 (RGBA: one 4-byte load per texel)
-  const double* rot = nullptr;        // (V,9) row-major R = Ry*Rx*Rz
-  int n_views = 0, h = 0, w = 0;
+  const RasterScan* scans = nullptr;  // n_scans entries (host memory)
+  int n_scans = 1;
+  const double* rot = nullptr;        // (S*V,9) row-major R = Ry*Rx*Rz
+  int n_views = 0, h = 0, w = 0;      // n_views per scan
   int channel_mode = 0;               // 0 RGB+depth, 1 geometry+depth, 2 RGB, 3 depth, 4 geometry
-  unsigned long long* zbuf = nullptr;  // workspace of raster_workspace_bytes(): (V,H,W) keys, then transformed vertices
+  unsigned long long* zbuf = nullptr;  // workspace of raster_workspace_bytes(): (S*V,H,W) keys, then transformed vertices
   size_t workspace_bytes = 0;
-  unsigned char* out_u8 = nullptr;     // (V,H,W,4) packed channels (CNN stem input) or null
-  float* out_f32 = nullptr;            // (V,H,W,C) reference-layout stack or null
-  int* out_tri = nullptr;              // (V,H,W) or null
-  float* out_z = nullptr;              // (V,H,W) or null
+  unsigned char* out_u8 = nullptr;     // (S*V,H,W,4) packed channels (CNN stem input) or null
+  float* out_f32 = nullptr;            // (S*V,H,W,C) reference-layout stack or null
+  int* out_tri = nullptr;              // (S*V,H,W) or null
+  float* out_z = nullptr;              // (S*V,H,W) or null
 };
 int raster_channels(int mode);
-size_t raster_workspace_bytes(int n_views, int h, int w, int n_verts);
+// total_views = S * V, n_verts = the largest vertex count of the pass
+size_t raster_workspace_bytes(int total_views, int h, int w, int n_verts);
 int raster_launch(const RasterArgs& a, cudaStream_t stream);
 
 // ---- peaks.cu -------------------------------------------------------------
@@ -47,26 +54,33 @@ int rays_from_peaks(const float* peaks, const double* rot, int l, int v, int ima
 
 // ---- consensus.cu ---------------------------------------------------------
 struct ConsensusArgs {
-  const float* peaks = nullptr;    // (L,V,3) f32, [..,2] = heat-map value
-  const double* starts = nullptr;  // (L,V,3)
-  const double* ends = nullptr;    // (L,V,3)
-  int l = 0, v = 0;
+  const float* peaks = nullptr;    // (L,S*V,3) f32, [..,2] = heat-map value
+  const double* starts = nullptr;  // (L,S*V,3)
+  const double* ends = nullptr;    // (L,S*V,3)
+  int l = 0, v = 0;                // v: views per scan
+  int n_scans = 1;
   int mode = 0;                    // 0 quantile, 1 absolute
   double threshold_quantile = 0.5;
   float threshold_absolute = 0.5f;
-  const unsigned int* draws = nullptr;  // (L,H,8) uint32 raw draws, index = draw mod n_lines
+  const unsigned int* draws = nullptr;  // (L,H,8) uint32 raw draws, index = draw mod n_lines; (S,L,H,8) per scan
+  size_t draws_scan_stride = 0;         // 0: every scan uses the same (L,H,8) table, else L*H*8
   int n_hyp = 1;
   double dist_thres = 100.0;
   void* workspace = nullptr;
   size_t workspace_bytes = 0;
-  double* out_landmarks = nullptr;  // (L,3)
-  double* out_errors = nullptr;     // (L)
-  int* out_nlines = nullptr;        // (L) lines kept by the filter (optional)
+  double* out_landmarks = nullptr;  // (S,L,3)
+  double* out_errors = nullptr;     // (S,L)
+  int* out_nlines = nullptr;        // (S,L) lines kept by the filter (optional)
 };
-size_t consensus_workspace_bytes(int l, int v, int n_hyp);
+size_t consensus_workspace_bytes(int l, int v, int n_hyp, int n_scans = 1);
 int consensus_launch(const ConsensusArgs& a, cudaStream_t s);
 
 // ---- snap.cu --------------------------------------------------------------
+struct SnapMesh {
+  const float* verts;  // (Nv,3)
+  const int* tris;     // (Nt,3)
+  int nt;
+};
 size_t snap_workspace_bytes(int l, int nt);
 int snap_launch(const float* verts, const int* tris, int nt, const double* lm, int l, void* workspace,
                 size_t workspace_bytes, double* out, int* out_tri, cudaStream_t s);
@@ -78,6 +92,11 @@ int snap_grid_query(const float* verts, const int* tris, int nt, const void* gri
                     int l, void* workspace, size_t workspace_bytes, double* out, int* out_tri, int* out_stats,
                     cudaStream_t s);
 int snap_grid_describe(const void* grid, int* dims_nover, double* edge_tau, cudaStream_t s);
+// several scans of a pass: landmarks (S,L,3) -> out (S,L,3), out_tri (S,L); grids[s] = scan s's snap grid or null
+// (the brute-force scan), the same points and triangles as one snap_launch / snap_grid_query per scan
+size_t snap_meshes_workspace_bytes(const SnapMesh* meshes, int n_scans, int l);
+int snap_meshes_launch(const SnapMesh* meshes, const void* const* grids, int n_scans, const double* lm, int l,
+                       void* workspace, size_t workspace_bytes, double* out, int* out_tri, cudaStream_t s);
 
 // ---- eltwise.cu / stem.cu ---------------------------------------------------
 // out_raw/out_act may be null; scale/shift are fp32[c] (folded BN) used only when out_act != null

@@ -112,6 +112,39 @@ def raster_multiview(verts, uvs, tris, tex, rot, h: int, w: int, channel_mode: s
     return {"u8": out_u8, "f32": f32, "tri": tri, "z": z}
 
 
+def raster_multiscan(scans, rot, h: int, w: int, channel_mode: str = "RGB+depth", want_f32: bool = False,
+                     want_tri: bool = False, want_z: bool = False, zbuf=None, out_u8=None):
+    """Several scans in one pass.  scans: list of (verts, uvs|None, tris, tex|None) cuda tensors as in raster_multiview;
+    rot (S*V,9|3,3) f64, scan-major (scan s owns views [s*V, (s+1)*V)).  zbuf: optional persistent workspace (a new
+    one is allocated when it is smaller than mvlm_raster_multiscan_workspace_bytes).
+    Returns dict(u8=(S*V,H,W,4), f32, tri, z) like raster_multiview; each scan's views equal raster_multiview's."""
+    lib = _lib.load()
+    n = len(scans)
+    if not 1 <= n <= _lib.MAX_SCANS:
+        raise ValueError(f"1 to {_lib.MAX_SCANS} scans per pass (got {n})")
+    total = rot.shape[0]
+    if total % n:
+        raise ValueError(f"{total} views do not split evenly over {n} scans")
+    v = total // n
+    dev = scans[0][0].device
+    mode = CHANNEL_MODES[channel_mode]
+    table = (_lib.RasterScan * n)()
+    for e, (verts, uvs, tris, tex) in zip(table, scans):
+        e.verts, e.n_verts, e.uvs, e.tris, e.n_tris = ptr(verts), verts.shape[0], ptr(uvs), ptr(tris), tris.shape[0]
+        e.tex, (e.tex_h, e.tex_w, e.tex_channels) = ptr(tex), (tex.shape[:3] if tex is not None else (0, 0, 3))
+    need = lib.mvlm_raster_multiscan_workspace_bytes(n, v, h, w, max(s[0].shape[0] for s in scans))
+    if zbuf is None or zbuf.numel() * zbuf.element_size() < need:
+        zbuf = torch.empty(((need + 7) // 8,), dtype=torch.int64, device=dev)
+    if out_u8 is None:
+        out_u8 = torch.empty((total, h, w, 4), dtype=torch.uint8, device=dev)
+    f32 = torch.empty((total, h, w, MODE_CHANNELS[mode]), dtype=torch.float32, device=dev) if want_f32 else None
+    tri = torch.empty((total, h, w), dtype=torch.int32, device=dev) if want_tri else None
+    z = torch.empty((total, h, w), dtype=torch.float32, device=dev) if want_z else None
+    check(lib.mvlm_raster_multiscan(table, n, ptr(rot), v, h, w, mode, ptr(zbuf), zbuf.numel() * zbuf.element_size(),
+                                    ptr(out_u8), ptr(f32), ptr(tri), ptr(z), cur_stream()), "mvlm_raster_multiscan")
+    return {"u8": out_u8, "f32": f32, "tri": tri, "z": z}
+
+
 def _on_device(device):
     device = torch.device(device)
     return torch.cuda.device(device) if device.type == "cuda" else contextlib.nullcontext()
@@ -286,6 +319,35 @@ def consensus(peaks, starts, ends, draws, mode: str = "quantile", threshold_quan
     return lm, err, nl
 
 
+def consensus_multiscan(peaks, starts, ends, draws, n_scans: int, mode: str = "quantile", threshold_quantile: float = 0.5,
+                        threshold_absolute: float = 0.5, dist_thres: float = 100.0, workspace=None):
+    """Consensus of the S scans of one pass: peaks (L,S*V,3) f32, starts / ends (L,S*V,3) f64, draws (L,H,8) shared by
+    every scan or (S,L,H,8) per scan.  Returns (landmarks (S,L,3) f64, errors (S,L) f64, n_lines (S,L) i32); scan s
+    gets what consensus() returns for its views alone."""
+    lib = _lib.load()
+    if mode not in ("quantile", "absolute"):
+        raise ValueError(f"Unknown mode for line matching in Estimator: {mode}")
+    l, sv = peaks.shape[:2]
+    if sv % n_scans:
+        raise ValueError(f"{sv} views do not split evenly over {n_scans} scans")
+    v = sv // n_scans
+    per_scan = draws.dim() == 4
+    if per_scan and draws.shape[0] != n_scans:
+        raise ValueError(f"per-scan draws for {draws.shape[0]} scans, the pass has {n_scans}")
+    n_hyp = draws.shape[-2]
+    nbytes = lib.mvlm_consensus_multiscan_workspace_bytes(n_scans, l, v, n_hyp)
+    if workspace is None or workspace.numel() < nbytes:
+        workspace = torch.empty((nbytes,), dtype=torch.uint8, device=peaks.device)
+    lm = torch.empty((n_scans, l, 3), dtype=torch.float64, device=peaks.device)
+    err = torch.empty((n_scans, l), dtype=torch.float64, device=peaks.device)
+    nl = torch.empty((n_scans, l), dtype=torch.int32, device=peaks.device)
+    check(lib.mvlm_consensus_multiscan(ptr(peaks), ptr(starts), ptr(ends), n_scans, l, v, 0 if mode == "quantile" else 1,
+                                       float(threshold_quantile), float(threshold_absolute), ptr(draws), int(per_scan),
+                                       n_hyp, float(dist_thres), ptr(workspace), workspace.numel(), ptr(lm), ptr(err),
+                                       ptr(nl), cur_stream()), "mvlm_consensus_multiscan")
+    return lm, err, nl
+
+
 # Above this many triangles building a uniform grid (memset + 7 small launches, 45-150 us) and querying it (20-50 us) beats
 # the brute-force scan for ONE batch of 73 landmarks: measured crossover ~110k triangles, 4.9x at 2M
 # (profiles/r1_snap_grid.txt).  A mesh that already has a grid uses it at any size (query alone: 3x at 100k, 20x at 2M).
@@ -341,4 +403,27 @@ def snap_to_mesh(verts, tris, landmarks, workspace=None, grid=None):
     tid = torch.empty((l,), dtype=torch.int32, device=verts.device)
     check(lib.mvlm_snap_to_mesh(ptr(verts), ptr(tris), nt, ptr(landmarks), l, ptr(workspace), workspace.numel(), ptr(out),
                                 ptr(tid), cur_stream()), "mvlm_snap_to_mesh")
+    return out, tid
+
+
+def snap_to_meshes(meshes, landmarks):
+    """Closest surface points of the S scans of one pass: meshes = list of (verts, tris, SnapGrid|None), landmarks
+    (S,L,3) f64.  Returns (points (S,L,3) f64, triangle ids (S,L) i32), equal to snap_to_mesh per scan."""
+    lib = _lib.load()
+    n, l = landmarks.shape[0], landmarks.shape[1]
+    if n != len(meshes):
+        raise ValueError(f"{len(meshes)} meshes for landmarks of {n} scans")
+    if not 1 <= n <= _lib.MAX_SCANS:
+        raise ValueError(f"1 to {_lib.MAX_SCANS} scans per pass (got {n})")
+    table = (_lib.SnapMesh * n)()
+    for e, (verts, tris, grid) in zip(table, meshes):
+        e.verts, e.tris, e.n_tris = ptr(verts), ptr(tris), tris.shape[0]
+        if grid is not None:
+            e.grid, e.grid_bytes = ptr(grid.buf), grid.buf.numel()
+    dev = landmarks.device
+    ws = torch.empty((lib.mvlm_snap_to_meshes_workspace_bytes(table, n, l),), dtype=torch.uint8, device=dev)
+    out = torch.empty((n, l, 3), dtype=torch.float64, device=dev)
+    tid = torch.empty((n, l), dtype=torch.int32, device=dev)
+    check(lib.mvlm_snap_to_meshes(table, n, ptr(landmarks), l, ptr(ws), ws.numel(), ptr(out), ptr(tid), cur_stream()),
+          "mvlm_snap_to_meshes")
     return out, tid

@@ -11,15 +11,33 @@ __all__ = ["Pipeline"]
 
 import abc
 import dataclasses
+import os
 import time
 from pathlib import Path
 
 import numpy as np
 import torch
 
+from .. import _lib
 from ..io_obj import Mesh, load_obj
 from ..prediction.paulsenpredictor import PaulsenModel
 from ..utils import Estimator3D, ObjRenderer3D, prealign
+
+# Pixels of one device pass of the batch drivers.  The premise -- a plan of 8 views of 256^2 cannot fill the GPU and
+# the views of several scans in one plan can -- is not measured yet (`tools/bench_batch.py --cnn --e2e` measures it),
+# so the default is 0: one scan per pass, the work of one scan at a time.  MVLM_PASS_PIXELS sets a budget for
+# measurements and tests; the candidate is about 96 views of 256^2 (12 scans of the 8-view preset per pass, while 100
+# views of 256^2 stay one scan per pass), the issue's estimate, not a measured figure.
+PASS_PIXELS = int(os.environ.get("MVLM_PASS_PIXELS", "0"))
+
+
+def scans_per_pass(n_views: int, h: int, w: int, max_views: int | None = None) -> int:
+    """Scans the batch drivers put into one device pass: as many as fit PASS_PIXELS (at least one, at most
+    MVLM_MAX_SCANS), and no more views than one CNN plan may take (`max_views`)."""
+    s = min(_lib.MAX_SCANS, max(1, PASS_PIXELS // (n_views * h * w)))
+    if max_views is not None:
+        s = min(s, max(1, max_views // n_views))
+    return s
 
 
 class _DeviceLock:
@@ -175,13 +193,17 @@ class Pipeline(abc.ABC, TimeMixin):
                 return load_obj(f, n_threads=4, texture_decoder=self.texture_decoder, device=self.device,
                                 parser=self.obj_parser)
 
+            # `prefetch` loader threads, with the scans of a whole pass queued for them: the driver takes a pass's scans
+            # at once and then waits for an earlier pass, the loaders keep working meanwhile
+            ahead = max(prefetch, self._scans_per_pass())
+
             def meshes():
                 with ThreadPoolExecutor(max_workers=max(1, prefetch)) as pool:
-                    pending = [pool.submit(load, f) for f in files[:prefetch]]
+                    pending = [pool.submit(load, f) for f in files[:ahead]]
                     for i, f in enumerate(files):
                         mesh = pending.pop(0).result()
-                        if i + prefetch < len(files):
-                            pending.append(pool.submit(load, files[i + prefetch]))
+                        if i + ahead < len(files):
+                            pending.append(pool.submit(load, files[i + ahead]))
                         if mesh is None:
                             print(f"File {f} does not exist")
                         yield mesh
@@ -213,85 +235,131 @@ class Pipeline(abc.ABC, TimeMixin):
             np.savetxt((out_dir / f"{f.stem}_{pname}.txt").as_posix(), lm, delimiter=",")
         return results
 
-    def _enqueue_mesh(self, mesh: Mesh, transforms: np.ndarray | None = None):
-        """Enqueues the whole hot path of one scan on the current stream WITHOUT waiting for it: host -> device copies
-        of the scan, raster, CNN, rays, consensus, snap, device -> pinned-host copy of the (L*3 + 1) result.
-        Returns (pinned host tensor, CUDA event recorded after the copy, objects to keep alive until then)."""
-        r, p, e = self.renderer_3d, self.predictor_2d, self.estimator_3d
-        if transforms is None:
-            transforms = r.generate_3d_transformations()
-        transforms = np.asarray(transforms)
-        back = None
-        if self.pre_align is not None:
-            # the whole path runs on the pre-aligned scan; the snapped landmarks are mapped back in _finish
-            verts = mesh.verts
-            if isinstance(verts, torch.Tensor):
-                # parser="gpu": prealign runs on numpy, so the vertices come back to the host (12 bytes per vertex, and
-                # this thread waits for the scan's parse); the aligned copy is uploaded like host-parsed vertices
-                mesh.geometry_ready.synchronize()
-                verts = verts.cpu().numpy()
-            a, b = prealign.affine(verts, self.pre_align)
-            mesh = dataclasses.replace(mesh, verts=prealign.apply(verts, a, b))
-            back = (a, b)
-        dmesh = r.upload(mesh)
-        out = r.render_device(dmesh, transforms)
-        peaks = p.predict_landmarks_device(out["u8"])
-        starts, ends = e.estimate_landmark_lines_device(peaks, transforms, r.image_size[0], rot=r.rotations_device(transforms))
-        if e.seed is not None:
-            draws_d = e.seeded_draws_device(peaks.shape[0])
-        else:
-            # reference RNG replay needs the per-landmark line counts -> one small D2H of the peak values (synchronises)
-            draws = e.reference_draws(peaks.cpu().numpy())
-            draws_d = torch.from_numpy(draws.view(np.int32)).to(self.device)
-        lm, err, _ = e.estimate_landmarks_from_lines_device(peaks, starts, ends, draws_d)
+    def _scans_per_pass(self) -> int:
+        """Pass size of the batch drivers (scans_per_pass for this pipeline's views).  One scan per pass when both the
+        view list (random views) and the consensus draws (seed=None) come from the global numpy RNG: one scan at a time
+        draws scan i's consensus draws, which depend on its peaks, before scan i+1's views, and a pass could not."""
+        r, e = self.renderer_3d, self.estimator_3d
+        if r.transforms is None and r.n_views != 8 and e.seed is None:
+            return 1
+        h, w = r.image_size[0], r.image_size[1]
+        v = r.n_views if r.transforms is None else len(r.transforms)
+        s = scans_per_pass(v, h, w)
+        return s if s == 1 else scans_per_pass(v, h, w, self.predictor_2d.max_views_per_launch(s * v, h, w))
+
+    def _enqueue_pass(self, meshes: list, transforms: np.ndarray | None = None, reserve_scans: int = 1):
+        """Enqueues the whole hot path of the scans of one pass on the current stream WITHOUT waiting for it: host ->
+        device copies of every scan, one raster sequence, one CNN plan over all views, rays, consensus and snap of all
+        scans, device -> pinned-host copy of the (S, L*3 + 1) result.  Each scan's landmarks equal those of a pass of
+        that scan alone.  `reserve_scans`: the pass size the caller plans (the persistent image and the result ring
+        are sized for it, so that a shorter last pass allocates nothing).
+        Returns (pinned host rows, CUDA event recorded after the copy, objects to keep alive until then)."""
         from .. import ops
 
-        snapped, _ = ops.snap_to_mesh(dmesh.verts, dmesh.tris, lm, grid=dmesh.snap_grid())
-        result = torch.cat([snapped.reshape(-1), err.sum().reshape(1) / err.numel()])
-        # ring of page-locked result buffers, allocated together on first use (cudaHostAlloc synchronises the device)
+        r, p, e = self.renderer_3d, self.predictor_2d, self.estimator_3d
+        n = len(meshes)
+        stacks, dmeshes, backs = [], [], []
+        for mesh in meshes:  # views drawn scan by scan, in the order of one scan at a time
+            t = np.asarray(r.generate_3d_transformations() if transforms is None else transforms)
+            back = None
+            if self.pre_align is not None:
+                # the whole path runs on the pre-aligned scan; the snapped landmarks are mapped back in _finish_pass
+                verts = mesh.verts
+                if isinstance(verts, torch.Tensor):
+                    # parser="gpu": prealign runs on numpy, so the vertices come back to the host (12 bytes per vertex,
+                    # and this thread waits for the scan's parse); the aligned copy is uploaded like host-parsed vertices
+                    mesh.geometry_ready.synchronize()
+                    verts = verts.cpu().numpy()
+                a, b = prealign.affine(verts, self.pre_align)
+                mesh = dataclasses.replace(mesh, verts=prealign.apply(verts, a, b))
+                back = (a, b)
+            stacks.append(t)
+            dmeshes.append(r.upload(mesh))
+            backs.append(back)
+        v = stacks[0].shape[0]
+        out = r.render_pass(dmeshes, stacks, reserve_views=reserve_scans * v)
+        all_views = np.concatenate(stacks)
+        peaks = p.predict_landmarks_device(out["u8"])
+        starts, ends = e.estimate_landmark_lines_device(peaks, all_views, r.image_size[0],
+                                                        rot=r.rotations_device(all_views))
+        if e.seed is not None:
+            draws_d = e.seeded_draws_device(peaks.shape[0])  # one (L,H,8) table for every scan
+        else:
+            # reference RNG replay needs the per-landmark line counts -> one small D2H of the peak values (synchronises);
+            # the draws are taken scan by scan, in the order of one scan at a time
+            pk = peaks.cpu().numpy()
+            draws = np.stack([e.reference_draws(pk[:, i * v:(i + 1) * v]) for i in range(n)])
+            draws_d = torch.from_numpy(draws.view(np.int32)).to(self.device)
+        lm, err, _ = e.estimate_landmarks_from_lines_device(peaks, starts, ends, draws_d, n_scans=n)
+        snapped, _ = ops.snap_to_meshes([(d.verts, d.tris, d.snap_grid()) for d in dmeshes], lm)
+        # the mean error per scan as one scan's (L,) sum, so last_error has the same bits in a pass of any size: one
+        # (S,L) row reduction would not guarantee that, torch sizes its reduction blocks (and so the order of the sums
+        # within a row) from the number of rows as well
+        mean_err = torch.stack([x.sum() for x in err]).reshape(n, 1) / err.shape[1]
+        result = torch.cat([snapped.reshape(n, -1), mean_err], dim=1)
+        # ring of page-locked result buffers, allocated together on first use (cudaHostAlloc synchronises the device) and
+        # sized for the planned pass: a shorter pass uses a prefix
         ring = self.__dict__.setdefault("_result_ring", [])
-        if not ring or ring[0].numel() != result.numel():
+        if not ring or ring[0].shape[1] != result.shape[1] or ring[0].shape[0] < n:
             ring.clear()
-            ring.extend(torch.empty(result.shape, dtype=result.dtype, pin_memory=True) for _ in range(8))
+            ring.extend(torch.empty((max(n, reserve_scans), result.shape[1]), dtype=result.dtype, pin_memory=True)
+                        for _ in range(8))
         self._result_i = (getattr(self, "_result_i", -1) + 1) % len(ring)
-        host = ring[self._result_i]
+        host = ring[self._result_i][:n]
         host.copy_(result, non_blocking=True)
         done = torch.cuda.Event()
         done.record()
-        return host, done, (dmesh, result, peaks, starts, ends, lm, back)
+        return host, done, (dmeshes, result, peaks, starts, ends, lm, backs)
 
-    def _finish(self, host: torch.Tensor, done, keep=None) -> np.ndarray:
+    def _finish_pass(self, host: torch.Tensor, done, keep) -> list:
+        """Waits for a pass of _enqueue_pass; returns its (L,3) landmarks per scan.  last_error and the prints follow
+        the scans in order."""
         done.synchronize()
-        result = host.numpy().copy()
-        self.last_error = float(result[-1])
-        self._print("Landmarks [Error]: ", f"{self.last_error:08.6f}", " mm")
-        lm = result[:-1].reshape(-1, 3)
-        back = keep[-1] if keep else None
-        return lm if back is None else prealign.invert(lm, *back)
+        rows = host.numpy().copy()
+        out = []
+        for row, back in zip(rows, keep[-1]):
+            self.last_error = float(row[-1])
+            self._print("Landmarks [Error]: ", f"{self.last_error:08.6f}", " mm")
+            lm = row[:-1].reshape(-1, 3)
+            out.append(lm if back is None else prealign.invert(lm, *back))
+        return out
 
     def predict_mesh(self, mesh: Mesh, transforms: np.ndarray | None = None) -> np.ndarray:
         """Fused device path for an already loaded scan (host arrays in, (L,3) float64 out)."""
         with self._lock:
-            host, done, keep = self._enqueue_mesh(mesh, transforms)
-            return self._finish(host, done, keep)
+            return self._finish_pass(*self._enqueue_pass([mesh], transforms))[0]
 
     def predict_meshes(self, meshes, depth: int = 2) -> list:
-        """Batch form of predict_mesh: same results, but up to `depth` scans are in flight -- the copies and launches of
-        the next scan are enqueued (one stream, so buffers are reused in order) before the host waits for the landmarks
-        of the previous one, which keeps host-side latency off the GPU's critical path.  A None entry yields None."""
+        """Batch form of predict_mesh: same results, bit for bit, and the same use of the global numpy RNG.  Several
+        scans share one device pass when PASS_PIXELS allows it (_scans_per_pass; one scan per pass by default), and up to
+        `depth` passes are in flight -- the copies and launches of the next pass are enqueued (one stream, so buffers
+        are reused in order) before the host waits for the landmarks of an earlier one, which keeps host-side latency
+        off the GPU's critical path.  A None entry yields None."""
         with self._lock:
             assert depth < 8, "depth is bounded by the ring of result buffers"
-            results, inflight = [], []
+            per_pass = self._scans_per_pass()
+            self.renderer_3d.reserve_upload_slots(per_pass * (depth + 1))
+            results, batch, where, inflight = [], [], [], []
+
+            def finish(keep_in_flight: int):
+                while len(inflight) > keep_in_flight:
+                    handle, idx = inflight.pop(0)
+                    for i, lm in zip(idx, self._finish_pass(*handle)):
+                        results[i] = lm
+
             for mesh in meshes:
+                results.append(None)
                 if mesh is None:
-                    inflight.append(None)
-                else:
-                    inflight.append(self._enqueue_mesh(mesh))
-                while len([x for x in inflight if x is not None]) > depth or (inflight and inflight[0] is None):
-                    head = inflight.pop(0)
-                    results.append(None if head is None else self._finish(*head))
-            for head in inflight:
-                results.append(None if head is None else self._finish(*head))
+                    continue
+                batch.append(mesh)
+                where.append(len(results) - 1)
+                if len(batch) == per_pass:
+                    inflight.append((self._enqueue_pass(batch, reserve_scans=per_pass), where))
+                    batch, where = [], []
+                    finish(depth)
+            if batch:
+                inflight.append((self._enqueue_pass(batch, reserve_scans=per_pass), where))
+            finish(0)
             return results
 
     def _predict_seams(self, file_name: Path, full_s: float):

@@ -92,9 +92,14 @@ class Estimator3D:
         err = err.cpu().numpy()
         return lm.cpu().numpy(), float(np.sum(err) / len(err))
 
-    def estimate_landmarks_from_lines_device(self, peaks, starts, ends, draws):
-        return ops.consensus(peaks, starts, ends, draws, mode=self.mode, threshold_quantile=self.threshold_quantile,
-                             threshold_absolute=self.threshold_absolute, dist_thres=float(self.dist_thres))
+    def estimate_landmarks_from_lines_device(self, peaks, starts, ends, draws, n_scans: int | None = None):
+        """n_scans: peaks / starts / ends are the (L, S*V, 3) arrays of a pass of S scans (draws (L,H,8) shared or
+        (S,L,H,8)); the results are then (S,L,3), (S,L), (S,L)."""
+        kw = dict(mode=self.mode, threshold_quantile=self.threshold_quantile, threshold_absolute=self.threshold_absolute,
+                  dist_thres=float(self.dist_thres))
+        if n_scans is None:
+            return ops.consensus(peaks, starts, ends, draws, **kw)
+        return ops.consensus_multiscan(peaks, starts, ends, draws, n_scans, **kw)
 
     # ---------------------------------------------------------------- snap (estimator3d.py:252-285)
     def project_landmarks_to_surface(self, pd, landmarks):

@@ -216,6 +216,17 @@ class ObjRenderer3D:
         self._stage_i += 1
         return DeviceMesh(mesh, self.device, st)
 
+    def reserve_upload_slots(self, n: int) -> None:
+        """At least `n` pinned staging slots: the batch drivers keep up to (scans per pass) x (passes in flight + 1)
+        scans between their upload and the end of their transfer, and a slot reused sooner makes the host wait for
+        the transfer of an earlier pass."""
+        if self.device.type != "cuda":
+            return
+        if not hasattr(self, "_stages"):
+            self._stages = [_PinnedStage() for _ in range(4)]
+            self._stage_i = 0
+        self._stages += [_PinnedStage() for _ in range(n - len(self._stages))]
+
     def rotations_device(self, transform_stack: np.ndarray) -> torch.Tensor:
         """(V,9) float64 device tensor of R = Ry@Rx@Rz per view; cached for the last transform stack
         (the per-view numpy evaluation that mirrors the reference dtype flow costs ~20 us per view)."""
@@ -227,21 +238,32 @@ class ObjRenderer3D:
 
     def render_device(self, dmesh: DeviceMesh, transform_stack: np.ndarray, want_f32=False, want_tri=False, want_z=False):
         """All views in one launch pair; returns the dict of device tensors of ops.raster_multiview."""
-        rot = self.rotations_device(np.asarray(transform_stack))
+        return self.render_pass([dmesh], [transform_stack], want_f32=want_f32, want_tri=want_tri, want_z=want_z)
+
+    def render_pass(self, dmeshes: list, transform_stacks: list, want_f32=False, want_tri=False, want_z=False,
+                    reserve_views: int = 0):
+        """The views of several scans in one launch sequence (ops.raster_multiscan), scan-major; every scan's images
+        equal render_device's.  `reserve_views`: the persistent image is sized for at least this many views (the
+        pass size the batch driver plans), so that a shorter pass uses a prefix of it at the same address."""
+        rot = self.rotations_device(np.concatenate([np.asarray(t) for t in transform_stacks]))
         h, w = self.image_size[0], self.image_size[1]
+        total = rot.shape[0]
         # persistent z-buffer / u8 image (overwritten by the next render): stable pointers let the CNN replay
         # its CUDA graph, and no allocation happens per scan
-        key = (rot.shape[0], h, w)
-        if getattr(self, "_buf_key", None) != key:
-            self._u8 = torch.empty((rot.shape[0], h, w, 4), dtype=torch.uint8, device=self.device)
+        if getattr(self, "_buf_key", None) != (h, w) or self._u8.shape[0] < total:
+            self._u8 = torch.empty((max(total, reserve_views), h, w, 4), dtype=torch.uint8, device=self.device)
             self._zbuf = None
-            self._buf_key = key
+            self._buf_key = (h, w)
         # the rasteriser's scratch also holds the per-(view, vertex) window coordinates: it grows with the largest scan
-        need = ops._lib.load().mvlm_raster_workspace_bytes(rot.shape[0], h, w, dmesh.verts.shape[0])
+        max_nv = max(d.verts.shape[0] for d in dmeshes)
+        lib = ops._lib.load()
+        need = lib.mvlm_raster_multiscan_workspace_bytes(len(dmeshes), total // len(dmeshes), h, w, max_nv)
         if self._zbuf is None or self._zbuf.numel() * 8 < need:
-            self._zbuf = ops.raster_workspace(rot.shape[0], h, w, int(dmesh.verts.shape[0] * 1.25), self.device)
-        return ops.raster_multiview(dmesh.verts, dmesh.uvs, dmesh.tris, dmesh.tex4(), rot, h, w, self.channel_mode,
-                                    want_f32=want_f32, want_tri=want_tri, want_z=want_z, zbuf=self._zbuf, out_u8=self._u8)
+            n = lib.mvlm_raster_multiscan_workspace_bytes(len(dmeshes), total // len(dmeshes), h, w, int(max_nv * 1.25))
+            self._zbuf = torch.empty(((n + 7) // 8,), dtype=torch.int64, device=self.device)
+        return ops.raster_multiscan([(d.verts, d.uvs, d.tris, d.tex4()) for d in dmeshes], rot, h, w, self.channel_mode,
+                                    want_f32=want_f32, want_tri=want_tri, want_z=want_z, zbuf=self._zbuf,
+                                    out_u8=self._u8[:total])
 
     # render3d.py:114-177
     def render_3d_multi_rgb_geometry_depth(self, transform_stack, file_name):

@@ -18,12 +18,12 @@ meshes = [load_obj(p) for p in paths]
 pinned = Mesh(*[torch.from_numpy(np.array(a)).pin_memory().numpy() for a in (meshes[0].verts, meshes[0].tris, meshes[0].uvs, meshes[0].texture)])
 dm.predict_meshes([meshes[0], pinned])
 enq, fin = [], []
-oe, of = dm._enqueue_mesh, dm._finish
-def e2(m, tr=None):
-    t0 = time.perf_counter(); r = oe(m, tr); enq.append(time.perf_counter() - t0); return r
-def f2(h, d):
-    t0 = time.perf_counter(); r = of(h, d); fin.append(time.perf_counter() - t0); return r
-dm._enqueue_mesh, dm._finish = e2, f2
+oe, of = dm._enqueue_pass, dm._finish_pass
+def e2(m, tr=None, **kw):
+    t0 = time.perf_counter(); r = oe(m, tr, **kw); enq.append(time.perf_counter() - t0); return r
+def f2(h, d, k):
+    t0 = time.perf_counter(); r = of(h, d, k); fin.append(time.perf_counter() - t0); return r
+dm._enqueue_pass, dm._finish_pass = e2, f2
 for name, batch in (("same pinned mesh", [pinned] * 16), ("same pageable mesh", [meshes[0]] * 16), ("4 pageable meshes", [meshes[i % 4] for i in range(16)])):
     for depth in (1, 2):
         enq.clear(); fin.clear()
@@ -31,7 +31,7 @@ for name, batch in (("same pinned mesh", [pinned] * 16), ("same pageable mesh", 
         dm.predict_meshes(batch, depth=depth)
         torch.cuda.synchronize(); dt = time.perf_counter() - t0
         print(f"{name:20s} depth {depth}: {16/dt:5.1f} scans/s; enqueue {np.mean(enq)*1e3:5.2f} ms (max {np.max(enq)*1e3:5.2f}), finish wait {np.mean(fin)*1e3:5.2f} ms")
-dm._enqueue_mesh, dm._finish = oe, of
+dm._enqueue_pass, dm._finish_pass = oe, of
 import mvlm_b200.pipeline.general_pipeline as gp
 orig = gp.load_obj
 for nt in (0, 4):

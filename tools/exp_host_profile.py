@@ -20,7 +20,7 @@ t0 = time.perf_counter()
 for _ in range(20): dm.predict_mesh(mesh)
 print(f"blocking calls: {20/(time.perf_counter()-t0):.1f} scans/s")
 t0 = time.perf_counter()
-hs = [dm._enqueue_mesh(mesh) for _ in range(20)]
+hs = [dm._enqueue_pass([mesh]) for _ in range(20)]
 t_enq = time.perf_counter() - t0
 torch.cuda.synchronize()
 print(f"enqueue only: {t_enq/20*1e3:.2f} ms per scan of host time; all done after {(time.perf_counter()-t0)/20*1e3:.2f} ms per scan")
