@@ -125,6 +125,50 @@ int mvlm_debug_obj_parse_lines(const char* text, size_t len, int max_lines, int*
                                int32_t* status, float* values, int32_t* n_tris, long long* corners,
                                long long max_corners);
 
+/* ------------------------------------------------------------------------- */
+/* Scan loader (host): PLY (ascii / binary little / big endian) and STL       */
+/* (ascii / binary) -> flat arrays; the format is chosen by the suffix (.ply,  */
+/* .stl, any case).  The legacy Deep-MVLM Utils3D read these formats too.      */
+/* Rules (DESIGN.md 7f): PLY `vertex` x y z as float32, red green blue as      */
+/* colours when all three are uchar, `face` vertex_indices fan-triangulated;   */
+/* STL is binary iff its size is 84 + 50 n, and its corners are welded: equal  */
+/* float32 coordinates (+0 == -0, NaN never) give one vertex, numbered in      */
+/* order of first occurrence; facets made degenerate by the weld are dropped.  */
+/* Errors as mvlm_obj_load ("does not exist", "does not contain any points",  */
+/* "face references vertex i of n") plus malformed header / body messages.     */
+/* n_threads <= 0: one thread per host core (at most 16; ASCII bodies only).   */
+/* ------------------------------------------------------------------------- */
+typedef struct mvlm_mesh mvlm_mesh;
+int mvlm_mesh_load(const char* path, int n_threads, mvlm_mesh** out);
+int mvlm_mesh_counts(const mvlm_mesh* mesh, int* n_verts, int* n_tris, int* has_colors);
+/* verts f32[n_verts*3], colors u8[n_verts*3] (may be NULL), tris i32[n_tris*3]: host memory */
+int mvlm_mesh_copy(const mvlm_mesh* mesh, float* verts, uint8_t* colors, int32_t* tris);
+void mvlm_mesh_free(mvlm_mesh* mesh);
+
+/* PLY / STL decoder on the GPU (mesh_parse.cu): the arrays of mvlm_mesh_load, bit for bit, for binary PLY whose faces */
+/* are all triangles and for binary STL (welded on the device).  Two phases on the caller's stream, like the OBJ      */
+/* parser:                                                                                                             */
+/*   mvlm_mesh_parse_device  file bytes in page-locked host memory (`host`, n_bytes): parses the PLY header or checks   */
+/*                           the STL size rule on the host, copies the bytes into the workspace, decodes (and welds)  */
+/*                           up to the output sizes, synchronises `stream` and fills *info.  info->fallback = 1: read */
+/*                           the file with mvlm_mesh_load (ASCII, a face that is not a triangle, an index out of       */
+/*                           range, any PLY the fixed-stride layout does not prove, beyond capacity); errors of the    */
+/*                           header are returned like mvlm_mesh_load's                                                  */
+/*   mvlm_mesh_parse_write   writes verts f32[n_verts*3], colors u8[n_verts*3] (only when has_colors), tris            */
+/*                           i32[n_tris*3] into device buffers; asynchronous, reads the workspace of the first phase.  */
+/* workspace: mvlm_mesh_parse_workspace_bytes(n_bytes, is_stl) bytes of device memory, 256-byte aligned (0: beyond the */
+/* decoder's capacity, 5.5M STL facets = the 16.7M items of one device scan, or not a binary STL size).               */
+typedef struct mvlm_mesh_parse_info {
+  int32_t n_verts, n_tris, has_colors, fallback;
+  int32_t is_stl;
+  size_t n_bytes;
+} mvlm_mesh_parse_info;
+size_t mvlm_mesh_parse_workspace_bytes(size_t n_bytes, int is_stl);
+int mvlm_mesh_parse_device(const uint8_t* host, size_t n_bytes, int is_stl, const char* path, void* workspace,
+                           size_t workspace_bytes, void* stream, mvlm_mesh_parse_info* info);
+int mvlm_mesh_parse_write(const mvlm_mesh_parse_info* info, const void* workspace, float* verts, uint8_t* colors,
+                          int32_t* tris, void* stream);
+
 /* Texture decode on the GPU (nvJPEG); replaces vtkJPEGReader in obj_to_actor, src/mvlm/utils/utils3d.py:26-36.  */
 /* data/len: the compressed file in host memory; out_rgb_dev: device buffer u8[height][width][3], row 0 = top.    */
 /* Thread-safe (one decoder state per calling thread); asynchronous on `stream` after the host-side parse.        */
@@ -173,6 +217,16 @@ int mvlm_raster_multiscan(const mvlm_raster_scan* scans /* host, n_scans entries
                           const double* rot /* (S*V,9) */, int n_views, int h, int w, int channel_mode, void* workspace,
                           size_t workspace_bytes, uint8_t* out_u8 /* (S*V,H,W,4) */, float* out_f32 /* (S*V,H,W,C) */,
                           int32_t* out_tri_id /* (S*V,H,W) */, float* out_depth /* (S*V,H,W) */, void* stream);
+/* The same pass with per-vertex colours: vertex_rgba[s] = scan s's (Nv,4) u8 RGBA colours in device memory (4-byte    */
+/* aligned).  The entries, or the whole array (= mvlm_raster_multiscan), may be NULL.  In the RGB modes (0, 2) a scan  */
+/* with colours and no (tex, uvs) pair is shaded per pixel with the barycentrics the texture lookup uses, in fp32:    */
+/* c = (l0*c0 + l1*c1) + l2*c2, q = (int)(c + 0.5f) clamped to [0,255]; a texture always wins; modes 1, 3 and 4 ignore */
+/* the colours.                                                                                                          */
+int mvlm_raster_multiscan_colored(const mvlm_raster_scan* scans /* host, n_scans entries */,
+                                  const uint8_t* const* vertex_rgba /* host array of n_scans device pointers, or NULL */,
+                                  int n_scans, const double* rot /* (S*V,9) */, int n_views, int h, int w,
+                                  int channel_mode, void* workspace, size_t workspace_bytes, uint8_t* out_u8,
+                                  float* out_f32, int32_t* out_tri_id, float* out_depth, void* stream);
 
 /* ------------------------------------------------------------------------- */
 /* Stage 2: stacked-hourglass heat-map CNN (MVLMModel),                       */

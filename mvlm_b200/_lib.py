@@ -48,6 +48,12 @@ class ObjParseInfo(C.Structure):
                 ("n_positions", C.c_int32), ("n_bytes", C.c_size_t)]
 
 
+class MeshParseInfo(C.Structure):
+    """mvlm_mesh_parse_info: what the first phase of the GPU PLY / STL decoder found."""
+    _fields_ = [("n_verts", C.c_int32), ("n_tris", C.c_int32), ("has_colors", C.c_int32), ("fallback", C.c_int32),
+                ("is_stl", C.c_int32), ("n_bytes", C.c_size_t)]
+
+
 class RasterScan(C.Structure):
     """mvlm_raster_scan: one scan of a multi-scan raster pass (device pointers)."""
     _fields_ = [("verts", C.c_void_p), ("n_verts", C.c_int), ("uvs", C.c_void_p), ("tris", C.c_void_p),
@@ -95,6 +101,8 @@ def _declare(lib: C.CDLL) -> None:
         "mvlm_raster_multiscan_workspace_bytes": ([i32, i32, i32, i32, i32], C.c_size_t),
         "mvlm_raster_multiscan": ([C.POINTER(RasterScan), i32, vp, i32, i32, i32, i32, vp, C.c_size_t, vp, vp, vp, vp, vp],
                                   i32),
+        "mvlm_raster_multiscan_colored": ([C.POINTER(RasterScan), C.POINTER(vp), i32, vp, i32, i32, i32, i32, vp,
+                                           C.c_size_t, vp, vp, vp, vp, vp], i32),
         "mvlm_hourglass_workspace_bytes": ([i32, i32, i32, i32, i32], C.c_size_t),
         "mvlm_hourglass_flops_per_view": ([i32, i32, i32, i32], f64),
         "mvlm_hourglass_create": ([C.POINTER(C.c_char_p), C.POINTER(vp), C.POINTER(C.c_longlong), i32, i32, i32, i32,
@@ -120,6 +128,13 @@ def _declare(lib: C.CDLL) -> None:
         "mvlm_obj_parse_write": ([C.POINTER(ObjParseInfo), vp, vp, vp, vp, vp], i32),
         "mvlm_debug_obj_parse_lines": ([C.c_char_p, C.c_size_t, i32, C.POINTER(i32), vp, vp, vp, vp, vp, C.c_longlong],
                                        i32),
+        "mvlm_mesh_load": ([C.c_char_p, i32, C.POINTER(vp)], i32),
+        "mvlm_mesh_counts": ([vp, C.POINTER(i32), C.POINTER(i32), C.POINTER(i32)], i32),
+        "mvlm_mesh_copy": ([vp, vp, vp, vp], i32),
+        "mvlm_mesh_free": ([vp], None),
+        "mvlm_mesh_parse_workspace_bytes": ([C.c_size_t, i32], C.c_size_t),
+        "mvlm_mesh_parse_device": ([vp, C.c_size_t, i32, C.c_char_p, vp, C.c_size_t, vp, C.POINTER(MeshParseInfo)], i32),
+        "mvlm_mesh_parse_write": ([C.POINTER(MeshParseInfo), vp, vp, vp, vp, vp], i32),
         "mvlm_jpeg_info": ([C.c_char_p, C.c_size_t, C.POINTER(i32), C.POINTER(i32)], i32),
         "mvlm_jpeg_decode_rgb": ([C.c_char_p, C.c_size_t, vp, i32, i32, vp], i32),
         "mvlm_heatmap_peaks": ([vp, i32, i32, i32, i32, i32, vp, vp], i32),

@@ -134,13 +134,23 @@ size_t mvlm_raster_multiscan_workspace_bytes(int n_scans, int n_views, int h, in
 int mvlm_raster_multiscan(const mvlm_raster_scan* scans, int n_scans, const double* rot, int n_views, int h, int w,
                           int channel_mode, void* workspace, size_t workspace_bytes, uint8_t* out_u8, float* out_f32,
                           int32_t* out_tri_id, float* out_depth, void* stream) {
+  return mvlm_raster_multiscan_colored(scans, nullptr, n_scans, rot, n_views, h, w, channel_mode, workspace,
+                                       workspace_bytes, out_u8, out_f32, out_tri_id, out_depth, stream);
+}
+
+int mvlm_raster_multiscan_colored(const mvlm_raster_scan* scans, const uint8_t* const* vertex_rgba, int n_scans,
+                                  const double* rot, int n_views, int h, int w, int channel_mode, void* workspace,
+                                  size_t workspace_bytes, uint8_t* out_u8, float* out_f32, int32_t* out_tri_id,
+                                  float* out_depth, void* stream) {
   MVLM_REQUIRE(scans, "mvlm_raster_multiscan: null scan table");
   MVLM_REQUIRE(n_scans > 0 && n_scans <= kMaxScans, "mvlm_raster_multiscan: 1 to %d scans per pass (got %d)", kMaxScans,
                n_scans);
   RasterScan table[kMaxScans];
   for (int s = 0; s < n_scans; ++s) {
     const mvlm_raster_scan& q = scans[s];
-    table[s] = RasterScan{q.verts, q.uvs, q.tris, q.tex, q.n_verts, q.n_tris, q.tex_h, q.tex_w, q.tex_channels};
+    const uchar4* colors = vertex_rgba ? reinterpret_cast<const uchar4*>(vertex_rgba[s]) : nullptr;
+    MVLM_REQUIRE((reinterpret_cast<uintptr_t>(colors) & 3) == 0, "mvlm_raster_multiscan: vertex colours of scan %d not 4-byte aligned", s);
+    table[s] = RasterScan{q.verts, q.uvs, q.tris, q.tex, colors, q.n_verts, q.n_tris, q.tex_h, q.tex_w, q.tex_channels};
   }
   RasterArgs a;
   a.scans = table; a.n_scans = n_scans;

@@ -19,8 +19,9 @@
 //                  screen tiles with a shared-memory z-tile (the textbook design for LARGE triangles) costs two more
 //                  passes over the (view, triangle) pairs to save less than one global atomic each: DESIGN.md 7d.
 //   raster_resolve one thread per pixel: winner triangle -> barycentric uv -> nearest texel (one 4-byte load from
-//                  the RGBA texture), depth byte, optional geometry shade; writes the u8 NHWC4 image the CNN stem
-//                  consumes and, on request, the fp32 (V,H,W,C) stack / triangle-id / z maps.
+//                  the RGBA texture) or, for a scan with vertex colours and no texture, the barycentric blend of its
+//                  three RGBA vertex colours; depth byte, optional geometry shade; writes the u8 NHWC4 image the CNN
+//                  stem consumes and, on request, the fp32 (V,H,W,C) stack / triangle-id / z maps.
 //
 // This file is compiled with --fmad=false: every fp32 operation rounds separately, in the same
 // order as oracle/csrc/oracle_native.c (built with -ffp-contract=off), so triangle-id maps and
@@ -57,6 +58,12 @@ __device__ __forceinline__ SV xform_vertex(const float* __restrict__ v, const do
   o.sy = (150.0f - yr) * ky;
   o.zb = (500.0f - zr) * (1.0f / 1500.0f);
   return o;
+}
+
+__device__ __forceinline__ unsigned char blend_u8(float l0, float l1, float l2, unsigned char c0, unsigned char c1,
+                                                  unsigned char c2) {
+  const float c = (l0 * static_cast<float>(c0) + l1 * static_cast<float>(c1)) + l2 * static_cast<float>(c2);
+  return static_cast<unsigned char>(static_cast<int>(fminf(fmaxf(c + 0.5f, 0.0f), 255.0f)));
 }
 
 struct RasterScans {
@@ -154,7 +161,8 @@ __global__ void __launch_bounds__(256) raster_resolve_kernel(RasterArgs g, const
     zval = __uint_as_float(static_cast<unsigned int>(key >> 32));
     const int i0 = __ldg(sc.tris + 3 * tid), i1 = __ldg(sc.tris + 3 * tid + 1), i2 = __ldg(sc.tris + 3 * tid + 2);
     const double* R = g.rot + view * 9;
-    if (sc.tex && sc.uvs && (mode == 0 || mode == 2)) {
+    const bool textured = sc.tex && sc.uvs;
+    if ((textured || sc.colors) && (mode == 0 || mode == 2)) {
       const float4* svv = sv + static_cast<size_t>(blockIdx.y) * sv_stride;
       const SV a = load_sv(svv, i0), b = load_sv(svv, i1), c = load_sv(svv, i2);
       const float cx = static_cast<float>(px) + 0.5f, cy = static_cast<float>(py) + 0.5f;
@@ -162,22 +170,28 @@ __global__ void __launch_bounds__(256) raster_resolve_kernel(RasterArgs g, const
       const float l0 = edge_fn(b.sx, b.sy, c.sx, c.sy, cx, cy) / area;
       const float l1 = edge_fn(c.sx, c.sy, a.sx, a.sy, cx, cy) / area;
       const float l2 = edge_fn(a.sx, a.sy, b.sx, b.sy, cx, cy) / area;
-      const float u = (l0 * sc.uvs[2 * i0] + l1 * sc.uvs[2 * i1]) + l2 * sc.uvs[2 * i2];
-      const float v = (l0 * sc.uvs[2 * i0 + 1] + l1 * sc.uvs[2 * i1 + 1]) + l2 * sc.uvs[2 * i2 + 1];
-      int tx = static_cast<int>(floorf(u * static_cast<float>(sc.tw)));
-      int ty = static_cast<int>(floorf(v * static_cast<float>(sc.th)));
-      // repeat wrap; texture coordinates inside [0, 1) (the usual case) skip the two integer divisions
-      if (tx < 0 || tx >= sc.tw) { tx %= sc.tw; if (tx < 0) tx += sc.tw; }
-      if (ty < 0 || ty >= sc.th) { ty %= sc.th; if (ty < 0) ty += sc.th; }
-      const size_t ti = static_cast<size_t>(sc.th - 1 - ty) * sc.tw + tx;
-      if (sc.tex_c == 4) {  // RGBA texture: one 4-byte load per texel
-        const uchar4 q4 = __ldg(reinterpret_cast<const uchar4*>(sc.tex) + ti);
-        r8 = q4.x; g8 = q4.y; b8 = q4.z;
-      } else {
-        const unsigned char* texel = sc.tex + ti * 3;
-        r8 = texel[0]; g8 = texel[1]; b8 = texel[2];
+      if (textured) {  // a texture always wins over vertex colours
+        const float u = (l0 * sc.uvs[2 * i0] + l1 * sc.uvs[2 * i1]) + l2 * sc.uvs[2 * i2];
+        const float v = (l0 * sc.uvs[2 * i0 + 1] + l1 * sc.uvs[2 * i1 + 1]) + l2 * sc.uvs[2 * i2 + 1];
+        int tx = static_cast<int>(floorf(u * static_cast<float>(sc.tw)));
+        int ty = static_cast<int>(floorf(v * static_cast<float>(sc.th)));
+        // repeat wrap; texture coordinates inside [0, 1) (the usual case) skip the two integer divisions
+        if (tx < 0 || tx >= sc.tw) { tx %= sc.tw; if (tx < 0) tx += sc.tw; }
+        if (ty < 0 || ty >= sc.th) { ty %= sc.th; if (ty < 0) ty += sc.th; }
+        const size_t ti = static_cast<size_t>(sc.th - 1 - ty) * sc.tw + tx;
+        if (sc.tex_c == 4) {  // RGBA texture: one 4-byte load per texel
+          const uchar4 q4 = __ldg(reinterpret_cast<const uchar4*>(sc.tex) + ti);
+          r8 = q4.x; g8 = q4.y; b8 = q4.z;
+        } else {
+          const unsigned char* texel = sc.tex + ti * 3;
+          r8 = texel[0]; g8 = texel[1]; b8 = texel[2];
+        }
+      } else {  // vertex colours (Gouraud): c = (l0*c0 + l1*c1) + l2*c2 per channel, rounded half up, clamped to [0,255]
+        const uchar4 c0 = __ldg(sc.colors + i0), c1 = __ldg(sc.colors + i1), c2 = __ldg(sc.colors + i2);
+        r8 = blend_u8(l0, l1, l2, c0.x, c1.x, c2.x);
+        g8 = blend_u8(l0, l1, l2, c0.y, c1.y, c2.y);
+        b8 = blend_u8(l0, l1, l2, c0.z, c1.z, c2.z);
       }
-
     }
     if (mode == 1 || mode == 4) {
       double p[3][3];

@@ -13,6 +13,7 @@ struct RasterScan {
   const float* uvs;            // (Nv,2) or null
   const int* tris;             // (Nt,3)
   const unsigned char* tex;    // (Th,Tw,tex_c) or null
+  const uchar4* colors;        // (Nv) RGBA vertex colours or null; used in the RGB modes when there is no (tex, uvs)
   int nv, nt;
   int th, tw, tex_c;           // tex_c = 3 (RGB) or 4 (RGBA: one 4-byte load per texel)
 };

@@ -23,6 +23,7 @@ class Mesh:
     path: Path | None = None
     texture_ready: object | None = None  # CUDA event recorded after a device-side decode (texture is a CUDA tensor)
     geometry_ready: object | None = None  # CUDA event recorded after a device-side parse (verts / uvs / tris are CUDA tensors)
+    colors: object | None = None  # (Nv,3) uint8 per-vertex RGB (PLY scans, io_mesh): numpy array, or a CUDA tensor
 
     @property
     def bbox_diagonal(self) -> float:

@@ -19,7 +19,8 @@ import numpy as np
 import torch
 
 from .. import _lib
-from ..io_obj import Mesh, load_obj
+from ..io_mesh import SUFFIXES, check_scan_file, check_scan_formats, is_scan_file, load_mesh
+from ..io_obj import Mesh
 from ..prediction.paulsenpredictor import PaulsenModel
 from ..utils import Estimator3D, ObjRenderer3D, prealign
 
@@ -95,7 +96,8 @@ class Pipeline(abc.ABC, TimeMixin):
                  screenshot_folder: Path | None = None, *, image_size: tuple = (256, 256),
                  channel_mode: str = "RGB+depth", n_hypotheses: int = 1, seed: int | None = None,
                  transforms: np.ndarray | None = None, device: str = "cuda", verbose: bool = True,
-                 texture_decoder: str = "pil", pre_align: dict | None = None, obj_parser: str = "host"):
+                 texture_decoder: str = "pil", pre_align: dict | None = None, obj_parser: str = "host",
+                 scan_formats: tuple = ("obj",)):
         TimeMixin.__init__(self)
         self.render_image_stack = render_image_stack
         self.render_image_folder = render_image_folder
@@ -113,6 +115,10 @@ class Pipeline(abc.ABC, TimeMixin):
         if obj_parser not in ("host", "gpu"):
             raise ValueError(f"Unknown OBJ parser: {obj_parser}")
         self.obj_parser = obj_parser
+        # scan file formats predict_one_file / predict_files / predict_folder / the seam renderer accept: ("obj",) (the
+        # default: the OBJ-only checks and messages) or any of "obj", "ply", "stl" (io_mesh; obj_parser then selects
+        # the host or the device decoder for every format)
+        self.scan_formats = check_scan_formats(scan_formats)
         # legacy "pre-align" block (configs/*.json:59-84): {"align_center_of_mass", "rot_x", "rot_y", "rot_z", "scale"};
         # None / identity = off, see utils/prealign.py
         self.pre_align = None if prealign.is_identity(pre_align) else dict(pre_align)
@@ -122,6 +128,7 @@ class Pipeline(abc.ABC, TimeMixin):
         self.renderer_3d.transforms = transforms
         self.renderer_3d.verbose = verbose
         self.renderer_3d.pre_align = self.pre_align
+        self.renderer_3d.scan_formats = self.scan_formats
         self.estimator_3d = Estimator3D(n_hypotheses=n_hypotheses, seed=seed, device=device)
         self.estimator_3d.verbose = verbose
         # One pipeline object = one set of device buffers (renderer images, CNN workspace, CUDA graphs): calls from
@@ -158,11 +165,10 @@ class Pipeline(abc.ABC, TimeMixin):
                 r = self.renderer_3d
                 if not file_name.is_file():
                     raise FileNotFoundError(f"File {file_name} is not a file")
-                if not file_name.suffix == ".obj":
-                    raise ValueError(f"File {file_name} is not an .obj file. Only .obj files are supported.")
+                check_scan_file(file_name, self.scan_formats)
                 self.tic()
-                mesh = load_obj(file_name, texture_decoder=self.texture_decoder, device=self.device,
-                                parser=self.obj_parser)
+                mesh = load_mesh(file_name, texture_decoder=self.texture_decoder, device=self.device,
+                                 parser=self.obj_parser)
                 self._print("Render [1] - Setup time: ", self.toc_p())
                 landmarks = self.predict_mesh(mesh)
                 self._print("Landmarks 3D Total: ", self.p_time(time.time() - full_s))
@@ -186,12 +192,11 @@ class Pipeline(abc.ABC, TimeMixin):
                     return None
                 if not f.is_file():
                     raise FileNotFoundError(f"File {f} is not a file")
-                if not f.suffix == ".obj":
-                    raise ValueError(f"File {f} is not an .obj file. Only .obj files are supported.")
+                check_scan_file(f, self.scan_formats)
                 # four parser threads per scan: with more, the loaders of `prefetch` scans oversubscribe the host and the
                 # thread that feeds the GPU gets descheduled (measured on the 16-core box: 36 scans/s with 16, 51 with 4)
-                return load_obj(f, n_threads=4, texture_decoder=self.texture_decoder, device=self.device,
-                                parser=self.obj_parser)
+                return load_mesh(f, n_threads=4, texture_decoder=self.texture_decoder, device=self.device,
+                                 parser=self.obj_parser)
 
             # `prefetch` loader threads, with the scans of a whole pass queued for them: the driver takes a pass's scans
             # at once and then waits for an earlier pass, the loaders keep working meanwhile
@@ -211,20 +216,29 @@ class Pipeline(abc.ABC, TimeMixin):
             return self.predict_meshes(meshes())
 
     def predict_folder(self, path, out=None) -> dict:
-        """The reference's batch loop (main.py:23-62) for this pipeline: every `*.obj` of a folder (sorted), or one
-        file; landmarks are written as `<out>/<stem>_<pipeline name>.txt` with `np.savetxt(..., delimiter=",")`, files
+        """The reference's batch loop (main.py:23-62) for this pipeline: every `*.obj` of a folder (sorted; with
+        scan_formats, every file of an enabled format), or one file; landmarks are written as `<out>/<stem>_<pipeline name>.txt` with `np.savetxt(..., delimiter=",")`, files
         whose landmarks could not be predicted are skipped.  Returns {file: landmarks | None}."""
         path = Path(path)
         if not path.exists():
             raise FileNotFoundError(f"{path.as_posix()} does not exist.")
+        default = self.scan_formats == ("obj",)
         if path.is_file():
-            if path.suffix.lower() != ".obj":
+            if default and path.suffix.lower() != ".obj":
                 raise ValueError(f"{path.as_posix()} is not an .obj file.")
+            if not default:
+                check_scan_file(path, self.scan_formats)
             files, out_dir = [path], Path(out) if out is not None else path.parent
-        else:
+        elif default:
             files, out_dir = sorted(path.glob("*.obj")), Path(out) if out is not None else path
             if len(files) == 0:
                 raise ValueError("Given folder does not contain any .obj files.")
+        else:
+            files = sorted(f for f in path.iterdir() if f.is_file() and is_scan_file(f, self.scan_formats))
+            out_dir = Path(out) if out is not None else path
+            if len(files) == 0:
+                names = ", ".join(SUFFIXES[f] for f in self.scan_formats)
+                raise ValueError(f"Given folder does not contain any {names} files.")
         out_dir.mkdir(parents=True, exist_ok=True)
         pname = getattr(self, "name", type(self).__name__.lower())
         results = dict(zip(files, self.predict_files(files)))

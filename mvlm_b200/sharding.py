@@ -122,14 +122,16 @@ def upload_mesh_sharded(renderer, mesh, group=None):
     verts = allgather_bytes(mesh.verts, device, stage, "verts", group)
     tris = allgather_bytes(mesh.tris, device, stage, "tris", group)
     uvs = None if mesh.uvs is None else allgather_bytes(mesh.uvs, device, stage, "uvs", group)
+    colors = None if mesh.colors is None else allgather_bytes(mesh.colors, device, stage, "colors", group)
     if stage is not None:
         stage.done = torch.cuda.Event()
         stage.done.record()
-    return DeviceMesh.from_device(mesh, verts, tris, uvs, tex_d)
+    return DeviceMesh.from_device(mesh, verts, tris, uvs, tex_d, colors)
 
 
 def _mesh_bytes(mesh) -> int:
-    return sum(a.nbytes for a in (mesh.verts, mesh.tris, mesh.uvs, mesh.texture) if isinstance(a, np.ndarray))
+    return sum(a.nbytes for a in (mesh.verts, mesh.tris, mesh.uvs, mesh.texture, mesh.colors)
+               if isinstance(a, np.ndarray))
 
 
 def predict_mesh_view_split(pipeline, mesh, transforms: np.ndarray, group=None) -> np.ndarray:

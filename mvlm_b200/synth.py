@@ -1,4 +1,4 @@
-"""Seeded synthetic inputs: a textured face-like mesh (OBJ + JPG), view transforms, ray sets.
+"""Seeded synthetic inputs: a textured face-like mesh (OBJ + JPG, PLY, STL), view transforms, ray sets.
 
 The reference's sample scans are missing blobs (.MISSING_LARGE_BLOBS) and there is no network,
 so every benchmark and parity test runs on these (SURVEY.md section 8d).
@@ -85,6 +85,83 @@ def write_obj(path: Path, verts, uvs, tris, texture: np.ndarray | None = None, j
         from PIL import Image
 
         Image.fromarray(texture).save(path.with_suffix(".jpg"), quality=jpeg_quality)
+    return path
+
+
+_PLY_NUMPY = {"char": "i1", "uchar": "u1", "short": "i2", "ushort": "u2", "int": "i4", "uint": "u4", "float": "f4",
+              "double": "f8", "int8": "i1", "uint8": "u1", "int16": "i2", "uint16": "u2", "int32": "i4", "uint32": "u4",
+              "float32": "f4", "float64": "f8"}
+
+
+def write_ply(path: Path, verts, faces, colors=None, fmt: str = "binary_little_endian", pos_type: str = "float",
+              count_type: str = "uchar", index_type: str = "int") -> Path:
+    """Writes a PLY scan: `vertex` x y z of `pos_type` (+ uchar red green blue when `colors` (Nv,3) uint8 is given) and
+    `face` vertex_indices lists.  faces: (F,3) int array, or a list of index sequences (polygons of any length).
+    fmt: "ascii", "binary_little_endian" or "binary_big_endian"."""
+    path = Path(path)
+    verts = np.asarray(verts)
+    polys = [list(map(int, f)) for f in faces]
+    end = {"binary_little_endian": "<", "binary_big_endian": ">", "ascii": "<"}[fmt]
+    head = ["ply", f"format {fmt} 1.0", "comment mvlm_b200 synthetic scan", f"element vertex {len(verts)}",
+            f"property {pos_type} x", f"property {pos_type} y", f"property {pos_type} z"]
+    if colors is not None:
+        head += ["property uchar red", "property uchar green", "property uchar blue"]
+    head += [f"element face {len(polys)}", f"property list {count_type} {index_type} vertex_indices", "end_header"]
+    with open(path, "wb") as f:
+        f.write(("\n".join(head) + "\n").encode())
+        if fmt == "ascii":
+            pos = verts.astype(_PLY_NUMPY[pos_type])
+            for i in range(len(verts)):
+                row = [repr(float(x)) if pos.dtype.kind == "f" else str(int(x)) for x in pos[i]]
+                if colors is not None:
+                    row += [str(int(c)) for c in colors[i]]
+                f.write((" ".join(row) + "\n").encode())
+            for p in polys:
+                f.write((" ".join(map(str, [len(p)] + p)) + "\n").encode())
+            return path
+        fields = [(c, end + _PLY_NUMPY[pos_type]) for c in "xyz"]
+        if colors is not None:
+            fields += [("red", "u1"), ("green", "u1"), ("blue", "u1")]
+        rec = np.empty(len(verts), dtype=fields)
+        for k, c in enumerate("xyz"):
+            rec[c] = verts[:, k]
+        if colors is not None:
+            for k, c in enumerate(("red", "green", "blue")):
+                rec[c] = np.asarray(colors)[:, k]
+        f.write(rec.tobytes())
+        cdt, idt = np.dtype(end + _PLY_NUMPY[count_type]), np.dtype(end + _PLY_NUMPY[index_type])
+        if all(len(p) == 3 for p in polys):  # one record array for the usual all-triangle file
+            frec = np.empty(len(polys), dtype=[("n", cdt), ("i", idt, (3,))])
+            frec["n"] = 3
+            frec["i"] = np.asarray(polys, dtype=np.int64).reshape(-1, 3)
+            f.write(frec.tobytes())
+        else:
+            for p in polys:
+                f.write(np.array([len(p)], cdt).tobytes() + np.array(p, idt).tobytes())
+    return path
+
+
+def write_stl(path: Path, verts, tris, binary: bool = True, header: bytes = b"mvlm_b200 synthetic scan") -> Path:
+    """Writes an STL triangle soup (three corners per facet, facet normals zero): binary (80-byte `header`, count,
+    50-byte records) or ASCII (`solid` ... `endsolid`, coordinates printed with repr, which round-trips float32
+    through float64)."""
+    path = Path(path)
+    corners = np.asarray(verts, np.float32)[np.asarray(tris, np.int64)]  # (F,3,3)
+    if binary:
+        rec = np.zeros(len(corners), dtype=[("n", "<f4", (3,)), ("v", "<f4", (9,)), ("a", "<u2")])
+        rec["v"] = corners.reshape(-1, 9)
+        with open(path, "wb") as f:
+            f.write(header[:80].ljust(80, b" "))
+            f.write(np.array([len(corners)], "<u4").tobytes())
+            f.write(rec.tobytes())
+        return path
+    lines = ["solid synthetic"]
+    for c in corners:
+        lines += ["facet normal 0 0 0", "  outer loop"]
+        lines += [f"    vertex {float(x)!r} {float(y)!r} {float(z)!r}" for x, y, z in c]
+        lines += ["  endloop", "endfacet"]
+    lines.append("endsolid synthetic")
+    Path(path).write_text("\n".join(lines) + "\n")
     return path
 
 

@@ -14,7 +14,8 @@ import numpy as np
 import torch
 
 from .. import ops
-from ..io_obj import Mesh, load_obj
+from ..io_mesh import check_scan_file, load_mesh
+from ..io_obj import Mesh
 
 __all__ = ["ObjRenderer3D", "ObjVTKRenderer3D", "fixed_eight_views", "rotation_matrices"]
 
@@ -121,15 +122,16 @@ class DeviceMesh:
             stage.done.synchronize()                          # the slot's previous transfer has left the host buffers
         self.verts, self.tris = up("verts", mesh.verts), up("tris", mesh.tris)
         self.uvs, self.tex = up("uvs", mesh.uvs), up("tex", mesh.texture)
+        self.colors = up("colors", mesh.colors)
         if stage is not None and device.type == "cuda":
             stage.done = torch.cuda.Event()
             stage.done.record()
 
     @classmethod
-    def from_device(cls, mesh: Mesh, verts, tris, uvs, tex) -> "DeviceMesh":
+    def from_device(cls, mesh: Mesh, verts, tris, uvs, tex, colors=None) -> "DeviceMesh":
         """Wraps arrays that are on the device already (sharding.upload_mesh_sharded)."""
         self = cls.__new__(cls)
-        self.mesh, self.verts, self.tris, self.uvs, self.tex = mesh, verts, tris, uvs, tex
+        self.mesh, self.verts, self.tris, self.uvs, self.tex, self.colors = mesh, verts, tris, uvs, tex, colors
         return self
 
     def tex4(self):
@@ -147,6 +149,19 @@ class DeviceMesh:
             self._tex4 = t
         return t
 
+    def colors4(self):
+        """The per-vertex colours as (Nv,4) RGBA (one 4-byte load per vertex in the rasteriser), expanded once per device
+        mesh; None without colours."""
+        if self.colors is None:
+            return None
+        c = self.__dict__.get("_colors4")
+        if c is None:
+            c = torch.empty((self.colors.shape[0], 4), dtype=torch.uint8, device=self.colors.device)
+            c[:, :3] = self.colors
+            c[:, 3] = 255
+            self._colors4 = c
+        return c
+
     def snap_grid(self):
         """Spatial index for the surface snap, built at most once per device mesh (None below ops.SNAP_GRID_MIN_TRIS,
         where the brute-force scan is faster than building the grid)."""
@@ -156,7 +171,8 @@ class DeviceMesh:
 
     @property
     def h2d_bytes(self) -> int:
-        return sum(t.numel() * t.element_size() for t in (self.verts, self.tris, self.uvs, self.tex) if t is not None)
+        return sum(t.numel() * t.element_size() for t in (self.verts, self.tris, self.uvs, self.tex, self.colors)
+                   if t is not None)
 
 
 class ObjRenderer3D:
@@ -183,6 +199,8 @@ class ObjRenderer3D:
         # injected view list (tests / benchmarks); None -> generate like the reference
         self.transforms: np.ndarray | None = None
         self.verbose = True
+        # suffixes multiview_render accepts (set by the pipeline's scan_formats)
+        self.scan_formats = ("obj",)
 
     # render3d.py:79-89 (GLOBAL np.random, same draw order)
     def random_transform(self, size=1):
@@ -261,14 +279,15 @@ class ObjRenderer3D:
         if self._zbuf is None or self._zbuf.numel() * 8 < need:
             n = lib.mvlm_raster_multiscan_workspace_bytes(len(dmeshes), total // len(dmeshes), h, w, int(max_nv * 1.25))
             self._zbuf = torch.empty(((n + 7) // 8,), dtype=torch.int64, device=self.device)
-        return ops.raster_multiscan([(d.verts, d.uvs, d.tris, d.tex4()) for d in dmeshes], rot, h, w, self.channel_mode,
+        return ops.raster_multiscan([(d.verts, d.uvs, d.tris, d.tex4(), d.colors4()) for d in dmeshes], rot, h, w,
+                                    self.channel_mode,
                                     want_f32=want_f32, want_tri=want_tri, want_z=want_z, zbuf=self._zbuf,
                                     out_u8=self._u8[:total])
 
     # render3d.py:114-177
     def render_3d_multi_rgb_geometry_depth(self, transform_stack, file_name):
         tt = time.time()
-        mesh = file_name if isinstance(file_name, Mesh) else load_obj(file_name)
+        mesh = file_name if isinstance(file_name, Mesh) else load_mesh(file_name)
         if self.pre_align is not None:  # legacy "pre-align" block, see utils/prealign.py; the seam path's back-transform
             import dataclasses           # is Pipeline._predict_seams'
 
@@ -294,8 +313,7 @@ class ObjRenderer3D:
             raise FileNotFoundError(f"File {file_name} does not exist")
         if not file_name.is_file():
             raise FileNotFoundError(f"File {file_name} is not a file")
-        if not file_name.suffix == ".obj":
-            raise ValueError(f"File {file_name} is not an .obj file. Only .obj files are supported.")
+        check_scan_file(file_name, self.scan_formats)
         if self.verbose:
             print("Render [0] - Prepare", f"{time.time() - t:08.6f} s")
         transformation_stack = self.generate_3d_transformations()
