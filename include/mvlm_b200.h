@@ -98,6 +98,20 @@ int mvlm_obj_counts(const mvlm_obj* obj, int* n_verts, int* n_tris, int* has_uv)
 /* verts f32[n_verts*3], uvs f32[n_verts*2] (may be NULL), tris i32[n_tris*3]: host memory */
 int mvlm_obj_copy(const mvlm_obj* obj, float* verts, float* uvs, int32_t* tris);
 void mvlm_obj_free(mvlm_obj* obj);
+/* Materials (DESIGN.md 7g): mvlm_obj_load_ex(..., MVLM_OBJ_MATERIALS, ...) loads the same arrays as mvlm_obj_load and */
+/* also keeps the `mtllib` names (rest of the line, trimmed; in file order), the distinct `usemtl` names (rest of the  */
+/* line, trimmed) in order of first appearance, and each triangle's material: the index of the name of the last       */
+/* `usemtl` line before its `f` line, -1 before the first.  flags = 0 is mvlm_obj_load.                                */
+#define MVLM_OBJ_MATERIALS 1
+int mvlm_obj_load_ex(const char* path, int n_threads, int flags, mvlm_obj** out);
+/* tri_material i32[n_tris] host memory (may be NULL); an error for a scan loaded without MVLM_OBJ_MATERIALS */
+int mvlm_obj_materials(const mvlm_obj* obj, int32_t* tri_material, int* n_materials, int* n_libraries);
+/* NUL-terminated names owned by obj (bytes as in the file); NULL for an index out of range */
+const char* mvlm_obj_material_name(const mvlm_obj* obj, int i);
+const char* mvlm_obj_library_name(const mvlm_obj* obj, int i);
+/* Debug (host, no file): the byte offsets where mvlm_obj_load's parallel chunks of text[0, len) start, for n_threads  */
+/* as mvlm_obj_load takes it; starts holds up to 16 (or n_threads) entries; returns the number of chunks.               */
+int mvlm_debug_obj_chunk_starts(const char* text, size_t len, int n_threads, long long* starts);
 
 /* Scan loader on the GPU (obj_parse.cu): the same language, arrays and error messages as mvlm_obj_load, bit for bit, */
 /* parsed from the file's bytes in device memory.  Two phases on the caller's stream:                                 */
@@ -118,6 +132,27 @@ int mvlm_obj_parse_device(const char* text_dev, size_t n_bytes, const char* path
                           size_t workspace_bytes, void* stream, mvlm_obj_parse_info* info);
 int mvlm_obj_parse_write(const mvlm_obj_parse_info* info, const void* workspace, float* verts, float* uvs,
                          int32_t* tris, void* stream);
+/* Materials on the GPU (DESIGN.md 7g): mvlm_obj_parse_device_ex with MVLM_OBJ_MATERIALS parses like                    */
+/* mvlm_obj_parse_device and also returns, in file order, every `usemtl` / `mtllib` line: its byte offset in the file,   */
+/* its kind (1 usemtl, 2 mtllib) and the triangles of the faces before it.  The names are read by the caller from its  */
+/* copy of the file (the rest of the line, trimmed, as mvlm_obj_load_ex).  name_lines: host buffer of at least          */
+/* MVLM_OBJ_MAX_NAME_LINES entries; a file with more name lines sets info->fallback (mvlm_obj_load_ex reads it).        */
+/* workspace: mvlm_obj_parse_workspace_bytes_ex(n_bytes, MVLM_OBJ_MATERIALS) bytes.  After mvlm_obj_parse_write,        */
+/* mvlm_obj_parse_tri_page copies line_page (host, the page of every `usemtl` ordinal in file order) into the workspace */
+/* and writes tri_page i32[n_tris] (device): line_page[ordinal of the last `usemtl` before the triangle], -1 before the */
+/* first.  flags = 0 is mvlm_obj_parse_device / mvlm_obj_parse_workspace_bytes.                                         */
+#define MVLM_OBJ_MAX_NAME_LINES 65536
+typedef struct mvlm_obj_name_line {
+  int64_t offset;       /* byte offset of the line's first character */
+  int32_t kind;         /* 1 usemtl, 2 mtllib */
+  int32_t tris_before;  /* triangles of the faces before the line */
+} mvlm_obj_name_line;
+size_t mvlm_obj_parse_workspace_bytes_ex(size_t n_bytes, int flags);
+int mvlm_obj_parse_device_ex(const char* text_dev, size_t n_bytes, const char* path, void* workspace,
+                             size_t workspace_bytes, int flags, void* stream, mvlm_obj_parse_info* info,
+                             mvlm_obj_name_line* name_lines, int max_name_lines, int* n_name_lines);
+int mvlm_obj_parse_tri_page(const mvlm_obj_parse_info* info, void* workspace, const int32_t* line_page, int n_usemtl,
+                            int32_t* tri_page, void* stream);
 /* Debug (host memory, no GPU): the GPU parser's per-line code run serially over text[0, len).  Per line: kind (0 other, */
 /* 1 v, 2 vt, 3 f), status (0 ok, 1 malformed, 2 host fallback), values f32[3] (v: x y z, vt: u v), n_tris (f), and   */
 /* for f lines the raw (a, b) of each triangulated corner appended to corners i64[2*max_corners] (b = 0: no uv).      */
@@ -227,6 +262,21 @@ int mvlm_raster_multiscan_colored(const mvlm_raster_scan* scans /* host, n_scans
                                   int n_scans, const double* rot /* (S*V,9) */, int n_views, int h, int w,
                                   int channel_mode, void* workspace, size_t workspace_bytes, uint8_t* out_u8,
                                   float* out_f32, int32_t* out_tri_id, float* out_depth, void* stream);
+/* The same pass with texture pages (several textures per scan, DESIGN.md 7g): pages[s] = NULL, or scan s's int32      */
+/* device array of n_tris + 3 P entries: the page of every triangle (-1 = none: white), then per page (texel offset,   */
+/* height, width) into the scan's tex, which then holds all P pages packed as RGBA texels (tex_channels 4; tex_h and   */
+/* tex_w are unused) and needs uvs.  In the RGB modes a triangle of page p takes                                       */
+/* page_p[h_p-1-(floor(v h_p) mod h_p)][floor(u w_p) mod w_p], the single-texture rule with the page's sizes; a paged   */
+/* scan ignores vertex colours; modes 1, 3 and 4 ignore pages.  pages (the whole array) may be NULL                    */
+/* (= mvlm_raster_multiscan_colored).  Preconditions the kernels do not check (device data): every page index is -1  */
+/* or in [0, P), every page has height and width >= 1, and offset + height * width <= the texels in tex; anything else */
+/* is undefined behaviour (render3d.DeviceMesh.paged builds a table that satisfies them).                             */
+int mvlm_raster_multiscan_paged(const mvlm_raster_scan* scans /* host, n_scans entries */,
+                                const uint8_t* const* vertex_rgba /* host array of n_scans device pointers, or NULL */,
+                                const int32_t* const* pages /* host array of n_scans device pointers, or NULL */,
+                                int n_scans, const double* rot /* (S*V,9) */, int n_views, int h, int w, int channel_mode,
+                                void* workspace, size_t workspace_bytes, uint8_t* out_u8, float* out_f32,
+                                int32_t* out_tri_id, float* out_depth, void* stream);
 
 /* ------------------------------------------------------------------------- */
 /* Stage 2: stacked-hourglass heat-map CNN (MVLMModel),                       */

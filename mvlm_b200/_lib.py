@@ -48,6 +48,11 @@ class ObjParseInfo(C.Structure):
                 ("n_positions", C.c_int32), ("n_bytes", C.c_size_t)]
 
 
+class ObjNameLine(C.Structure):
+    """mvlm_obj_name_line: one `usemtl` (kind 1) / `mtllib` (kind 2) line found by the GPU OBJ parser."""
+    _fields_ = [("offset", C.c_int64), ("kind", C.c_int32), ("tris_before", C.c_int32)]
+
+
 class MeshParseInfo(C.Structure):
     """mvlm_mesh_parse_info: what the first phase of the GPU PLY / STL decoder found."""
     _fields_ = [("n_verts", C.c_int32), ("n_tris", C.c_int32), ("has_colors", C.c_int32), ("fallback", C.c_int32),
@@ -68,6 +73,8 @@ class SnapMesh(C.Structure):
 
 
 MAX_SCANS = 64  # MVLM_MAX_SCANS
+OBJ_MATERIALS = 1  # MVLM_OBJ_MATERIALS
+OBJ_MAX_NAME_LINES = 65536  # MVLM_OBJ_MAX_NAME_LINES
 
 _lib = None
 
@@ -103,6 +110,8 @@ def _declare(lib: C.CDLL) -> None:
                                   i32),
         "mvlm_raster_multiscan_colored": ([C.POINTER(RasterScan), C.POINTER(vp), i32, vp, i32, i32, i32, i32, vp,
                                            C.c_size_t, vp, vp, vp, vp, vp], i32),
+        "mvlm_raster_multiscan_paged": ([C.POINTER(RasterScan), C.POINTER(vp), C.POINTER(vp), i32, vp, i32, i32, i32,
+                                         i32, vp, C.c_size_t, vp, vp, vp, vp, vp], i32),
         "mvlm_hourglass_workspace_bytes": ([i32, i32, i32, i32, i32], C.c_size_t),
         "mvlm_hourglass_flops_per_view": ([i32, i32, i32, i32], f64),
         "mvlm_hourglass_create": ([C.POINTER(C.c_char_p), C.POINTER(vp), C.POINTER(C.c_longlong), i32, i32, i32, i32,
@@ -123,9 +132,18 @@ def _declare(lib: C.CDLL) -> None:
         "mvlm_obj_counts": ([vp, C.POINTER(i32), C.POINTER(i32), C.POINTER(i32)], i32),
         "mvlm_obj_copy": ([vp, vp, vp, vp], i32),
         "mvlm_obj_free": ([vp], None),
+        "mvlm_obj_load_ex": ([C.c_char_p, i32, i32, C.POINTER(vp)], i32),
+        "mvlm_obj_materials": ([vp, vp, C.POINTER(i32), C.POINTER(i32)], i32),
+        "mvlm_obj_material_name": ([vp, i32], C.c_char_p),
+        "mvlm_obj_library_name": ([vp, i32], C.c_char_p),
+        "mvlm_debug_obj_chunk_starts": ([C.c_char_p, C.c_size_t, i32, vp], i32),
         "mvlm_obj_parse_workspace_bytes": ([C.c_size_t], C.c_size_t),
         "mvlm_obj_parse_device": ([vp, C.c_size_t, C.c_char_p, vp, C.c_size_t, vp, C.POINTER(ObjParseInfo)], i32),
         "mvlm_obj_parse_write": ([C.POINTER(ObjParseInfo), vp, vp, vp, vp, vp], i32),
+        "mvlm_obj_parse_workspace_bytes_ex": ([C.c_size_t, i32], C.c_size_t),
+        "mvlm_obj_parse_device_ex": ([vp, C.c_size_t, C.c_char_p, vp, C.c_size_t, i32, vp, C.POINTER(ObjParseInfo),
+                                      C.POINTER(ObjNameLine), i32, C.POINTER(i32)], i32),
+        "mvlm_obj_parse_tri_page": ([C.POINTER(ObjParseInfo), vp, vp, i32, vp, vp], i32),
         "mvlm_debug_obj_parse_lines": ([C.c_char_p, C.c_size_t, i32, C.POINTER(i32), vp, vp, vp, vp, vp, C.c_longlong],
                                        i32),
         "mvlm_mesh_load": ([C.c_char_p, i32, C.POINTER(vp)], i32),

@@ -142,6 +142,14 @@ int mvlm_raster_multiscan_colored(const mvlm_raster_scan* scans, const uint8_t* 
                                   const double* rot, int n_views, int h, int w, int channel_mode, void* workspace,
                                   size_t workspace_bytes, uint8_t* out_u8, float* out_f32, int32_t* out_tri_id,
                                   float* out_depth, void* stream) {
+  return mvlm_raster_multiscan_paged(scans, vertex_rgba, nullptr, n_scans, rot, n_views, h, w, channel_mode, workspace,
+                                     workspace_bytes, out_u8, out_f32, out_tri_id, out_depth, stream);
+}
+
+int mvlm_raster_multiscan_paged(const mvlm_raster_scan* scans, const uint8_t* const* vertex_rgba,
+                                const int32_t* const* pages, int n_scans, const double* rot, int n_views, int h, int w,
+                                int channel_mode, void* workspace, size_t workspace_bytes, uint8_t* out_u8,
+                                float* out_f32, int32_t* out_tri_id, float* out_depth, void* stream) {
   MVLM_REQUIRE(scans, "mvlm_raster_multiscan: null scan table");
   MVLM_REQUIRE(n_scans > 0 && n_scans <= kMaxScans, "mvlm_raster_multiscan: 1 to %d scans per pass (got %d)", kMaxScans,
                n_scans);
@@ -150,7 +158,11 @@ int mvlm_raster_multiscan_colored(const mvlm_raster_scan* scans, const uint8_t* 
     const mvlm_raster_scan& q = scans[s];
     const uchar4* colors = vertex_rgba ? reinterpret_cast<const uchar4*>(vertex_rgba[s]) : nullptr;
     MVLM_REQUIRE((reinterpret_cast<uintptr_t>(colors) & 3) == 0, "mvlm_raster_multiscan: vertex colours of scan %d not 4-byte aligned", s);
-    table[s] = RasterScan{q.verts, q.uvs, q.tris, q.tex, colors, q.n_verts, q.n_tris, q.tex_h, q.tex_w, q.tex_channels};
+    const int* paged = pages ? pages[s] : nullptr;
+    MVLM_REQUIRE(!paged || (q.tex && q.uvs && q.tex_channels == 4 && (reinterpret_cast<uintptr_t>(q.tex) & 3) == 0),
+                 "mvlm_raster_multiscan: scan %d has pages but no 4-byte aligned RGBA texel buffer and uvs", s);
+    table[s] = RasterScan{q.verts, q.uvs, q.tris, q.tex, colors, paged, q.n_verts, q.n_tris, q.tex_h, q.tex_w,
+                          q.tex_channels};
   }
   RasterArgs a;
   a.scans = table; a.n_scans = n_scans;

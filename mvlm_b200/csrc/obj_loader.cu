@@ -11,6 +11,11 @@
 // scan; 1.05 s in numpy): the file is split at line boundaries into one chunk per thread, every chunk is
 // parsed independently (std::from_chars: correctly rounded like Python's float()), and the chunks are
 // concatenated in file order.
+//
+// With MVLM_OBJ_MATERIALS (mvlm_obj_load_ex) the loader also keeps the `mtllib` names, the distinct `usemtl` names in
+// order of first appearance, and every triangle's material ordinal (the last `usemtl` before its `f` line; -1 before
+// the first).  A chunk numbers only its own `usemtl` lines; the join offsets them by the lines of earlier chunks, and
+// a chunk's triangles before its first `usemtl` inherit the last one of the chunks before it (DESIGN.md 7g).
 #include <algorithm>
 #include <charconv>
 #include <cstdio>
@@ -18,6 +23,7 @@
 #include <cstring>
 #include <string>
 #include <thread>
+#include <unordered_map>
 #include <vector>
 
 #include "../../include/mvlm_b200.h"
@@ -35,6 +41,11 @@ struct Chunk {
   std::vector<long long> cv, ct;
   std::vector<int> v_before, vt_before;  // per triangle
   bool bad = false;
+  // MVLM_OBJ_MATERIALS: this chunk's `usemtl` / `mtllib` names in file order, and per triangle the index of the last
+  // `usemtl` line of this chunk before it (-1: none yet in this chunk)
+  bool materials = false;
+  std::vector<std::string> usemtl, mtllib;
+  std::vector<int> mat_local;
 };
 
 inline const char* skip_ws(const char* p, const char* end) {
@@ -49,6 +60,17 @@ inline bool parse_double(const char*& p, const char* end, double* out) {
   if (r.ec != std::errc()) return false;
   p = r.ptr;
   return true;
+}
+
+// the rest of a `usemtl` / `mtllib` line, trimmed of blanks and a CR
+inline std::string rest_trimmed(const char* p, const char* end) {
+  p = skip_ws(p, end);
+  while (end > p && (end[-1] == ' ' || end[-1] == '\t' || end[-1] == '\r')) --end;
+  return std::string(p, static_cast<size_t>(end - p));
+}
+
+inline bool is_statement(const char* p, const char* eol, const char* word, size_t n) {
+  return static_cast<size_t>(eol - p) > n && (p[n] == ' ' || p[n] == '\t') && memcmp(p, word, n) == 0;
 }
 
 inline bool parse_int(const char*& p, const char* end, long long* out) {
@@ -119,10 +141,35 @@ void parse_chunk(const char* begin, const char* end, Chunk* c) {
         }
         c->v_before.push_back(n_v);
         c->vt_before.push_back(n_vt);
+        if (c->materials) c->mat_local.push_back(static_cast<int>(c->usemtl.size()) - 1);
       }
+    } else if (c->materials && is_statement(p, eol, "usemtl", 6)) {
+      c->usemtl.push_back(rest_trimmed(p + 7, eol));
+    } else if (c->materials && is_statement(p, eol, "mtllib", 6)) {
+      c->mtllib.push_back(rest_trimmed(p + 7, eol));
     }
     p = eol + 1;
   }
+}
+
+int chunk_count(size_t size, int n_threads) {
+  if (n_threads <= 0) n_threads = static_cast<int>(std::min(16u, std::max(1u, std::thread::hardware_concurrency())));
+  return size < (1u << 16) ? 1 : n_threads;
+}
+
+// chunk boundaries at line starts: cuts[0] = base, cuts[n] = end
+std::vector<const char*> chunk_cuts(const char* base, const char* end, int n_threads) {
+  const size_t size = static_cast<size_t>(end - base);
+  std::vector<const char*> cuts(static_cast<size_t>(n_threads) + 1);
+  cuts[0] = base;
+  for (int i = 1; i < n_threads; ++i) {
+    const char* p = base + size * static_cast<size_t>(i) / static_cast<size_t>(n_threads);
+    if (p < cuts[static_cast<size_t>(i) - 1]) p = cuts[static_cast<size_t>(i) - 1];
+    const char* nl = p < end ? static_cast<const char*>(memchr(p, '\n', static_cast<size_t>(end - p))) : nullptr;
+    cuts[static_cast<size_t>(i)] = nl ? nl + 1 : end;
+  }
+  cuts[static_cast<size_t>(n_threads)] = end;
+  return cuts;
 }
 
 }  // namespace
@@ -132,14 +179,21 @@ struct mvlm_obj {
   std::vector<float> verts, uvs;
   std::vector<int32_t> tris;
   bool has_uv = false;
+  bool has_materials = false;                 // loaded with MVLM_OBJ_MATERIALS
+  std::vector<int32_t> tri_material;          // per triangle: index into materials, -1 = none
+  std::vector<std::string> materials, libraries;
 };
 
 using namespace mvlm;
 
 extern "C" {
 
-int mvlm_obj_load(const char* path, int n_threads, mvlm_obj** out) {
+int mvlm_obj_load(const char* path, int n_threads, mvlm_obj** out) { return mvlm_obj_load_ex(path, n_threads, 0, out); }
+
+int mvlm_obj_load_ex(const char* path, int n_threads, int flags, mvlm_obj** out) {
   MVLM_REQUIRE(path && out, "mvlm_obj_load: null pointer");
+  MVLM_REQUIRE((flags & ~MVLM_OBJ_MATERIALS) == 0, "mvlm_obj_load_ex: unknown flags 0x%x", flags);
+  const bool materials = (flags & MVLM_OBJ_MATERIALS) != 0;
   *out = nullptr;
   FILE* fh = fopen(path, "rb");
   MVLM_REQUIRE(fh != nullptr, "File %s does not exist.", path);
@@ -152,19 +206,10 @@ int mvlm_obj_load(const char* path, int n_threads, mvlm_obj** out) {
   MVLM_REQUIRE(static_cast<long>(got) == size, "mvlm_obj_load: short read on %s", path);
   const char* base = buf.data();
   const char* end = base + buf.size();
-  if (n_threads <= 0) n_threads = static_cast<int>(std::min(16u, std::max(1u, std::thread::hardware_concurrency())));
-  if (buf.size() < (1u << 16)) n_threads = 1;
-  // chunk boundaries at line starts
-  std::vector<const char*> cuts(static_cast<size_t>(n_threads) + 1);
-  cuts[0] = base;
-  for (int i = 1; i < n_threads; ++i) {
-    const char* p = base + buf.size() * static_cast<size_t>(i) / static_cast<size_t>(n_threads);
-    if (p < cuts[static_cast<size_t>(i) - 1]) p = cuts[static_cast<size_t>(i) - 1];
-    const char* nl = p < end ? static_cast<const char*>(memchr(p, '\n', static_cast<size_t>(end - p))) : nullptr;
-    cuts[static_cast<size_t>(i)] = nl ? nl + 1 : end;
-  }
-  cuts[static_cast<size_t>(n_threads)] = end;
+  n_threads = chunk_count(buf.size(), n_threads);
+  const std::vector<const char*> cuts = chunk_cuts(base, end, n_threads);
   std::vector<Chunk> chunks(static_cast<size_t>(n_threads));
+  for (Chunk& c : chunks) c.materials = materials;
   {
     std::vector<std::thread> th;
     for (int i = 1; i < n_threads; ++i)
@@ -209,6 +254,29 @@ int mvlm_obj_load(const char* path, int n_threads, mvlm_obj** out) {
       ot += c.tex.size();
     }
     mvlm_obj* o = new mvlm_obj();
+    if (materials) {
+      // usemtl line (file order) -> distinct name; triangles -> the last usemtl line before them
+      o->has_materials = true;
+      std::unordered_map<std::string, int32_t> ids;
+      std::vector<int32_t> line_id;
+      for (const Chunk& c : chunks) {
+        for (const std::string& name : c.usemtl) {
+          auto it = ids.emplace(name, static_cast<int32_t>(o->materials.size())).first;
+          if (it->second == static_cast<int32_t>(o->materials.size())) o->materials.push_back(name);
+          line_id.push_back(it->second);
+        }
+        o->libraries.insert(o->libraries.end(), c.mtllib.begin(), c.mtllib.end());
+      }
+      o->tri_material.reserve(n_tri);
+      long long base = 0;  // usemtl lines of the chunks before this one
+      for (const Chunk& c : chunks) {
+        for (int local : c.mat_local) {
+          const long long line = base + local;  // local = -1: the last line of the earlier chunks (or none)
+          o->tri_material.push_back(line >= 0 ? line_id[static_cast<size_t>(line)] : -1);
+        }
+        base += static_cast<long long>(c.usemtl.size());
+      }
+    }
     o->tris.resize(n_tri * 3);
     if (n_tex == 0 || !any_uv) {
       // no texture coordinates in use: positions as they are, faces index them directly
@@ -278,6 +346,33 @@ int mvlm_obj_copy(const mvlm_obj* obj, float* verts, float* uvs, int32_t* tris) 
   return MVLM_OK;
 }
 
+int mvlm_obj_materials(const mvlm_obj* obj, int32_t* tri_material, int* n_materials, int* n_libraries) {
+  MVLM_REQUIRE(obj && n_materials && n_libraries, "mvlm_obj_materials: null pointer");
+  MVLM_REQUIRE(obj->has_materials, "mvlm_obj_materials: the scan was loaded without MVLM_OBJ_MATERIALS");
+  *n_materials = static_cast<int>(obj->materials.size());
+  *n_libraries = static_cast<int>(obj->libraries.size());
+  if (tri_material) memcpy(tri_material, obj->tri_material.data(), obj->tri_material.size() * sizeof(int32_t));
+  return MVLM_OK;
+}
+
+const char* mvlm_obj_material_name(const mvlm_obj* obj, int i) {
+  if (!obj || i < 0 || static_cast<size_t>(i) >= obj->materials.size()) return nullptr;
+  return obj->materials[static_cast<size_t>(i)].c_str();
+}
+
+const char* mvlm_obj_library_name(const mvlm_obj* obj, int i) {
+  if (!obj || i < 0 || static_cast<size_t>(i) >= obj->libraries.size()) return nullptr;
+  return obj->libraries[static_cast<size_t>(i)].c_str();
+}
+
 void mvlm_obj_free(mvlm_obj* obj) { delete obj; }
+
+int mvlm_debug_obj_chunk_starts(const char* text, size_t len, int n_threads, long long* starts) {
+  MVLM_REQUIRE((text || len == 0) && starts, "mvlm_debug_obj_chunk_starts: null pointer");
+  const int n = chunk_count(len, n_threads);
+  const std::vector<const char*> cuts = chunk_cuts(text, text + len, n);
+  for (int i = 0; i < n; ++i) starts[i] = cuts[static_cast<size_t>(i)] - text;
+  return n;
+}
 
 }  // extern "C"

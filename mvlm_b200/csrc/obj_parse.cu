@@ -16,6 +16,14 @@
 //          into per-position buckets, per-bucket insertion sort + unique (deterministic), scan of the unique counts
 //   write  (phase 2) output vertices = unique (position, uv) pairs in ascending order, and each corner's vertex
 //
+// Materials (MVLM_OBJ_MATERIALS, DESIGN.md 7g): the count pass also counts the `usemtl` lines and the name lines
+// (`usemtl` + `mtllib`) that start in every item, two more exclusive scans give each item its first `usemtl` ordinal
+// and its first name-line slot, and the parse pass stores every triangle's ordinal (the item's base plus the `usemtl`
+// lines it has walked, minus one: -1 before the first) and every name line's (offset, kind, triangles before it).  The
+// name lines come back to the host with the output sizes; the host reads the names from its copy of the file, maps
+// each `usemtl` ordinal to a texture page and mvlm_obj_parse_tri_page writes the page of every triangle.  A file with
+// more than MVLM_OBJ_MAX_NAME_LINES name lines takes the host fallback.
+//
 // Numbers: a token of at most 19 significant digits is converted exactly: Clinger's fast path (mantissa <= 2^53,
 // |exp10| <= 22; one correctly rounded multiply or divide) or Eisel-Lemire with 128-bit products over a table of
 // powers of five (the algorithm of fast_float, which libstdc++'s from_chars uses).  A token of more digits, and the
@@ -42,7 +50,8 @@ constexpr int kItemBytes = 32;    // bytes of the file per thread of the count /
 constexpr int kMaxBucket = 1024;  // corners of one position the per-bucket insertion sort takes (else host fallback)
 
 enum { kOk = 0, kBad = 1, kFallback = 2 };
-enum { kOther = 0, kV = 1, kVT = 2, kF = 3 };
+enum { kOther = 0, kV = 1, kVT = 2, kF = 3, kUsemtl = 4, kMtllib = 5 };
+constexpr int kInlineNames = 64;  // name lines copied back in the same synchronisation as the sizes
 
 #define MVLM_POW10_TABLE                                                                                                \
   1e0, 1e1, 1e2, 1e3, 1e4, 1e5, 1e6, 1e7, 1e8, 1e9, 1e10, 1e11, 1e12, 1e13, 1e14, 1e15, 1e16, 1e17, 1e18, 1e19, 1e20, \
@@ -349,6 +358,20 @@ HD int line_kind(const char* p, const char* eol) {
   return kOther;
 }
 
+HD bool is_statement(const char* p, const char* eol, const char* word) {  // obj_loader.cu is_statement, 6 letters
+  if (eol - p <= 6 || !(p[6] == ' ' || p[6] == '\t')) return false;
+  for (int i = 0; i < 6; ++i)
+    if (p[i] != word[i]) return false;
+  return true;
+}
+
+// kUsemtl / kMtllib for a name line, else kOther (only asked for lines line_kind calls kOther)
+HD int name_kind(const char* p, const char* eol) {
+  if (is_statement(p, eol, "usemtl")) return kUsemtl;
+  if (is_statement(p, eol, "mtllib")) return kMtllib;
+  return kOther;
+}
+
 // the first k numbers of a `v` (k = 3, from p + 2) or `vt` (k = 2, from p + 3) line
 HD int parse_numbers(const char* q, const char* eol, int k, float* out) {
   for (int i = 0; i < k; ++i) {
@@ -427,6 +450,7 @@ struct ParseHdr {
   int n_corners_dedup;      // total of the histogram scan
   int n_out;                // total of the unique-count scan
   int bad, fallback, any_uv;
+  int n_usemtl, n_names;    // totals of the two material scans
   unsigned int err_ord;     // first out-of-range corner (triangulated order); 0xffffffff: none
   int err_kind;             // 1 vertex, 2 vt
   long long err_a, err_b;
@@ -437,9 +461,11 @@ struct Layout {
   int items, items_pad, p_cap, t_cap, tri_cap, p_pad;
   size_t hdr, cnt_v, cnt_vt, cnt_tri, off_v, off_vt, off_tri, block_sums, pos, tex, keys, hist, bstart, ucnt, ustart,
       bucket, total;
+  // MVLM_OBJ_MATERIALS only, after everything else (the arrays above keep their offsets)
+  size_t cnt_mat, cnt_name, off_mat, off_name, names, line_page, tri_ord;
 };
 
-Layout layout(size_t n) {
+Layout layout(size_t n, bool materials = false) {
   Layout L{};
   const size_t items = (n + kItemBytes - 1) / kItemBytes;
   const size_t items_pad = (items + kScanItems) / kScanItems * kScanItems;  // at least one block, room for a sentinel
@@ -475,6 +501,15 @@ Layout layout(size_t n) {
   L.ucnt = take(p_pad * 4);
   L.ustart = take(p_pad * 4);
   L.bucket = take(tri_cap * 3 * 4);
+  if (materials) {
+    L.cnt_mat = take(items_pad * 4);  // contiguous with cnt_name (one memset)
+    L.cnt_name = take(items_pad * 4);
+    L.off_mat = take(items_pad * 4);
+    L.off_name = take(items_pad * 4);
+    L.names = take(static_cast<size_t>(MVLM_OBJ_MAX_NAME_LINES) * sizeof(mvlm_obj_name_line));
+    L.line_page = take(static_cast<size_t>(MVLM_OBJ_MAX_NAME_LINES) * 4);
+    L.tri_ord = take(tri_cap * 4);
+  }
   L.total = o;
   return L;
 }
@@ -494,11 +529,12 @@ __device__ __forceinline__ long long find_eol(const char* text, long long s, lon
 
 __global__ void __launch_bounds__(256) obj_count_kernel(const char* __restrict__ text, long long n, int items,
                                                         int* __restrict__ cnt_v, int* __restrict__ cnt_vt,
-                                                        int* __restrict__ cnt_tri, ParseHdr* __restrict__ hdr) {
+                                                        int* __restrict__ cnt_tri, int* __restrict__ cnt_mat,
+                                                        int* __restrict__ cnt_name, ParseHdr* __restrict__ hdr) {
   const int c = blockIdx.x * blockDim.x + threadIdx.x;
   if (c >= items) return;
   const long long lo = static_cast<long long>(c) * kItemBytes, hi = min(n, lo + kItemBytes);
-  int nv = 0, nvt = 0, ntri = 0;
+  int nv = 0, nvt = 0, ntri = 0, nmat = 0, nname = 0;
   bool bad = false;
   for (long long s = first_line_start(text, lo, hi); s < hi;) {
     const long long eol = find_eol(text, s, n);
@@ -511,12 +547,20 @@ __global__ void __launch_bounds__(256) obj_count_kernel(const char* __restrict__
       int k = 0;
       if (parse_face(text + s, text + eol, [&](long long, long long) { ++k; }) != kOk) bad = true;
       ntri += k > 2 ? k - 2 : 0;
+    } else if (cnt_name) {
+      const int nk = name_kind(text + s, text + eol);
+      nmat += nk == kUsemtl;
+      nname += nk != kOther;
     }
     s = eol + 1;
   }
   cnt_v[c] = nv;
   cnt_vt[c] = nvt;
   cnt_tri[c] = ntri;
+  if (cnt_name) {
+    cnt_mat[c] = nmat;
+    cnt_name[c] = nname;
+  }
   if (bad) atomicOr(&hdr->bad, 1);
 }
 
@@ -528,7 +572,10 @@ __global__ void __launch_bounds__(256) obj_parse_kernel(const char* __restrict__
                                                         const int* __restrict__ off_tri, ParseHdr* __restrict__ hdr,
                                                         int p_cap, int t_cap, unsigned int key_cap,
                                                         float* __restrict__ pos, float* __restrict__ tex,
-                                                        unsigned long long* __restrict__ keys) {
+                                                        unsigned long long* __restrict__ keys,
+                                                        const int* __restrict__ off_mat, const int* __restrict__ off_name,
+                                                        mvlm_obj_name_line* __restrict__ names,
+                                                        int32_t* __restrict__ tri_ord) {
   const int c = blockIdx.x * blockDim.x + threadIdx.x;
   if (c >= items) return;
   const long long lo = static_cast<long long>(c) * kItemBytes, hi = min(n, lo + kItemBytes);
@@ -536,6 +583,9 @@ __global__ void __launch_bounds__(256) obj_parse_kernel(const char* __restrict__
   unsigned int ord = 3u * static_cast<unsigned int>(off_tri[c]);
   const long long n_pos = hdr->n_pos, n_tex = hdr->n_tex;
   const unsigned int err_ord = kReport ? hdr->err_ord : 0u;
+  const bool materials = !kReport && names != nullptr;
+  int mat = materials ? off_mat[c] - 1 : -1;  // ordinal of the last `usemtl` line before the current line
+  int name = materials ? off_name[c] : 0;
   int bad = 0, fallback = 0, any_uv = 0;
   for (long long s = first_line_start(text, lo, hi); s < hi;) {
     const long long eol = find_eol(text, s, n);
@@ -553,7 +603,8 @@ __global__ void __launch_bounds__(256) obj_parse_kernel(const char* __restrict__
       else fallback = 1;
     } else if (kind == kF) {
       const long long v_seen = vi, vt_seen = ti;
-      parse_face_triangles(p, e, [&](int, long long a, long long b) {
+      parse_face_triangles(p, e, [&](int j, long long a, long long b) {
+        if (materials && j == 0 && ord < key_cap) tri_ord[ord / 3] = mat;
         unsigned long long key = 0;
         const int r = resolve_corner(a, b, v_seen, vt_seen, n_pos, n_tex, &key);
         if (kReport) {
@@ -570,6 +621,17 @@ __global__ void __launch_bounds__(256) obj_parse_kernel(const char* __restrict__
         }
         ++ord;
       });
+    } else if (materials) {
+      const int nk = name_kind(p, e);
+      if (nk != kOther) {
+        if (nk == kUsemtl) ++mat;
+        if (name < MVLM_OBJ_MAX_NAME_LINES) {
+          names[name].offset = s;
+          names[name].kind = nk == kUsemtl ? 1 : 2;
+          names[name].tris_before = static_cast<int32_t>(ord / 3);
+        }
+        ++name;
+      }
     }
     if (kind == kV) ++vi;
     if (kind == kVT) ++ti;
@@ -660,6 +722,16 @@ __global__ void __launch_bounds__(256) obj_map_corners_kernel(const unsigned lon
   tris[i] = ustart[v] + u;
 }
 
+// the page of every triangle: line_page[its `usemtl` ordinal], -1 before the first `usemtl`
+__global__ void __launch_bounds__(256) obj_tri_page_kernel(const int32_t* __restrict__ tri_ord, int n_tris,
+                                                           const int32_t* __restrict__ line_page,
+                                                           int32_t* __restrict__ tri_page) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n_tris) return;
+  const int m = tri_ord[i];
+  tri_page[i] = m >= 0 ? line_page[m] : -1;
+}
+
 __global__ void __launch_bounds__(256) obj_positions_kernel(const unsigned long long* __restrict__ keys, int n_corners,
                                                             int32_t* __restrict__ tris) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -675,18 +747,31 @@ using namespace mvlm;
 
 extern "C" {
 
-size_t mvlm_obj_parse_workspace_bytes(size_t n_bytes) {
-  const Layout L = layout(n_bytes);
+size_t mvlm_obj_parse_workspace_bytes(size_t n_bytes) { return mvlm_obj_parse_workspace_bytes_ex(n_bytes, 0); }
+
+size_t mvlm_obj_parse_workspace_bytes_ex(size_t n_bytes, int flags) {
+  const Layout L = layout(n_bytes, (flags & MVLM_OBJ_MATERIALS) != 0);
   return L.fits ? L.total : 0;
 }
 
 int mvlm_obj_parse_device(const char* text, size_t n_bytes, const char* path, void* workspace, size_t workspace_bytes,
                           void* stream, mvlm_obj_parse_info* info) {
+  return mvlm_obj_parse_device_ex(text, n_bytes, path, workspace, workspace_bytes, 0, stream, info, nullptr, 0, nullptr);
+}
+
+int mvlm_obj_parse_device_ex(const char* text, size_t n_bytes, const char* path, void* workspace,
+                             size_t workspace_bytes, int flags, void* stream, mvlm_obj_parse_info* info,
+                             mvlm_obj_name_line* name_lines, int max_name_lines, int* n_name_lines) {
   MVLM_REQUIRE(info && path, "mvlm_obj_parse_device: null pointer");
+  MVLM_REQUIRE((flags & ~MVLM_OBJ_MATERIALS) == 0, "mvlm_obj_parse_device_ex: unknown flags 0x%x", flags);
+  const bool materials = (flags & MVLM_OBJ_MATERIALS) != 0;
+  MVLM_REQUIRE(!materials || (name_lines && n_name_lines && max_name_lines >= MVLM_OBJ_MAX_NAME_LINES),
+               "mvlm_obj_parse_device_ex: materials need a host buffer of MVLM_OBJ_MAX_NAME_LINES name lines");
   memset(info, 0, sizeof(*info));
   info->n_bytes = n_bytes;
+  if (n_name_lines) *n_name_lines = 0;
   MVLM_REQUIRE(n_bytes > 0, "File %s does not contain any points.", path);
-  const Layout L = layout(n_bytes);
+  const Layout L = layout(n_bytes, materials);
   if (!L.fits) {  // beyond the scan capacity: the host parser takes it
     info->fallback = 1;
     return MVLM_OK;
@@ -708,20 +793,35 @@ int mvlm_obj_parse_device(const char* text, size_t n_bytes, const char* path, vo
   float* pos = reinterpret_cast<float*>(ws + L.pos);
   float* tex = reinterpret_cast<float*>(ws + L.tex);
   unsigned long long* keys = reinterpret_cast<unsigned long long*>(ws + L.keys);
+  int* cnt_mat = materials ? reinterpret_cast<int*>(ws + L.cnt_mat) : nullptr;
+  int* cnt_name = materials ? reinterpret_cast<int*>(ws + L.cnt_name) : nullptr;
+  int* off_mat = materials ? reinterpret_cast<int*>(ws + L.off_mat) : nullptr;
+  int* off_name = materials ? reinterpret_cast<int*>(ws + L.off_name) : nullptr;
+  mvlm_obj_name_line* names = materials ? reinterpret_cast<mvlm_obj_name_line*>(ws + L.names) : nullptr;
+  int32_t* tri_ord = materials ? reinterpret_cast<int32_t*>(ws + L.tri_ord) : nullptr;
   const long long n = static_cast<long long>(n_bytes);
 
   MVLM_CHECK_CUDA(cudaMemsetAsync(ws, 0, L.off_v, s));  // header + the three count arrays (padding zero)
   MVLM_CHECK_CUDA(cudaMemsetAsync(&hdr->err_ord, 0xff, sizeof(unsigned int), s));
-  obj_count_kernel<<<blocks_for(L.items), 256, 0, s>>>(text, n, L.items, cnt_v, cnt_vt, cnt_tri, hdr);
+  if (materials) MVLM_CHECK_CUDA(cudaMemsetAsync(cnt_mat, 0, L.off_mat - L.cnt_mat, s));
+  obj_count_kernel<<<blocks_for(L.items), 256, 0, s>>>(text, n, L.items, cnt_v, cnt_vt, cnt_tri, cnt_mat, cnt_name, hdr);
   exclusive_scan(cnt_v, L.items_pad, block_sums, off_v, &hdr->n_pos, s);
   exclusive_scan(cnt_vt, L.items_pad, block_sums, off_vt, &hdr->n_tex, s);
   exclusive_scan(cnt_tri, L.items_pad, block_sums, off_tri, &hdr->n_tri, s);
+  if (materials) {
+    exclusive_scan(cnt_mat, L.items_pad, block_sums, off_mat, &hdr->n_usemtl, s);
+    exclusive_scan(cnt_name, L.items_pad, block_sums, off_name, &hdr->n_names, s);
+    count_launch(6);
+  }
   obj_parse_kernel<false><<<blocks_for(L.items), 256, 0, s>>>(text, n, L.items, off_v, off_vt, off_tri, hdr, L.p_cap,
-                                                              L.t_cap, 3u * L.tri_cap, pos, tex, keys);
+                                                              L.t_cap, 3u * L.tri_cap, pos, tex, keys, off_mat,
+                                                              off_name, names, tri_ord);
   count_launch(11);
   MVLM_CHECK_CUDA(cudaGetLastError());
   ParseHdr h;
   MVLM_CHECK_CUDA(cudaMemcpyAsync(&h, hdr, sizeof(h), cudaMemcpyDeviceToHost, s));
+  if (materials)  // the first name lines travel with the sizes; a file with more takes one more copy below
+    MVLM_CHECK_CUDA(cudaMemcpyAsync(name_lines, names, kInlineNames * sizeof(mvlm_obj_name_line), cudaMemcpyDeviceToHost, s));
   MVLM_CHECK_CUDA(cudaStreamSynchronize(s));
   // the host parser's order of precedence: malformed line, no points, first out-of-range corner
   if (h.fallback) {
@@ -732,7 +832,8 @@ int mvlm_obj_parse_device(const char* text, size_t n_bytes, const char* path, vo
   MVLM_REQUIRE(h.n_pos > 0, "File %s does not contain any points.", path);
   if (h.err_ord != 0xffffffffu) {
     obj_parse_kernel<true><<<blocks_for(L.items), 256, 0, s>>>(text, n, L.items, off_v, off_vt, off_tri, hdr, L.p_cap,
-                                                               L.t_cap, 3u * L.tri_cap, pos, tex, keys);
+                                                               L.t_cap, 3u * L.tri_cap, pos, tex, keys, nullptr,
+                                                               nullptr, nullptr, nullptr);
     count_launch(1);
     MVLM_CHECK_CUDA(cudaGetLastError());
     MVLM_CHECK_CUDA(cudaMemcpyAsync(&h, hdr, sizeof(h), cudaMemcpyDeviceToHost, s));
@@ -774,6 +875,19 @@ int mvlm_obj_parse_device(const char* text, size_t n_bytes, const char* path, vo
       return MVLM_OK;
     }
   }
+  if (materials) {
+    if (h.n_names > MVLM_OBJ_MAX_NAME_LINES) {
+      info->fallback = 1;
+      return MVLM_OK;
+    }
+    if (h.n_names > kInlineNames) {
+      MVLM_CHECK_CUDA(cudaMemcpyAsync(name_lines + kInlineNames, names + kInlineNames,
+                                      static_cast<size_t>(h.n_names - kInlineNames) * sizeof(mvlm_obj_name_line),
+                                      cudaMemcpyDeviceToHost, s));
+      MVLM_CHECK_CUDA(cudaStreamSynchronize(s));
+    }
+    *n_name_lines = h.n_names;
+  }
   info->n_verts = h.any_uv ? h.n_out : h.n_pos;
   info->n_tris = h.n_tri;
   info->has_uv = h.any_uv ? 1 : 0;
@@ -807,6 +921,28 @@ int mvlm_obj_parse_write(const mvlm_obj_parse_info* info, const void* workspace,
                                                                         info->n_positions, verts, uvs);
     obj_map_corners_kernel<<<blocks_for(n_corners), 256, 0, s>>>(keys, n_corners, bstart, ustart, bucket, tris);
     count_launch(2);
+  }
+  MVLM_CHECK_CUDA(cudaGetLastError());
+  return MVLM_OK;
+}
+
+int mvlm_obj_parse_tri_page(const mvlm_obj_parse_info* info, void* workspace, const int32_t* line_page, int n_usemtl,
+                            int32_t* tri_page, void* stream) {
+  MVLM_REQUIRE(info && workspace && (line_page || n_usemtl == 0) && (tri_page || info->n_tris == 0),
+               "mvlm_obj_parse_tri_page: null pointer");
+  MVLM_REQUIRE(!info->fallback && info->n_positions > 0, "mvlm_obj_parse_tri_page: no parse to write");
+  MVLM_REQUIRE(n_usemtl >= 0 && n_usemtl <= MVLM_OBJ_MAX_NAME_LINES, "mvlm_obj_parse_tri_page: %d usemtl lines",
+               n_usemtl);
+  const Layout L = layout(info->n_bytes, true);
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  uint8_t* ws = static_cast<uint8_t*>(workspace);
+  int32_t* table = reinterpret_cast<int32_t*>(ws + L.line_page);
+  if (n_usemtl > 0)
+    MVLM_CHECK_CUDA(cudaMemcpyAsync(table, line_page, static_cast<size_t>(n_usemtl) * 4, cudaMemcpyHostToDevice, s));
+  if (info->n_tris > 0) {
+    obj_tri_page_kernel<<<blocks_for(info->n_tris), 256, 0, s>>>(reinterpret_cast<const int32_t*>(ws + L.tri_ord),
+                                                                 info->n_tris, table, tri_page);
+    count_launch(1);
   }
   MVLM_CHECK_CUDA(cudaGetLastError());
   return MVLM_OK;

@@ -19,9 +19,10 @@
 //                  screen tiles with a shared-memory z-tile (the textbook design for LARGE triangles) costs two more
 //                  passes over the (view, triangle) pairs to save less than one global atomic each: DESIGN.md 7d.
 //   raster_resolve one thread per pixel: winner triangle -> barycentric uv -> nearest texel (one 4-byte load from
-//                  the RGBA texture) or, for a scan with vertex colours and no texture, the barycentric blend of its
-//                  three RGBA vertex colours; depth byte, optional geometry shade; writes the u8 NHWC4 image the CNN
-//                  stem consumes and, on request, the fp32 (V,H,W,C) stack / triangle-id / z maps.
+//                  the RGBA texture, or from the triangle's page of a scan with texture pages) or, for a scan with
+//                  vertex colours and no texture, the barycentric blend of its three RGBA vertex colours; depth byte,
+//                  optional geometry shade; writes the u8 NHWC4 image the CNN stem consumes and, on request, the fp32
+//                  (V,H,W,C) stack / triangle-id / z maps.
 //
 // This file is compiled with --fmad=false: every fp32 operation rounds separately, in the same
 // order as oracle/csrc/oracle_native.c (built with -ffp-contract=off), so triangle-id maps and
@@ -170,7 +171,22 @@ __global__ void __launch_bounds__(256) raster_resolve_kernel(RasterArgs g, const
       const float l0 = edge_fn(b.sx, b.sy, c.sx, c.sy, cx, cy) / area;
       const float l1 = edge_fn(c.sx, c.sy, a.sx, a.sy, cx, cy) / area;
       const float l2 = edge_fn(a.sx, a.sy, b.sx, b.sy, cx, cy) / area;
-      if (textured) {  // a texture always wins over vertex colours
+      if (sc.pages) {  // texture pages: the single-texture rule below with the sizes of the triangle's page
+        const int page = __ldg(sc.pages + tid);
+        if (page >= 0) {  // -1: no page, white
+          const int* e = sc.pages + sc.nt + 3 * page;
+          const int off = __ldg(e), th = __ldg(e + 1), tw = __ldg(e + 2);
+          const float u = (l0 * sc.uvs[2 * i0] + l1 * sc.uvs[2 * i1]) + l2 * sc.uvs[2 * i2];
+          const float v = (l0 * sc.uvs[2 * i0 + 1] + l1 * sc.uvs[2 * i1 + 1]) + l2 * sc.uvs[2 * i2 + 1];
+          int tx = static_cast<int>(floorf(u * static_cast<float>(tw)));
+          int ty = static_cast<int>(floorf(v * static_cast<float>(th)));
+          if (tx < 0 || tx >= tw) { tx %= tw; if (tx < 0) tx += tw; }
+          if (ty < 0 || ty >= th) { ty %= th; if (ty < 0) ty += th; }
+          const size_t ti = static_cast<size_t>(off) + static_cast<size_t>(th - 1 - ty) * tw + tx;
+          const uchar4 q4 = __ldg(reinterpret_cast<const uchar4*>(sc.tex) + ti);
+          r8 = q4.x; g8 = q4.y; b8 = q4.z;
+        }
+      } else if (textured) {  // a texture always wins over vertex colours
         const float u = (l0 * sc.uvs[2 * i0] + l1 * sc.uvs[2 * i1]) + l2 * sc.uvs[2 * i2];
         const float v = (l0 * sc.uvs[2 * i0 + 1] + l1 * sc.uvs[2 * i1 + 1]) + l2 * sc.uvs[2 * i2 + 1];
         int tx = static_cast<int>(floorf(u * static_cast<float>(sc.tw)));

@@ -14,6 +14,8 @@ struct RasterScan {
   const int* tris;             // (Nt,3)
   const unsigned char* tex;    // (Th,Tw,tex_c) or null
   const uchar4* colors;        // (Nv) RGBA vertex colours or null; used in the RGB modes when there is no (tex, uvs)
+  // texture pages or null: (Nt) page per triangle (-1 = white), then (P,3) texel offset into tex (RGBA), height, width
+  const int* pages;
   int nv, nt;
   int th, tw, tex_c;           // tex_c = 3 (RGB) or 4 (RGBA: one 4-byte load per texel)
 };

@@ -11,7 +11,7 @@ from pathlib import Path
 
 import numpy as np
 
-from .io_obj import Mesh, load_obj, loader_state, read_pinned
+from .io_obj import Mesh, check_texture_source, load_obj, loader_state, read_pinned
 
 SUFFIXES = {"obj": ".obj", "ply": ".ply", "stl": ".stl"}
 
@@ -127,14 +127,15 @@ def load_ply_stl(path: Path | str, n_threads: int = 0, device="cuda", parser: st
 
 
 def load_mesh(path: Path | str, load_texture: bool = True, n_threads: int = 0, texture_decoder: str = "pil",
-              device="cuda", parser: str = "host") -> Mesh:
+              device="cuda", parser: str = "host", texture_source: str = "stem") -> Mesh:
     """Any supported scan by its suffix: `.obj` -> io_obj.load_obj (all arguments apply), `.ply` / `.stl` (any case)
-    -> load_ply_stl (no texture: load_texture and texture_decoder do not apply)."""
+    -> load_ply_stl (no texture: load_texture, texture_decoder and texture_source do not apply)."""
     path = Path(path)
     suffix = path.suffix.lower()
+    check_texture_source(texture_source)
     if path.suffix == ".obj":
         return load_obj(path, load_texture=load_texture, n_threads=n_threads, texture_decoder=texture_decoder,
-                        device=device, parser=parser)
+                        device=device, parser=parser, texture_source=texture_source)
     if suffix in (".ply", ".stl"):
         return load_ply_stl(path, n_threads=n_threads, device=device, parser=parser)
     raise ValueError(f"File {path} is not an .obj, .ply or .stl file.")

@@ -114,8 +114,10 @@ def raster_multiview(verts, uvs, tris, tex, rot, h: int, w: int, channel_mode: s
 
 def raster_multiscan(scans, rot, h: int, w: int, channel_mode: str = "RGB+depth", want_f32: bool = False,
                      want_tri: bool = False, want_z: bool = False, zbuf=None, out_u8=None):
-    """Several scans in one pass.  scans: list of (verts, uvs|None, tris, tex|None[, colors|None]) cuda tensors as in
-    raster_multiview, colors (Nv,4) u8 RGBA per-vertex colours (used in the RGB modes by a scan without a texture);
+    """Several scans in one pass.  scans: list of (verts, uvs|None, tris, tex|None[, colors|None[, pages|None]]) cuda
+    tensors as in raster_multiview, colors (Nv,4) u8 RGBA per-vertex colours (used in the RGB modes by a scan without a
+    texture), pages the int32 (Nt + 3P,) page table of mvlm_raster_multiscan_paged (page per triangle, then texel
+    offset, height, width per page) with tex the RGBA texels of all P pages (render3d.DeviceMesh.paged builds both);
     rot (S*V,9|3,3) f64, scan-major (scan s owns views [s*V, (s+1)*V)).  zbuf: optional persistent workspace (a new
     one is allocated when it is smaller than mvlm_raster_multiscan_workspace_bytes).
     Returns dict(u8=(S*V,H,W,4), f32, tri, z) like raster_multiview; each scan's views equal raster_multiview's."""
@@ -131,13 +133,19 @@ def raster_multiscan(scans, rot, h: int, w: int, channel_mode: str = "RGB+depth"
     mode = CHANNEL_MODES[channel_mode]
     table = (_lib.RasterScan * n)()
     rgba = (C.c_void_p * n)()
+    paged = (C.c_void_p * n)()
     for i, (e, scan) in enumerate(zip(table, scans)):
-        if len(scan) not in (4, 5):
-            raise ValueError("a scan is (verts, uvs, tris, tex) or (verts, uvs, tris, tex, colors)")
+        if len(scan) not in (4, 5, 6):
+            raise ValueError("a scan is (verts, uvs, tris, tex[, colors[, pages]])")
         verts, uvs, tris, tex = scan[:4]
-        colors = scan[4] if len(scan) == 5 else None
+        colors = scan[4] if len(scan) >= 5 else None
+        pages = scan[5] if len(scan) == 6 else None
         if colors is not None and (colors.dtype != torch.uint8 or tuple(colors.shape) != (verts.shape[0], 4)):
             raise ValueError(f"vertex colours must be ({verts.shape[0]}, 4) uint8 RGBA")
+        if pages is not None and (pages.dtype != torch.int32 or pages.dim() != 1 or pages.numel() < tris.shape[0]
+                                  or (pages.numel() - tris.shape[0]) % 3 or tex is None or tex.shape[-1] != 4):
+            raise ValueError("pages must be an int32 (Nt + 3P,) table with an RGBA texel buffer as tex")
+        paged[i] = ptr(pages)
         e.verts, e.n_verts, e.uvs, e.tris, e.n_tris = ptr(verts), verts.shape[0], ptr(uvs), ptr(tris), tris.shape[0]
         e.tex, (e.tex_h, e.tex_w, e.tex_channels) = ptr(tex), (tex.shape[:3] if tex is not None else (0, 0, 3))
         rgba[i] = ptr(colors)
@@ -149,9 +157,9 @@ def raster_multiscan(scans, rot, h: int, w: int, channel_mode: str = "RGB+depth"
     f32 = torch.empty((total, h, w, MODE_CHANNELS[mode]), dtype=torch.float32, device=dev) if want_f32 else None
     tri = torch.empty((total, h, w), dtype=torch.int32, device=dev) if want_tri else None
     z = torch.empty((total, h, w), dtype=torch.float32, device=dev) if want_z else None
-    check(lib.mvlm_raster_multiscan_colored(table, rgba, n, ptr(rot), v, h, w, mode, ptr(zbuf),
-                                            zbuf.numel() * zbuf.element_size(), ptr(out_u8), ptr(f32), ptr(tri), ptr(z),
-                                            cur_stream()), "mvlm_raster_multiscan_colored")
+    check(lib.mvlm_raster_multiscan_paged(table, rgba, paged, n, ptr(rot), v, h, w, mode, ptr(zbuf),
+                                          zbuf.numel() * zbuf.element_size(), ptr(out_u8), ptr(f32), ptr(tri), ptr(z),
+                                          cur_stream()), "mvlm_raster_multiscan_paged")
     return {"u8": out_u8, "f32": f32, "tri": tri, "z": z}
 
 

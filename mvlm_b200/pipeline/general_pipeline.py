@@ -20,7 +20,7 @@ import torch
 
 from .. import _lib
 from ..io_mesh import SUFFIXES, check_scan_file, check_scan_formats, is_scan_file, load_mesh
-from ..io_obj import Mesh
+from ..io_obj import Mesh, check_texture_source
 from ..prediction.paulsenpredictor import PaulsenModel
 from ..utils import Estimator3D, ObjRenderer3D, prealign
 
@@ -97,7 +97,7 @@ class Pipeline(abc.ABC, TimeMixin):
                  channel_mode: str = "RGB+depth", n_hypotheses: int = 1, seed: int | None = None,
                  transforms: np.ndarray | None = None, device: str = "cuda", verbose: bool = True,
                  texture_decoder: str = "pil", pre_align: dict | None = None, obj_parser: str = "host",
-                 scan_formats: tuple = ("obj",)):
+                 scan_formats: tuple = ("obj",), texture_source: str = "stem"):
         TimeMixin.__init__(self)
         self.render_image_stack = render_image_stack
         self.render_image_folder = render_image_folder
@@ -119,6 +119,9 @@ class Pipeline(abc.ABC, TimeMixin):
         # default: the OBJ-only checks and messages) or any of "obj", "ply", "stl" (io_mesh; obj_parser then selects
         # the host or the device decoder for every format)
         self.scan_formats = check_scan_formats(scan_formats)
+        # where an OBJ scan's texture comes from: "stem" (the reference's `<stem>.jpg` rule, the default) or "mtl" (its
+        # MTL materials, several texture pages per scan; DESIGN.md 7g) in every entry point and the seam renderer
+        self.texture_source = check_texture_source(texture_source)
         # legacy "pre-align" block (configs/*.json:59-84): {"align_center_of_mass", "rot_x", "rot_y", "rot_z", "scale"};
         # None / identity = off, see utils/prealign.py
         self.pre_align = None if prealign.is_identity(pre_align) else dict(pre_align)
@@ -129,6 +132,7 @@ class Pipeline(abc.ABC, TimeMixin):
         self.renderer_3d.verbose = verbose
         self.renderer_3d.pre_align = self.pre_align
         self.renderer_3d.scan_formats = self.scan_formats
+        self.renderer_3d.texture_source = self.texture_source
         self.estimator_3d = Estimator3D(n_hypotheses=n_hypotheses, seed=seed, device=device)
         self.estimator_3d.verbose = verbose
         # One pipeline object = one set of device buffers (renderer images, CNN workspace, CUDA graphs): calls from
@@ -168,7 +172,7 @@ class Pipeline(abc.ABC, TimeMixin):
                 check_scan_file(file_name, self.scan_formats)
                 self.tic()
                 mesh = load_mesh(file_name, texture_decoder=self.texture_decoder, device=self.device,
-                                 parser=self.obj_parser)
+                                 parser=self.obj_parser, texture_source=self.texture_source)
                 self._print("Render [1] - Setup time: ", self.toc_p())
                 landmarks = self.predict_mesh(mesh)
                 self._print("Landmarks 3D Total: ", self.p_time(time.time() - full_s))
@@ -196,7 +200,7 @@ class Pipeline(abc.ABC, TimeMixin):
                 # four parser threads per scan: with more, the loaders of `prefetch` scans oversubscribe the host and the
                 # thread that feeds the GPU gets descheduled (measured on the 16-core box: 36 scans/s with 16, 51 with 4)
                 return load_mesh(f, n_threads=4, texture_decoder=self.texture_decoder, device=self.device,
-                                 parser=self.obj_parser)
+                                 parser=self.obj_parser, texture_source=self.texture_source)
 
             # `prefetch` loader threads, with the scans of a whole pass queued for them: the driver takes a pass's scans
             # at once and then waits for an earlier pass, the loaders keep working meanwhile

@@ -1,4 +1,4 @@
-"""Seeded synthetic inputs: a textured face-like mesh (OBJ + JPG, PLY, STL), view transforms, ray sets.
+"""Seeded synthetic inputs: a textured face-like mesh (OBJ + JPG, OBJ + MTL pages, PLY, STL), view transforms, ray sets.
 
 The reference's sample scans are missing blobs (.MISSING_LARGE_BLOBS) and there is no network,
 so every benchmark and parity test runs on these (SURVEY.md section 8d).
@@ -85,6 +85,39 @@ def write_obj(path: Path, verts, uvs, tris, texture: np.ndarray | None = None, j
         from PIL import Image
 
         Image.fromarray(texture).save(path.with_suffix(".jpg"), quality=jpeg_quality)
+    return path
+
+
+def write_obj_mtl(path: Path, verts, uvs, tris, pages: list, tri_page, formats=None, jpeg_quality: int = 95) -> Path:
+    """Writes an OBJ scan textured through MTL materials (DESIGN.md 7g): `<path>.obj` with `mtllib <stem>.mtl`, its
+    faces in file order split into `usemtl` groups wherever `tri_page` changes, `<stem>.mtl` with one material per page
+    (`map_Kd <stem>_<i>.<format>`) and one without a texture for page -1, and the pages themselves.
+    pages: (Th,Tw,3) uint8 images of any sizes; tri_page: (Nt,) page of every triangle (-1: the untextured material);
+    formats: file format per page, "jpg" (default) or "png"."""
+    from PIL import Image
+
+    path = Path(path)
+    tri_page = np.asarray(tri_page)
+    formats = formats or ["jpg"] * len(pages)
+    files = [f"{path.stem}_{i}.{fmt}" for i, fmt in enumerate(formats)]
+    for img, fmt, name in zip(pages, formats, files):
+        Image.fromarray(img).save(path.parent / name, **({"quality": jpeg_quality} if fmt == "jpg" else {}))
+    lines = []
+    for i, name in enumerate(files):
+        lines += [f"newmtl page{i}", "Ka 1 1 1", "Kd 1 1 1", f"map_Kd {name}", ""]
+    lines += ["newmtl untextured", "Kd 1 1 1", ""]
+    path.with_suffix(".mtl").write_text("\n".join(lines))
+    t = np.asarray(tris) + 1
+    cuts = np.flatnonzero(np.diff(tri_page)) + 1
+    with open(path, "w") as f:
+        f.write(f"# mvlm_b200 synthetic scan\nmtllib {path.stem}.mtl\n")
+        np.savetxt(f, verts, fmt="v %.6f %.6f %.6f")
+        np.savetxt(f, uvs, fmt="vt %.6f %.6f")
+        for lo, hi in zip(np.concatenate(([0], cuts)), np.concatenate((cuts, [len(t)]))):
+            f.write(f"usemtl {'untextured' if tri_page[lo] < 0 else f'page{tri_page[lo]}'}\n")
+            tt = t[lo:hi]
+            np.savetxt(f, np.stack([tt[:, 0], tt[:, 0], tt[:, 1], tt[:, 1], tt[:, 2], tt[:, 2]], 1),
+                       fmt="f %d/%d %d/%d %d/%d")
     return path
 
 

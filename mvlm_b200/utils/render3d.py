@@ -93,6 +93,15 @@ class _PinnedStage:
         return view.view(a.shape)
 
 
+def page_table(pages) -> np.ndarray:
+    """(3P,) int32: texel offset, height and width of every page in the packed RGBA buffer of DeviceMesh.paged."""
+    table, off = [], 0
+    for p in pages:
+        table += [off, p.shape[0], p.shape[1]]
+        off += p.shape[0] * p.shape[1]
+    return np.asarray(table, dtype=np.int32)
+
+
 class DeviceMesh:
     """Device-resident copy of a Mesh (uploaded once per scan)."""
 
@@ -103,7 +112,7 @@ class DeviceMesh:
             if a is None:
                 return None
             if isinstance(a, torch.Tensor):  # decoded (nvJPEG) or parsed (parser="gpu") on the loader's side stream
-                ready = mesh.texture_ready if name == "tex" else mesh.geometry_ready
+                ready = mesh.texture_ready if name == "tex" or name.startswith("page") else mesh.geometry_ready
                 if ready is not None:
                     torch.cuda.current_stream().wait_event(ready)
                 a.record_stream(torch.cuda.current_stream())
@@ -123,16 +132,40 @@ class DeviceMesh:
         self.verts, self.tris = up("verts", mesh.verts), up("tris", mesh.tris)
         self.uvs, self.tex = up("uvs", mesh.uvs), up("tex", mesh.texture)
         self.colors = up("colors", mesh.colors)
+        self.pages = None if mesh.pages is None else [up(f"page{i}", p) for i, p in enumerate(mesh.pages)]
+        self.tri_page = up("tri_page", mesh.tri_page)
+        self.page_table = None if mesh.pages is None else up("page_table", page_table(mesh.pages))
         if stage is not None and device.type == "cuda":
             stage.done = torch.cuda.Event()
             stage.done.record()
 
     @classmethod
-    def from_device(cls, mesh: Mesh, verts, tris, uvs, tex, colors=None) -> "DeviceMesh":
+    def from_device(cls, mesh: Mesh, verts, tris, uvs, tex, colors=None, pages=None, tri_page=None,
+                    page_table=None) -> "DeviceMesh":
         """Wraps arrays that are on the device already (sharding.upload_mesh_sharded)."""
         self = cls.__new__(cls)
         self.mesh, self.verts, self.tris, self.uvs, self.tex, self.colors = mesh, verts, tris, uvs, tex, colors
+        self.pages, self.tri_page, self.page_table = pages, tri_page, page_table
         return self
+
+    def paged(self):
+        """Texture pages for the rasteriser, packed once per device mesh: (RGBA texels of all pages (1, N, 4) u8, int32
+        (Nt + 3P,) table = the page of every triangle, then texel offset, height and width of every page), or
+        (None, None) for a scan without pages."""
+        if self.pages is None:
+            return None, None
+        t = self.__dict__.get("_paged")
+        if t is None:
+            dev = self.tri_page.device
+            texels = torch.empty((1, sum(p.shape[0] * p.shape[1] for p in self.pages), 4), dtype=torch.uint8, device=dev)
+            texels[..., 3] = 255
+            off = 0
+            for p in self.pages:
+                n = p.shape[0] * p.shape[1]
+                texels[0, off:off + n, :3] = p.reshape(n, 3)
+                off += n
+            t = self._paged = (texels, torch.cat([self.tri_page.reshape(-1), self.page_table]))
+        return t
 
     def tex4(self):
         """The texture as RGBA (one 4-byte load per texel in the rasteriser), expanded once per device mesh."""
@@ -171,7 +204,8 @@ class DeviceMesh:
 
     @property
     def h2d_bytes(self) -> int:
-        return sum(t.numel() * t.element_size() for t in (self.verts, self.tris, self.uvs, self.tex, self.colors)
+        return sum(t.numel() * t.element_size()
+                   for t in (self.verts, self.tris, self.uvs, self.tex, self.colors, self.tri_page, *(self.pages or ()))
                    if t is not None)
 
 
@@ -201,6 +235,8 @@ class ObjRenderer3D:
         self.verbose = True
         # suffixes multiview_render accepts (set by the pipeline's scan_formats)
         self.scan_formats = ("obj",)
+        # where multiview_render finds an OBJ's texture (set by the pipeline's texture_source)
+        self.texture_source = "stem"
 
     # render3d.py:79-89 (GLOBAL np.random, same draw order)
     def random_transform(self, size=1):
@@ -279,15 +315,18 @@ class ObjRenderer3D:
         if self._zbuf is None or self._zbuf.numel() * 8 < need:
             n = lib.mvlm_raster_multiscan_workspace_bytes(len(dmeshes), total // len(dmeshes), h, w, int(max_nv * 1.25))
             self._zbuf = torch.empty(((n + 7) // 8,), dtype=torch.int64, device=self.device)
-        return ops.raster_multiscan([(d.verts, d.uvs, d.tris, d.tex4(), d.colors4()) for d in dmeshes], rot, h, w,
-                                    self.channel_mode,
+        scans = []
+        for d in dmeshes:
+            texels, pages = d.paged()
+            scans.append((d.verts, d.uvs, d.tris, d.tex4() if pages is None else texels, d.colors4(), pages))
+        return ops.raster_multiscan(scans, rot, h, w, self.channel_mode,
                                     want_f32=want_f32, want_tri=want_tri, want_z=want_z, zbuf=self._zbuf,
                                     out_u8=self._u8[:total])
 
     # render3d.py:114-177
     def render_3d_multi_rgb_geometry_depth(self, transform_stack, file_name):
         tt = time.time()
-        mesh = file_name if isinstance(file_name, Mesh) else load_mesh(file_name)
+        mesh = file_name if isinstance(file_name, Mesh) else load_mesh(file_name, texture_source=self.texture_source)
         if self.pre_align is not None:  # legacy "pre-align" block, see utils/prealign.py; the seam path's back-transform
             import dataclasses           # is Pipeline._predict_seams'
 
