@@ -171,36 +171,31 @@ __global__ void __launch_bounds__(256) raster_resolve_kernel(RasterArgs g, const
       const float l0 = edge_fn(b.sx, b.sy, c.sx, c.sy, cx, cy) / area;
       const float l1 = edge_fn(c.sx, c.sy, a.sx, a.sy, cx, cy) / area;
       const float l2 = edge_fn(a.sx, a.sy, b.sx, b.sy, cx, cy) / area;
-      if (sc.pages) {  // texture pages: the single-texture rule below with the sizes of the triangle's page
-        const int page = __ldg(sc.pages + tid);
-        if (page >= 0) {  // -1: no page, white
-          const int* e = sc.pages + sc.nt + 3 * page;
-          const int off = __ldg(e), th = __ldg(e + 1), tw = __ldg(e + 2);
+      if (textured) {  // a texture always wins over vertex colours (pages imply a texture, mvlm_raster_multiscan_paged)
+        // a single texture is page 0 at texel offset 0; a paged scan reads its triangle's page (-1: no page, white)
+        const int page = sc.pages ? __ldg(sc.pages + tid) : 0;
+        if (page >= 0) {
+          size_t off = 0;
+          int th = sc.th, tw = sc.tw;
+          if (sc.pages) {
+            const int* e = sc.pages + sc.nt + 3 * page;
+            off = static_cast<size_t>(__ldg(e)); th = __ldg(e + 1); tw = __ldg(e + 2);
+          }
           const float u = (l0 * sc.uvs[2 * i0] + l1 * sc.uvs[2 * i1]) + l2 * sc.uvs[2 * i2];
           const float v = (l0 * sc.uvs[2 * i0 + 1] + l1 * sc.uvs[2 * i1 + 1]) + l2 * sc.uvs[2 * i2 + 1];
           int tx = static_cast<int>(floorf(u * static_cast<float>(tw)));
           int ty = static_cast<int>(floorf(v * static_cast<float>(th)));
+          // repeat wrap; texture coordinates inside [0, 1) (the usual case) skip the two integer divisions
           if (tx < 0 || tx >= tw) { tx %= tw; if (tx < 0) tx += tw; }
           if (ty < 0 || ty >= th) { ty %= th; if (ty < 0) ty += th; }
-          const size_t ti = static_cast<size_t>(off) + static_cast<size_t>(th - 1 - ty) * tw + tx;
-          const uchar4 q4 = __ldg(reinterpret_cast<const uchar4*>(sc.tex) + ti);
-          r8 = q4.x; g8 = q4.y; b8 = q4.z;
-        }
-      } else if (textured) {  // a texture always wins over vertex colours
-        const float u = (l0 * sc.uvs[2 * i0] + l1 * sc.uvs[2 * i1]) + l2 * sc.uvs[2 * i2];
-        const float v = (l0 * sc.uvs[2 * i0 + 1] + l1 * sc.uvs[2 * i1 + 1]) + l2 * sc.uvs[2 * i2 + 1];
-        int tx = static_cast<int>(floorf(u * static_cast<float>(sc.tw)));
-        int ty = static_cast<int>(floorf(v * static_cast<float>(sc.th)));
-        // repeat wrap; texture coordinates inside [0, 1) (the usual case) skip the two integer divisions
-        if (tx < 0 || tx >= sc.tw) { tx %= sc.tw; if (tx < 0) tx += sc.tw; }
-        if (ty < 0 || ty >= sc.th) { ty %= sc.th; if (ty < 0) ty += sc.th; }
-        const size_t ti = static_cast<size_t>(sc.th - 1 - ty) * sc.tw + tx;
-        if (sc.tex_c == 4) {  // RGBA texture: one 4-byte load per texel
-          const uchar4 q4 = __ldg(reinterpret_cast<const uchar4*>(sc.tex) + ti);
-          r8 = q4.x; g8 = q4.y; b8 = q4.z;
-        } else {
-          const unsigned char* texel = sc.tex + ti * 3;
-          r8 = texel[0]; g8 = texel[1]; b8 = texel[2];
+          const size_t ti = off + static_cast<size_t>(th - 1 - ty) * tw + tx;
+          if (sc.tex_c == 4) {  // RGBA texture or pages: one 4-byte load per texel
+            const uchar4 q4 = __ldg(reinterpret_cast<const uchar4*>(sc.tex) + ti);
+            r8 = q4.x; g8 = q4.y; b8 = q4.z;
+          } else {
+            const unsigned char* texel = sc.tex + ti * 3;
+            r8 = texel[0]; g8 = texel[1]; b8 = texel[2];
+          }
         }
       } else {  // vertex colours (Gouraud): c = (l0*c0 + l1*c1) + l2*c2 per channel, rounded half up, clamped to [0,255]
         const uchar4 c0 = __ldg(sc.colors + i0), c1 = __ldg(sc.colors + i1), c2 = __ldg(sc.colors + i2);

@@ -13,7 +13,7 @@ page of every triangle (Mesh.tri_page).
 from __future__ import annotations
 
 import os
-from dataclasses import dataclass
+from dataclasses import dataclass, replace
 from pathlib import Path
 
 import numpy as np
@@ -37,6 +37,20 @@ class Mesh:
     @property
     def bbox_diagonal(self) -> float:
         return float(np.linalg.norm(self.verts.max(0) - self.verts.min(0)))
+
+    def arrays(self) -> list:
+        """(name, array, ready event) of every array of the scan that is present, in upload order: verts, tris, uvs,
+        tex, colors, tri_page, page0 .. page{P-1} and page_table (render3d.page_table, computed from the pages).  A
+        CUDA tensor is read only after its event: texture_ready for the texture and the pages, geometry_ready for the
+        rest.  The names key the pinned staging buffers of the uploads, which are reused from scan to scan."""
+        g, t = self.geometry_ready, self.texture_ready
+        out = [("verts", self.verts, g), ("tris", self.tris, g), ("uvs", self.uvs, g), ("tex", self.texture, t),
+               ("colors", self.colors, g), ("tri_page", self.tri_page, g)]
+        if self.pages is not None:
+            from .utils.render3d import page_table
+
+            out += [(f"page{i}", p, t) for i, p in enumerate(self.pages)] + [("page_table", page_table(self.pages), g)]
+        return [e for e in out if e[1] is not None]
 
 
 def _texture_file(path: Path):
@@ -63,11 +77,29 @@ def _read_image(file: Path):
         return None
 
 
-def _load_texture(path: Path):
+TEXTURE_DECODERS = ("pil", "nvjpeg")
+
+
+def _check_texture_decoder(texture_decoder: str) -> None:
+    if texture_decoder not in TEXTURE_DECODERS:
+        raise ValueError(f"Unknown texture decoder: {texture_decoder}")
+
+
+def _read_texture(file: Path, texture_decoder: str, device):
+    """One image file -> ((Th,Tw,3) uint8, event recorded after a device-side decode or None), or (None, None) when it
+    is missing or unreadable.  JPEG files under texture_decoder="nvjpeg" are decoded on the GPU (a CUDA tensor),
+    everything else through PIL (a numpy array)."""
+    _check_texture_decoder(texture_decoder)
+    if texture_decoder == "nvjpeg" and file.suffix.lower() in (".jpg", ".jpeg"):
+        return _decode_jpeg_nvjpeg(file, device)
+    return _read_image(file), None
+
+
+def _load_texture(path: Path, texture_decoder: str = "pil", device=None):
+    """The `<stem>.jpg` rule (_texture_file) through _read_texture: (texture, event | None)."""
+    _check_texture_decoder(texture_decoder)  # also for a scan without a texture file
     jpg = _texture_file(path)
-    if jpg is None:
-        return None
-    return _read_image(jpg)
+    return (None, None) if jpg is None else _read_texture(jpg, texture_decoder, device)
 
 
 TEXTURE_SOURCES = ("stem", "mtl")
@@ -127,17 +159,10 @@ def loader_state(device):
     return _tls
 
 
-def _decode_texture_nvjpeg(path: Path, device):
-    """`<stem>.jpg` -> (Th,Tw,3) uint8 CUDA tensor + the event recorded behind the decode (mvlm_jpeg_decode_rgb on a
-    per-thread side stream: the loader threads of Pipeline.predict_files decode while the main stream computes)."""
-    jpg = _texture_file(path)
-    if jpg is None:
-        return None, None
-    return _decode_jpeg_nvjpeg(jpg, device)
-
-
 def _decode_jpeg_nvjpeg(jpg: Path, device):
-    """One JPEG file -> (Th,Tw,3) uint8 CUDA tensor + event, or (None, None) when it is missing or unreadable."""
+    """One JPEG file -> (Th,Tw,3) uint8 CUDA tensor + the event recorded behind the decode, or (None, None) when it is
+    missing or unreadable (mvlm_jpeg_decode_rgb on a per-thread side stream: the loader threads of
+    Pipeline.predict_files decode while the main stream computes)."""
     import torch
 
     from . import _lib
@@ -303,12 +328,7 @@ def _load_pages(path: Path, order: list, names: list, libraries: list, texture_d
             continue
         key = os.path.normpath(file)
         if key not in by_file:
-            if texture_decoder == "nvjpeg" and file.suffix.lower() in (".jpg", ".jpeg"):
-                img, ev = _decode_jpeg_nvjpeg(file, device)
-            elif texture_decoder in ("nvjpeg", "pil"):
-                img, ev = _read_image(file), None
-            else:
-                raise ValueError(f"Unknown texture decoder: {texture_decoder}")
+            img, ev = _read_texture(file, texture_decoder, device)
             if img is None:
                 print("Could not load texture", file)
                 by_file[key] = -1
@@ -325,10 +345,8 @@ def _load_pages(path: Path, order: list, names: list, libraries: list, texture_d
 def _paged_mesh(mesh: Mesh, pages: list, one_page: bool, tri_page, ready, geometry_ready) -> Mesh:
     """A scan whose triangles all use one page (`one_page`) is an ordinary single-texture scan."""
     if one_page:
-        return Mesh(verts=mesh.verts, tris=mesh.tris, uvs=mesh.uvs, texture=pages[0], path=mesh.path,
-                    texture_ready=ready, geometry_ready=mesh.geometry_ready)
-    return Mesh(verts=mesh.verts, tris=mesh.tris, uvs=mesh.uvs, texture=None, path=mesh.path, texture_ready=ready,
-                geometry_ready=geometry_ready, pages=pages, tri_page=tri_page)
+        return replace(mesh, texture=pages[0], texture_ready=ready)
+    return replace(mesh, texture_ready=ready, geometry_ready=geometry_ready, pages=pages, tri_page=tri_page)
 
 
 def _with_materials(mesh: Mesh, materials, texture_decoder: str, device) -> Mesh | None:
@@ -420,7 +438,7 @@ def load_obj(path: Path | str, load_texture: bool = True, n_threads: int = 0, te
                 textured = _with_device_materials(mesh, *parsed[4], texture_decoder, device)
                 if textured is not None:
                     return textured
-            texture, ready = _load_texture_as(path, texture_decoder, device) if load_texture and uvs is not None \
+            texture, ready = _load_texture(path, texture_decoder, device) if load_texture and uvs is not None \
                 else (None, None)
             return Mesh(verts=verts, tris=tris, uvs=uvs, texture=texture, path=path, texture_ready=ready,
                         geometry_ready=geometry_ready)
@@ -455,14 +473,5 @@ def load_obj(path: Path | str, load_texture: bool = True, n_threads: int = 0, te
         if textured is not None:
             return textured
     if load_texture and uvs is not None:
-        mesh.texture, mesh.texture_ready = _load_texture_as(path, texture_decoder, device)
+        mesh.texture, mesh.texture_ready = _load_texture(path, texture_decoder, device)
     return mesh
-
-
-def _load_texture_as(path: Path, texture_decoder: str, device):
-    """(texture, event recorded after a device-side decode or None)."""
-    if texture_decoder == "nvjpeg":
-        return _decode_texture_nvjpeg(path, device)
-    if texture_decoder == "pil":
-        return _load_texture(path), None
-    raise ValueError(f"Unknown texture decoder: {texture_decoder}")

@@ -8,6 +8,7 @@ import contextlib
 import ctypes as C
 
 import os
+from typing import NamedTuple
 
 import torch
 
@@ -112,12 +113,22 @@ def raster_multiview(verts, uvs, tris, tex, rot, h: int, w: int, channel_mode: s
     return {"u8": out_u8, "f32": f32, "tri": tri, "z": z}
 
 
+class RasterInput(NamedTuple):
+    """One scan of raster_multiscan, cuda tensors as in raster_multiview.  colors: (Nv,4) u8 RGBA per-vertex colours,
+    used in the RGB modes by a scan without a texture.  pages: the int32 (Nt + 3P,) table of
+    mvlm_raster_multiscan_paged (the page of every triangle, then texel offset, height and width of every page), with
+    tex the RGBA texels of all P pages.  render3d.DeviceMesh.raster_input builds it from a scan."""
+    verts: torch.Tensor
+    uvs: torch.Tensor | None
+    tris: torch.Tensor
+    tex: torch.Tensor | None
+    colors: torch.Tensor | None = None
+    pages: torch.Tensor | None = None
+
+
 def raster_multiscan(scans, rot, h: int, w: int, channel_mode: str = "RGB+depth", want_f32: bool = False,
                      want_tri: bool = False, want_z: bool = False, zbuf=None, out_u8=None):
-    """Several scans in one pass.  scans: list of (verts, uvs|None, tris, tex|None[, colors|None[, pages|None]]) cuda
-    tensors as in raster_multiview, colors (Nv,4) u8 RGBA per-vertex colours (used in the RGB modes by a scan without a
-    texture), pages the int32 (Nt + 3P,) page table of mvlm_raster_multiscan_paged (page per triangle, then texel
-    offset, height, width per page) with tex the RGBA texels of all P pages (render3d.DeviceMesh.paged builds both);
+    """Several scans in one pass.  scans: list of RasterInput, or of tuples of its fields in order;
     rot (S*V,9|3,3) f64, scan-major (scan s owns views [s*V, (s+1)*V)).  zbuf: optional persistent workspace (a new
     one is allocated when it is smaller than mvlm_raster_multiscan_workspace_bytes).
     Returns dict(u8=(S*V,H,W,4), f32, tri, z) like raster_multiview; each scan's views equal raster_multiview's."""
@@ -135,20 +146,20 @@ def raster_multiscan(scans, rot, h: int, w: int, channel_mode: str = "RGB+depth"
     rgba = (C.c_void_p * n)()
     paged = (C.c_void_p * n)()
     for i, (e, scan) in enumerate(zip(table, scans)):
-        if len(scan) not in (4, 5, 6):
-            raise ValueError("a scan is (verts, uvs, tris, tex[, colors[, pages]])")
-        verts, uvs, tris, tex = scan[:4]
-        colors = scan[4] if len(scan) >= 5 else None
-        pages = scan[5] if len(scan) == 6 else None
-        if colors is not None and (colors.dtype != torch.uint8 or tuple(colors.shape) != (verts.shape[0], 4)):
-            raise ValueError(f"vertex colours must be ({verts.shape[0]}, 4) uint8 RGBA")
-        if pages is not None and (pages.dtype != torch.int32 or pages.dim() != 1 or pages.numel() < tris.shape[0]
-                                  or (pages.numel() - tris.shape[0]) % 3 or tex is None or tex.shape[-1] != 4):
+        try:
+            s = RasterInput(*scan)
+        except TypeError:
+            raise ValueError("a scan is (verts, uvs, tris, tex[, colors[, pages]])") from None
+        if s.colors is not None and (s.colors.dtype != torch.uint8 or tuple(s.colors.shape) != (s.verts.shape[0], 4)):
+            raise ValueError(f"vertex colours must be ({s.verts.shape[0]}, 4) uint8 RGBA")
+        if s.pages is not None and (s.pages.dtype != torch.int32 or s.pages.dim() != 1
+                                    or s.pages.numel() < s.tris.shape[0] or (s.pages.numel() - s.tris.shape[0]) % 3
+                                    or s.tex is None or s.tex.shape[-1] != 4):
             raise ValueError("pages must be an int32 (Nt + 3P,) table with an RGBA texel buffer as tex")
-        paged[i] = ptr(pages)
-        e.verts, e.n_verts, e.uvs, e.tris, e.n_tris = ptr(verts), verts.shape[0], ptr(uvs), ptr(tris), tris.shape[0]
-        e.tex, (e.tex_h, e.tex_w, e.tex_channels) = ptr(tex), (tex.shape[:3] if tex is not None else (0, 0, 3))
-        rgba[i] = ptr(colors)
+        e.verts, e.n_verts, e.uvs = ptr(s.verts), s.verts.shape[0], ptr(s.uvs)
+        e.tris, e.n_tris = ptr(s.tris), s.tris.shape[0]
+        e.tex, (e.tex_h, e.tex_w, e.tex_channels) = ptr(s.tex), (s.tex.shape[:3] if s.tex is not None else (0, 0, 3))
+        rgba[i], paged[i] = ptr(s.colors), ptr(s.pages)
     need = lib.mvlm_raster_multiscan_workspace_bytes(n, v, h, w, max(s[0].shape[0] for s in scans))
     if zbuf is None or zbuf.numel() * zbuf.element_size() < need:
         zbuf = torch.empty(((need + 7) // 8,), dtype=torch.int64, device=dev)

@@ -100,7 +100,7 @@ def allgather_bytes(array: np.ndarray, device, stage=None, name: str = "a", grou
 
 def upload_mesh_sharded(renderer, mesh, group=None):
     """DeviceMesh of a scan every rank holds in host memory, each rank uploading 1/world of it (allgather_bytes)."""
-    from .utils.render3d import DeviceMesh, _PinnedStage, page_table
+    from .utils.render3d import DeviceMesh, _on_current_stream, _PinnedStage
 
     device = renderer.device
     stage = None
@@ -110,32 +110,18 @@ def upload_mesh_sharded(renderer, mesh, group=None):
         stage = ring[renderer._shard_i % len(ring)]
         if stage.done is not None:
             stage.done.synchronize()  # the slot's previous transfer has left the host buffers
-    def texture(tex, name):
-        if isinstance(tex, torch.Tensor):  # decoded on the device already
-            if mesh.texture_ready is not None:
-                torch.cuda.current_stream().wait_event(mesh.texture_ready)
-            if tex.is_cuda:
-                tex.record_stream(torch.cuda.current_stream())  # decoded on a loader stream: keep its memory until we are done
-            return tex
-        return None if tex is None else allgather_bytes(tex, device, stage, name, group)
-
-    tex_d = texture(mesh.texture, "tex")
-    pages = None if mesh.pages is None else [texture(p, f"page{i}") for i, p in enumerate(mesh.pages)]
-    verts = allgather_bytes(mesh.verts, device, stage, "verts", group)
-    tris = allgather_bytes(mesh.tris, device, stage, "tris", group)
-    uvs = None if mesh.uvs is None else allgather_bytes(mesh.uvs, device, stage, "uvs", group)
-    colors = None if mesh.colors is None else allgather_bytes(mesh.colors, device, stage, "colors", group)
-    tri_page = None if mesh.tri_page is None else allgather_bytes(mesh.tri_page, device, stage, "tri_page", group)
-    table = None if mesh.pages is None else allgather_bytes(page_table(mesh.pages), device, stage, "page_table", group)
+    arrays = {name: _on_current_stream(a, ready) if isinstance(a, torch.Tensor)  # on the device already
+              else allgather_bytes(a, device, stage, name, group) for name, a, ready in mesh.arrays()}
     if stage is not None:
         stage.done = torch.cuda.Event()
         stage.done.record()
-    return DeviceMesh.from_device(mesh, verts, tris, uvs, tex_d, colors, pages, tri_page, table)
+    return DeviceMesh.from_device(mesh, arrays)
 
 
 def _mesh_bytes(mesh) -> int:
-    return sum(a.nbytes for a in (mesh.verts, mesh.tris, mesh.uvs, mesh.texture, mesh.colors, mesh.tri_page,
-                                  *(mesh.pages or ())) if isinstance(a, np.ndarray))
+    """Bytes of the scan's host arrays (Mesh.arrays), the upload that upload_mesh_sharded splits over the ranks; for a
+    scan with texture pages this includes their 12-byte-per-page table."""
+    return sum(a.nbytes for _, a, _ in mesh.arrays() if isinstance(a, np.ndarray))
 
 
 def predict_mesh_view_split(pipeline, mesh, transforms: np.ndarray, group=None) -> np.ndarray:

@@ -94,7 +94,8 @@ class _PinnedStage:
 
 
 def page_table(pages) -> np.ndarray:
-    """(3P,) int32: texel offset, height and width of every page in the packed RGBA buffer of DeviceMesh.paged."""
+    """(3P,) int32: texel offset, height and width of every page in the packed RGBA texels of
+    DeviceMesh.raster_input."""
     table, off = [], 0
     for p in pages:
         table += [off, p.shape[0], p.shape[1]]
@@ -102,21 +103,23 @@ def page_table(pages) -> np.ndarray:
     return np.asarray(table, dtype=np.int32)
 
 
+def _on_current_stream(a: torch.Tensor, ready) -> torch.Tensor:
+    """A device-side array of a scan (decoded or parsed on a loader's side stream) for use on the current stream."""
+    if ready is not None:
+        torch.cuda.current_stream().wait_event(ready)
+    if a.is_cuda:
+        a.record_stream(torch.cuda.current_stream())  # keep its memory until the current stream is done with it
+    return a
+
+
 class DeviceMesh:
-    """Device-resident copy of a Mesh (uploaded once per scan)."""
+    """Device-resident copy of a Mesh (uploaded once per scan): `arrays` maps the names of Mesh.arrays to device
+    tensors; verts, tris, uvs, tex, colors, tri_page, pages and page_table name them (None when absent)."""
 
     def __init__(self, mesh: Mesh, device: torch.device, stage: _PinnedStage | None = None):
-        self.mesh = mesh
-
-        def up(name, a):
-            if a is None:
-                return None
+        def up(name, a, ready):
             if isinstance(a, torch.Tensor):  # decoded (nvJPEG) or parsed (parser="gpu") on the loader's side stream
-                ready = mesh.texture_ready if name == "tex" or name.startswith("page") else mesh.geometry_ready
-                if ready is not None:
-                    torch.cuda.current_stream().wait_event(ready)
-                a.record_stream(torch.cuda.current_stream())
-                return a
+                return _on_current_stream(a, ready)
             a = np.ascontiguousarray(a)
             if device.type != "cuda":
                 return torch.from_numpy(a.copy()).to(device)
@@ -129,43 +132,55 @@ class DeviceMesh:
 
         if stage is not None and stage.done is not None:
             stage.done.synchronize()                          # the slot's previous transfer has left the host buffers
-        self.verts, self.tris = up("verts", mesh.verts), up("tris", mesh.tris)
-        self.uvs, self.tex = up("uvs", mesh.uvs), up("tex", mesh.texture)
-        self.colors = up("colors", mesh.colors)
-        self.pages = None if mesh.pages is None else [up(f"page{i}", p) for i, p in enumerate(mesh.pages)]
-        self.tri_page = up("tri_page", mesh.tri_page)
-        self.page_table = None if mesh.pages is None else up("page_table", page_table(mesh.pages))
+        arrays = {name: up(name, a, ready) for name, a, ready in mesh.arrays()}
         if stage is not None and device.type == "cuda":
             stage.done = torch.cuda.Event()
             stage.done.record()
+        self._wrap(mesh, arrays)
 
     @classmethod
-    def from_device(cls, mesh: Mesh, verts, tris, uvs, tex, colors=None, pages=None, tri_page=None,
-                    page_table=None) -> "DeviceMesh":
-        """Wraps arrays that are on the device already (sharding.upload_mesh_sharded)."""
+    def from_device(cls, mesh: Mesh, arrays: dict) -> "DeviceMesh":
+        """Wraps the device tensors of Mesh.arrays, by name (sharding.upload_mesh_sharded)."""
         self = cls.__new__(cls)
-        self.mesh, self.verts, self.tris, self.uvs, self.tex, self.colors = mesh, verts, tris, uvs, tex, colors
-        self.pages, self.tri_page, self.page_table = pages, tri_page, page_table
+        self._wrap(mesh, arrays)
         return self
 
+    def _wrap(self, mesh: Mesh, arrays: dict) -> None:
+        self.mesh, self.arrays = mesh, arrays
+        self.verts, self.tris, self.uvs, self.tex, self.colors, self.tri_page, self.page_table = \
+            (arrays.get(k) for k in ("verts", "tris", "uvs", "tex", "colors", "tri_page", "page_table"))
+        self.pages = None if mesh.pages is None else [arrays[f"page{i}"] for i in range(len(mesh.pages))]
+
+    def raster_input(self) -> ops.RasterInput:
+        """The scan as ops.raster_multiscan reads it, built once per device mesh: the texture as RGBA (tex4), the
+        vertex colours as (Nv,4) RGBA (one 4-byte load per texel or vertex in the rasteriser), and for a scan with
+        pages, the RGBA texels of all pages packed into one (1, N, 4) u8 buffer (offsets in page_table) as the texture
+        with the int32 (Nt + 3P,) table: the page of every triangle, then page_table."""
+        r = self.__dict__.get("_raster_input")
+        if r is None:
+            tex, table = self.tex4(), None
+            if self.pages is not None:
+                tex = torch.empty((1, sum(p.shape[0] * p.shape[1] for p in self.pages), 4), dtype=torch.uint8,
+                                  device=self.tri_page.device)
+                tex[..., 3] = 255
+                off = 0
+                for p in self.pages:
+                    n = p.shape[0] * p.shape[1]
+                    tex[0, off:off + n, :3] = p.reshape(n, 3)
+                    off += n
+                table = torch.cat([self.tri_page.reshape(-1), self.page_table])
+            colors = None
+            if self.colors is not None:
+                colors = torch.empty((self.colors.shape[0], 4), dtype=torch.uint8, device=self.colors.device)
+                colors[:, :3] = self.colors
+                colors[:, 3] = 255
+            r = self._raster_input = ops.RasterInput(self.verts, self.uvs, self.tris, tex, colors, table)
+        return r
+
     def paged(self):
-        """Texture pages for the rasteriser, packed once per device mesh: (RGBA texels of all pages (1, N, 4) u8, int32
-        (Nt + 3P,) table = the page of every triangle, then texel offset, height and width of every page), or
-        (None, None) for a scan without pages."""
-        if self.pages is None:
-            return None, None
-        t = self.__dict__.get("_paged")
-        if t is None:
-            dev = self.tri_page.device
-            texels = torch.empty((1, sum(p.shape[0] * p.shape[1] for p in self.pages), 4), dtype=torch.uint8, device=dev)
-            texels[..., 3] = 255
-            off = 0
-            for p in self.pages:
-                n = p.shape[0] * p.shape[1]
-                texels[0, off:off + n, :3] = p.reshape(n, 3)
-                off += n
-            t = self._paged = (texels, torch.cat([self.tri_page.reshape(-1), self.page_table]))
-        return t
+        """(packed RGBA texels of all pages, int32 (Nt + 3P,) table) of raster_input, or (None, None) without pages."""
+        r = self.raster_input()
+        return (None, None) if r.pages is None else (r.tex, r.pages)
 
     def tex4(self):
         """The texture as RGBA (one 4-byte load per texel in the rasteriser), expanded once per device mesh."""
@@ -182,19 +197,6 @@ class DeviceMesh:
             self._tex4 = t
         return t
 
-    def colors4(self):
-        """The per-vertex colours as (Nv,4) RGBA (one 4-byte load per vertex in the rasteriser), expanded once per device
-        mesh; None without colours."""
-        if self.colors is None:
-            return None
-        c = self.__dict__.get("_colors4")
-        if c is None:
-            c = torch.empty((self.colors.shape[0], 4), dtype=torch.uint8, device=self.colors.device)
-            c[:, :3] = self.colors
-            c[:, 3] = 255
-            self._colors4 = c
-        return c
-
     def snap_grid(self):
         """Spatial index for the surface snap, built at most once per device mesh (None below ops.SNAP_GRID_MIN_TRIS,
         where the brute-force scan is faster than building the grid)."""
@@ -204,9 +206,7 @@ class DeviceMesh:
 
     @property
     def h2d_bytes(self) -> int:
-        return sum(t.numel() * t.element_size()
-                   for t in (self.verts, self.tris, self.uvs, self.tex, self.colors, self.tri_page, *(self.pages or ()))
-                   if t is not None)
+        return sum(t.numel() * t.element_size() for t in self.arrays.values())
 
 
 class ObjRenderer3D:
@@ -315,11 +315,7 @@ class ObjRenderer3D:
         if self._zbuf is None or self._zbuf.numel() * 8 < need:
             n = lib.mvlm_raster_multiscan_workspace_bytes(len(dmeshes), total // len(dmeshes), h, w, int(max_nv * 1.25))
             self._zbuf = torch.empty(((n + 7) // 8,), dtype=torch.int64, device=self.device)
-        scans = []
-        for d in dmeshes:
-            texels, pages = d.paged()
-            scans.append((d.verts, d.uvs, d.tris, d.tex4() if pages is None else texels, d.colors4(), pages))
-        return ops.raster_multiscan(scans, rot, h, w, self.channel_mode,
+        return ops.raster_multiscan([d.raster_input() for d in dmeshes], rot, h, w, self.channel_mode,
                                     want_f32=want_f32, want_tri=want_tri, want_z=want_z, zbuf=self._zbuf,
                                     out_u8=self._u8[:total])
 

@@ -61,6 +61,6 @@ def load_obj_python(path: Path | str, load_texture: bool = True) -> Mesh:
         verts = pos[uniq[:, 0]]
         uvs = np.where(uniq[:, 1:2] >= 0, tex[np.clip(uniq[:, 1], 0, None)], 0.0).astype(np.float32)
         tris = inv.reshape(-1, 3).astype(np.int32)
-    texture = _load_texture(path) if (load_texture and uvs is not None) else None
+    texture = _load_texture(path)[0] if (load_texture and uvs is not None) else None
     return Mesh(verts=np.ascontiguousarray(verts), tris=np.ascontiguousarray(tris),
                 uvs=None if uvs is None else np.ascontiguousarray(uvs), texture=texture, path=path)
