@@ -10,18 +10,16 @@
 //
 // ASCII bodies are split at line boundaries into one chunk per thread and each chunk is converted with std::from_chars
 // (correctly rounded, like the OBJ loader) before one serial pass interprets the values.
-#include <algorithm>
 #include <charconv>
 #include <cmath>
-#include <cstdio>
 #include <cstdlib>
 #include <cstring>
 #include <string>
-#include <thread>
 #include <vector>
 
 #include "../../include/mvlm_b200.h"
 #include "common.cuh"
+#include "host_text.cuh"
 #include "mesh_format.cuh"
 
 struct mvlm_mesh {
@@ -158,44 +156,7 @@ namespace {
 
 using namespace mesh;
 
-inline bool parse_double(const char*& p, const char* end, double* out) {
-  while (p < end && (*p == ' ' || *p == '\t' || *p == '\r')) ++p;
-  if (p < end && *p == '+') ++p;
-  const auto r = std::from_chars(p, end, *out);
-  if (r.ec != std::errc()) return false;
-  p = r.ptr;
-  return true;
-}
-
 inline bool is_space(char c) { return c == ' ' || c == '\t' || c == '\r' || c == '\n'; }
-
-// line-aligned chunks of [begin, end), one per thread
-std::vector<const char*> line_cuts(const char* begin, const char* end, int n_threads) {
-  const size_t n = static_cast<size_t>(end - begin);
-  if (n < (1u << 16)) n_threads = 1;
-  std::vector<const char*> cuts(static_cast<size_t>(n_threads) + 1);
-  cuts[0] = begin;
-  for (int i = 1; i < n_threads; ++i) {
-    const char* p = begin + n * static_cast<size_t>(i) / static_cast<size_t>(n_threads);
-    if (p < cuts[static_cast<size_t>(i) - 1]) p = cuts[static_cast<size_t>(i) - 1];
-    const char* nl = p < end ? static_cast<const char*>(memchr(p, '\n', static_cast<size_t>(end - p))) : nullptr;
-    cuts[static_cast<size_t>(i)] = nl ? nl + 1 : end;
-  }
-  cuts[static_cast<size_t>(n_threads)] = end;
-  return cuts;
-}
-
-template <class T, class F>
-std::vector<T> parallel_chunks(const char* begin, const char* end, int n_threads, F&& fn) {
-  const std::vector<const char*> cuts = line_cuts(begin, end, n_threads);
-  const size_t k = cuts.size() - 1;
-  std::vector<T> out(k);
-  std::vector<std::thread> th;
-  for (size_t i = 1; i < k; ++i) th.emplace_back([&, i] { fn(cuts[i], cuts[i + 1], &out[i]); });
-  fn(cuts[0], cuts[1], &out[0]);
-  for (auto& t : th) t.join();
-  return out;
-}
 
 // ---- PLY body readers ------------------------------------------------------------------------------------------------
 struct BinReader {
@@ -511,18 +472,11 @@ int mvlm_mesh_load(const char* path, int n_threads, mvlm_mesh** out) {
   *out = nullptr;
   const bool ply = has_suffix(path, ".ply"), stl = has_suffix(path, ".stl");
   MVLM_REQUIRE(ply || stl, "mvlm_mesh_load: %s is not a .ply or .stl file", path);
-  FILE* fh = fopen(path, "rb");
-  MVLM_REQUIRE(fh != nullptr, "File %s does not exist.", path);
-  fseek(fh, 0, SEEK_END);
-  const long size = ftell(fh);
-  fseek(fh, 0, SEEK_SET);
-  std::string buf(static_cast<size_t>(size > 0 ? size : 0), '\0');
-  const size_t got = size > 0 ? fread(&buf[0], 1, static_cast<size_t>(size), fh) : 0;
-  fclose(fh);
-  MVLM_REQUIRE(static_cast<long>(got) == size, "mvlm_mesh_load: short read on %s", path);
-  if (n_threads <= 0) n_threads = static_cast<int>(std::min(16u, std::max(1u, std::thread::hardware_concurrency())));
+  std::string buf;
+  int rc = read_file(path, "mvlm_mesh_load", &buf);
+  if (rc != MVLM_OK) return rc;
   mvlm_mesh* m = new mvlm_mesh();
-  const int rc = ply ? load_ply(buf, path, n_threads, m) : load_stl(buf, path, n_threads, m);
+  rc = ply ? load_ply(buf, path, n_threads, m) : load_stl(buf, path, n_threads, m);
   if (rc != MVLM_OK) {
     delete m;
     return rc;

@@ -9,8 +9,8 @@
 //
 // At ~50 scans/s on the GPU the text parse is the bottleneck of predict_one_file(path) (6 MB of text per
 // scan; 1.05 s in numpy): the file is split at line boundaries into one chunk per thread, every chunk is
-// parsed independently (std::from_chars: correctly rounded like Python's float()), and the chunks are
-// concatenated in file order.
+// parsed independently (std::from_chars: correctly rounded like Python's float(); both in host_text.cuh), and
+// the chunks are concatenated in file order.
 //
 // With MVLM_OBJ_MATERIALS (mvlm_obj_load_ex) the loader also keeps the `mtllib` names, the distinct `usemtl` names in
 // order of first appearance, and every triangle's material ordinal (the last `usemtl` before its `f` line; -1 before
@@ -18,16 +18,15 @@
 // a chunk's triangles before its first `usemtl` inherit the last one of the chunks before it (DESIGN.md 7g).
 #include <algorithm>
 #include <charconv>
-#include <cstdio>
 #include <cstdlib>
 #include <cstring>
 #include <string>
-#include <thread>
 #include <unordered_map>
 #include <vector>
 
 #include "../../include/mvlm_b200.h"
 #include "common.cuh"
+#include "host_text.cuh"
 
 namespace mvlm {
 namespace {
@@ -47,20 +46,6 @@ struct Chunk {
   std::vector<std::string> usemtl, mtllib;
   std::vector<int> mat_local;
 };
-
-inline const char* skip_ws(const char* p, const char* end) {
-  while (p < end && (*p == ' ' || *p == '\t' || *p == '\r')) ++p;
-  return p;
-}
-
-inline bool parse_double(const char*& p, const char* end, double* out) {
-  p = skip_ws(p, end);
-  if (p < end && *p == '+') ++p;  // from_chars rejects a leading '+', Python's float() accepts it
-  auto r = std::from_chars(p, end, *out);
-  if (r.ec != std::errc()) return false;
-  p = r.ptr;
-  return true;
-}
 
 // the rest of a `usemtl` / `mtllib` line, trimmed of blanks and a CR
 inline std::string rest_trimmed(const char* p, const char* end) {
@@ -152,26 +137,6 @@ void parse_chunk(const char* begin, const char* end, Chunk* c) {
   }
 }
 
-int chunk_count(size_t size, int n_threads) {
-  if (n_threads <= 0) n_threads = static_cast<int>(std::min(16u, std::max(1u, std::thread::hardware_concurrency())));
-  return size < (1u << 16) ? 1 : n_threads;
-}
-
-// chunk boundaries at line starts: cuts[0] = base, cuts[n] = end
-std::vector<const char*> chunk_cuts(const char* base, const char* end, int n_threads) {
-  const size_t size = static_cast<size_t>(end - base);
-  std::vector<const char*> cuts(static_cast<size_t>(n_threads) + 1);
-  cuts[0] = base;
-  for (int i = 1; i < n_threads; ++i) {
-    const char* p = base + size * static_cast<size_t>(i) / static_cast<size_t>(n_threads);
-    if (p < cuts[static_cast<size_t>(i) - 1]) p = cuts[static_cast<size_t>(i) - 1];
-    const char* nl = p < end ? static_cast<const char*>(memchr(p, '\n', static_cast<size_t>(end - p))) : nullptr;
-    cuts[static_cast<size_t>(i)] = nl ? nl + 1 : end;
-  }
-  cuts[static_cast<size_t>(n_threads)] = end;
-  return cuts;
-}
-
 }  // namespace
 }  // namespace mvlm
 
@@ -195,28 +160,12 @@ int mvlm_obj_load_ex(const char* path, int n_threads, int flags, mvlm_obj** out)
   MVLM_REQUIRE((flags & ~MVLM_OBJ_MATERIALS) == 0, "mvlm_obj_load_ex: unknown flags 0x%x", flags);
   const bool materials = (flags & MVLM_OBJ_MATERIALS) != 0;
   *out = nullptr;
-  FILE* fh = fopen(path, "rb");
-  MVLM_REQUIRE(fh != nullptr, "File %s does not exist.", path);
-  fseek(fh, 0, SEEK_END);
-  const long size = ftell(fh);
-  fseek(fh, 0, SEEK_SET);
-  std::string buf(static_cast<size_t>(size > 0 ? size : 0), '\0');
-  const size_t got = size > 0 ? fread(&buf[0], 1, static_cast<size_t>(size), fh) : 0;
-  fclose(fh);
-  MVLM_REQUIRE(static_cast<long>(got) == size, "mvlm_obj_load: short read on %s", path);
-  const char* base = buf.data();
-  const char* end = base + buf.size();
-  n_threads = chunk_count(buf.size(), n_threads);
-  const std::vector<const char*> cuts = chunk_cuts(base, end, n_threads);
-  std::vector<Chunk> chunks(static_cast<size_t>(n_threads));
-  for (Chunk& c : chunks) c.materials = materials;
-  {
-    std::vector<std::thread> th;
-    for (int i = 1; i < n_threads; ++i)
-      th.emplace_back(parse_chunk, cuts[static_cast<size_t>(i)], cuts[static_cast<size_t>(i) + 1], &chunks[static_cast<size_t>(i)]);
-    parse_chunk(cuts[0], cuts[1], &chunks[0]);
-    for (auto& t : th) t.join();
-  }
+  std::string buf;
+  const int rc = read_file(path, "mvlm_obj_load", &buf);
+  if (rc != MVLM_OK) return rc;
+  const std::vector<Chunk> chunks = parallel_chunks<Chunk>(
+      buf.data(), buf.data() + buf.size(), n_threads,
+      [materials](const char* b, const char* e, Chunk* c) { c->materials = materials; parse_chunk(b, e, c); });
   size_t n_pos = 0, n_tex = 0, n_tri = 0;
   for (const Chunk& c : chunks) {
     MVLM_REQUIRE(!c.bad, "mvlm_obj_load: malformed v / vt / f line in %s", path);
@@ -369,10 +318,9 @@ void mvlm_obj_free(mvlm_obj* obj) { delete obj; }
 
 int mvlm_debug_obj_chunk_starts(const char* text, size_t len, int n_threads, long long* starts) {
   MVLM_REQUIRE((text || len == 0) && starts, "mvlm_debug_obj_chunk_starts: null pointer");
-  const int n = chunk_count(len, n_threads);
-  const std::vector<const char*> cuts = chunk_cuts(text, text + len, n);
-  for (int i = 0; i < n; ++i) starts[i] = cuts[static_cast<size_t>(i)] - text;
-  return n;
+  const std::vector<const char*> cuts = line_cuts(text, text + len, n_threads);
+  for (size_t i = 0; i + 1 < cuts.size(); ++i) starts[i] = cuts[i] - text;
+  return static_cast<int>(cuts.size()) - 1;
 }
 
 }  // extern "C"

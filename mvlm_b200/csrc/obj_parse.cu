@@ -324,7 +324,7 @@ HD int from_chars_double(const char*& p, const char* end, double* out) {
   return kOk;
 }
 
-// obj_loader.cu parse_double: whitespace, one optional '+', from_chars
+// host_text.cuh parse_double: whitespace, one optional '+', from_chars
 HD int parse_double(const char*& p, const char* end, double* out) {
   while (p < end && is_ws(*p)) ++p;
   if (p < end && *p == '+') ++p;

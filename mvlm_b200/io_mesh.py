@@ -11,7 +11,7 @@ from pathlib import Path
 
 import numpy as np
 
-from .io_obj import Mesh, check_texture_source, load_obj, loader_state, read_pinned
+from .io_obj import Mesh, check_texture_source, decode_on_device, load_obj, read_pinned
 
 SUFFIXES = {"obj": ".obj", "ply": ".ply", "stl": ".stl"}
 
@@ -47,6 +47,14 @@ def check_scan_file(path: Path, scan_formats) -> None:
     raise ValueError(f"File {path} is not a scan file. Only {names} files are supported.")
 
 
+def check_scan_path(path: Path, scan_formats) -> None:
+    """check_scan_file for an existing path that is about to be loaded, after a FileNotFoundError when it is not a
+    regular file.  A missing path is the caller's to handle."""
+    if not path.is_file():
+        raise FileNotFoundError(f"File {path} is not a file")
+    check_scan_file(path, scan_formats)
+
+
 def parse_mesh_device(path: Path, device):
     """parser="gpu" for a PLY / STL file: the bytes are read into the calling thread's page-locked buffer and decoded
     by csrc/mesh_parse.cu on the thread's side stream.  Returns (verts, colors | None, tris, event recorded after the
@@ -64,30 +72,21 @@ def parse_mesh_device(path: Path, device):
     ws_bytes = lib.mvlm_mesh_parse_workspace_bytes(n, is_stl)
     if ws_bytes == 0:
         return None
-    device = torch.device(device)
     host = read_pinned(path, device)
-    st = loader_state(device)
-    with torch.cuda.device(device), torch.cuda.stream(st.stream):
-        if st.workspace is None or st.workspace.numel() < ws_bytes:
-            st.workspace = None
-            st.workspace = torch.empty((ws_bytes,), dtype=torch.uint8, device=device)
-        info = _lib.MeshParseInfo()
-        # synchronises the side stream (the output sizes come back to the host, and the page-locked buffer is free
-        # for the next file); the main stream never waits
-        if lib.mvlm_mesh_parse_device(host.data_ptr(), n, is_stl, str(path).encode(), st.workspace.data_ptr(), ws_bytes,
-                                      st.stream.cuda_stream, C.byref(info)) != 0:
-            raise ValueError(lib.mvlm_last_error().decode("utf-8", "replace"))
-        if info.fallback:
-            return None
+    info = _lib.MeshParseInfo()
+
+    def outputs(ws, stream):
         verts = torch.empty((info.n_verts, 3), dtype=torch.float32, device=device)
         tris = torch.empty((info.n_tris, 3), dtype=torch.int32, device=device)
         colors = torch.empty((info.n_verts, 3), dtype=torch.uint8, device=device) if info.has_colors else None
-        _lib.check(lib.mvlm_mesh_parse_write(C.byref(info), st.workspace.data_ptr(), verts.data_ptr(),
-                                             None if colors is None else colors.data_ptr(), tris.data_ptr(),
-                                             st.stream.cuda_stream), "mvlm_mesh_parse_write")
-        ready = torch.cuda.Event(enable_timing=True)
-        ready.record(st.stream)
-    return verts, colors, tris, ready
+        _lib.check(lib.mvlm_mesh_parse_write(C.byref(info), ws, verts.data_ptr(),
+                                             None if colors is None else colors.data_ptr(), tris.data_ptr(), stream),
+                   "mvlm_mesh_parse_write")
+        return verts, colors, tris
+
+    # once phase 1 returns (it synchronises the side stream), the page-locked buffer is free for the next file
+    return decode_on_device(device, ws_bytes, info, lambda ws, stream: lib.mvlm_mesh_parse_device(
+        host.data_ptr(), n, is_stl, str(path).encode(), ws, ws_bytes, stream, C.byref(info)), outputs)
 
 
 def load_ply_stl(path: Path | str, n_threads: int = 0, device="cuda", parser: str = "host") -> Mesh:

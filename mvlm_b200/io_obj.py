@@ -159,6 +159,40 @@ def loader_state(device):
     return _tls
 
 
+def _grown(st, name: str, n: int, **alloc):
+    """The loader state's uint8 buffer `name` (pinned, text, workspace), reallocated with max(n, 1) bytes when it holds
+    fewer than n.  The old buffer is dropped first, so that a large file can reuse its memory."""
+    import torch
+
+    if getattr(st, name) is None or getattr(st, name).numel() < n:
+        setattr(st, name, None)
+        setattr(st, name, torch.empty((max(n, 1),), dtype=torch.uint8, **alloc))
+    return getattr(st, name)
+
+
+def decode_on_device(device, ws_bytes: int, info, phase1, phase2):
+    """Runs a two-phase device decoder (csrc/obj_parse.cu, csrc/mesh_parse.cu) on the calling thread's side stream.
+    phase1(workspace, stream) fills `info` and returns the status (it synchronises the side stream; the main stream
+    never waits); phase2(workspace, stream) allocates and writes the outputs.  Returns phase2's tuple + (event behind
+    the outputs,), None on info.fallback (the host loader reads the file), or raises ValueError when phase 1 fails."""
+    import torch
+
+    from . import _lib
+
+    device = torch.device(device)
+    st = loader_state(device)
+    with torch.cuda.device(device), torch.cuda.stream(st.stream):
+        ws = _grown(st, "workspace", ws_bytes, device=device).data_ptr()
+        if phase1(ws, st.stream.cuda_stream) != 0:
+            raise ValueError(_lib.load().mvlm_last_error().decode("utf-8", "replace"))
+        if info.fallback:
+            return None
+        out = phase2(ws, st.stream.cuda_stream)
+        ready = torch.cuda.Event(enable_timing=True)
+        ready.record(st.stream)
+    return out + (ready,)
+
+
 def _decode_jpeg_nvjpeg(jpg: Path, device):
     """One JPEG file -> (Th,Tw,3) uint8 CUDA tensor + the event recorded behind the decode, or (None, None) when it is
     missing or unreadable (mvlm_jpeg_decode_rgb on a per-thread side stream: the loader threads of
@@ -191,14 +225,9 @@ def _decode_jpeg_nvjpeg(jpg: Path, device):
 def read_pinned(path: Path, device):
     """The bytes of `path` in the calling thread's page-locked buffer (grown to the largest file read): a uint8 tensor
     view of exactly the file's size."""
-    import torch
-
-    st = loader_state(device)
     n = path.stat().st_size
-    if st.pinned is None or st.pinned.numel() < n:
-        st.pinned = None
-        st.pinned = torch.empty((max(n, 1),), dtype=torch.uint8, pin_memory=True)
-    view = memoryview(st.pinned.numpy())[:n]
+    pinned = _grown(loader_state(device), "pinned", n, pin_memory=True)
+    view = memoryview(pinned.numpy())[:n]
     got = 0
     with open(path, "rb", buffering=0) as fh:
         while got < n:
@@ -208,7 +237,7 @@ def read_pinned(path: Path, device):
             got += k
     if got != n:
         raise ValueError(f"mvlm_obj_load: short read on {path}")
-    return st.pinned[:n]
+    return pinned[:n]
 
 
 def parse_obj_device(text, path: Path, device):
@@ -230,41 +259,35 @@ def _parse_device(text, path: Path, device, materials: bool = False):
     from . import _lib
 
     lib = _lib.load()
-    device = torch.device(device)
-    st = loader_state(device)
     n = text.numel()
     flags = _lib.OBJ_MATERIALS if materials else 0
     ws_bytes = lib.mvlm_obj_parse_workspace_bytes_ex(n, flags)
     if ws_bytes == 0:
         return None
-    with torch.cuda.device(device), torch.cuda.stream(st.stream):
-        if st.workspace is None or st.workspace.numel() < ws_bytes:
-            st.workspace = None
-            st.workspace = torch.empty((ws_bytes,), dtype=torch.uint8, device=device)
-        info = _lib.ObjParseInfo()
-        lines, n_lines = None, C.c_int()
-        if materials:
-            if getattr(st, "name_lines", None) is None:
-                st.name_lines = (_lib.ObjNameLine * _lib.OBJ_MAX_NAME_LINES)()
-            lines = st.name_lines
-        # synchronises the side stream (the sizes of the outputs come back to the host); the main stream never waits
-        if lib.mvlm_obj_parse_device_ex(text.data_ptr(), n, str(path).encode(), st.workspace.data_ptr(), ws_bytes,
-                                        flags, st.stream.cuda_stream, C.byref(info), lines,
-                                        _lib.OBJ_MAX_NAME_LINES if materials else 0, C.byref(n_lines)) != 0:
-            raise ValueError(lib.mvlm_last_error().decode("utf-8", "replace"))
-        if info.fallback:
-            return None
+    info, lines, n_lines = _lib.ObjParseInfo(), None, C.c_int()
+    if materials:
+        st = loader_state(device)
+        if getattr(st, "name_lines", None) is None:
+            st.name_lines = (_lib.ObjNameLine * _lib.OBJ_MAX_NAME_LINES)()
+        lines = st.name_lines
+
+    def outputs(ws, stream):
         verts = torch.empty((info.n_verts, 3), dtype=torch.float32, device=device)
         tris = torch.empty((info.n_tris, 3), dtype=torch.int32, device=device)
         uvs = torch.empty((info.n_verts, 2), dtype=torch.float32, device=device) if info.has_uv else None
-        _lib.check(lib.mvlm_obj_parse_write(C.byref(info), st.workspace.data_ptr(), verts.data_ptr(),
-                                            None if uvs is None else uvs.data_ptr(), tris.data_ptr(),
-                                            st.stream.cuda_stream), "mvlm_obj_parse_write")
-        ready = torch.cuda.Event(enable_timing=True)
-        ready.record(st.stream)
+        _lib.check(lib.mvlm_obj_parse_write(C.byref(info), ws, verts.data_ptr(),
+                                            None if uvs is None else uvs.data_ptr(), tris.data_ptr(), stream),
+                   "mvlm_obj_parse_write")
+        return verts, uvs, tris
+
+    parsed = decode_on_device(device, ws_bytes, info, lambda ws, stream: lib.mvlm_obj_parse_device_ex(
+        text.data_ptr(), n, str(path).encode(), ws, ws_bytes, flags, stream, C.byref(info), lines,
+        _lib.OBJ_MAX_NAME_LINES if materials else 0, C.byref(n_lines)), outputs)
+    if parsed is None:
+        return None
     extra = (info, [(lines[i].offset, lines[i].kind, lines[i].tris_before) for i in range(n_lines.value)]) \
         if materials else None
-    return verts, uvs, tris, ready, extra
+    return parsed + (extra,)
 
 
 def _load_geometry_gpu(path: Path, device, materials: bool = False):
@@ -280,11 +303,7 @@ def _load_geometry_gpu(path: Path, device, materials: bool = False):
     host = read_pinned(path, device)
     st = loader_state(device)
     with torch.cuda.device(device), torch.cuda.stream(st.stream):
-        n = host.numel()
-        if st.text is None or st.text.numel() < n:
-            st.text = None
-            st.text = torch.empty((max(n, 1),), dtype=torch.uint8, device=device)
-        text = st.text[:n]
+        text = _grown(st, "text", host.numel(), device=device)[:host.numel()]
         text.copy_(host, non_blocking=True)
     parsed = _parse_device(text, path, device, materials)
     if parsed is None or not materials:

@@ -19,7 +19,7 @@ import numpy as np
 import torch
 
 from .. import _lib
-from ..io_mesh import SUFFIXES, check_scan_file, check_scan_formats, is_scan_file, load_mesh
+from ..io_mesh import SUFFIXES, check_scan_file, check_scan_formats, check_scan_path, is_scan_file, load_mesh
 from ..io_obj import Mesh, check_texture_source
 from ..prediction.paulsenpredictor import PaulsenModel
 from ..utils import Estimator3D, ObjRenderer3D, prealign
@@ -167,9 +167,7 @@ class Pipeline(abc.ABC, TimeMixin):
                      and self.predictor_2d.selection_method in ("simple", "moment"))
             if fused:
                 r = self.renderer_3d
-                if not file_name.is_file():
-                    raise FileNotFoundError(f"File {file_name} is not a file")
-                check_scan_file(file_name, self.scan_formats)
+                check_scan_path(file_name, self.scan_formats)
                 self.tic()
                 mesh = load_mesh(file_name, texture_decoder=self.texture_decoder, device=self.device,
                                  parser=self.obj_parser, texture_source=self.texture_source)
@@ -194,9 +192,7 @@ class Pipeline(abc.ABC, TimeMixin):
             def load(f: Path):
                 if not f.exists():
                     return None
-                if not f.is_file():
-                    raise FileNotFoundError(f"File {f} is not a file")
-                check_scan_file(f, self.scan_formats)
+                check_scan_path(f, self.scan_formats)
                 # four parser threads per scan: with more, the loaders of `prefetch` scans oversubscribe the host and the
                 # thread that feeds the GPU gets descheduled (measured on the 16-core box: 36 scans/s with 16, 51 with 4)
                 return load_mesh(f, n_threads=4, texture_decoder=self.texture_decoder, device=self.device,

@@ -14,7 +14,7 @@ import numpy as np
 import torch
 
 from .. import ops
-from ..io_mesh import check_scan_file, load_mesh
+from ..io_mesh import check_scan_path, load_mesh
 from ..io_obj import Mesh
 
 __all__ = ["ObjRenderer3D", "ObjVTKRenderer3D", "fixed_eight_views", "rotation_matrices"]
@@ -346,9 +346,7 @@ class ObjRenderer3D:
         file_name = Path(file_name)
         if not file_name.exists():
             raise FileNotFoundError(f"File {file_name} does not exist")
-        if not file_name.is_file():
-            raise FileNotFoundError(f"File {file_name} is not a file")
-        check_scan_file(file_name, self.scan_formats)
+        check_scan_path(file_name, self.scan_formats)
         if self.verbose:
             print("Render [0] - Prepare", f"{time.time() - t:08.6f} s")
         transformation_stack = self.generate_3d_transformations()

@@ -7,7 +7,7 @@ import pytest
 
 import mesh_ref
 from mvlm_b200 import synth
-from mvlm_b200.io_mesh import check_scan_file, is_scan_file, load_mesh, load_ply_stl
+from mvlm_b200.io_mesh import check_scan_file, check_scan_path, is_scan_file, load_mesh, load_ply_stl
 
 
 def _same(a, b):
@@ -248,6 +248,11 @@ def test_load_mesh_dispatch_and_scan_file_checks(lib, tmp_path, face):
         check_scan_file(Path("a.ply"), ("obj",))
     with pytest.raises(ValueError, match="Only .obj, .ply, .stl files are supported"):
         check_scan_file(Path("a.wrl"), ("obj", "ply", "stl"))
+    check_scan_path(tmp_path / "A.STL", ("obj", "stl"))
+    with pytest.raises(ValueError, match=r"^File .*A.STL is not an .obj file. Only .obj files are supported.$"):
+        check_scan_path(tmp_path / "A.STL", ("obj",))
+    with pytest.raises(FileNotFoundError, match=r"^File .* is not a file$"):
+        check_scan_path(tmp_path, ("obj",))  # checked before the suffix
 
 
 def test_mesh_symbols_and_info_layout(lib):
