@@ -35,23 +35,6 @@ int sm_count() {
   return n;
 }
 
-__global__ void pack_conv_weight_kernel(const float* __restrict__ w, int cout, int cin, int kh, int kw,
-                                        int cout_pad, int cin_pad, __nv_bfloat16* __restrict__ out) {
-  const long long total = 1ll * cout_pad * kw * kh * cin_pad;
-  for (long long i = blockIdx.x * 1ll * blockDim.x + threadIdx.x; i < total;
-       i += 1ll * gridDim.x * blockDim.x) {
-    const int ci = static_cast<int>(i % cin_pad);
-    long long r = i / cin_pad;
-    const int ky = static_cast<int>(r % kh);
-    r /= kh;
-    const int kx = static_cast<int>(r % kw);
-    const int co = static_cast<int>(r / kw);
-    float v = 0.f;
-    if (co < cout && ci < cin) v = w[((1ll * co * cin + ci) * kh + ky) * kw + kx];
-    out[i] = __float2bfloat16_rn(v);
-  }
-}
-
 }  // namespace mvlm
 
 using namespace mvlm;
@@ -104,14 +87,10 @@ int mvlm_pack_conv_weight(const float* w_oihw, int cout, int cin, int kh, int kw
                           void* out_bf16, void* stream) {
   MVLM_REQUIRE(w_oihw && out_bf16, "mvlm_pack_conv_weight: null pointer");
   MVLM_REQUIRE(cout_pad >= cout && cin_pad >= cin, "mvlm_pack_conv_weight: pads smaller than dims");
-  const long long total = 1ll * cout_pad * kw * kh * cin_pad;
-  const int block = 256;
-  const int grid = static_cast<int>((total + block - 1) / block > 4096 ? 4096 : (total + block - 1) / block);
-  pack_conv_weight_kernel<<<grid, block, 0, static_cast<cudaStream_t>(stream)>>>(
-      w_oihw, cout, cin, kh, kw, cout_pad, cin_pad, static_cast<__nv_bfloat16*>(out_bf16));
+  const int rc = pack_conv_weight(w_oihw, cout, cin, kh, kw, cout_pad, cin_pad, static_cast<__nv_bfloat16*>(out_bf16),
+                                  static_cast<cudaStream_t>(stream));
   count_launch();
-  MVLM_CHECK_CUDA(cudaGetLastError());
-  return MVLM_OK;
+  return rc;
 }
 
 size_t mvlm_raster_workspace_bytes(int n_views, int h, int w, int n_verts) {

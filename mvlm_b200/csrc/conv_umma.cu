@@ -30,8 +30,6 @@
 // MMAs of tile i+1.
 #include "conv_epilogue.cuh"
 
-#include <stdlib.h>
-
 #include <algorithm>
 #include <type_traits>
 #include <atomic>
@@ -490,9 +488,6 @@ EncodeTiledFn get_encode_fn() {
   return fn;
 }
 
-// programmatic dependent launch of consecutive conv kernels (MVLM_CONV_NO_PDL=1 switches it off)
-const bool g_pdl = getenv("MVLM_CONV_NO_PDL") == nullptr;
-
 template <int F>
 int launch_t(const ConvParams& p, cudaStream_t stream) {
   // the attribute is per device (and per kernel instantiation): one flag per device ordinal
@@ -510,9 +505,10 @@ int launch_t(const ConvParams& p, cudaStream_t stream) {
   cfg.blockDim = dim3(kThreads);
   cfg.dynamicSmemBytes = kSmemBytes;
   cfg.stream = stream;
+  // programmatic dependent launch of consecutive conv kernels
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = g_pdl ? 1 : 0;
+  attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
   MVLM_CHECK_CUDA(cudaLaunchKernelEx(&cfg, conv_umma_kernel<F>, p));
@@ -584,12 +580,8 @@ int conv_plan(const ConvShape& s, const ConvEpilogue& e, ConvParams* out) {
     // conv11 phase kernels: 8 x 10 KB; the 64 -> 128 resample)
     const bool fits_128 = m_tile == kMTile && s.cout_pad <= kMTile && n_wtiles <= kMaxWSlots &&
                           nh * p.h_slot_bytes + n_wtiles * wslot <= kPoolBytes;
-    p.w_stationary = ((m_tile == 64 ? n_wtiles * wslot <= kMaxWSlots * 8192 : fits_128) && getenv("MVLM_CONV_NO_STATIONARY") == nullptr) ? 1 : 0;
+    p.w_stationary = (m_tile == 64 ? n_wtiles * wslot <= kMaxWSlots * 8192 : fits_128) ? 1 : 0;
     if (p.w_stationary) nw = n_wtiles;
-    if (const char* env = getenv("MVLM_CONV_RING")) {  // experiment knob: "halo_slots,weight_slots"
-      int a = 0, b = 0;
-      if (sscanf(env, "%d,%d", &a, &b) == 2 && a >= 2 && a <= kMaxHSlots && b >= 2 && b <= kMaxWSlots && !p.w_stationary) { nh = a; nw = b; }
-    }
     while (nh * p.h_slot_bytes + nw * wslot > kPoolBytes && nw > 2 && !p.w_stationary) --nw;
     while (nh * p.h_slot_bytes + nw * wslot > kPoolBytes && nh > 2) --nh;
     MVLM_REQUIRE(nh * p.h_slot_bytes + nw * wslot <= kPoolBytes, "conv_plan: operand rings do not fit");

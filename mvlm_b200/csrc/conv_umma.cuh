@@ -102,6 +102,10 @@ struct alignas(64) ConvParams {
 int conv_plan(const ConvShape& s, const ConvEpilogue& e, ConvParams* out);
 // Launches the persistent kernel for a planned conv.
 int conv_launch(const ConvParams& p, cudaStream_t stream);
+// OIHW fp32 weights -> the packed layout above, [cout_pad][kw][kh][cin_pad] bf16 with zero rows / channels past
+// cout / cin (hourglass.cu).  Counts no launch: the plan build's packing is not part of a forward pass.
+int pack_conv_weight(const float* w_oihw, int cout, int cin, int kh, int kw, int cout_pad, int cin_pad,
+                     __nv_bfloat16* out, cudaStream_t stream);
 // Debug: when non-null, the next conv_launch calls record role timings there (148 x 8 int64) followed by the
 // per-tile timeline of CTA 0 (kConvTraceTiles x 16 int64, see conv_umma.cu).
 constexpr int kConvTraceTiles = 64;

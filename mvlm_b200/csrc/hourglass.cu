@@ -35,18 +35,19 @@ __global__ void fold_bn_kernel(const float* w, const float* b, const float* m, c
 }
 
 // OIHW fp32 -> [cout_pad][kw][kh][cin_pad] bf16
-__global__ void pack_weight_kernel(const float* __restrict__ w, int cout, int cin, int k, int cout_pad, int cin_pad,
-                                   __nv_bfloat16* __restrict__ out) {
-  const long long total = 1ll * cout_pad * k * k * cin_pad;
-  for (long long i = blockIdx.x * 1ll * blockDim.x + threadIdx.x; i < total; i += 1ll * gridDim.x * blockDim.x) {
+__global__ void pack_conv_weight_kernel(const float* __restrict__ w, int cout, int cin, int kh, int kw,
+                                        int cout_pad, int cin_pad, __nv_bfloat16* __restrict__ out) {
+  const long long total = 1ll * cout_pad * kw * kh * cin_pad;
+  for (long long i = blockIdx.x * 1ll * blockDim.x + threadIdx.x; i < total;
+       i += 1ll * gridDim.x * blockDim.x) {
     const int ci = static_cast<int>(i % cin_pad);
     long long r = i / cin_pad;
-    const int ky = static_cast<int>(r % k);
-    r /= k;
-    const int kx = static_cast<int>(r % k);
-    const int co = static_cast<int>(r / k);
+    const int ky = static_cast<int>(r % kh);
+    r /= kh;
+    const int kx = static_cast<int>(r % kw);
+    const int co = static_cast<int>(r / kw);
     float v = 0.f;
-    if (co < cout && ci < cin) v = w[((1ll * co * cin + ci) * k + ky) * k + kx];
+    if (co < cout && ci < cin) v = w[((1ll * co * cin + ci) * kh + ky) * kw + kx];
     out[i] = __float2bfloat16_rn(v);
   }
 }
@@ -106,16 +107,27 @@ inline int pad_to(int x, int m) { return (x + m - 1) / m * m; }
 
 }  // namespace
 
+int pack_conv_weight(const float* w_oihw, int cout, int cin, int kh, int kw, int cout_pad, int cin_pad,
+                     __nv_bfloat16* out, cudaStream_t stream) {
+  const long long total = 1ll * cout_pad * kw * kh * cin_pad;
+  const int block = 256;
+  const int grid = static_cast<int>((total + block - 1) / block > 4096 ? 4096 : (total + block - 1) / block);
+  pack_conv_weight_kernel<<<grid, block, 0, stream>>>(w_oihw, cout, cin, kh, kw, cout_pad, cin_pad, out);
+  MVLM_CHECK_CUDA(cudaGetLastError());
+  return MVLM_OK;
+}
+
 HourglassNet::~HourglassNet() {
   for (auto& g : graphs_) cudaGraphExecDestroy(g.second);
   for (void* p : owned_) cudaFree(p);
 }
 
-// Workspace allocation with buffer reuse.  The plan is emitted twice: a LAYOUT pass (no CUDA calls) hands out fake,
-// never-reused addresses and records for every buffer the first and the last op that touches it; assign_offsets()
-// then packs the buffers so that two share memory only when their lifetimes are disjoint (launches are stream-
-// ordered, and programmatic dependent launch only overlaps a kernel's prologue, which touches no activation); the
-// real pass hands out the packed addresses in the same allocation order.  20.3 GB -> a few GB at 100 views of 256^2.
+// Workspace allocation with buffer reuse.  emit() runs twice through the same calls: the LAYOUT pass (no CUDA calls)
+// hands out fake, never-reused addresses, records for every buffer the first and the last op that touches it, and
+// sizes the parameter arena; assign_offsets() then packs the buffers so that two share memory only when their
+// lifetimes are disjoint (launches are stream-ordered, and programmatic dependent launch only overlaps a kernel's
+// prologue, which touches no activation); the real pass hands out the packed addresses in the same allocation order,
+// fills the parameters and plans the convolutions.  20.3 GB -> a few GB at 100 views of 256^2.
 static uint8_t* const kFakeBase = reinterpret_cast<uint8_t*>(static_cast<uintptr_t>(1) << 44);
 
 void* HourglassNet::ws_alloc(size_t bytes) {
@@ -128,7 +140,7 @@ void* HourglassNet::ws_alloc(size_t bytes) {
     fake_off_ += aligned;
     return kFakeBase + b.fake_off;
   }
-  if (dry_ || ws_ == nullptr || next_buf_ >= bufs_.size()) return nullptr;
+  if (ws_ == nullptr || next_buf_ >= bufs_.size()) return nullptr;
   return ws_ + bufs_[next_buf_++].offset;
 }
 
@@ -224,11 +236,19 @@ HourglassNet::T HourglassNet::alloc(int h, int w, int c) {
 
 // Device memory for the plan's parameters (packed bf16 weights, folded BatchNorm affines, padded biases): sized in the
 // layout pass, ONE cudaMalloc for the real pass (round 1 made 271 allocations and as many NULL-stream launches per plan).
-void* HourglassNet::param_alloc(size_t bytes) {
+// Every parameter tensor reserves its bytes here, by the same call in both passes, so the real pass's offsets are the
+// ones the layout pass counted.  Layout pass: only the offset advances (*dst = *src = null).  Real pass: *dst = the
+// tensor's slice of the arena, *src = state_dict entry `name` (`numel` elements), which the caller packs into *dst.
+int HourglassNet::param(const std::string& name, long long numel, size_t bytes, void** dst, const float** src) {
   const size_t aligned = (bytes + 255) & ~static_cast<size_t>(255);
-  void* p = (layout_pass_ || params_ == nullptr || param_off_ + aligned > param_cap_) ? nullptr : params_ + param_off_;
+  *dst = (layout_pass_ || params_ == nullptr || param_off_ + aligned > param_cap_) ? nullptr : params_ + param_off_;
+  *src = nullptr;
   param_off_ += aligned;
-  return p;
+  if (layout_pass_) return MVLM_OK;
+  const int rc = sd_get(name, numel, src);
+  if (rc) return rc;
+  MVLM_REQUIRE(*dst, "hourglass: parameter arena exhausted (%s)", name.c_str());
+  return MVLM_OK;
 }
 
 int HourglassNet::sd_get(const std::string& name, long long numel, const float** out) const {
@@ -242,25 +262,23 @@ int HourglassNet::sd_get(const std::string& name, long long numel, const float**
   return MVLM_OK;
 }
 
+// a BatchNorm several convs apply is folded once per pass
 int HourglassNet::bn(const std::string& name, int c, const float** scale, const float** shift) {
-  *scale = *shift = nullptr;
-  if (dry_) {
-    if (layout_pass_ && bn_seen_.insert(name).second) param_alloc(sizeof(float) * 2 * c);
-    return MVLM_OK;
-  }
   auto it = bn_cache_.find(name);
   if (it == bn_cache_.end()) {
-    const char* suffix[4] = {".weight", ".bias", ".running_mean", ".running_var"};
+    void* buf;
     const float* src[4];
-    for (int k = 0; k < 4; ++k) {
-      const int rc = sd_get(name + suffix[k], c, &src[k]);
-      if (rc) return rc;
+    int rc = param(name + ".weight", c, sizeof(float) * 2 * c, &buf, &src[0]);
+    if (rc) return rc;
+    float* f = static_cast<float*>(buf);
+    if (!layout_pass_) {
+      const char* suffix[3] = {".bias", ".running_mean", ".running_var"};
+      for (int k = 0; k < 3; ++k)
+        if ((rc = sd_get(name + suffix[k], c, &src[k + 1]))) return rc;
+      fold_bn_kernel<<<ceil_div(c, 128), 128, 0, build_stream_>>>(src[0], src[1], src[2], src[3], 1e-5f, c, f, f + c);
+      MVLM_CHECK_CUDA(cudaGetLastError());
     }
-    float* buf = static_cast<float*>(param_alloc(sizeof(float) * 2 * c));
-    MVLM_REQUIRE(buf, "hourglass: parameter arena exhausted (%s)", name.c_str());
-    fold_bn_kernel<<<ceil_div(c, 128), 128, 0, build_stream_>>>(src[0], src[1], src[2], src[3], 1e-5f, c, buf, buf + c);
-    MVLM_CHECK_CUDA(cudaGetLastError());
-    it = bn_cache_.emplace(name, std::make_pair(buf, buf + c)).first;
+    it = bn_cache_.emplace(name, std::make_pair(f, f ? f + c : nullptr)).first;
   }
   *scale = it->second.first;
   *shift = it->second.second;
@@ -269,69 +287,64 @@ int HourglassNet::bn(const std::string& name, int c, const float** scale, const 
 
 int HourglassNet::packed(const std::string& name, int cout, int cin, int k, int cout_pad, int cin_pad,
                          const __nv_bfloat16** out) {
-  *out = nullptr;
-  const size_t n = static_cast<size_t>(cout_pad) * k * k * cin_pad;
-  if (dry_) {
-    if (layout_pass_) param_alloc(n * sizeof(__nv_bfloat16));
-    return MVLM_OK;
-  }
-  const float* src = nullptr;
-  const int rc = sd_get(name, 1ll * cout * cin * k * k, &src);
-  if (rc) return rc;
-  __nv_bfloat16* buf = static_cast<__nv_bfloat16*>(param_alloc(n * sizeof(__nv_bfloat16)));
-  MVLM_REQUIRE(buf, "hourglass: parameter arena exhausted (%s)", name.c_str());
-  pack_weight_kernel<<<256, 256, 0, build_stream_>>>(src, cout, cin, k, cout_pad, cin_pad, buf);
-  MVLM_CHECK_CUDA(cudaGetLastError());
-  *out = buf;
-  return MVLM_OK;
+  void* buf;
+  const float* src;
+  const int rc = param(name, 1ll * cout * cin * k * k, sizeof(__nv_bfloat16) * cout_pad * k * k * cin_pad, &buf, &src);
+  *out = static_cast<__nv_bfloat16*>(buf);
+  if (rc || layout_pass_) return rc;
+  return pack_conv_weight(src, cout, cin, k, k, cout_pad, cin_pad, static_cast<__nv_bfloat16*>(buf), build_stream_);
 }
 
 int HourglassNet::bias(const std::string& name, int cout, int cout_pad, const float** out) {
-  *out = nullptr;
-  if (dry_) {
-    if (layout_pass_) param_alloc(sizeof(float) * cout_pad);
-    return MVLM_OK;
-  }
-  const float* src = nullptr;
-  const int rc = sd_get(name, cout, &src);
-  if (rc) return rc;
-  float* buf = static_cast<float*>(param_alloc(sizeof(float) * cout_pad));
-  MVLM_REQUIRE(buf, "hourglass: parameter arena exhausted (%s)", name.c_str());
-  pad_bias_kernel<<<ceil_div(cout_pad, 128), 128, 0, build_stream_>>>(src, cout, cout_pad, buf);
+  void* buf;
+  const float* src;
+  const int rc = param(name, cout, sizeof(float) * cout_pad, &buf, &src);
+  *out = static_cast<float*>(buf);
+  if (rc || layout_pass_) return rc;
+  pad_bias_kernel<<<ceil_div(cout_pad, 128), 128, 0, build_stream_>>>(src, cout, cout_pad, static_cast<float*>(buf));
   MVLM_CHECK_CUDA(cudaGetLastError());
-  *out = buf;
   return MVLM_OK;
 }
 
-int HourglassNet::emit_conv(const char* tag, T in, int cin, const std::string& wname, int cout, int cout_pad,
-                            int n_tile, int k, ConvEpilogue e, bool with_bias) {
-  // algorithmic FLOPs use the true (unpadded) channel counts of the reference layer
-  const int cin_real = (wname == "conv7") ? L_ : cin;
-  flops_ += 2.0 * cout * cin_real * k * k * in.h * in.w;
+// conv1.weight for the stem's 16-channel hi / lo input
+int HourglassNet::stem_weight(const __nv_bfloat16** out) {
+  void* buf;
+  const float* src;
+  const int rc = param("conv1.weight", 64ll * cin_ * 9, sizeof(__nv_bfloat16) * 64 * 9 * 16, &buf, &src);
+  *out = static_cast<__nv_bfloat16*>(buf);
+  if (rc || layout_pass_) return rc;
+  pack_stem_weight_kernel<<<36, 256, 0, build_stream_>>>(src, 64, cin_, 64, static_cast<__nv_bfloat16*>(buf));
+  MVLM_CHECK_CUDA(cudaGetLastError());
+  return MVLM_OK;
+}
+
+// conv11.weight folded into the 2x2 kernel of up-sampling phase (a, b)
+int HourglassNet::phase_weight(int a, int b, const __nv_bfloat16** out) {
+  void* buf;
+  const float* src;
+  const int rc = param("conv11.weight", 9ll * L_ * L_, sizeof(__nv_bfloat16) * Lp_ * 4 * Lp_, &buf, &src);
+  *out = static_cast<__nv_bfloat16*>(buf);
+  if (rc || layout_pass_) return rc;
+  pack_phase_weight_kernel<<<64, 256, 0, build_stream_>>>(src, L_, L_, a, b, Lp_, Lp_, static_cast<__nv_bfloat16*>(buf));
+  MVLM_CHECK_CUDA(cudaGetLastError());
+  return MVLM_OK;
+}
+
+int HourglassNet::emit_conv(const char* tag, T in, int cin, const __nv_bfloat16* w, int cout_pad, int n_tile, int kh,
+                            int kw, int y_off0, int x_off0, const ConvEpilogue& e, double flops, bool is_head) {
+  flops_ += flops;
   note_conv(in.p, e);
   NetOp op;
   op.kind = NetOp::CONV;
   op.tag = tag;
+  op.is_head = is_head;
   op.h = in.h; op.w = in.w;
-  if (layout_pass_) {  // parameter bytes of this layer (packed weights, bias), allocated by the real pass below
-    const __nv_bfloat16* dw;
-    const float* db;
-    packed(wname + ".weight", cout, cin_real, k, cout_pad, cin, &dw);
-    if (with_bias) bias(wname + ".bias", cout, cout_pad, &db);
-  }
-  if (!dry_) {
+  if (!layout_pass_) {
     ConvShape s;
     s.in = in.p; s.n = V_; s.h = in.h; s.w = in.w; s.cin = cin; s.in_cs = in.c;
-    const __nv_bfloat16* wp;
-    int rc = packed(wname + ".weight", cout, cin_real, k, cout_pad, cin, &wp);
-    if (rc) return rc;
-    s.wpacked = wp; s.cout_pad = cout_pad; s.n_tile = n_tile; s.kh = k; s.kw = k;
-    s.y_off0 = -(k / 2); s.x_off0 = -(k / 2);
-    if (with_bias) {
-      rc = bias(wname + ".bias", cout, cout_pad, &e.bias);
-      if (rc) return rc;
-    }
-    rc = conv_plan(s, e, &op.conv);
+    s.wpacked = w; s.cout_pad = cout_pad; s.n_tile = n_tile; s.kh = kh; s.kw = kw;
+    s.y_off0 = y_off0; s.x_off0 = x_off0;
+    const int rc = conv_plan(s, e, &op.conv);
     if (rc) return rc;
   }
   ops_.push_back(op);
@@ -347,8 +360,11 @@ int HourglassNet::rb(const std::string& p, T x, T a_in, T ar, int cin, int cout,
   if (cin != cout) {
     ConvEpilogue e;
     e.out_raw = y.p; e.raw_cs = cout; e.raw_co = 0;
-    rc = emit_conv("rb.resample", ar, cin, p + ".resample.2", cout, cout, cout < 128 ? cout : 128, 1, e, false);
-    if (rc) return rc;
+    const __nv_bfloat16* wr;
+    if ((rc = packed(p + ".resample.2.weight", cout, cin, 1, cout, cin, &wr)) ||
+        (rc = emit_conv("rb.resample", ar, cin, wr, cout, cout < 128 ? cout : 128, 1, 1, 0, 0, e,
+                        2.0 * cout * cin * ar.h * ar.w)))
+      return rc;
     skip = y;  // the three convs accumulate in place
   }
   const float *ps = nullptr, *pt = nullptr;
@@ -390,20 +406,23 @@ int HourglassNet::rb(const std::string& p, T x, T a_in, T ar, int cin, int cout,
     e.out_raw = pool_raw ? pool_raw->p : y.p; e.raw_cs = cout; e.raw_co = offs[i];
     e.pool2 = pool_raw != nullptr;
     if (post_bn) {
-      e.post_scale = dry_ ? nullptr : ps + offs[i];
-      e.post_shift = dry_ ? nullptr : pt + offs[i];
+      e.post_scale = layout_pass_ ? nullptr : ps + offs[i];
+      e.post_shift = layout_pass_ ? nullptr : pt + offs[i];
       e.out_post = post_act->p; e.post_cs = cout; e.post_co = offs[i];
     }
     if (aux) {
       e.aux_mode = aux->mode;
-      e.aux_scale = dry_ ? nullptr : as + offs[i];
-      e.aux_shift = dry_ ? nullptr : at + offs[i];
+      e.aux_scale = layout_pass_ ? nullptr : as + offs[i];
+      e.aux_shift = layout_pass_ ? nullptr : at + offs[i];
       e.out_aux1 = aux->out1->p; e.aux1_cs = cout; e.aux1_co = offs[i];
       if (aux->mode == 2) { e.out_aux2 = aux->out2->p; e.aux2_cs = cout; e.aux2_co = offs[i]; }
     }
     const int nt = widths[i] < 128 ? widths[i] : 128;
-    rc = emit_conv("rb.conv", ins[i], cins[i], p + names[i], widths[i], widths[i], nt, 3, e, false);
-    if (rc) return rc;
+    const __nv_bfloat16* wc;
+    if ((rc = packed(p + names[i] + ".weight", widths[i], cins[i], 3, widths[i], cins[i], &wc)) ||
+        (rc = emit_conv("rb.conv", ins[i], cins[i], wc, widths[i], nt, 3, 3, -1, -1, e,
+                        2.0 * widths[i] * cins[i] * 9 * h * w)))
+      return rc;
   }
   *y_out = y;
   return MVLM_OK;
@@ -515,8 +534,7 @@ int HourglassNet::build(const StateDict* sd, int n_landmarks, int cin, int n_vie
   fuse_elt_ = !(getenv("MVLM_HG_ELT_FUSION") != nullptr && atoi(getenv("MVLM_HG_ELT_FUSION")) == 0);
   // layout pass: lifetimes and packed offsets
   bufs_.clear(); fake_off_ = 0; ws_needed_ = 0; next_buf_ = 0;
-  param_off_ = 0; bn_seen_.clear();
-  dry_ = true; layout_pass_ = true;
+  layout_pass_ = true;
   int rc = emit();
   layout_pass_ = false;
   if (rc) return rc;
@@ -529,9 +547,7 @@ int HourglassNet::build(const StateDict* sd, int n_landmarks, int cin, int n_vie
   MVLM_CHECK_CUDA(cudaMalloc(&params_, param_bytes));
   owned_.push_back(params_);
   param_cap_ = param_bytes;
-  param_off_ = 0;
   MVLM_CHECK_CUDA(cudaStreamCreateWithFlags(&build_stream_, cudaStreamNonBlocking));
-  dry_ = false;
   rc = emit();
   if (rc == MVLM_OK && param_off_ > param_bytes) {
     set_error("hourglass: parameter arena overrun (%zu of %zu bytes)", param_off_, param_bytes);
@@ -554,10 +570,11 @@ void HourglassNet::probe(const char* name, const T& t) {
   }
 }
 
-// emits the plan: ops_, probes, flops_ (layout pass: fake addresses, no CUDA calls)
+// emits the plan: ops_, probes, flops_, the parameter arena (layout pass: fake addresses, no CUDA calls)
 int HourglassNet::emit() {
   const int h = H_, w = W_, cin = cin_;
   ops_.clear(); flops_ = 0.0; probes.clear();
+  param_off_ = 0; bn_cache_.clear();
   int rc;
   const int F = 256, h2 = h / 2, w2 = w / 2;
 
@@ -571,40 +588,16 @@ int HourglassNet::emit() {
     op.kind = NetOp::STEM;
     op.out_raw = img16.p; op.h = h; op.w = w; op.c = cin;
     ops_.push_back(op);
-    flops_ += 2.0 * 64 * cin * 9 * h * w;
-    note_use(img16.p); note_use(a_c2.p); note_use(ar_c2.p);
-    NetOp cv;
-    cv.kind = NetOp::CONV;
-    cv.tag = "conv1";
-    cv.h = h; cv.w = w;
-    if (layout_pass_) {  // what the real pass allocates in this block, in the same order
-      param_alloc(sizeof(__nv_bfloat16) * 64 * 9 * 16);
-      const float* dummy;
-      bias("conv1.bias", 64, 64, &dummy);
-      bn("bn1", 64, &dummy, &dummy);
-      bn("conv2.bn1", 64, &dummy, &dummy);
-      bn("conv2.resample.0", 64, &dummy, &dummy);
-    }
-    if (!dry_) {
-      const float* w1 = nullptr;
-      if ((rc = sd_get("conv1.weight", 64ll * cin * 9, &w1))) return rc;
-      __nv_bfloat16* wp = static_cast<__nv_bfloat16*>(param_alloc(sizeof(__nv_bfloat16) * 64 * 9 * 16));
-      MVLM_REQUIRE(wp, "hourglass: parameter arena exhausted (conv1)");
-      pack_stem_weight_kernel<<<36, 256, 0, build_stream_>>>(w1, 64, cin, 64, wp);
-      MVLM_CHECK_CUDA(cudaGetLastError());
-      ConvShape s;
-      s.in = img16.p; s.n = V_; s.h = h; s.w = w; s.cin = 16; s.in_cs = 16;
-      s.wpacked = wp; s.cout_pad = 64; s.n_tile = 64; s.kh = 3; s.kw = 3; s.y_off0 = -1; s.x_off0 = -1;
-      ConvEpilogue e;
-      if ((rc = bias("conv1.bias", 64, 64, &e.bias))) return rc;
-      if ((rc = bn("bn1", 64, &e.mid_scale, &e.mid_shift))) return rc;
-      if ((rc = bn("conv2.bn1", 64, &e.pre_scale, &e.pre_shift))) return rc;
-      if ((rc = bn("conv2.resample.0", 64, &e.post_scale, &e.post_shift))) return rc;
-      e.out_pre = a_c2.p; e.pre_cs = 64; e.pre_co = 0;
-      e.out_post = ar_c2.p; e.post_cs = 64; e.post_co = 0;
-      if ((rc = conv_plan(s, e, &cv.conv))) return rc;
-    }
-    ops_.push_back(cv);
+    const __nv_bfloat16* w1;
+    ConvEpilogue e;
+    if ((rc = stem_weight(&w1))) return rc;
+    if ((rc = bias("conv1.bias", 64, 64, &e.bias))) return rc;
+    if ((rc = bn("bn1", 64, &e.mid_scale, &e.mid_shift))) return rc;
+    if ((rc = bn("conv2.bn1", 64, &e.pre_scale, &e.pre_shift))) return rc;
+    if ((rc = bn("conv2.resample.0", 64, &e.post_scale, &e.post_shift))) return rc;
+    e.out_pre = a_c2.p; e.pre_cs = 64; e.pre_co = 0;
+    e.out_post = ar_c2.p; e.post_cs = 64; e.post_co = 0;
+    if ((rc = emit_conv("conv1", img16, 16, w1, 64, 64, 3, 3, -1, -1, e, 2.0 * 64 * cin * 9 * h * w))) return rc;
   }
   T none, y2, y3, r3, a3, a4, a_h1, ar4;
   // conv2 block: its output is only consumed through the max-pool (:411) -> pooled outputs straight from the epilogues
@@ -636,18 +629,25 @@ int HourglassNet::emit() {
   T hg1;
   if ((rc = hourglass("hg1", r3, a_h1, &hg1, fuse_elt_ ? &p1 : nullptr, fuse_elt_ ? &pa1 : nullptr))) return rc;
   probe("hg1", hg1);
+  // conv5..conv10 read all channels of their input; their FLOPs count the true (unpadded) channels
   T ll1 = alloc(h2, w2, F);
   {
     ConvEpilogue e;
+    const __nv_bfloat16* w5;
     if ((rc = bn("bn2", F, &e.pre_scale, &e.pre_shift))) return rc;
     e.out_pre = ll1.p; e.pre_cs = F; e.pre_co = 0;
-    if ((rc = emit_conv("conv5", hg1, F, "conv5", F, F, 128, 3, e, true))) return rc;
+    if ((rc = packed("conv5.weight", F, F, 3, F, F, &w5)) || (rc = bias("conv5.bias", F, F, &e.bias)) ||
+        (rc = emit_conv("conv5", hg1, F, w5, F, 128, 3, 3, -1, -1, e, 2.0 * F * F * 9 * h2 * w2)))
+      return rc;
   }
   T x6 = alloc(h2, w2, Lp_);
   {
     ConvEpilogue e;
+    const __nv_bfloat16* w6;
     e.out_raw = x6.p; e.raw_cs = Lp_; e.raw_co = 0;
-    if ((rc = emit_conv("conv6", ll1, F, "conv6", L_, Lp_, Lp_, 3, e, true))) return rc;
+    if ((rc = packed("conv6.weight", L_, F, 3, Lp_, F, &w6)) || (rc = bias("conv6.bias", L_, Lp_, &e.bias)) ||
+        (rc = emit_conv("conv6", ll1, F, w6, Lp_, Lp_, 3, 3, -1, -1, e, 2.0 * L_ * F * 9 * h2 * w2)))
+      return rc;
   }
   T sum = alloc(h2, w2, F), a_h2;
   {
@@ -666,7 +666,10 @@ int HourglassNet::emit() {
       e.out_aux1 = p2.p; e.aux1_cs = F; e.aux1_co = 0;
       e.out_aux2 = pa2.p; e.aux2_cs = F; e.aux2_co = 0;
     }
-    if ((rc = emit_conv("conv7", x6, Lp_, "conv7", F, F, 128, 3, e, true))) return rc;
+    const __nv_bfloat16* w7;
+    if ((rc = packed("conv7.weight", F, L_, 3, F, Lp_, &w7)) || (rc = bias("conv7.bias", F, F, &e.bias)) ||
+        (rc = emit_conv("conv7", x6, Lp_, w7, F, 128, 3, 3, -1, -1, e, 2.0 * F * L_ * 9 * h2 * w2)))
+      return rc;
   }
   probe("sum_temp", sum);
   // ---- hourglass 2 (:424), conv9+bn3+relu (:426), conv10 (:427)
@@ -675,15 +678,21 @@ int HourglassNet::emit() {
   T ll2 = alloc(h2, w2, F);
   {
     ConvEpilogue e;
+    const __nv_bfloat16* w9;
     if ((rc = bn("bn3", F, &e.pre_scale, &e.pre_shift))) return rc;
     e.out_pre = ll2.p; e.pre_cs = F; e.pre_co = 0;
-    if ((rc = emit_conv("conv9", hg2, F, "conv9", F, F, 128, 3, e, true))) return rc;
+    if ((rc = packed("conv9.weight", F, F, 3, F, F, &w9)) || (rc = bias("conv9.bias", F, F, &e.bias)) ||
+        (rc = emit_conv("conv9", hg2, F, w9, F, 128, 3, 3, -1, -1, e, 2.0 * F * F * 9 * h2 * w2)))
+      return rc;
   }
   T x10 = alloc(h2, w2, Lp_);
   {
     ConvEpilogue e;
+    const __nv_bfloat16* w10;
     e.out_raw = x10.p; e.raw_cs = Lp_; e.raw_co = 0;
-    if ((rc = emit_conv("conv10", ll2, F, "conv10", L_, Lp_, Lp_, 3, e, true))) return rc;
+    if ((rc = packed("conv10.weight", L_, F, 3, Lp_, F, &w10)) || (rc = bias("conv10.bias", L_, Lp_, &e.bias)) ||
+        (rc = emit_conv("conv10", ll2, F, w10, Lp_, Lp_, 3, 3, -1, -1, e, 2.0 * L_ * F * 9 * h2 * w2)))
+      return rc;
   }
   probe("x10", x10);
   // ---- conv11 on nearest-x2(conv10) (:428-429) as four 2x2 phase convs with fused arg-max
@@ -692,43 +701,23 @@ int HourglassNet::emit() {
     note_use(keys_);
     NetOp op;
     op.kind = NetOp::MEMSET;
-    op.ptr = keys_; op.bytes = sizeof(unsigned long long) * V_ * L_;
+    op.bytes = sizeof(unsigned long long) * V_ * L_;
     ops_.push_back(op);
   }
-  flops_ += 2.0 * L_ * L_ * 9 * h * w;  // algorithmic FLOPs of the reference's conv11
-  const float* b11 = nullptr;
-  if ((rc = bias("conv11.bias", L_, Lp_, &b11))) return rc;
-  b11_ = b11;
+  if ((rc = bias("conv11.bias", L_, Lp_, &b11_))) return rc;
   x10_ = x10.p;
   for (int a = 0; a < 2; ++a) {
     for (int b = 0; b < 2; ++b) {
-      note_use(x10.p); note_use(keys_);
-      NetOp op;
-      op.kind = NetOp::CONV;
-      op.is_head = true;
-      op.tag = "conv11.phase";
-      op.h = h2; op.w = w2;
-      if (layout_pass_) param_alloc(sizeof(__nv_bfloat16) * Lp_ * 4 * Lp_);
-      if (!dry_) {
-        const float* w11 = nullptr;
-        if ((rc = sd_get("conv11.weight", 9ll * L_ * L_, &w11))) return rc;
-        __nv_bfloat16* wp = static_cast<__nv_bfloat16*>(param_alloc(sizeof(__nv_bfloat16) * Lp_ * 4 * Lp_));
-        MVLM_REQUIRE(wp, "hourglass: parameter arena exhausted (conv11)");
-        pack_phase_weight_kernel<<<64, 256, 0, build_stream_>>>(w11, L_, L_, a, b, Lp_, Lp_, wp);
-        MVLM_CHECK_CUDA(cudaGetLastError());
-        phase_w_[2 * a + b] = wp;
-        ConvShape s;
-        s.in = x10.p; s.n = V_; s.h = h2; s.w = w2; s.cin = Lp_; s.in_cs = Lp_;
-        s.wpacked = wp; s.cout_pad = Lp_; s.n_tile = Lp_; s.kh = 2; s.kw = 2;
-        s.y_off0 = a - 1; s.x_off0 = b - 1;
-        ConvEpilogue e;
-        e.bias = b11;
-        e.argmax_keys = keys_;
-        e.cout_real = L_;
-        e.up_sy = 2; e.up_sx = 2; e.up_py = a; e.up_px = b;
-        if ((rc = conv_plan(s, e, &op.conv))) return rc;
-      }
-      ops_.push_back(op);
+      ConvEpilogue e;
+      e.bias = b11_;
+      e.argmax_keys = keys_;
+      e.cout_real = L_;
+      e.up_sy = 2; e.up_sx = 2; e.up_py = a; e.up_px = b;
+      // each phase computes a quarter of the reference conv11's output pixels
+      if ((rc = phase_weight(a, b, &phase_w_[2 * a + b])) ||
+          (rc = emit_conv("conv11.phase", x10, Lp_, phase_w_[2 * a + b], Lp_, Lp_, 2, 2, a - 1, b - 1, e,
+                          2.0 * L_ * L_ * 9 * h2 * w2, true)))
+        return rc;
     }
   }
   {
@@ -797,7 +786,7 @@ int HourglassNet::forward_keys(const unsigned char* img_u8, const float* img_f32
 
 int HourglassNet::forward(const unsigned char* img_u8, const float* img_f32, float* out_heatmaps, float* out_peaks,
                           cudaStream_t stream) {
-  MVLM_REQUIRE(!dry_, "hourglass: forward on a dry plan");
+  MVLM_REQUIRE(params_, "hourglass: forward on a dry plan");
   MVLM_REQUIRE(out_peaks || out_heatmaps, "hourglass: no output requested");
   for (NetOp& op : ops_) {
     const int rc = run_op(op, img_u8, img_f32, out_heatmaps, out_peaks, stream);
@@ -809,7 +798,7 @@ int HourglassNet::forward(const unsigned char* img_u8, const float* img_f32, flo
 int HourglassNet::profile_ops(const unsigned char* img_u8, const float* img_f32, float* out_peaks, int reps,
                               float* ms_out, double* roles_out, int trace_op, long long* trace_out,
                               cudaStream_t stream) {
-  MVLM_REQUIRE(!dry_ && out_peaks && ms_out && reps > 0, "hourglass: bad profile_ops arguments");
+  MVLM_REQUIRE(params_ && out_peaks && ms_out && reps > 0, "hourglass: bad profile_ops arguments");
   const size_t n = ops_.size();
   std::vector<cudaEvent_t> ev(n + 1);
   for (auto& e : ev) MVLM_CHECK_CUDA(cudaEventCreate(&e));

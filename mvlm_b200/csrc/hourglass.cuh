@@ -1,7 +1,6 @@
 // Stacked-hourglass heat-map CNN plan: the whole network as a static list of fused launches.
 #pragma once
 #include <map>
-#include <set>
 #include <string>
 #include <vector>
 
@@ -22,13 +21,11 @@ struct NetOp {
   ConvParams conv;  // CONV
   // eltwise / memset
   const __nv_bfloat16* in0 = nullptr;
-  const __nv_bfloat16* in1 = nullptr;
   __nv_bfloat16* out_raw = nullptr;
   __nv_bfloat16* out_act = nullptr;
   const float* scale = nullptr;
   const float* shift = nullptr;
   int h = 0, w = 0, c = 0;
-  void* ptr = nullptr;
   size_t bytes = 0;
   bool is_head = false;  // conv11 phase: out_f32 patched per forward call
   const char* tag = "";
@@ -92,20 +89,24 @@ class HourglassNet {
   void note_conv(const void* in, const ConvEpilogue& e);
   void assign_offsets();
   void probe(const char* name, const T& t);
-  void* param_alloc(size_t bytes);
+  int param(const std::string& name, long long numel, size_t bytes, void** dst, const float** src);
   unsigned char* params_ = nullptr;  // one arena for packed weights / folded BatchNorm affines / biases
   size_t param_off_ = 0, param_cap_ = 0;
-  std::set<std::string> bn_seen_;
   cudaStream_t build_stream_ = nullptr;  // plan-build kernels (weight repacking) run here, not on the NULL stream
   static constexpr size_t kMaxGraphs = 8;
   std::vector<Buf> bufs_;
   size_t fake_off_ = 0, ws_needed_ = 0, next_buf_ = 0;
   bool layout_pass_ = false, keep_probes_ = false, reuse_ = true, fuse_elt_ = false;
+  // parameter tensors (see param): null in the layout pass, filled on build_stream_ in the real pass
   int bn(const std::string& name, int c, const float** scale, const float** shift);
   int packed(const std::string& name, int cout, int cin, int k, int cout_pad, int cin_pad, const __nv_bfloat16** out);
   int bias(const std::string& name, int cout, int cout_pad, const float** out);
-  int emit_conv(const char* tag, T in, int cin, const std::string& wname, int cout, int cout_pad, int n_tile, int k,
-                ConvEpilogue e, bool with_bias);
+  int stem_weight(const __nv_bfloat16** out);
+  int phase_weight(int a, int b, const __nv_bfloat16** out);
+  // one convolution op: the first `cin` channels of `in` through the packed weights `w` (kh x kw taps, tap (0,0) at
+  // input offset (y_off0, x_off0)); `flops` = the algorithmic FLOPs of the reference layer's share this op computes
+  int emit_conv(const char* tag, T in, int cin, const __nv_bfloat16* w, int cout_pad, int n_tile, int kh, int kw,
+                int y_off0, int x_off0, const ConvEpilogue& e, double flops, bool is_head = false);
   // pool_raw != nullptr: the block output is only consumed through a 2x2 max-pool (conv2 block, :410-411):
   // the three convs write the pooled raw tensor and relu(post_bn(pooled)) directly; no full-resolution output
   // up_low != nullptr: the nearest-x2 up-sampled half-resolution tensor is added to the block output
@@ -121,12 +122,11 @@ class HourglassNet {
   const StateDict* sd_ = nullptr;
   // state_dict entry `name` with exactly `numel` elements (a checkpoint of another model must not be misread)
   int sd_get(const std::string& name, long long numel, const float** out) const;
-  bool dry_ = true;
   int V_ = 0, H_ = 0, W_ = 0, L_ = 0, Lp_ = 0, cin_ = 0;
   uint8_t* ws_ = nullptr;
   size_t ws_size_ = 0;
   std::vector<void*> owned_;
-  std::map<std::string, std::pair<float*, float*>> bn_cache_;
+  std::map<std::string, std::pair<float*, float*>> bn_cache_;  // folded BatchNorm scale / shift by name, per pass
   std::vector<NetOp> ops_;
   unsigned long long* keys_ = nullptr;
   unsigned long long* out_keys_ = nullptr;  // set for the duration of forward_keys
