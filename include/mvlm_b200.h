@@ -327,6 +327,42 @@ int mvlm_debug_hourglass_profile(mvlm_hourglass* net, const uint8_t* img_u8, con
                                  long long* trace_out /* 64 x 16 int64 timeline of CTA 0 of conv op trace_op, or NULL */,
                                  void* stream);
 int mvlm_debug_hourglass_describe(const mvlm_hourglass* net, int op, char* buf, int buf_len);
+/* What every op computes, for the layer-wise tests (tests/test_plan_layers_*.py).  operands[] in the order in, res1,
+ * res2, res_up, out_pre, out_raw, out_post, out_aux1, out_aux2, keys (pool / bnrelu: in, out_raw = pooled, out_post =
+ * act; stem: out_raw = hi/lo staging; memset / peaks: keys, peaks: in = conv11's input).  An absent operand has cs 0.
+ * buf = allocation index of the plan buffer (-1: not the start of one), ws_offset = its byte offset in the workspace.
+ * terms[] = BatchNorm affines mid, pre, post, aux, scale (pool / bnrelu): name ("" = none) + channel offset. */
+#define MVLM_HG_OPERANDS 10
+#define MVLM_HG_TERMS 5
+typedef struct {
+  int32_t buf, cs, co, pad_;
+  int64_t ws_offset;
+} mvlm_hg_operand;
+typedef struct {
+  char bn[64];
+  int32_t off;
+} mvlm_hg_term;
+typedef struct {
+  int32_t kind; /* 0 conv, 1 pool, 2 bnrelu, 3 stem, 4 memset, 5 peaks */
+  char layer[64], bias[64];
+  int32_t phase_a, phase_b;
+  mvlm_hg_term terms[MVLM_HG_TERMS];
+  int32_t h, w, cin, in_cs, kh, kw, y_off0, x_off0, cout_pad, n_tile, cout_real, pool2, aux_mode;
+  mvlm_hg_operand operands[MVLM_HG_OPERANDS];
+} mvlm_hg_op;
+typedef struct {
+  int64_t bytes, offset;
+} mvlm_hg_buffer;
+/* The records of a plan that is only laid out (no device, no state_dict; honours the MVLM_HG_* switches) or of a
+ * created one.  Writes min(n, max) entries of ops / bufs (either may be NULL) and the counts to *n_ops / *n_bufs. */
+int mvlm_debug_hourglass_dry_ops(int n_landmarks, int cin, int n_views, int h, int w, mvlm_hg_op* ops, int max_ops,
+                                 int* n_ops, mvlm_hg_buffer* bufs, int max_bufs, int* n_bufs);
+int mvlm_debug_hourglass_ops(const mvlm_hourglass* net, mvlm_hg_op* ops, int max_ops, int* n_ops, mvlm_hg_buffer* bufs,
+                             int max_bufs, int* n_bufs);
+/* Runs op `op` of the plan alone (arguments as mvlm_hourglass_forward; out_heatmaps makes the conv11 phases write
+ * their fp32 maps). */
+int mvlm_debug_hourglass_run_op(mvlm_hourglass* net, int op, const uint8_t* img_u8, const float* img_f32,
+                                float* out_heatmaps, float* out_peaks, void* stream);
 /* layer-wise parity probes: "r3", "hg1", "sum_temp", "x10" -> NHWC bf16 tensor in the workspace */
 int mvlm_hourglass_probe(const mvlm_hourglass* net, const char* name, const void** ptr, int* h, int* w, int* c);
 void mvlm_hourglass_destroy(mvlm_hourglass* net);

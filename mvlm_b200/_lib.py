@@ -72,6 +72,34 @@ class SnapMesh(C.Structure):
                 ("grid_bytes", C.c_size_t)]
 
 
+class HgOperand(C.Structure):
+    """mvlm_hg_operand: one tensor operand of a CNN plan op (plan buffer, channel stride / offset, workspace offset)."""
+    _fields_ = [("buf", C.c_int32), ("cs", C.c_int32), ("co", C.c_int32), ("pad_", C.c_int32), ("ws_offset", C.c_int64)]
+
+
+class HgTerm(C.Structure):
+    """mvlm_hg_term: a BatchNorm affine an op applies, and the channel offset into it."""
+    _fields_ = [("bn", C.c_char * 64), ("off", C.c_int32)]
+
+
+HG_OPERANDS = ("in", "res1", "res2", "res_up", "out_pre", "out_raw", "out_post", "out_aux1", "out_aux2", "keys")
+HG_TERMS = ("mid", "pre", "post", "aux", "scale")
+HG_KINDS = ("conv", "pool", "bnrelu", "stem", "memset", "peaks")
+
+
+class HgOp(C.Structure):
+    """mvlm_hg_op: what one op of the CNN plan computes (include/mvlm_b200.h)."""
+    _fields_ = [("kind", C.c_int32), ("layer", C.c_char * 64), ("bias", C.c_char * 64),
+                ("phase_a", C.c_int32), ("phase_b", C.c_int32), ("terms", HgTerm * len(HG_TERMS))] + \
+        [(f, C.c_int32) for f in ("h", "w", "cin", "in_cs", "kh", "kw", "y_off0", "x_off0", "cout_pad", "n_tile",
+                                  "cout_real", "pool2", "aux_mode")] + [("operands", HgOperand * len(HG_OPERANDS))]
+
+
+class HgBuffer(C.Structure):
+    """mvlm_hg_buffer: bytes and workspace offset of one plan buffer."""
+    _fields_ = [("bytes", C.c_int64), ("offset", C.c_int64)]
+
+
 MAX_SCANS = 64  # MVLM_MAX_SCANS
 OBJ_MATERIALS = 1  # MVLM_OBJ_MATERIALS
 OBJ_MAX_NAME_LINES = 65536  # MVLM_OBJ_MAX_NAME_LINES
@@ -126,6 +154,11 @@ def _declare(lib: C.CDLL) -> None:
                                          C.POINTER(C.c_longlong), vp], i32),
         "mvlm_debug_conv_profile_ints": ([], i32),
         "mvlm_debug_hourglass_describe": ([vp, i32, C.c_char_p, i32], i32),
+        "mvlm_debug_hourglass_dry_ops": ([i32, i32, i32, i32, i32, C.POINTER(HgOp), i32, C.POINTER(i32),
+                                          C.POINTER(HgBuffer), i32, C.POINTER(i32)], i32),
+        "mvlm_debug_hourglass_ops": ([vp, C.POINTER(HgOp), i32, C.POINTER(i32), C.POINTER(HgBuffer), i32,
+                                      C.POINTER(i32)], i32),
+        "mvlm_debug_hourglass_run_op": ([vp, i32, vp, vp, vp, vp, vp], i32),
         "mvlm_hourglass_probe": ([vp, C.c_char_p, C.POINTER(vp), C.POINTER(i32), C.POINTER(i32), C.POINTER(i32)], i32),
         "mvlm_hourglass_destroy": ([vp], None),
         "mvlm_obj_load": ([C.c_char_p, i32, C.POINTER(vp)], i32),

@@ -1,5 +1,6 @@
 // C-ABI glue (include/mvlm_b200.h): error state, launch counter, thin wrappers.
 #include <stdarg.h>
+#include <string.h>
 
 #include <atomic>
 
@@ -230,6 +231,58 @@ int mvlm_debug_hourglass_describe(const mvlm_hourglass* net, int op, char* buf, 
   MVLM_REQUIRE(net && buf && buf_len > 0, "mvlm_debug_hourglass_describe: null pointer");
   snprintf(buf, buf_len, "%s", net->net.describe_op(op).c_str());
   return MVLM_OK;
+}
+
+static int hourglass_ops(const HourglassNet& net, mvlm_hg_op* ops, int max_ops, int* n_ops, mvlm_hg_buffer* bufs,
+                         int max_bufs, int* n_bufs) {
+  MVLM_REQUIRE(n_ops && n_bufs, "mvlm_debug_hourglass_ops: null count pointer");
+  static_assert(kOpOperands == MVLM_HG_OPERANDS && kOpTerms == MVLM_HG_TERMS, "op record layout");
+  *n_ops = net.n_ops();
+  *n_bufs = net.n_buffers();
+  for (int i = 0; ops && i < max_ops && i < net.n_ops(); ++i) {
+    const NetOp& op = net.ops()[i];
+    const OpRecord& r = op.rec;
+    mvlm_hg_op& o = ops[i];
+    memset(&o, 0, sizeof(o));
+    o.kind = static_cast<int32_t>(op.kind);
+    snprintf(o.layer, sizeof(o.layer), "%s", r.layer.c_str());
+    snprintf(o.bias, sizeof(o.bias), "%s", r.bias.c_str());
+    o.phase_a = r.phase_a; o.phase_b = r.phase_b;
+    for (int k = 0; k < kOpTerms; ++k) {
+      snprintf(o.terms[k].bn, sizeof(o.terms[k].bn), "%s", r.terms[k].bn.c_str());
+      o.terms[k].off = r.terms[k].off;
+    }
+    o.h = r.h; o.w = r.w; o.cin = r.cin; o.in_cs = r.in_cs; o.kh = r.kh; o.kw = r.kw; o.y_off0 = r.y_off0;
+    o.x_off0 = r.x_off0; o.cout_pad = r.cout_pad; o.n_tile = r.n_tile; o.cout_real = r.cout_real; o.pool2 = r.pool2;
+    o.aux_mode = r.aux_mode;
+    for (int k = 0; k < kOpOperands; ++k)
+      o.operands[k] = mvlm_hg_operand{r.opnd[k].buf, r.opnd[k].cs, r.opnd[k].co, 0, r.opnd[k].ws_off};
+  }
+  for (int i = 0; bufs && i < max_bufs && i < net.n_buffers(); ++i)
+    bufs[i] = mvlm_hg_buffer{static_cast<int64_t>(net.buffer_bytes(i)), static_cast<int64_t>(net.buffer_offset(i))};
+  return MVLM_OK;
+}
+
+int mvlm_debug_hourglass_dry_ops(int n_landmarks, int cin, int n_views, int h, int w, mvlm_hg_op* ops, int max_ops,
+                                 int* n_ops, mvlm_hg_buffer* bufs, int max_bufs, int* n_bufs) {
+  HourglassNet dry;
+  const int rc = dry.build(nullptr, n_landmarks, cin, n_views, h, w, nullptr, 0, true);
+  if (rc != MVLM_OK) return rc;
+  return hourglass_ops(dry, ops, max_ops, n_ops, bufs, max_bufs, n_bufs);
+}
+
+int mvlm_debug_hourglass_ops(const mvlm_hourglass* net, mvlm_hg_op* ops, int max_ops, int* n_ops, mvlm_hg_buffer* bufs,
+                             int max_bufs, int* n_bufs) {
+  MVLM_REQUIRE(net, "mvlm_debug_hourglass_ops: null handle");
+  return hourglass_ops(net->net, ops, max_ops, n_ops, bufs, max_bufs, n_bufs);
+}
+
+int mvlm_debug_hourglass_run_op(mvlm_hourglass* net, int op, const uint8_t* img_u8, const float* img_f32,
+                                float* out_heatmaps, float* out_peaks, void* stream) {
+  MVLM_REQUIRE(net, "mvlm_debug_hourglass_run_op: null handle");
+  MVLM_REQUIRE(op >= 0 && op < net->net.n_ops(), "mvlm_debug_hourglass_run_op: op %d of %d", op, net->net.n_ops());
+  return net->net.run_op(net->net.ops_mut()[op], img_u8, img_f32, out_heatmaps, out_peaks,
+                         static_cast<cudaStream_t>(stream));
 }
 
 int mvlm_hourglass_num_launches(const mvlm_hourglass* net) { return net ? net->net.n_ops() : 0; }

@@ -167,6 +167,31 @@ void HourglassNet::note_conv(const void* in, const ConvEpilogue& e) {
   note_use(e.out_post); note_use(e.argmax_keys); note_use(e.out_aux1); note_use(e.out_aux2);
 }
 
+// Independent of note_use on purpose: the layer-wise tests derive the lifetimes from these records and check the
+// packing that note_use drove.  Layout pass: the allocation index of the buffer starting at `p` (-1 if `p` is not the
+// start of one); real pass: the byte offset of `p` in the workspace (push_op adds the layout pass's index).
+void HourglassNet::record(OpRecord& r, int slot, const void* p, int cs, int co) const {
+  if (p == nullptr) return;
+  OpRecord::Operand& o = r.opnd[slot];
+  o.cs = cs; o.co = co;
+  const uint8_t* q = static_cast<const uint8_t*>(p);
+  if (layout_pass_) {
+    if (q < kFakeBase || q >= kFakeBase + fake_off_) return;
+    const size_t off = static_cast<size_t>(q - kFakeBase);
+    for (size_t i = 0; i < bufs_.size(); ++i)
+      if (bufs_[i].fake_off == off) o.buf = static_cast<int>(i);
+  } else if (ws_ != nullptr && q >= ws_ && q < ws_ + ws_size_) {
+    o.ws_off = static_cast<long long>(q - ws_);
+  }
+}
+
+void HourglassNet::push_op(NetOp& op) {
+  const size_t i = ops_.size();
+  if (!layout_pass_ && i < layout_recs_.size())
+    for (int k = 0; k < kOpOperands; ++k) op.rec.opnd[k].buf = layout_recs_[i].opnd[k].buf;
+  ops_.push_back(op);
+}
+
 void HourglassNet::assign_offsets() {
   const int n_ops = static_cast<int>(ops_.size());
   for (Buf& b : bufs_) {
@@ -331,7 +356,8 @@ int HourglassNet::phase_weight(int a, int b, const __nv_bfloat16** out) {
 }
 
 int HourglassNet::emit_conv(const char* tag, T in, int cin, const __nv_bfloat16* w, int cout_pad, int n_tile, int kh,
-                            int kw, int y_off0, int x_off0, const ConvEpilogue& e, double flops, bool is_head) {
+                            int kw, int y_off0, int x_off0, const ConvEpilogue& e, double flops, OpRecord rec,
+                            bool is_head) {
   flops_ += flops;
   note_conv(in.p, e);
   NetOp op;
@@ -339,6 +365,20 @@ int HourglassNet::emit_conv(const char* tag, T in, int cin, const __nv_bfloat16*
   op.tag = tag;
   op.is_head = is_head;
   op.h = in.h; op.w = in.w;
+  rec.h = in.h; rec.w = in.w; rec.cin = cin; rec.in_cs = in.c; rec.kh = kh; rec.kw = kw;
+  rec.y_off0 = y_off0; rec.x_off0 = x_off0; rec.cout_pad = cout_pad; rec.n_tile = n_tile;
+  rec.cout_real = e.cout_real; rec.pool2 = e.pool2 ? 1 : 0; rec.aux_mode = e.aux_mode;
+  record(rec, kOpIn, in.p, in.c, 0);
+  record(rec, kOpRes1, e.res1, e.res1_cs, e.res1_co);
+  record(rec, kOpRes2, e.res2, e.res2_cs, e.res2_co);
+  record(rec, kOpResUp, e.res_up, e.up_cs, e.up_co);
+  record(rec, kOpOutPre, e.out_pre, e.pre_cs, e.pre_co);
+  record(rec, kOpOutRaw, e.out_raw, e.raw_cs, e.raw_co);
+  record(rec, kOpOutPost, e.out_post, e.post_cs, e.post_co);
+  record(rec, kOpOutAux1, e.out_aux1, e.aux1_cs, e.aux1_co);
+  record(rec, kOpOutAux2, e.out_aux2, e.aux2_cs, e.aux2_co);
+  record(rec, kOpKeys, e.argmax_keys, L_, 0);
+  op.rec = rec;
   if (!layout_pass_) {
     ConvShape s;
     s.in = in.p; s.n = V_; s.h = in.h; s.w = in.w; s.cin = cin; s.in_cs = in.c;
@@ -347,7 +387,7 @@ int HourglassNet::emit_conv(const char* tag, T in, int cin, const __nv_bfloat16*
     const int rc = conv_plan(s, e, &op.conv);
     if (rc) return rc;
   }
-  ops_.push_back(op);
+  push_op(op);
   return MVLM_OK;
 }
 
@@ -361,9 +401,11 @@ int HourglassNet::rb(const std::string& p, T x, T a_in, T ar, int cin, int cout,
     ConvEpilogue e;
     e.out_raw = y.p; e.raw_cs = cout; e.raw_co = 0;
     const __nv_bfloat16* wr;
+    OpRecord rec;
+    rec.layer = p + ".resample.2";
     if ((rc = packed(p + ".resample.2.weight", cout, cin, 1, cout, cin, &wr)) ||
         (rc = emit_conv("rb.resample", ar, cin, wr, cout, cout < 128 ? cout : 128, 1, 1, 0, 0, e,
-                        2.0 * cout * cin * ar.h * ar.w)))
+                        2.0 * cout * cin * ar.h * ar.w, rec)))
       return rc;
     skip = y;  // the three convs accumulate in place
   }
@@ -396,11 +438,16 @@ int HourglassNet::rb(const std::string& p, T x, T a_in, T ar, int cin, int cout,
   const char* names[3] = {".conv1", ".conv2", ".conv3"};
   for (int i = 0; i < 3; ++i) {
     ConvEpilogue e;
+    OpRecord rec;
+    rec.layer = p + names[i];
     if (pre_bn[i]) {
       rc = bn(p + pre_bn[i], widths[i], &e.pre_scale, &e.pre_shift);
       if (rc) return rc;
       e.out_pre = pres[i].p; e.pre_cs = pres[i].c; e.pre_co = 0;
+      rec.terms[kTermPre] = {p + pre_bn[i], 0};
     }
+    if (post_bn) rec.terms[kTermPost] = {post_bn, offs[i]};
+    if (aux) rec.terms[kTermAux] = {aux->bn, offs[i]};
     e.res1 = skip.p; e.res1_cs = skip.c; e.res1_co = offs[i];
     if (up_low) { e.res_up = up_low->p; e.up_cs = up_low->c; e.up_co = offs[i]; }
     e.out_raw = pool_raw ? pool_raw->p : y.p; e.raw_cs = cout; e.raw_co = offs[i];
@@ -421,7 +468,7 @@ int HourglassNet::rb(const std::string& p, T x, T a_in, T ar, int cin, int cout,
     const __nv_bfloat16* wc;
     if ((rc = packed(p + names[i] + ".weight", widths[i], cins[i], 3, widths[i], cins[i], &wc)) ||
         (rc = emit_conv("rb.conv", ins[i], cins[i], wc, widths[i], nt, 3, 3, -1, -1, e,
-                        2.0 * widths[i] * cins[i] * 9 * h * w)))
+                        2.0 * widths[i] * cins[i] * 9 * h * w, rec)))
       return rc;
   }
   *y_out = y;
@@ -437,8 +484,13 @@ int HourglassNet::emit_pool(T in, T out_raw, const char* bn_name, T out_act) {
   if (bn_name) {
     int rc = bn(bn_name, in.c, &op.scale, &op.shift);
     if (rc) return rc;
+    op.rec.terms[kTermScale] = {bn_name, 0};
   }
-  ops_.push_back(op);
+  op.rec.h = in.h; op.rec.w = in.w; op.rec.cin = in.c; op.rec.in_cs = in.c;
+  record(op.rec, kOpIn, in.p, in.c, 0);
+  record(op.rec, kOpOutRaw, out_raw.p, out_raw.c, 0);
+  record(op.rec, kOpOutPost, out_act.p, out_act.c, 0);
+  push_op(op);
   return MVLM_OK;
 }
 
@@ -539,6 +591,12 @@ int HourglassNet::build(const StateDict* sd, int n_landmarks, int cin, int n_vie
   layout_pass_ = false;
   if (rc) return rc;
   assign_offsets();
+  layout_recs_.clear();
+  for (NetOp& op : ops_) {
+    for (auto& o : op.rec.opnd)
+      if (o.buf >= 0) o.ws_off = static_cast<long long>(bufs_[o.buf].offset);
+    layout_recs_.push_back(op.rec);
+  }
   if (dry) return MVLM_OK;
   MVLM_REQUIRE(ws_needed_ <= ws_size_, "hourglass: workspace too small (%zu needed, %zu given)", ws_needed_, ws_size_);
   // real pass: one arena for every parameter tensor, repacking kernels on a private stream (the state_dict tensors must
@@ -577,6 +635,14 @@ int HourglassNet::emit() {
   param_off_ = 0; bn_cache_.clear();
   int rc;
   const int F = 256, h2 = h / 2, w2 = w / 2;
+  // record of a top-level conv: weights "<layer>.weight", bias "<layer>.bias", optionally one BatchNorm term
+  auto conv_rec = [](const char* layer, const char* bn_name = nullptr, int term = kTermPre) {
+    OpRecord r;
+    r.layer = layer;
+    r.bias = std::string(layer) + ".bias";
+    if (bn_name) r.terms[term] = {bn_name, 0};
+    return r;
+  };
 
   // ---- stem (:405-407): image -> hi/lo bf16 staging, then conv1 on the tensor cores with the fused
   //      bias -> bn1+ReLU -> {conv2.bn1, conv2.resample.0} BatchNorm+ReLU epilogue; conv2 block (:410)
@@ -587,9 +653,16 @@ int HourglassNet::emit() {
     NetOp op;
     op.kind = NetOp::STEM;
     op.out_raw = img16.p; op.h = h; op.w = w; op.c = cin;
-    ops_.push_back(op);
+    op.rec.h = h; op.rec.w = w; op.rec.cin = cin;
+    record(op.rec, kOpOutRaw, img16.p, 16, 0);
+    push_op(op);
     const __nv_bfloat16* w1;
     ConvEpilogue e;
+    OpRecord rec;
+    rec.layer = "conv1"; rec.bias = "conv1.bias";
+    rec.terms[kTermMid] = {"bn1", 0};
+    rec.terms[kTermPre] = {"conv2.bn1", 0};
+    rec.terms[kTermPost] = {"conv2.resample.0", 0};
     if ((rc = stem_weight(&w1))) return rc;
     if ((rc = bias("conv1.bias", 64, 64, &e.bias))) return rc;
     if ((rc = bn("bn1", 64, &e.mid_scale, &e.mid_shift))) return rc;
@@ -597,7 +670,7 @@ int HourglassNet::emit() {
     if ((rc = bn("conv2.resample.0", 64, &e.post_scale, &e.post_shift))) return rc;
     e.out_pre = a_c2.p; e.pre_cs = 64; e.pre_co = 0;
     e.out_post = ar_c2.p; e.post_cs = 64; e.post_co = 0;
-    if ((rc = emit_conv("conv1", img16, 16, w1, 64, 64, 3, 3, -1, -1, e, 2.0 * 64 * cin * 9 * h * w))) return rc;
+    if ((rc = emit_conv("conv1", img16, 16, w1, 64, 64, 3, 3, -1, -1, e, 2.0 * 64 * cin * 9 * h * w, rec))) return rc;
   }
   T none, y2, y3, r3, a3, a4, a_h1, ar4;
   // conv2 block: its output is only consumed through the max-pool (:411) -> pooled outputs straight from the epilogues
@@ -618,7 +691,11 @@ int HourglassNet::emit() {
     op.kind = NetOp::BNRELU;
     op.in0 = y3.p; op.out_act = ar4.p; op.h = h2; op.w = w2; op.c = 128;
     if ((rc = bn("conv4.resample.0", 128, &op.scale, &op.shift))) return rc;
-    ops_.push_back(op);
+    op.rec.terms[kTermScale] = {"conv4.resample.0", 0};
+    op.rec.h = h2; op.rec.w = w2; op.rec.cin = 128; op.rec.in_cs = 128;
+    record(op.rec, kOpIn, y3.p, 128, 0);
+    record(op.rec, kOpOutPost, ar4.p, 128, 0);
+    push_op(op);
   }
   // the first max-pool of each hourglass (:309) is written by the block that produces its input: conv4 / conv7
   T p1, pa1, p2, pa2;
@@ -637,7 +714,8 @@ int HourglassNet::emit() {
     if ((rc = bn("bn2", F, &e.pre_scale, &e.pre_shift))) return rc;
     e.out_pre = ll1.p; e.pre_cs = F; e.pre_co = 0;
     if ((rc = packed("conv5.weight", F, F, 3, F, F, &w5)) || (rc = bias("conv5.bias", F, F, &e.bias)) ||
-        (rc = emit_conv("conv5", hg1, F, w5, F, 128, 3, 3, -1, -1, e, 2.0 * F * F * 9 * h2 * w2)))
+        (rc = emit_conv("conv5", hg1, F, w5, F, 128, 3, 3, -1, -1, e, 2.0 * F * F * 9 * h2 * w2,
+                         conv_rec("conv5", "bn2", kTermPre))))
       return rc;
   }
   T x6 = alloc(h2, w2, Lp_);
@@ -646,7 +724,7 @@ int HourglassNet::emit() {
     const __nv_bfloat16* w6;
     e.out_raw = x6.p; e.raw_cs = Lp_; e.raw_co = 0;
     if ((rc = packed("conv6.weight", L_, F, 3, Lp_, F, &w6)) || (rc = bias("conv6.bias", L_, Lp_, &e.bias)) ||
-        (rc = emit_conv("conv6", ll1, F, w6, Lp_, Lp_, 3, 3, -1, -1, e, 2.0 * L_ * F * 9 * h2 * w2)))
+        (rc = emit_conv("conv6", ll1, F, w6, Lp_, Lp_, 3, 3, -1, -1, e, 2.0 * L_ * F * 9 * h2 * w2, conv_rec("conv6"))))
       return rc;
   }
   T sum = alloc(h2, w2, F), a_h2;
@@ -667,8 +745,10 @@ int HourglassNet::emit() {
       e.out_aux2 = pa2.p; e.aux2_cs = F; e.aux2_co = 0;
     }
     const __nv_bfloat16* w7;
+    OpRecord rec = conv_rec("conv7", "hg2.rb1.bn1", kTermPost);
+    if (fuse_elt_) rec.terms[kTermAux] = {"hg2.rb2.bn1", 0};
     if ((rc = packed("conv7.weight", F, L_, 3, F, Lp_, &w7)) || (rc = bias("conv7.bias", F, F, &e.bias)) ||
-        (rc = emit_conv("conv7", x6, Lp_, w7, F, 128, 3, 3, -1, -1, e, 2.0 * F * L_ * 9 * h2 * w2)))
+        (rc = emit_conv("conv7", x6, Lp_, w7, F, 128, 3, 3, -1, -1, e, 2.0 * F * L_ * 9 * h2 * w2, rec)))
       return rc;
   }
   probe("sum_temp", sum);
@@ -682,7 +762,8 @@ int HourglassNet::emit() {
     if ((rc = bn("bn3", F, &e.pre_scale, &e.pre_shift))) return rc;
     e.out_pre = ll2.p; e.pre_cs = F; e.pre_co = 0;
     if ((rc = packed("conv9.weight", F, F, 3, F, F, &w9)) || (rc = bias("conv9.bias", F, F, &e.bias)) ||
-        (rc = emit_conv("conv9", hg2, F, w9, F, 128, 3, 3, -1, -1, e, 2.0 * F * F * 9 * h2 * w2)))
+        (rc = emit_conv("conv9", hg2, F, w9, F, 128, 3, 3, -1, -1, e, 2.0 * F * F * 9 * h2 * w2,
+                         conv_rec("conv9", "bn3", kTermPre))))
       return rc;
   }
   T x10 = alloc(h2, w2, Lp_);
@@ -691,7 +772,8 @@ int HourglassNet::emit() {
     const __nv_bfloat16* w10;
     e.out_raw = x10.p; e.raw_cs = Lp_; e.raw_co = 0;
     if ((rc = packed("conv10.weight", L_, F, 3, Lp_, F, &w10)) || (rc = bias("conv10.bias", L_, Lp_, &e.bias)) ||
-        (rc = emit_conv("conv10", ll2, F, w10, Lp_, Lp_, 3, 3, -1, -1, e, 2.0 * L_ * F * 9 * h2 * w2)))
+        (rc = emit_conv("conv10", ll2, F, w10, Lp_, Lp_, 3, 3, -1, -1, e, 2.0 * L_ * F * 9 * h2 * w2,
+                         conv_rec("conv10"))))
       return rc;
   }
   probe("x10", x10);
@@ -702,7 +784,8 @@ int HourglassNet::emit() {
     NetOp op;
     op.kind = NetOp::MEMSET;
     op.bytes = sizeof(unsigned long long) * V_ * L_;
-    ops_.push_back(op);
+    record(op.rec, kOpKeys, keys_, L_, 0);
+    push_op(op);
   }
   if ((rc = bias("conv11.bias", L_, Lp_, &b11_))) return rc;
   x10_ = x10.p;
@@ -713,10 +796,12 @@ int HourglassNet::emit() {
       e.argmax_keys = keys_;
       e.cout_real = L_;
       e.up_sy = 2; e.up_sx = 2; e.up_py = a; e.up_px = b;
+      OpRecord rec = conv_rec("conv11");
+      rec.phase_a = a; rec.phase_b = b;
       // each phase computes a quarter of the reference conv11's output pixels
       if ((rc = phase_weight(a, b, &phase_w_[2 * a + b])) ||
           (rc = emit_conv("conv11.phase", x10, Lp_, phase_w_[2 * a + b], Lp_, Lp_, 2, 2, a - 1, b - 1, e,
-                          2.0 * L_ * L_ * 9 * h2 * w2, true)))
+                          2.0 * L_ * L_ * 9 * h2 * w2, rec, true)))
         return rc;
     }
   }
@@ -725,7 +810,10 @@ int HourglassNet::emit() {
     note_use(x10.p);  // the "moment" selection re-evaluates windows of the last layer from its input
     NetOp op;
     op.kind = NetOp::PEAKS;
-    ops_.push_back(op);
+    op.rec.h = H_; op.rec.w = W_;
+    record(op.rec, kOpIn, x10.p, Lp_, 0);
+    record(op.rec, kOpKeys, keys_, L_, 0);
+    push_op(op);
   }
   return MVLM_OK;
 }

@@ -16,6 +16,20 @@ struct SdEntry {
 };
 typedef std::map<std::string, SdEntry> StateDict;
 
+// What one op computes, for the layer-wise tests (mvlm_debug_hourglass_ops): the state_dict names it applies and the
+// plan buffer (allocation index, the same in both passes of emit()) and channel slice of every tensor it touches.
+enum { kOpIn, kOpRes1, kOpRes2, kOpResUp, kOpOutPre, kOpOutRaw, kOpOutPost, kOpOutAux1, kOpOutAux2, kOpKeys,
+       kOpOperands };
+enum { kTermMid, kTermPre, kTermPost, kTermAux, kTermScale, kOpTerms };  // BatchNorm affines (pool / bnrelu: scale)
+struct OpRecord {
+  std::string layer, bias;  // conv: weight prefix ("hg1.rb5.conv2", "conv2.resample.2", "conv11"), bias key or ""
+  int phase_a = -1, phase_b = -1;  // conv11 up-sampling phase
+  struct Term { std::string bn; int off = 0; } terms[kOpTerms];  // BN name ("" = none) + channel offset into it
+  int h = 0, w = 0, cin = 0, in_cs = 0, kh = 0, kw = 0, y_off0 = 0, x_off0 = 0, cout_pad = 0, n_tile = 0,
+      cout_real = 0, pool2 = 0, aux_mode = 0;
+  struct Operand { int buf = -1, cs = 0, co = 0; long long ws_off = -1; } opnd[kOpOperands];  // ws_off: real pass
+};
+
 struct NetOp {
   enum Kind { CONV, POOL, BNRELU, STEM, MEMSET, PEAKS } kind;  // STEM = image -> hi/lo bf16 staging
   ConvParams conv;  // CONV
@@ -29,6 +43,7 @@ struct NetOp {
   size_t bytes = 0;
   bool is_head = false;  // conv11 phase: out_f32 patched per forward call
   const char* tag = "";
+  OpRecord rec;
 };
 
 class HourglassNet {
@@ -62,6 +77,11 @@ class HourglassNet {
   // one-line description of op i ("conv rb.conv 128x128 256->128 k3 pre res1 raw", "pool 64x64x256", ...)
   std::string describe_op(int i) const;
 
+  // bytes and workspace offset of plan buffer i (allocation order)
+  int n_buffers() const { return static_cast<int>(bufs_.size()); }
+  size_t buffer_bytes(int i) const { return bufs_[i].bytes; }
+  size_t buffer_offset(int i) const { return bufs_[i].offset; }
+
   size_t workspace_needed() const { return ws_needed_; }
   int n_views() const { return V_; }
   int n_landmarks() const { return L_; }
@@ -70,6 +90,7 @@ class HourglassNet {
   double flops_per_view() const { return flops_; }
   int n_ops() const { return static_cast<int>(ops_.size()); }
   const std::vector<NetOp>& ops() const { return ops_; }
+  std::vector<NetOp>& ops_mut() { return ops_; }
   // intermediate tensors exposed for layer-wise parity tests: name -> (ptr, h, w, c)
   struct Probe { const __nv_bfloat16* p; int h, w, c; };
   std::map<std::string, Probe> probes;
@@ -105,8 +126,13 @@ class HourglassNet {
   int phase_weight(int a, int b, const __nv_bfloat16** out);
   // one convolution op: the first `cin` channels of `in` through the packed weights `w` (kh x kw taps, tap (0,0) at
   // input offset (y_off0, x_off0)); `flops` = the algorithmic FLOPs of the reference layer's share this op computes
+  // `rec` carries the op's state_dict names; emit_conv adds the shape and the operands
   int emit_conv(const char* tag, T in, int cin, const __nv_bfloat16* w, int cout_pad, int n_tile, int kh, int kw,
-                int y_off0, int x_off0, const ConvEpilogue& e, double flops, bool is_head = false);
+                int y_off0, int x_off0, const ConvEpilogue& e, double flops, OpRecord rec, bool is_head = false);
+  // operand `slot` of `r` is the workspace tensor at `p` (channel stride cs, first channel co); see OpRecord
+  void record(OpRecord& r, int slot, const void* p, int cs, int co) const;
+  void push_op(NetOp& op);
+  std::vector<OpRecord> layout_recs_;  // the layout pass's records: buffer indices of the real pass's operands
   // pool_raw != nullptr: the block output is only consumed through a 2x2 max-pool (conv2 block, :410-411):
   // the three convs write the pooled raw tensor and relu(post_bn(pooled)) directly; no full-resolution output
   // up_low != nullptr: the nearest-x2 up-sampled half-resolution tensor is added to the block output
