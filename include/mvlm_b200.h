@@ -67,6 +67,17 @@ typedef struct mvlm_conv_args {
   int pool2;              /* 1: out_raw / out_post are the 2x2 max-pooled (half resolution) tensors */
   const void* res_up;     /* optional bf16 (n, h/2, w/2, up_cs): v += nearest-x2 up-sampled res_up (with res1/res2) */
   int up_cs, up_co;
+  /* optional copies for a second consumer (needs out_raw / out_post, no mid / pool2 / fp32 outputs):
+   *   aux_mode 1: out_aux1 = relu(aux_scale*bf16(raw)+aux_shift) at full resolution
+   *   aux_mode 2: out_aux1 = 2x2 max-pool of bf16(raw), out_aux2 = relu(aux_scale*out_aux1+aux_shift), both at half
+   *               resolution (even h, w) */
+  int aux_mode;
+  const float* aux_scale;
+  const float* aux_shift;
+  void* out_aux1;
+  int aux1_cs, aux1_co;
+  void* out_aux2;
+  int aux2_cs, aux2_co;
 } mvlm_conv_args;
 
 int mvlm_conv2d_bf16(const mvlm_conv_args* args, void* stream);
@@ -80,6 +91,15 @@ void mvlm_debug_conv_profile(long long* dev_buf);
 int mvlm_debug_conv_profile_ints(void);
 /* Debug experiment switch: 1 = tensor-pipe-only timing (no TMA loads; outputs are garbage), 0 = normal. */
 void mvlm_debug_conv_mode(int mode);
+/* Debug: the following conv launches of the calling thread use at most n persistent CTAs (n <= 0: one per SM), so
+ * that every CTA runs several tiles.  The kernels are unchanged. */
+void mvlm_debug_conv_max_ctas(int n);
+/* Debug: the conv kernel instantiations the library holds (feature flags, conv_epilogue.cuh); writes up to max of
+ * them and returns their number. */
+int mvlm_debug_conv_variants(int32_t* flags, int max);
+/* Debug: plans a conv without launching it: out = {instantiation flags it would run (-1: none), tile_h, n_hslots,
+ * n_wslots, w_stationary, tail, total_tiles, grid under the current mvlm_debug_conv_max_ctas}. */
+int mvlm_debug_conv_describe(const mvlm_conv_args* args, int32_t out[8]);
 
 /* fp32 OIHW (device) -> packed bf16 [cout_pad][kw][kh][cin_pad] (device), zero padded. */
 int mvlm_pack_conv_weight(const float* w_oihw, int cout, int cin, int kh, int kw, int cout_pad,

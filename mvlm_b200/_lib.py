@@ -39,6 +39,9 @@ class ConvArgs(C.Structure):
         ("mid_scale", C.c_void_p), ("mid_shift", C.c_void_p),
         ("pool2", C.c_int),
         ("res_up", C.c_void_p), ("up_cs", C.c_int), ("up_co", C.c_int),
+        ("aux_mode", C.c_int), ("aux_scale", C.c_void_p), ("aux_shift", C.c_void_p),
+        ("out_aux1", C.c_void_p), ("aux1_cs", C.c_int), ("aux1_co", C.c_int),
+        ("out_aux2", C.c_void_p), ("aux2_cs", C.c_int), ("aux2_co", C.c_int),
     ]
 
 
@@ -153,6 +156,9 @@ def _declare(lib: C.CDLL) -> None:
         "mvlm_debug_hourglass_profile": ([vp, vp, vp, vp, i32, C.POINTER(C.c_float), C.POINTER(C.c_double), i32,
                                          C.POINTER(C.c_longlong), vp], i32),
         "mvlm_debug_conv_profile_ints": ([], i32),
+        "mvlm_debug_conv_max_ctas": ([i32], None),
+        "mvlm_debug_conv_variants": ([C.POINTER(C.c_int32), i32], i32),
+        "mvlm_debug_conv_describe": ([C.POINTER(ConvArgs), C.POINTER(C.c_int32)], i32),
         "mvlm_debug_hourglass_describe": ([vp, i32, C.c_char_p, i32], i32),
         "mvlm_debug_hourglass_dry_ops": ([i32, i32, i32, i32, i32, C.POINTER(HgOp), i32, C.POINTER(i32),
                                           C.POINTER(HgBuffer), i32, C.POINTER(i32)], i32),

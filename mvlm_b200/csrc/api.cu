@@ -54,8 +54,13 @@ long long mvlm_launch_count(int reset) {
 void mvlm_debug_conv_profile(long long* dev_buf) { conv_set_profile_buffer(dev_buf); }
 int mvlm_debug_conv_profile_ints(void) { return kConvProfInts; }
 void mvlm_debug_conv_mode(int mode) { conv_set_debug_mode(mode); }
+void mvlm_debug_conv_max_ctas(int n) { conv_set_max_ctas(n); }
+int mvlm_debug_conv_variants(int32_t* flags, int max) { return conv_variants(flags, flags ? max : 0); }
 
-int mvlm_conv2d_bf16(const mvlm_conv_args* a, void* stream) {
+}  // extern "C"
+
+// mvlm_conv_args -> a planned conv
+static int plan_conv_args(const mvlm_conv_args* a, ConvParams* p) {
   MVLM_REQUIRE(a != nullptr, "mvlm_conv2d_bf16: null args");
   ConvShape s;
   s.in = static_cast<const __nv_bfloat16*>(a->in);
@@ -78,10 +83,28 @@ int mvlm_conv2d_bf16(const mvlm_conv_args* a, void* stream) {
   e.out_f32 = a->out_f32; e.argmax_keys = a->argmax_keys; e.cout_real = a->cout_real;
   e.up_sy = a->up_sy > 0 ? a->up_sy : 1; e.up_sx = a->up_sx > 0 ? a->up_sx : 1;
   e.up_py = a->up_py; e.up_px = a->up_px;
+  e.aux_mode = a->aux_mode; e.aux_scale = a->aux_scale; e.aux_shift = a->aux_shift;
+  e.out_aux1 = static_cast<__nv_bfloat16*>(a->out_aux1); e.aux1_cs = a->aux1_cs; e.aux1_co = a->aux1_co;
+  e.out_aux2 = static_cast<__nv_bfloat16*>(a->out_aux2); e.aux2_cs = a->aux2_cs; e.aux2_co = a->aux2_co;
+  return conv_plan(s, e, p);
+}
+
+extern "C" {
+
+int mvlm_conv2d_bf16(const mvlm_conv_args* a, void* stream) {
   ConvParams p;
-  int rc = conv_plan(s, e, &p);
+  const int rc = plan_conv_args(a, &p);
   if (rc != MVLM_OK) return rc;
   return conv_launch(p, static_cast<cudaStream_t>(stream));
+}
+
+int mvlm_debug_conv_describe(const mvlm_conv_args* a, int32_t out[8]) {
+  MVLM_REQUIRE(out != nullptr, "mvlm_debug_conv_describe: null output");
+  ConvParams p;
+  const int rc = plan_conv_args(a, &p);
+  if (rc != MVLM_OK) return rc;
+  conv_describe(p, out);
+  return MVLM_OK;
 }
 
 int mvlm_pack_conv_weight(const float* w_oihw, int cout, int cin, int kh, int kw, int cout_pad, int cin_pad,

@@ -488,6 +488,18 @@ EncodeTiledFn get_encode_fn() {
   return fn;
 }
 
+// debug hooks: set and read on the thread that profiles (thread-local: other threads' launches are unaffected)
+thread_local long long* g_prof_buf = nullptr;
+thread_local int g_debug_mode = 0;
+thread_local int g_max_ctas = 0;  // > 0: at most this many persistent CTAs (tests: several tiles per CTA)
+
+int launch_grid(const ConvParams& p) {
+  const int n_sms = sm_count();
+  int grid = p.total_tiles < n_sms ? p.total_tiles : n_sms;
+  if (g_max_ctas > 0 && g_max_ctas < grid) grid = g_max_ctas;
+  return grid;
+}
+
 template <int F>
 int launch_t(const ConvParams& p, cudaStream_t stream) {
   // the attribute is per device (and per kernel instantiation): one flag per device ordinal
@@ -498,8 +510,7 @@ int launch_t(const ConvParams& p, cudaStream_t stream) {
     MVLM_CHECK_CUDA(cudaFuncSetAttribute(conv_umma_kernel<F>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
     if (dev >= 0 && dev < kMaxDevices) configured[dev].store(true, std::memory_order_release);
   }
-  const int n_sms = sm_count();
-  const int grid = p.total_tiles < n_sms ? p.total_tiles : n_sms;
+  const int grid = launch_grid(p);
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(static_cast<unsigned>(grid));
   cfg.blockDim = dim3(kThreads);
@@ -517,9 +528,58 @@ int launch_t(const ConvParams& p, cudaStream_t stream) {
   return MVLM_OK;
 }
 
-// debug hooks: set and read on the thread that profiles (thread-local: other threads' launches are unaffected)
-thread_local long long* g_prof_buf = nullptr;
-thread_local int g_debug_mode = 0;
+// Every instantiation of conv_umma_kernel, X(flags).  The combinations the network plan uses (hourglass.cu) run at
+// M = 128 and, for cout <= 64, as the M = 64 .ws variant with streamed weights or, with 3 x 3 taps over stationary
+// weights, the variant whose MMA warp issues a tile's MMAs straight-line (MVLM_CONV_ALL_M); some exist at M = 128 only.
+#define MVLM_CONV_ALL_M(X, FLAGS) X(FLAGS) X((FLAGS) | F_M64) X((FLAGS) | F_M64 | F_STAT)
+#define MVLM_CONV_VARIANTS(X)                                                        \
+  MVLM_CONV_ALL_M(X, F_PRE | F_RES1 | F_RAW | F_POST)    /* RB conv1/2 */           \
+  MVLM_CONV_ALL_M(X, F_PRE | F_RES1 | F_RAW)                                        \
+  MVLM_CONV_ALL_M(X, F_RES1 | F_RAW | F_POST)            /* RB conv3 */             \
+  MVLM_CONV_ALL_M(X, F_RES1 | F_RAW)                                                \
+  MVLM_CONV_ALL_M(X, F_RAW)                              /* resample, conv6/10 */   \
+  X(F_PRE)                                               /* conv5, conv9 */         \
+  X(F_RES1 | F_RES2 | F_RAW | F_POST)                    /* conv7 */                \
+  X(F_ARGMAX)                                            /* conv11 phases */        \
+  X(F_ARGMAX | F_STAT)  /* conv11 phases: 2 x 2 taps over stationary weights at M = 128, straight-line issue */ \
+  MVLM_CONV_ALL_M(X, F_F32)                                                         \
+  MVLM_CONV_ALL_M(X, F_F32 | F_ARGMAX)                                              \
+  MVLM_CONV_ALL_M(X, F_MID | F_PRE | F_POST)             /* stem (conv1) */         \
+  MVLM_CONV_ALL_M(X, F_POOL | F_PRE | F_RES1 | F_RAW | F_POST)  /* conv2 block: pooled outputs only */ \
+  MVLM_CONV_ALL_M(X, F_POOL | F_RES1 | F_RAW | F_POST)                              \
+  MVLM_CONV_ALL_M(X, F_POOL | F_RAW)                                                \
+  X(F_PRE | F_RES1 | F_RES2 | F_RAW | F_POST)                                       \
+  /* skip-branch ResidualBlocks with the up-sampled low path added in the epilogue (hourglass up path) */ \
+  MVLM_CONV_ALL_M(X, F_UP | F_PRE | F_RES1 | F_RAW | F_POST)                        \
+  MVLM_CONV_ALL_M(X, F_UP | F_PRE | F_RES1 | F_RAW)                                 \
+  MVLM_CONV_ALL_M(X, F_UP | F_RES1 | F_RAW | F_POST)                                \
+  MVLM_CONV_ALL_M(X, F_UP | F_RES1 | F_RAW)                                         \
+  /* producers that also write the copies of a fused BatchNorm+ReLU / max-pool pass (aux_mode 1 / 2) */ \
+  MVLM_CONV_ALL_M(X, F_POST2 | F_PRE | F_RES1 | F_RAW | F_POST)                     \
+  MVLM_CONV_ALL_M(X, F_POST2 | F_RES1 | F_RAW | F_POST)                             \
+  MVLM_CONV_ALL_M(X, F_POOLX | F_PRE | F_RES1 | F_RAW | F_POST)                     \
+  MVLM_CONV_ALL_M(X, F_POOLX | F_RES1 | F_RAW | F_POST)                             \
+  X(F_POOLX | F_RES1 | F_RES2 | F_RAW | F_POST)
+
+#define MVLM_CONV_FLAGS(FLAGS) (FLAGS),
+constexpr int kConvVariants[] = {MVLM_CONV_VARIANTS(MVLM_CONV_FLAGS)};
+#undef MVLM_CONV_FLAGS
+constexpr int kNumConvVariants = static_cast<int>(sizeof(kConvVariants) / sizeof(kConvVariants[0]));
+
+// The instantiation a planned conv runs (its feature mask + F_M64 / F_STAT), or -1 when there is none.
+int conv_variant(const ConvParams& p) {
+  int v = feature_mask(p.e);
+  if (p.s.cout_pad <= 64) {
+    // cout <= 64 layers run the M = 64 variant (conv_plan chose the ring geometry accordingly), and, with 3 x 3 taps
+    // over stationary weights, the one whose MMA warp issues a tile's MMAs straight-line
+    v |= F_M64 | (p.w_stationary && p.s.kw == 3 && p.s.kh == 3 ? F_STAT : 0);
+  } else if (v == F_ARGMAX && p.w_stationary && p.s.kw == 2 && p.s.kh == 2) {
+    v |= F_STAT;  // the conv11 phase kernels
+  }
+  for (int i = 0; i < kNumConvVariants; ++i)
+    if (kConvVariants[i] == v) return v;
+  return -1;
+}
 
 }  // namespace
 
@@ -676,58 +736,36 @@ int conv_plan(const ConvShape& s, const ConvEpilogue& e, ConvParams* out) {
 
 void conv_set_profile_buffer(long long* dev_buf) { g_prof_buf = dev_buf; }
 void conv_set_debug_mode(int mode) { g_debug_mode = mode; }
+void conv_set_max_ctas(int n) { g_max_ctas = n > 0 ? n : 0; }
+
+int conv_variants(int32_t* flags, int max) {
+  for (int i = 0; i < kNumConvVariants && i < max; ++i) flags[i] = kConvVariants[i];
+  return kNumConvVariants;
+}
+
+void conv_describe(const ConvParams& p, int32_t out[8]) {
+  out[0] = conv_variant(p);
+  out[1] = p.tile_h;
+  out[2] = p.n_hslots;
+  out[3] = p.n_wslots;
+  out[4] = p.w_stationary;
+  out[5] = p.tail;
+  out[6] = p.total_tiles;
+  out[7] = launch_grid(p);
+}
 
 int conv_launch(const ConvParams& p_in, cudaStream_t stream) {
   ConvParams p = p_in;
   p.prof = g_prof_buf;
   p.debug_mode = g_debug_mode;
-  const ConvEpilogue& e = p.e;
-  const int f = feature_mask(e);
-  // cout <= 64 layers run the M = 64 variant (conv_plan chose the ring geometry accordingly)
-  const bool m64 = p.s.cout_pad <= 64;
-  // ... and, with 3 x 3 taps over stationary weights, the variant whose MMA warp issues a tile's MMAs straight-line
-  const bool stat = m64 && p.w_stationary && p.s.kw == 3 && p.s.kh == 3;
-#define MVLM_CASE_BOTH(FLAGS) \
+  switch (conv_variant(p)) {
+#define MVLM_CONV_CASE(FLAGS) \
   case (FLAGS):               \
-    return m64 ? (stat ? launch_t<(FLAGS) | F_M64 | F_STAT>(p, stream) : launch_t<(FLAGS) | F_M64>(p, stream)) : launch_t<(FLAGS)>(p, stream)
-#define MVLM_CASE_128(FLAGS) \
-  case (FLAGS):              \
-    if (!m64) return launch_t<(FLAGS)>(p, stream); \
-    break
-  // the conv11 phase kernels: 2 x 2 taps over stationary weights at M = 128, straight-line issue as well
-  if (f == F_ARGMAX && !m64 && p.w_stationary && p.s.kw == 2 && p.s.kh == 2) return launch_t<F_ARGMAX | F_STAT>(p, stream);
-  switch (f) {
-    // the combinations the network plan uses (hourglass.cu)
-    MVLM_CASE_BOTH(F_PRE | F_RES1 | F_RAW | F_POST);  // RB conv1/2
-    MVLM_CASE_BOTH(F_PRE | F_RES1 | F_RAW);
-    MVLM_CASE_BOTH(F_RES1 | F_RAW | F_POST);          // RB conv3
-    MVLM_CASE_BOTH(F_RES1 | F_RAW);
-    MVLM_CASE_BOTH(F_RAW);                            // resample, conv6/10
-    MVLM_CASE_128(F_PRE);                             // conv5, conv9
-    MVLM_CASE_128(F_RES1 | F_RES2 | F_RAW | F_POST);  // conv7
-    MVLM_CASE_128(F_ARGMAX);                          // conv11 phases
-    MVLM_CASE_BOTH(F_F32);
-    MVLM_CASE_BOTH(F_F32 | F_ARGMAX);
-    MVLM_CASE_BOTH(F_MID | F_PRE | F_POST);           // stem (conv1)
-    MVLM_CASE_BOTH(F_POOL | F_PRE | F_RES1 | F_RAW | F_POST);  // conv2 block: pooled outputs only
-    MVLM_CASE_BOTH(F_POOL | F_RES1 | F_RAW | F_POST);
-    MVLM_CASE_BOTH(F_POOL | F_RAW);
-    MVLM_CASE_128(F_PRE | F_RES1 | F_RES2 | F_RAW | F_POST);
-    // skip-branch ResidualBlocks with the up-sampled low path added in the epilogue (hourglass up path)
-    MVLM_CASE_BOTH(F_UP | F_PRE | F_RES1 | F_RAW | F_POST);
-    MVLM_CASE_BOTH(F_UP | F_PRE | F_RES1 | F_RAW);
-    MVLM_CASE_BOTH(F_UP | F_RES1 | F_RAW | F_POST);
-    MVLM_CASE_BOTH(F_UP | F_RES1 | F_RAW);
-    // producers that also write the copies of a fused BatchNorm+ReLU / max-pool pass (aux_mode 1 / 2)
-    MVLM_CASE_BOTH(F_POST2 | F_PRE | F_RES1 | F_RAW | F_POST);
-    MVLM_CASE_BOTH(F_POST2 | F_RES1 | F_RAW | F_POST);
-    MVLM_CASE_BOTH(F_POOLX | F_PRE | F_RES1 | F_RAW | F_POST);
-    MVLM_CASE_BOTH(F_POOLX | F_RES1 | F_RAW | F_POST);
-    MVLM_CASE_128(F_POOLX | F_RES1 | F_RES2 | F_RAW | F_POST);
+    return launch_t<(FLAGS)>(p, stream);
+    MVLM_CONV_VARIANTS(MVLM_CONV_CASE)
+#undef MVLM_CONV_CASE
   }
-#undef MVLM_CASE_BOTH
-#undef MVLM_CASE_128
-  set_error("conv_launch: unsupported epilogue combination 0x%x (cout_pad %d)", f, p.s.cout_pad);
+  set_error("conv_launch: unsupported epilogue combination 0x%x (cout_pad %d)", feature_mask(p.e), p.s.cout_pad);
   return MVLM_E_UNSUPPORTED;
 }
 

@@ -112,5 +112,12 @@ constexpr int kConvTraceTiles = 64;
 constexpr int kConvProfInts = 148 * 8 + kConvTraceTiles * 16;
 void conv_set_profile_buffer(long long* dev_buf);
 void conv_set_debug_mode(int mode);
+// Debug: at most n CTAs per launch on the calling thread (0: one per SM), so that tests run several tiles per CTA.
+void conv_set_max_ctas(int n);
+// The supported kernel instantiations (feature flags incl. F_M64 / F_STAT); returns their number, writes up to max.
+int conv_variants(int32_t* flags, int max);
+// What conv_launch would run for a planned conv: instantiation flags (-1: unsupported), tile_h, n_hslots, n_wslots,
+// w_stationary, tail, total_tiles and the grid under the calling thread's CTA cap.
+void conv_describe(const ConvParams& p, int32_t out[8]);
 
 }  // namespace mvlm

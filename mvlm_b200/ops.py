@@ -31,7 +31,7 @@ def conv2d_bf16(x: torch.Tensor, wpacked: torch.Tensor, *, cin: int | None = Non
                 kh: int = 3, kw: int = 3, y_off0: int | None = None, x_off0: int | None = None,
                 bias=None, mid=None, pre=None, res1=None, res2=None, out_raw=None, post=None,
                 out_f32=None, argmax_keys=None, cout_real: int | None = None,
-                up=(1, 1, 0, 0), pool2: bool = False, res_up=None) -> None:
+                up=(1, 1, 0, 0), pool2: bool = False, res_up=None, aux=None) -> None:
     """One fused conv launch.
 
     x          : (N,H,W,Cs) bf16; the first `cin` channels are read.
@@ -39,8 +39,57 @@ def conv2d_bf16(x: torch.Tensor, wpacked: torch.Tensor, *, cin: int | None = Non
     res1/res2  : (tensor bf16 (N,H,W,Cs'), channel offset)
     res_up     : (tensor bf16 (N,H/2,W/2,Cs'), channel offset), added with nearest x2 up-sampling
     out_raw    : (tensor bf16 (N,H,W,Cs'), channel offset)
+    aux        : (mode, scale f32[cout_pad], shift f32[cout_pad], out1 bf16, channel offset 1, out2 bf16 | None,
+                  channel offset 2): mode 1 out1 = relu(scale * bf16(raw) + shift); mode 2 out1 = max-pool 2x2 of
+                  bf16(raw), out2 = relu(scale * out1 + shift), both at half resolution
     """
+    a = _conv_args(x, wpacked, cin=cin, n_tile=n_tile, kh=kh, kw=kw, y_off0=y_off0, x_off0=x_off0, bias=bias, mid=mid,
+                   pre=pre, res1=res1, res2=res2, out_raw=out_raw, post=post, out_f32=out_f32, argmax_keys=argmax_keys,
+                   cout_real=cout_real, up=up, pool2=pool2, res_up=res_up, aux=aux)
+    check(_lib.load().mvlm_conv2d_bf16(C.byref(a), cur_stream()), "mvlm_conv2d_bf16")
+
+
+class ConvPlanInfo(NamedTuple):
+    """What one conv2d_bf16 call would run (mvlm_debug_conv_describe)."""
+    variant: int       # instantiation flags, -1: none
+    tile_h: int
+    n_hslots: int
+    n_wslots: int
+    w_stationary: int
+    tail: int
+    total_tiles: int
+    grid: int          # CTAs under the current conv_max_ctas cap
+
+
+def conv_describe(x: torch.Tensor, wpacked: torch.Tensor, **kw) -> ConvPlanInfo:
+    """Plans conv2d_bf16(x, wpacked, **kw) without launching it: kw are conv2d_bf16's keyword arguments (_conv_args
+    spells them out and raises on any other)."""
+    a = _conv_args(x, wpacked, **kw)
+    out = (C.c_int32 * 8)()
+    check(_lib.load().mvlm_debug_conv_describe(C.byref(a), out), "mvlm_debug_conv_describe")
+    return ConvPlanInfo(*out)
+
+
+def conv_variants() -> list[int]:
+    """Feature flags of every conv kernel instantiation the library holds."""
     lib = _lib.load()
+    n = lib.mvlm_debug_conv_variants(None, 0)
+    out = (C.c_int32 * n)()
+    lib.mvlm_debug_conv_variants(out, n)
+    return list(out)
+
+
+def set_conv_max_ctas(n: int) -> None:
+    """Debug: conv launches of this thread use at most n persistent CTAs (0: one per SM)."""
+    _lib.load().mvlm_debug_conv_max_ctas(n)
+
+
+def _conv_args(x: torch.Tensor, wpacked: torch.Tensor, *, cin: int | None = None, n_tile: int,
+               kh: int = 3, kw: int = 3, y_off0: int | None = None, x_off0: int | None = None,
+               bias=None, mid=None, pre=None, res1=None, res2=None, out_raw=None, post=None,
+               out_f32=None, argmax_keys=None, cout_real: int | None = None,
+               up=(1, 1, 0, 0), pool2: bool = False, res_up=None, aux=None) -> ConvArgs:
+    """The mvlm_conv_args of one conv2d_bf16 call (the arguments are conv2d_bf16's)."""
     n, h, w, cs = x.shape
     a = ConvArgs()
     a.in_ = ptr(x)
@@ -72,7 +121,13 @@ def conv2d_bf16(x: torch.Tensor, wpacked: torch.Tensor, *, cin: int | None = Non
     a.pool2 = 1 if pool2 else 0
     if res_up is not None:
         a.res_up, a.up_cs, a.up_co = ptr(res_up[0]), res_up[0].shape[-1], res_up[1]
-    check(lib.mvlm_conv2d_bf16(C.byref(a), cur_stream()), "mvlm_conv2d_bf16")
+    if aux is not None:
+        mode, scale, shift, out1, co1, out2, co2 = aux
+        a.aux_mode, a.aux_scale, a.aux_shift = mode, ptr(scale), ptr(shift)
+        a.out_aux1, a.aux1_cs, a.aux1_co = ptr(out1), out1.shape[-1], co1
+        if out2 is not None:
+            a.out_aux2, a.aux2_cs, a.aux2_co = ptr(out2), out2.shape[-1], co2
+    return a
 
 
 # --------------------------------------------------------------------------------------------

@@ -266,7 +266,7 @@ def layer_weight(sd, op, lp):
     return out
 
 
-def _conv(x_nhwc, w, y_off0, x_off0):
+def conv(x_nhwc, w, y_off0, x_off0):
     """NHWC fp64 conv whose tap (ky, kx) reads input (y + y_off0 + ky, x + x_off0 + kx), zero outside."""
     kh, kw = w.shape[-2:]
     x = x_nhwc.permute(0, 3, 1, 2)
@@ -299,8 +299,8 @@ def conv_ref(sd, op, x, res, lp, perturb=None):
         w = layer_weight(sd, wop, lp)
     if perturb == "shift_in":
         x = torch.roll(x, 1, dims=2)
-    v = _conv(x, w, op["y_off0"], op["x_off0"])
-    A = _conv(x.abs(), w.abs(), op["y_off0"], op["x_off0"])
+    v = conv(x, w, op["y_off0"], op["x_off0"])
+    A = conv(x.abs(), w.abs(), op["y_off0"], op["x_off0"])
     if op["bias"] and perturb != "bias":
         b = torch.zeros(cout, dtype=torch.float64, device=v.device)
         bb = sd[op["bias"]].double()
