@@ -426,6 +426,20 @@ int mvlm_consensus_multiscan(const float* peaks, const double* starts, const dou
                              double dist_thres, void* workspace, size_t workspace_bytes,
                              double* out_landmarks /* (S,L,3) */, double* out_errors /* (S,L) */,
                              int32_t* out_nlines /* (S,L) or NULL */, void* stream);
+/* The same consensus plus a per-landmark report of the final fit, one launch more (DESIGN.md 7h).  Landmarks,      */
+/* errors and line counts are exactly mvlm_consensus_multiscan's; the workspace is the same.  Report outputs, all   */
+/* required: status 0 = a hypothesis was accepted, 1 = none was (LSQ over all kept lines), 2 = fewer than 3 lines;  */
+/* n_inliers = lines of the final fit; inliers[s][l][v] = 1 when view v's line is one of them (views the filter     */
+/* removed: 0); rms = sqrt(mean squared distance of those lines to the landmark), NaN without lines; covariance =   */
+/* sigma^2 J^-1 row-major with J = sum (I - n n^T), sigma^2 = sum d^2 / (2k - 3), NaN when k < 2 or J is singular. */
+int mvlm_consensus_multiscan_report(const float* peaks, const double* starts, const double* ends, int n_scans,
+                                    int n_landmarks, int n_views, int mode, double threshold_quantile,
+                                    float threshold_absolute, const uint32_t* draws, int draws_per_scan, int n_hyp,
+                                    double dist_thres, void* workspace, size_t workspace_bytes,
+                                    double* out_landmarks /* (S,L,3) */, double* out_errors /* (S,L) */,
+                                    int32_t* out_nlines /* (S,L) or NULL */, int8_t* out_status /* (S,L) */,
+                                    int32_t* out_ninliers /* (S,L) */, uint8_t* out_inliers /* (S,L,V) */,
+                                    double* out_rms /* (S,L) */, double* out_covariance /* (S,L,9) */, void* stream);
 
 /* ------------------------------------------------------------------------- */
 /* Stage 5b: snap to the mesh surface.  Replaces                               */

@@ -4,7 +4,8 @@ import sys
 
 import mvlm_b200
 from mvlm_b200 import pipeline, prediction, utils  # noqa: F401
+from mvlm_b200.report import LandmarkReport  # noqa: F401
 
-__all__ = ["pipeline", "utils", "prediction"]
-for _n in __all__:
+__all__ = ["pipeline", "utils", "prediction", "LandmarkReport"]
+for _n in ("pipeline", "utils", "prediction"):
     sys.modules[f"mvlm.{_n}"] = getattr(mvlm_b200, _n)

@@ -7,12 +7,16 @@
 All device work goes through libmvlm_b200.so (hand-written sm_100a CUDA, C-ABI in
 include/mvlm_b200.h); there is no CPU fallback.
 """
-__all__ = ["pipeline", "utils", "prediction"]
+__all__ = ["pipeline", "utils", "prediction", "LandmarkReport"]
 __version__ = "0.1.0"
 
 
 def __getattr__(name):
     # lazy: `import mvlm_b200.build` must work before the shared library exists
+    if name == "LandmarkReport":
+        from .report import LandmarkReport
+
+        return LandmarkReport
     if name in __all__:
         import importlib
 

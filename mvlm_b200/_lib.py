@@ -201,6 +201,8 @@ def _declare(lib: C.CDLL) -> None:
         "mvlm_consensus_multiscan_workspace_bytes": ([i32, i32, i32, i32], C.c_size_t),
         "mvlm_consensus_multiscan": ([vp, vp, vp, i32, i32, i32, i32, f64, f32, vp, i32, i32, f64, vp, C.c_size_t, vp, vp,
                                       vp, vp], i32),
+        "mvlm_consensus_multiscan_report": ([vp, vp, vp, i32, i32, i32, i32, f64, f32, vp, i32, i32, f64, vp, C.c_size_t,
+                                             vp, vp, vp, vp, vp, vp, vp, vp, vp], i32),
         "mvlm_snap_workspace_bytes": ([i32, i32], C.c_size_t),
         "mvlm_snap_to_meshes_workspace_bytes": ([C.POINTER(SnapMesh), i32, i32], C.c_size_t),
         "mvlm_snap_to_meshes": ([C.POINTER(SnapMesh), i32, vp, i32, vp, C.c_size_t, vp, vp, vp], i32),

@@ -349,11 +349,12 @@ size_t mvlm_consensus_multiscan_workspace_bytes(int n_scans, int n_landmarks, in
   return consensus_workspace_bytes(n_landmarks, n_views, n_hyp, n_scans);
 }
 
-int mvlm_consensus_multiscan(const float* peaks, const double* starts, const double* ends, int n_scans,
+namespace {
+ConsensusArgs consensus_args(const float* peaks, const double* starts, const double* ends, int n_scans,
                              int n_landmarks, int n_views, int mode, double threshold_quantile,
                              float threshold_absolute, const uint32_t* draws, int draws_per_scan, int n_hyp,
                              double dist_thres, void* workspace, size_t workspace_bytes, double* out_landmarks,
-                             double* out_errors, int32_t* out_nlines, void* stream) {
+                             double* out_errors, int32_t* out_nlines) {
   ConsensusArgs a;
   a.peaks = peaks; a.starts = starts; a.ends = ends; a.l = n_landmarks; a.v = n_views; a.n_scans = n_scans;
   a.mode = mode;
@@ -362,7 +363,35 @@ int mvlm_consensus_multiscan(const float* peaks, const double* starts, const dou
   a.draws_scan_stride = draws_per_scan ? static_cast<size_t>(n_landmarks) * n_hyp * 8 : 0;
   a.workspace = workspace; a.workspace_bytes = workspace_bytes;
   a.out_landmarks = out_landmarks; a.out_errors = out_errors; a.out_nlines = out_nlines;
-  return consensus_launch(a, static_cast<cudaStream_t>(stream));
+  return a;
+}
+}  // namespace
+
+int mvlm_consensus_multiscan(const float* peaks, const double* starts, const double* ends, int n_scans,
+                             int n_landmarks, int n_views, int mode, double threshold_quantile,
+                             float threshold_absolute, const uint32_t* draws, int draws_per_scan, int n_hyp,
+                             double dist_thres, void* workspace, size_t workspace_bytes, double* out_landmarks,
+                             double* out_errors, int32_t* out_nlines, void* stream) {
+  return consensus_launch(consensus_args(peaks, starts, ends, n_scans, n_landmarks, n_views, mode, threshold_quantile,
+                                         threshold_absolute, draws, draws_per_scan, n_hyp, dist_thres, workspace,
+                                         workspace_bytes, out_landmarks, out_errors, out_nlines),
+                          static_cast<cudaStream_t>(stream));
+}
+
+int mvlm_consensus_multiscan_report(const float* peaks, const double* starts, const double* ends, int n_scans,
+                                    int n_landmarks, int n_views, int mode, double threshold_quantile,
+                                    float threshold_absolute, const uint32_t* draws, int draws_per_scan, int n_hyp,
+                                    double dist_thres, void* workspace, size_t workspace_bytes, double* out_landmarks,
+                                    double* out_errors, int32_t* out_nlines, int8_t* out_status,
+                                    int32_t* out_ninliers, uint8_t* out_inliers, double* out_rms,
+                                    double* out_covariance, void* stream) {
+  ConsensusReport r;
+  r.status = reinterpret_cast<signed char*>(out_status); r.n_inliers = out_ninliers; r.inliers = out_inliers;
+  r.rms = out_rms; r.covariance = out_covariance;
+  return consensus_launch(consensus_args(peaks, starts, ends, n_scans, n_landmarks, n_views, mode, threshold_quantile,
+                                         threshold_absolute, draws, draws_per_scan, n_hyp, dist_thres, workspace,
+                                         workspace_bytes, out_landmarks, out_errors, out_nlines),
+                          static_cast<cudaStream_t>(stream), &r);
 }
 
 size_t mvlm_snap_workspace_bytes(int n_landmarks, int n_tris) { return snap_workspace_bytes(n_landmarks, n_tris); }

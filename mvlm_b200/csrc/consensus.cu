@@ -25,6 +25,8 @@
 //                         normal-equation sums -> inlier refit -> score pass), warp-shuffle + shared
 //                         memory reduction of the lexicographic (error, hypothesis) minimum.
 //   consensus_finalize    lexicographic (error, hypothesis) minimum over splits, fallbacks.
+//   consensus_report      (only when report outputs are given) one block per (landmark, scan): status, inlier mask
+//                         in view order, counts, rms and covariance of the final fit (DESIGN.md 7h).
 #include "common.cuh"
 #include "stages.cuh"
 
@@ -37,11 +39,14 @@ constexpr int kMaxViews = 1024;
 constexpr int kPartDoubles = 5;   // err, hyp, p[3]
 constexpr double kNoFit = 100000000.0;  // estimator3d.py:95
 
-// Minimum-norm solve of the symmetric 3x3 system S p = c via Jacobi eigen-decomposition,
-// singular values below 1e-15 * max are dropped (np.linalg.pinv default rcond, utils3d.py:123).
-__device__ void sym3_pinv_solve(const double* S6, const double* c, double* p) {
+// Jacobi eigen-decomposition of the symmetric 3x3 matrix S6 = {xx,yy,zz,xy,xz,yz}: eigenvalues lam[k], eigenvector k
+// in column k of v.
+__device__ __forceinline__ void sym3_jacobi(const double* S6, double lam[3], double v[3][3]) {
   double a[3][3] = {{S6[0], S6[3], S6[4]}, {S6[3], S6[1], S6[5]}, {S6[4], S6[5], S6[2]}};
-  double v[3][3] = {{1, 0, 0}, {0, 1, 0}, {0, 0, 1}};
+#pragma unroll
+  for (int r = 0; r < 3; ++r)
+#pragma unroll
+    for (int k = 0; k < 3; ++k) v[r][k] = r == k ? 1.0 : 0.0;
   for (int sweep = 0; sweep < 12; ++sweep) {
     const double off = a[0][1] * a[0][1] + a[0][2] * a[0][2] + a[1][2] * a[1][2];
     const double diag = a[0][0] * a[0][0] + a[1][1] * a[1][1] + a[2][2] * a[2][2];
@@ -73,10 +78,20 @@ __device__ void sym3_pinv_solve(const double* S6, const double* c, double* p) {
       }
     }
   }
-  const double l0 = a[0][0], l1 = a[1][1], l2 = a[2][2];
-  const double lmax = fmax(fabs(l0), fmax(fabs(l1), fabs(l2)));
-  const double cut = 1e-15 * lmax;
-  const double lam[3] = {l0, l1, l2};
+  lam[0] = a[0][0]; lam[1] = a[1][1]; lam[2] = a[2][2];
+}
+
+// Eigenvalues at or below this are dropped as singular (np.linalg.pinv default rcond, utils3d.py:123).
+__device__ __forceinline__ double sym3_cut(const double lam[3]) {
+  return 1e-15 * fmax(fabs(lam[0]), fmax(fabs(lam[1]), fabs(lam[2])));
+}
+
+// Minimum-norm solve of the symmetric 3x3 system S p = c via the Jacobi eigen-decomposition, singular values at or
+// below sym3_cut dropped.
+__device__ void sym3_pinv_solve(const double* S6, const double* c, double* p) {
+  double lam[3], v[3][3];
+  sym3_jacobi(S6, lam, v);
+  const double cut = sym3_cut(lam);
   p[0] = p[1] = p[2] = 0.0;
 #pragma unroll
   for (int k = 0; k < 3; ++k) {
@@ -126,22 +141,23 @@ __host__ __device__ inline Layout carve(void* ws, int L, int V, int splits) {
   return o;
 }
 
-__global__ void __launch_bounds__(256) consensus_prepare_kernel(ConsensusArgs g, Layout ws) {
-  __shared__ float vals[kMaxViews];
-  __shared__ unsigned char keep[kMaxViews];
-  __shared__ float sel[2];
-  __shared__ int any_nan;
-  __shared__ double red[9][8];
+// Row of landmark l's views of scan s in the (L, S*V, 3) peaks / rays.
+__device__ __forceinline__ size_t view_row(const ConsensusArgs& g, int l, int s) {
+  return static_cast<size_t>(l) * g.n_scans * g.v + static_cast<size_t>(s) * g.v;
+}
+
+// Heat-value line filter of one (landmark, scan) slot, called by the whole block: keep[i] = 1 for the views i whose
+// value is strictly above the quantile / absolute threshold.  vals (V floats), keep (V bytes), sel (2 floats) and
+// any_nan are the caller's shared memory; returns after a barrier, with keep complete.
+__device__ void filter_keep_mask(const ConsensusArgs& g, size_t row, float* vals, unsigned char* keep, float* sel,
+                                 int* any_nan) {
   const int V = g.v, tid = threadIdx.x;
-  const int sl = blockIdx.y * g.l + blockIdx.x;  // (scan, landmark) slot
-  // row of this landmark's views of this scan in the (L, S*V, 3) peaks / rays
-  const size_t row = static_cast<size_t>(blockIdx.x) * g.n_scans * V + static_cast<size_t>(blockIdx.y) * V;
-  if (tid == 0) { any_nan = 0; sel[0] = sel[1] = 0.f; }
+  if (tid == 0) { *any_nan = 0; sel[0] = sel[1] = 0.f; }
   __syncthreads();
   for (int i = tid; i < V; i += blockDim.x) {
     const float x = g.peaks[(row + i) * 3 + 2];
     vals[i] = x;
-    if (x != x) any_nan = 1;
+    if (x != x) *any_nan = 1;
   }
   __syncthreads();
   float thr;
@@ -172,10 +188,22 @@ __global__ void __launch_bounds__(256) consensus_prepare_kernel(ConsensusArgs g,
     const float diff = b - a;
     thr = a + diff * t;
     if (t >= 0.5f) thr = b - diff * (1.0f - t);
-    if (any_nan) thr = NAN;  // np.quantile -> nan -> every comparison False
+    if (*any_nan) thr = NAN;  // np.quantile -> nan -> every comparison False
   }
   for (int i = tid; i < V; i += blockDim.x) keep[i] = vals[i] > thr ? 1 : 0;
   __syncthreads();
+}
+
+__global__ void __launch_bounds__(256) consensus_prepare_kernel(ConsensusArgs g, Layout ws) {
+  __shared__ float vals[kMaxViews];
+  __shared__ unsigned char keep[kMaxViews];
+  __shared__ float sel[2];
+  __shared__ int any_nan;
+  __shared__ double red[9][8];
+  const int V = g.v, tid = threadIdx.x;
+  const int sl = blockIdx.y * g.l + blockIdx.x;  // (scan, landmark) slot
+  const size_t row = view_row(g, blockIdx.x, blockIdx.y);
+  filter_keep_mask(g, row, vals, keep, sel, &any_nan);
   double acc[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
   int n_kept = 0;
   for (int i = 0; i < V; ++i) n_kept += keep[i];  // every thread: tiny V
@@ -312,21 +340,26 @@ __global__ void __launch_bounds__(256) consensus_hyp_kernel(ConsensusArgs g, Lay
   }
 }
 
+// Split holding a slot's winning hypothesis: the lexicographic (error, hypothesis) minimum over the splits' partial
+// results; -1 when no split accepted one.  part = the slot's `splits` records of kPartDoubles.
+__device__ __forceinline__ int winning_split(const double* part, int splits) {
+  int bs = -1;
+  for (int s = 0; s < splits; ++s) {
+    const double* q = part + s * kPartDoubles;
+    if (q[1] < 0.0) continue;
+    if (bs < 0 || q[0] < part[bs * kPartDoubles] ||
+        (q[0] == part[bs * kPartDoubles] && q[1] < part[bs * kPartDoubles + 1]))
+      bs = s;
+  }
+  return bs;
+}
+
 __global__ void consensus_finalize_kernel(ConsensusArgs g, Layout ws, int splits) {
   const int l = blockIdx.x * blockDim.x + threadIdx.x;  // (scan, landmark) slot
   if (l >= g.l * g.n_scans) return;
   const int n = ws.nl[l];
   const double* part = ws.part + static_cast<size_t>(l) * splits * kPartDoubles;
-  int bs = -1;
-  if (n >= 3) {
-    for (int s = 0; s < splits; ++s) {
-      const double* q = part + s * kPartDoubles;
-      if (q[1] < 0.0) continue;
-      if (bs < 0 || q[0] < part[bs * kPartDoubles] ||
-          (q[0] == part[bs * kPartDoubles] && q[1] < part[bs * kPartDoubles + 1]))
-        bs = s;
-    }
-  }
+  const int bs = n >= 3 ? winning_split(part, splits) : -1;
   double* o = g.out_landmarks + 3 * l;
   if (bs >= 0) {
     const double* q = part + bs * kPartDoubles;
@@ -338,6 +371,100 @@ __global__ void consensus_finalize_kernel(ConsensusArgs g, Layout ws, int splits
     // over all lines, error stays 1e8 (:131-133)
     g.out_errors[l] = n < 3 ? 0.0 : kNoFit;
   }
+}
+
+// One block per (landmark, scan) slot, after finalize, on the same workspace: which lines the final fit used and how
+// well they agree.  The filter and the winner are the ones prepare and finalize computed (same functions, same
+// inputs); the winner's 8-line point, inlier test, refit and squared distances repeat consensus_hyp_kernel's
+// arithmetic in its order, so the inlier set is the one the hypothesis kernel scored and the refit point is
+// out_landmarks bit for bit (status 0: rms^2 sums exactly what out_errors sums).  The per-line sums run on one thread
+// in line order; every other thread only rebuilds the filter and writes the mask.
+__global__ void __launch_bounds__(256) consensus_report_kernel(ConsensusArgs g, Layout ws, int splits,
+                                                               ConsensusReport r) {
+  __shared__ float vals[kMaxViews];
+  __shared__ unsigned char keep[kMaxViews];
+  __shared__ unsigned char used[kMaxViews];  // by compacted line position
+  __shared__ short pos_of[kMaxViews];        // compacted line position of each kept view
+  __shared__ float sel[2];
+  __shared__ int any_nan;
+  const int V = g.v, tid = threadIdx.x;
+  const int slot = blockIdx.y * g.l + blockIdx.x;  // (scan, landmark) slot
+  filter_keep_mask(g, view_row(g, blockIdx.x, blockIdx.y), vals, keep, sel, &any_nan);
+  for (int i = tid; i < V; i += blockDim.x) {
+    if (!keep[i]) continue;
+    int pos = 0;
+    for (int j = 0; j < i; ++j) pos += keep[j];
+    pos_of[i] = static_cast<short>(pos);
+  }
+  const int n = ws.nl[slot];
+  if (tid == 0) {
+    const double* lines = ws.lines + static_cast<size_t>(slot) * V * kLineDoubles;
+    const double* part = ws.part + static_cast<size_t>(slot) * splits * kPartDoubles;
+    const int bs = n >= 3 ? winning_split(part, splits) : -1;
+    double c[3];  // the consensus point
+    int k;        // lines of the final fit
+    signed char status;
+    if (bs >= 0) {
+      // --- the winner's 8-line LSQ, inliers and refit, as in consensus_hyp_kernel
+      const int h = static_cast<int>(part[bs * kPartDoubles + 1]);
+      const unsigned int* dr = g.draws + static_cast<size_t>(blockIdx.y) * g.draws_scan_stride +
+                               (static_cast<size_t>(blockIdx.x) * g.n_hyp + h) * 8;
+      double s9[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
+      for (int q = 0; q < 8; ++q) {
+        const double* ln = lines + static_cast<size_t>(dr[q] % static_cast<unsigned int>(n)) * kLineDoubles;
+#pragma unroll
+        for (int j = 0; j < 9; ++j) s9[j] += ln[6 + j];
+      }
+      double p[3];
+      sym3_pinv_solve(s9, s9 + 6, p);
+      double acc[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
+      k = 0;
+      for (int i = 0; i < n; ++i) {
+        const double* ln = lines + static_cast<size_t>(i) * kLineDoubles;
+        used[i] = line_sqdist(p, ln) < g.dist_thres ? 1 : 0;
+        if (used[i]) {
+          ++k;
+#pragma unroll
+          for (int j = 0; j < 9; ++j) acc[j] += ln[6 + j];
+        }
+      }
+      sym3_pinv_solve(acc, acc + 6, c);
+      status = 0;
+    } else {
+      // --- no accepted hypothesis (status 1) or fewer than 3 lines (status 2): LSQ over every kept line
+      for (int i = 0; i < n; ++i) used[i] = 1;
+      k = n;
+      c[0] = ws.p_all[3 * slot]; c[1] = ws.p_all[3 * slot + 1]; c[2] = ws.p_all[3 * slot + 2];
+      status = n < 3 ? 2 : 1;
+    }
+    // --- squared distances of the used lines and J = sum (I - n n^T) = -sum M_i
+    double ds = 0.0, J[6] = {0, 0, 0, 0, 0, 0};
+    for (int i = 0; i < n; ++i) {
+      if (!used[i]) continue;
+      const double* ln = lines + static_cast<size_t>(i) * kLineDoubles;
+      ds += line_sqdist(c, ln);
+#pragma unroll
+      for (int j = 0; j < 6; ++j) J[j] -= ln[6 + j];
+    }
+    r.status[slot] = status;
+    r.n_inliers[slot] = k;
+    r.rms[slot] = sqrt(ds / static_cast<double>(k));  // k = 0: NaN
+    // covariance sigma^2 J^-1, sigma^2 = ds / (2k - 3): each line constrains the two directions across it
+    double* cov = r.covariance + static_cast<size_t>(slot) * 9;
+    double lam[3], v[3][3];
+    sym3_jacobi(J, lam, v);
+    const double cut = sym3_cut(lam);
+    const bool full_rank = k >= 2 && fabs(lam[0]) > cut && fabs(lam[1]) > cut && fabs(lam[2]) > cut;
+    const double s2 = ds / static_cast<double>(2 * k - 3);
+    for (int a = 0; a < 3; ++a)
+      for (int b = 0; b < 3; ++b)
+        cov[3 * a + b] = full_rank ? s2 * (v[a][0] * v[b][0] / lam[0] + v[a][1] * v[b][1] / lam[1] +
+                                           v[a][2] * v[b][2] / lam[2])
+                                   : NAN;
+  }
+  __syncthreads();
+  unsigned char* mask = r.inliers + static_cast<size_t>(slot) * V;
+  for (int i = tid; i < V; i += blockDim.x) mask[i] = keep[i] ? used[pos_of[i]] : 0;
 }
 
 int pick_splits(int l, int n_hyp) {
@@ -358,9 +485,11 @@ size_t consensus_workspace_bytes(int l, int v, int n_hyp, int n_scans) {
   return d * sizeof(double) + static_cast<size_t>(l) * sizeof(int) + 64;
 }
 
-int consensus_launch(const ConsensusArgs& a, cudaStream_t s) {
+int consensus_launch(const ConsensusArgs& a, cudaStream_t s, const ConsensusReport* report) {
   MVLM_REQUIRE(a.peaks && a.starts && a.ends && a.draws && a.out_landmarks && a.out_errors && a.workspace,
                "consensus: null pointer");
+  MVLM_REQUIRE(!report || (report->status && report->n_inliers && report->inliers && report->rms && report->covariance),
+               "consensus: null report output");
   MVLM_REQUIRE(a.l > 0 && a.v > 0 && a.n_hyp > 0 && a.n_scans > 0 && a.n_scans <= 65535, "consensus: bad sizes");
   MVLM_REQUIRE(a.draws_scan_stride == 0 || a.draws_scan_stride == static_cast<size_t>(a.l) * a.n_hyp * 8,
                "consensus: draws are one shared (L,H,8) table or one (S,L,H,8) table");
@@ -382,6 +511,10 @@ int consensus_launch(const ConsensusArgs& a, cudaStream_t s) {
   consensus_hyp_kernel<<<dim3(a.l, splits, a.n_scans), 256, smem, s>>>(a, ws, splits, chunk);
   consensus_finalize_kernel<<<ceil_div(slots, 128), 128, 0, s>>>(a, ws, splits);
   count_launch(3);
+  if (report) {
+    consensus_report_kernel<<<dim3(a.l, a.n_scans), 256, 0, s>>>(a, ws, splits, *report);
+    count_launch(1);
+  }
   MVLM_CHECK_CUDA(cudaGetLastError());
   return MVLM_OK;
 }

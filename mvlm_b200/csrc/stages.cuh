@@ -75,8 +75,17 @@ struct ConsensusArgs {
   double* out_errors = nullptr;     // (S,L)
   int* out_nlines = nullptr;        // (S,L) lines kept by the filter (optional)
 };
+// Per-landmark report of the final fit (DESIGN.md 7h); every pointer (S,L,...) and required when the report is asked for.
+struct ConsensusReport {
+  signed char* status = nullptr;   // (S,L) 0 ransac, 1 all lines (no hypothesis accepted), 2 fewer than 3 lines
+  int* n_inliers = nullptr;        // (S,L) lines of the final fit
+  unsigned char* inliers = nullptr;  // (S,L,V) view v's line is one of them
+  double* rms = nullptr;           // (S,L)
+  double* covariance = nullptr;    // (S,L,9) row-major
+};
 size_t consensus_workspace_bytes(int l, int v, int n_hyp, int n_scans = 1);
-int consensus_launch(const ConsensusArgs& a, cudaStream_t s);
+// report: null runs the three consensus kernels; otherwise the report kernel runs after them (one launch more)
+int consensus_launch(const ConsensusArgs& a, cudaStream_t s, const ConsensusReport* report = nullptr);
 
 // ---- snap.cu --------------------------------------------------------------
 struct SnapMesh {

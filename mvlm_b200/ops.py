@@ -383,12 +383,29 @@ def rays_from_peaks(peaks: torch.Tensor, rot: torch.Tensor, image_size: int):
     return starts, ends
 
 
+class ConsensusReport(NamedTuple):
+    """Per-landmark report of the consensus's final fit (mvlm_consensus_multiscan_report, DESIGN.md 7h), on the device.
+    Leading dimensions (L,) from consensus(), (S,L) from consensus_multiscan()."""
+    status: torch.Tensor      # int8: 0 ransac, 1 all lines (no hypothesis accepted), 2 fewer than 3 lines
+    n_inliers: torch.Tensor   # int32: lines of the final fit
+    inliers: torch.Tensor     # bool (..., V): view v's line is one of them
+    rms: torch.Tensor         # f64
+    covariance: torch.Tensor  # f64 (..., 3, 3)
+
+
 def consensus(peaks, starts, ends, draws, mode: str = "quantile", threshold_quantile: float = 0.5,
-              threshold_absolute: float = 0.5, dist_thres: float = 100.0, workspace=None):
-    """Returns (landmarks (L,3) f64, errors (L,) f64, n_lines (L,) i32) on the device."""
+              threshold_absolute: float = 0.5, dist_thres: float = 100.0, workspace=None, report: bool = False):
+    """Returns (landmarks (L,3) f64, errors (L,) f64, n_lines (L,) i32) on the device; with report=True a fourth item,
+    the ConsensusReport (one launch more, the same landmarks, errors and line counts)."""
     lib = _lib.load()
     if mode not in ("quantile", "absolute"):
         raise ValueError(f"Unknown mode for line matching in Estimator: {mode}")
+    if report:
+        lm, err, nl, rep = consensus_multiscan(peaks, starts, ends, draws, 1, mode=mode,
+                                               threshold_quantile=threshold_quantile,
+                                               threshold_absolute=threshold_absolute, dist_thres=dist_thres,
+                                               workspace=workspace, report=True)
+        return lm[0], err[0], nl[0], ConsensusReport(*(t[0] for t in rep))
     l, v = peaks.shape[:2]
     n_hyp = draws.shape[1]
     nbytes = lib.mvlm_consensus_workspace_bytes(l, v, n_hyp)
@@ -404,10 +421,10 @@ def consensus(peaks, starts, ends, draws, mode: str = "quantile", threshold_quan
 
 
 def consensus_multiscan(peaks, starts, ends, draws, n_scans: int, mode: str = "quantile", threshold_quantile: float = 0.5,
-                        threshold_absolute: float = 0.5, dist_thres: float = 100.0, workspace=None):
+                        threshold_absolute: float = 0.5, dist_thres: float = 100.0, workspace=None, report: bool = False):
     """Consensus of the S scans of one pass: peaks (L,S*V,3) f32, starts / ends (L,S*V,3) f64, draws (L,H,8) shared by
     every scan or (S,L,H,8) per scan.  Returns (landmarks (S,L,3) f64, errors (S,L) f64, n_lines (S,L) i32); scan s
-    gets what consensus() returns for its views alone."""
+    gets what consensus() returns for its views alone.  report=True adds a fourth item, the (S,L,...) ConsensusReport."""
     lib = _lib.load()
     if mode not in ("quantile", "absolute"):
         raise ValueError(f"Unknown mode for line matching in Estimator: {mode}")
@@ -425,11 +442,21 @@ def consensus_multiscan(peaks, starts, ends, draws, n_scans: int, mode: str = "q
     lm = torch.empty((n_scans, l, 3), dtype=torch.float64, device=peaks.device)
     err = torch.empty((n_scans, l), dtype=torch.float64, device=peaks.device)
     nl = torch.empty((n_scans, l), dtype=torch.int32, device=peaks.device)
-    check(lib.mvlm_consensus_multiscan(ptr(peaks), ptr(starts), ptr(ends), n_scans, l, v, 0 if mode == "quantile" else 1,
-                                       float(threshold_quantile), float(threshold_absolute), ptr(draws), int(per_scan),
-                                       n_hyp, float(dist_thres), ptr(workspace), workspace.numel(), ptr(lm), ptr(err),
-                                       ptr(nl), cur_stream()), "mvlm_consensus_multiscan")
-    return lm, err, nl
+    args = (ptr(peaks), ptr(starts), ptr(ends), n_scans, l, v, 0 if mode == "quantile" else 1, float(threshold_quantile),
+            float(threshold_absolute), ptr(draws), int(per_scan), n_hyp, float(dist_thres), ptr(workspace),
+            workspace.numel(), ptr(lm), ptr(err), ptr(nl))
+    if not report:
+        check(lib.mvlm_consensus_multiscan(*args, cur_stream()), "mvlm_consensus_multiscan")
+        return lm, err, nl
+    dev = peaks.device
+    rep = ConsensusReport(status=torch.empty((n_scans, l), dtype=torch.int8, device=dev),
+                          n_inliers=torch.empty((n_scans, l), dtype=torch.int32, device=dev),
+                          inliers=torch.empty((n_scans, l, v), dtype=torch.bool, device=dev),
+                          rms=torch.empty((n_scans, l), dtype=torch.float64, device=dev),
+                          covariance=torch.empty((n_scans, l, 3, 3), dtype=torch.float64, device=dev))
+    check(lib.mvlm_consensus_multiscan_report(*args, *(ptr(t) for t in rep), cur_stream()),
+          "mvlm_consensus_multiscan_report")
+    return lm, err, nl, rep
 
 
 # Above this many triangles building a uniform grid (memset + 7 small launches, 45-150 us) and querying it (20-50 us) beats

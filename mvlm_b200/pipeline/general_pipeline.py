@@ -19,6 +19,7 @@ import numpy as np
 import torch
 
 from .. import _lib
+from .. import report as _report
 from ..io_mesh import SUFFIXES, check_scan_file, check_scan_formats, check_scan_path, is_scan_file, load_mesh
 from ..io_obj import Mesh, check_texture_source
 from ..prediction.paulsenpredictor import PaulsenModel
@@ -153,7 +154,11 @@ class Pipeline(abc.ABC, TimeMixin):
 
     # ------------------------------------------------------------------ general_pipeline.py:67-131
     def predict_one_file(self, file_name: Path, landmark_indices: list[int] | None = None,
-                         view_indices: list[int] | None = None, clip_rays_to_mesh: bool = True):
+                         view_indices: list[int] | None = None, clip_rays_to_mesh: bool = True, *,
+                         report: bool = False):
+        """(L,3) landmarks of one scan file, or None when the file does not exist.  report=True returns the scan's
+        LandmarkReport instead (its `landmarks` are the same array).  The report needs the fused device path: with
+        user-supplied components or render_image_stack=True (the seam-by-seam path) report=True raises ValueError."""
         with self._lock:
             if self.predictor_2d is None:
                 raise ValueError("Predictor2D is not initialized.")
@@ -172,16 +177,20 @@ class Pipeline(abc.ABC, TimeMixin):
                 mesh = load_mesh(file_name, texture_decoder=self.texture_decoder, device=self.device,
                                  parser=self.obj_parser, texture_source=self.texture_source)
                 self._print("Render [1] - Setup time: ", self.toc_p())
-                landmarks = self.predict_mesh(mesh)
+                landmarks = self.predict_mesh(mesh, report=report)
                 self._print("Landmarks 3D Total: ", self.p_time(time.time() - full_s))
                 return landmarks
+            if report:
+                raise ValueError("report=True needs the fused device path (the library's own renderer, predictor and "
+                                 "estimator, render_image_stack=False); this pipeline runs the seam-by-seam path")
             return self._predict_seams(file_name, full_s)
 
-    def predict_files(self, file_names, prefetch: int = 2) -> list:
+    def predict_files(self, file_names, prefetch: int = 2, *, report: bool = False) -> list:
         """Batch driver (the reference's main.py:50-62 loop is strictly serial): the native loader parses / decodes the
         next `prefetch` scans on background threads (the C parser and the JPEG decoder release the GIL) and the copies
         and launches of scan i+1 are enqueued while the GPU still works on scan i (see predict_meshes).
-        Returns one (L,3) array (or None for a missing file) per input, in order."""
+        Returns one (L,3) array (or None for a missing file) per input, in order; with report=True one LandmarkReport
+        (or None) per input."""
         with self._lock:
             from concurrent.futures import ThreadPoolExecutor
 
@@ -213,12 +222,13 @@ class Pipeline(abc.ABC, TimeMixin):
                             print(f"File {f} does not exist")
                         yield mesh
 
-            return self.predict_meshes(meshes())
+            return self.predict_meshes(meshes(), report=report)
 
-    def predict_folder(self, path, out=None) -> dict:
+    def predict_folder(self, path, out=None, *, report: bool = False) -> dict:
         """The reference's batch loop (main.py:23-62) for this pipeline: every `*.obj` of a folder (sorted; with
         scan_formats, every file of an enabled format), or one file; landmarks are written as `<out>/<stem>_<pipeline name>.txt` with `np.savetxt(..., delimiter=",")`, files
-        whose landmarks could not be predicted are skipped.  Returns {file: landmarks | None}."""
+        whose landmarks could not be predicted are skipped.  Returns {file: landmarks | None}.  report=True returns
+        {file: LandmarkReport | None} and also writes each report as `<out>/<stem>_<pipeline name>_report.npz`."""
         path = Path(path)
         if not path.exists():
             raise FileNotFoundError(f"{path.as_posix()} does not exist.")
@@ -241,11 +251,14 @@ class Pipeline(abc.ABC, TimeMixin):
                 raise ValueError(f"Given folder does not contain any {names} files.")
         out_dir.mkdir(parents=True, exist_ok=True)
         pname = getattr(self, "name", type(self).__name__.lower())
-        results = dict(zip(files, self.predict_files(files)))
+        results = dict(zip(files, self.predict_files(files, report=report)))
         for f, lm in results.items():
             if lm is None:
                 print(f"Landmarks for {f} could not be predicted -> skipping file [{f.stem}] for pipeline {pname}")
                 continue
+            if report:
+                lm.save((out_dir / f"{f.stem}_{pname}_report.npz").as_posix())
+                lm = lm.landmarks
             np.savetxt((out_dir / f"{f.stem}_{pname}.txt").as_posix(), lm, delimiter=",")
         return results
 
@@ -261,13 +274,16 @@ class Pipeline(abc.ABC, TimeMixin):
         s = scans_per_pass(v, h, w)
         return s if s == 1 else scans_per_pass(v, h, w, self.predictor_2d.max_views_per_launch(s * v, h, w))
 
-    def _enqueue_pass(self, meshes: list, transforms: np.ndarray | None = None, reserve_scans: int = 1):
+    def _enqueue_pass(self, meshes: list, transforms: np.ndarray | None = None, reserve_scans: int = 1,
+                      report: bool = False):
         """Enqueues the whole hot path of the scans of one pass on the current stream WITHOUT waiting for it: host ->
         device copies of every scan, one raster sequence, one CNN plan over all views, rays, consensus and snap of all
         scans, device -> pinned-host copy of the (S, L*3 + 1) result.  Each scan's landmarks equal those of a pass of
         that scan alone.  `reserve_scans`: the pass size the caller plans (the persistent image and the result ring
-        are sized for it, so that a shorter last pass allocates nothing).
-        Returns (pinned host rows, CUDA event recorded after the copy, objects to keep alive until then)."""
+        are sized for it, so that a shorter last pass allocates nothing).  report=True also runs the consensus report
+        kernel and copies the pass's packed reports (report.pack) to the host in one more page-locked copy.
+        Returns (pinned host rows, CUDA event recorded after the copies, objects to keep alive until then,
+        None or (pinned packed report rows, views per scan))."""
         from .. import ops
 
         r, p, e = self.renderer_3d, self.predictor_2d, self.estimator_3d
@@ -304,8 +320,9 @@ class Pipeline(abc.ABC, TimeMixin):
             pk = peaks.cpu().numpy()
             draws = np.stack([e.reference_draws(pk[:, i * v:(i + 1) * v]) for i in range(n)])
             draws_d = torch.from_numpy(draws.view(np.int32)).to(self.device)
-        lm, err, _ = e.estimate_landmarks_from_lines_device(peaks, starts, ends, draws_d, n_scans=n)
-        snapped, _ = ops.snap_to_meshes([(d.verts, d.tris, d.snap_grid()) for d in dmeshes], lm)
+        est = e.estimate_landmarks_from_lines_device(peaks, starts, ends, draws_d, n_scans=n, report=report)
+        lm, err = est[0], est[1]
+        snapped, tri = ops.snap_to_meshes([(d.verts, d.tris, d.snap_grid()) for d in dmeshes], lm)
         # the mean error per scan as one scan's (L,) sum, so last_error has the same bits in a pass of any size: one
         # (S,L) row reduction would not guarantee that, torch sizes its reduction blocks (and so the order of the sums
         # within a row) from the number of rows as well
@@ -321,34 +338,52 @@ class Pipeline(abc.ABC, TimeMixin):
         self._result_i = (getattr(self, "_result_i", -1) + 1) % len(ring)
         host = ring[self._result_i][:n]
         host.copy_(result, non_blocking=True)
+        rep = None
+        if report:
+            packed = _report.pack(lm, est[2], est[3], snapped, tri, [(d.verts, d.tris) for d in dmeshes], peaks)
+            rring = self.__dict__.setdefault("_report_ring", [])
+            if not rring or rring[0].shape[1] != packed.shape[1] or rring[0].shape[0] < n:
+                rring.clear()
+                rring.extend(torch.empty((max(n, reserve_scans), packed.shape[1]), dtype=torch.uint8, pin_memory=True)
+                             for _ in range(len(ring)))
+            rep = (rring[self._result_i][:n], v)
+            rep[0].copy_(packed, non_blocking=True)
+            result = (result, packed)
         done = torch.cuda.Event()
         done.record()
-        return host, done, (dmeshes, result, peaks, starts, ends, lm, backs)
+        return host, done, (dmeshes, result, peaks, starts, ends, lm, backs), rep
 
-    def _finish_pass(self, host: torch.Tensor, done, keep) -> list:
-        """Waits for a pass of _enqueue_pass; returns its (L,3) landmarks per scan.  last_error and the prints follow
-        the scans in order."""
+    def _finish_pass(self, host: torch.Tensor, done, keep, rep=None) -> list:
+        """Waits for a pass of _enqueue_pass; returns its (L,3) landmarks per scan, or its LandmarkReports when the pass
+        made them.  last_error and the prints follow the scans in order."""
         done.synchronize()
         rows = host.numpy().copy()
+        reps = None if rep is None else rep[0].numpy()
         out = []
-        for row, back in zip(rows, keep[-1]):
+        for i, (row, back) in enumerate(zip(rows, keep[-1])):
             self.last_error = float(row[-1])
             self._print("Landmarks [Error]: ", f"{self.last_error:08.6f}", " mm")
             lm = row[:-1].reshape(-1, 3)
-            out.append(lm if back is None else prealign.invert(lm, *back))
+            if reps is not None:
+                r = _report.unpack(reps[i], rep[1], lm, self.last_error)
+                out.append(r if back is None else _report.map_back(r, *back))
+            else:
+                out.append(lm if back is None else prealign.invert(lm, *back))
         return out
 
-    def predict_mesh(self, mesh: Mesh, transforms: np.ndarray | None = None) -> np.ndarray:
-        """Fused device path for an already loaded scan (host arrays in, (L,3) float64 out)."""
+    def predict_mesh(self, mesh: Mesh, transforms: np.ndarray | None = None, *, report: bool = False):
+        """Fused device path for an already loaded scan (host arrays in, (L,3) float64 out; report=True: the scan's
+        LandmarkReport)."""
         with self._lock:
-            return self._finish_pass(*self._enqueue_pass([mesh], transforms))[0]
+            return self._finish_pass(*self._enqueue_pass([mesh], transforms, report=report))[0]
 
-    def predict_meshes(self, meshes, depth: int = 2) -> list:
+    def predict_meshes(self, meshes, depth: int = 2, *, report: bool = False) -> list:
         """Batch form of predict_mesh: same results, bit for bit, and the same use of the global numpy RNG.  Several
         scans share one device pass when PASS_PIXELS allows it (_scans_per_pass; one scan per pass by default), and up to
         `depth` passes are in flight -- the copies and launches of the next pass are enqueued (one stream, so buffers
         are reused in order) before the host waits for the landmarks of an earlier one, which keeps host-side latency
-        off the GPU's critical path.  A None entry yields None."""
+        off the GPU's critical path.  A None entry yields None.  report=True: one LandmarkReport per scan, each equal to
+        the one predict_mesh(report=True) gives."""
         with self._lock:
             assert depth < 8, "depth is bounded by the ring of result buffers"
             per_pass = self._scans_per_pass()
@@ -368,11 +403,11 @@ class Pipeline(abc.ABC, TimeMixin):
                 batch.append(mesh)
                 where.append(len(results) - 1)
                 if len(batch) == per_pass:
-                    inflight.append((self._enqueue_pass(batch, reserve_scans=per_pass), where))
+                    inflight.append((self._enqueue_pass(batch, reserve_scans=per_pass, report=report), where))
                     batch, where = [], []
                     finish(depth)
             if batch:
-                inflight.append((self._enqueue_pass(batch, reserve_scans=per_pass), where))
+                inflight.append((self._enqueue_pass(batch, reserve_scans=per_pass, report=report), where))
             finish(0)
             return results
 

@@ -124,11 +124,12 @@ def _mesh_bytes(mesh) -> int:
     return sum(a.nbytes for _, a, _ in mesh.arrays() if isinstance(a, np.ndarray))
 
 
-def predict_mesh_view_split(pipeline, mesh, transforms: np.ndarray, group=None) -> np.ndarray:
+def predict_mesh_view_split(pipeline, mesh, transforms: np.ndarray, group=None, report: bool = False):
     """One scan whose views are split over the ranks of `group` (BASELINE.json config 4):
     every rank holds the whole mesh (uploaded in `world` slices and all-gathered when it is large), rasterises and runs
     the CNN on its block of views, the peaks are all-gathered, and every rank finishes rays / consensus / snap redundantly (it is microseconds of
-    work and removes a broadcast of the result)."""
+    work and removes a broadcast of the result).  Returns the (L,3) landmarks; report=True returns the scan's
+    LandmarkReport instead (every rank holds all peaks after the gather, so every rank builds it)."""
     from . import ops
 
     world = dist.get_world_size(group)
@@ -169,19 +170,29 @@ def predict_mesh_view_split(pipeline, mesh, transforms: np.ndarray, group=None) 
         pipeline._vs_rot_key = transforms.tobytes()
     starts, ends = e.estimate_landmark_lines_device(peaks, transforms, r.image_size[0], rot=pipeline._vs_rot)
     draws = e.seeded_draws_device(peaks.shape[0])
-    lm, err, _ = e.estimate_landmarks_from_lines_device(peaks, starts, ends, draws)
-    snapped, _ = ops.snap_to_mesh(dmesh.verts, dmesh.tris, lm, grid=dmesh.snap_grid())
+    est = e.estimate_landmarks_from_lines_device(peaks, starts, ends, draws, report=report)
+    lm, err = est[0], est[1]
+    snapped, tri = ops.snap_to_mesh(dmesh.verts, dmesh.tris, lm, grid=dmesh.snap_grid())
     pipeline.last_error = float((err.sum() / err.numel()).item())
-    return snapped.cpu().numpy()
+    landmarks = snapped.cpu().numpy()
+    if not report:
+        return landmarks
+    from .report import pack, unpack
+
+    one = lambda t: t.unsqueeze(0)  # noqa: E731  (a pass of one scan)
+    packed = pack(one(lm), one(est[2]), ops.ConsensusReport(*map(one, est[3])), one(snapped), one(tri),
+                  [(dmesh.verts, dmesh.tris)], peaks)
+    return unpack(packed[0].cpu().numpy(), n_views, landmarks, pipeline.last_error)
 
 
-def predict_files(pipeline, paths, group=None):
+def predict_files(pipeline, paths, group=None, report: bool = False):
     """Batch driver (reference main.py:50-62 is a serial loop): scans are dealt round-robin to the
-    ranks; rank 0 receives all results.  Returns {index: (L,3) array} on rank 0, own share elsewhere."""
+    ranks; rank 0 receives all results.  Returns {index: (L,3) array} on rank 0, own share elsewhere; report=True:
+    {index: LandmarkReport}."""
     world = dist.get_world_size(group) if dist.is_initialized() else 1
     rank = dist.get_rank(group) if dist.is_initialized() else 0
     idx = shard_scans(len(paths), rank, world)
-    mine = dict(zip(idx, pipeline.predict_files([paths[i] for i in idx])))  # prefetching loader, see Pipeline.predict_files
+    mine = dict(zip(idx, pipeline.predict_files([paths[i] for i in idx], report=report)))  # prefetching loader, see Pipeline.predict_files
     if world == 1:
         return mine
     gathered = [None] * world

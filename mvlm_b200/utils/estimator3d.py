@@ -92,11 +92,12 @@ class Estimator3D:
         err = err.cpu().numpy()
         return lm.cpu().numpy(), float(np.sum(err) / len(err))
 
-    def estimate_landmarks_from_lines_device(self, peaks, starts, ends, draws, n_scans: int | None = None):
+    def estimate_landmarks_from_lines_device(self, peaks, starts, ends, draws, n_scans: int | None = None,
+                                             report: bool = False):
         """n_scans: peaks / starts / ends are the (L, S*V, 3) arrays of a pass of S scans (draws (L,H,8) shared or
-        (S,L,H,8)); the results are then (S,L,3), (S,L), (S,L)."""
+        (S,L,H,8)); the results are then (S,L,3), (S,L), (S,L).  report=True adds the ops.ConsensusReport."""
         kw = dict(mode=self.mode, threshold_quantile=self.threshold_quantile, threshold_absolute=self.threshold_absolute,
-                  dist_thres=float(self.dist_thres))
+                  dist_thres=float(self.dist_thres), report=report)
         if n_scans is None:
             return ops.consensus(peaks, starts, ends, draws, **kw)
         return ops.consensus_multiscan(peaks, starts, ends, draws, n_scans, **kw)

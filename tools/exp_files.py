@@ -21,8 +21,8 @@ enq, fin = [], []
 oe, of = dm._enqueue_pass, dm._finish_pass
 def e2(m, tr=None, **kw):
     t0 = time.perf_counter(); r = oe(m, tr, **kw); enq.append(time.perf_counter() - t0); return r
-def f2(h, d, k):
-    t0 = time.perf_counter(); r = of(h, d, k); fin.append(time.perf_counter() - t0); return r
+def f2(*handle):
+    t0 = time.perf_counter(); r = of(*handle); fin.append(time.perf_counter() - t0); return r
 dm._enqueue_pass, dm._finish_pass = e2, f2
 for name, batch in (("same pinned mesh", [pinned] * 16), ("same pageable mesh", [meshes[0]] * 16), ("4 pageable meshes", [meshes[i % 4] for i in range(16)])):
     for depth in (1, 2):
